@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — `kmercamel compute` hot path on B200 (driver contract, see DESIGN.md "Measurement").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W]                 our CUDA path
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   our CUDA path
   python bench.py --impl reference [--gpus N] [--steps K] [--warmup W]   the reference's own CPU path (oracle/_ref)
 
 A step = one pass of the whole hot path (extract -> count -> overlap levels -> emission) over one synthetic input.
@@ -102,6 +102,27 @@ def make_workload(rank: int):
     from kmercamel_b200 import synth
     recs = synth.random_genome_records(N_RECORDS, RECORD_LEN, SEED + rank)
     return recs, synth.frame_records(recs)
+
+
+DUMP_SAMPLE = 1 << 22   # superstring bytes written by --dump-outputs: 16 MB of float32 values + 32 MB of float64 positions
+
+
+def dump_outputs(out_dir: str, ms: bytes, n_kmers: int):
+    """Writes what one `compute` returned, so that two builds can be compared output for output:
+      result.npy                        float64 [superstring length, distinct k-mers]
+      superstring_sample_positions.npy  float64 positions in the masked superstring: one per equal stratum, drawn with a fixed seed
+                                        (every position when the superstring has at most DUMP_SAMPLE bytes)
+      superstring_sample.npy            float32 byte values of the superstring at those positions"""
+    n = len(ms)
+    if n <= DUMP_SAMPLE:
+        pos = np.arange(n, dtype=np.int64)
+    else:
+        edges = np.arange(DUMP_SAMPLE + 1, dtype=np.int64) * n // DUMP_SAMPLE
+        pos = edges[:-1] + np.random.default_rng(SEED).integers(0, np.diff(edges))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "result.npy"), np.array([n, n_kmers], dtype=np.float64))
+    np.save(os.path.join(out_dir, "superstring_sample.npy"), np.frombuffer(ms, dtype=np.uint8)[pos].astype(np.float32))
+    np.save(os.path.join(out_dir, "superstring_sample_positions.npy"), pos.astype(np.float64))
 
 
 def ref_binary():
@@ -376,10 +397,14 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/*.npy (see dump_outputs; one GPU only)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (world > 1 or args.impl != "ours"):
+        raise SystemExit("--dump-outputs: only for our path on one GPU")
 
     if args.impl == "reference":
         run_reference_arm(args, rank, world)
@@ -438,6 +463,8 @@ def main():
     e1.record(stream)
     barrier()
     dev_ms = e0.elapsed_time(e1)
+    if args.dump_outputs:   # the next call reuses the result buffer of the last timed step
+        last_ms, last_n_kmers = ctx.copy_to_host(res.ms_ptr, res.length), res.n_kmers
     ctx.profile_enable(True)
     ctx.profile_reset()
     barrier()
@@ -561,6 +588,8 @@ def main():
                        "sig_fallbacks": int(ctx.stat("sig_fallbacks"))},
         }
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_ms, last_n_kmers)
     if world > 1:
         dist.destroy_process_group()
 
