@@ -269,7 +269,7 @@ static int camel_compute(int argc, char **argv, bool lower_bound) {
     restrict_visible_devices(devices);
     device = devices[0];
     // several devices: the k-mer set construction of the from-FASTA greedy is sharded over them; every other mode runs on the first
-    const bool multi = devices.size() > 1 && !lower_bound && algorithm == "greedy" && !assume_simplitigs && mask_path.empty();
+    bool multi = devices.size() > 1 && !lower_bound && algorithm == "greedy" && !assume_simplitigs && mask_path.empty();
     if (devices.size() > 1 && !multi) write_log("Note: -S, -M, streaming and lowerbound run on one GPU; using device " + std::to_string(device_asked) + ".");
     // the CUDA context(s) (~1 s) are created while the file is read and framed
     kc_ctx *ctx = nullptr;
@@ -306,9 +306,23 @@ static int camel_compute(int argc, char **argv, bool lower_bound) {
     }
     std::vector<unsigned char>().swap(data);
     const double t_frame = now_ms();
+    // 64-bit window positions (include/kcgpu.h KC_POS32_BYTES): one GPU, and no digest to verify with
+    const bool large = n_bytes >= KC_POS32_BYTES;
+    if (large && verify) {
+        std::cerr << "kmercamel compute: verification not available for inputs of 2^32 bytes or more (" << n_bytes << " sequence bytes)" << std::endl;
+        return 1;
+    }
 
     init_thread.join();
     rc = rc_init;
+    if (rc == KC_OK && multi && large) {
+        kc_group_destroy(group);
+        group = nullptr;
+        ctx = nullptr;
+        multi = false;
+        write_log("Note: inputs of 2^32 bytes or more run on one GPU; using device " + std::to_string(device_asked) + ".");
+        rc = kc_init(device, nullptr, &ctx);
+    }
     const double t_init = now_ms();
     if (rc != KC_OK) {
         std::cerr << "cannot initialise CUDA device " << device_asked << (multi ? " (and the other devices of -g; all need peer access to each other)" : "") << ": "

@@ -34,9 +34,17 @@ extern "C" {
 #define KC_ERR_OOM (-3)
 #define KC_ERR_EMPTY (-4)     /* no k-mer in the input (reference src/main.cpp:155-158) / empty node list (src/global.h:219-221) */
 #define KC_ERR_BAD_SEQ (-5)   /* -S record with a non-ACGT byte (reference src/simplitigs.h:82 asserts) or shorter than k */
-#define KC_ERR_TOO_LARGE (-6) /* more than 2^32-2 virtual nodes or sequence bytes on one GPU */
+#define KC_ERR_TOO_LARGE (-6) /* more than 2^32-2 virtual nodes on one GPU, or an input of KC_POS32_BYTES or more that the call
+                               * cannot take (see KC_POS32_BYTES); kc_last_error says why */
 #define KC_ERR_INTERNAL (-7)
 #define KC_ERR_NO_DEVICE (-8)
+
+/* Inputs of KC_POS32_BYTES sequence bytes or more (about 2^32) need 64-bit window positions.  kc_compute and
+ * kc_compute_device take them on one GPU through the signature-bucket k-mer set construction, which applies with k >= 26,
+ * min_frequency 1, no want_maxone and no assume_simplitigs; outside those conditions, or when a signature bucket overflows on
+ * such an input (heavily repeated sequence), they fail with KC_ERR_TOO_LARGE.  Every other entry point (streaming, maskopt,
+ * lower bound, count_kmers, kmer_digest, groups) refuses such inputs with KC_ERR_TOO_LARGE. */
+#define KC_POS32_BYTES 0xFFFFFFF0ULL
 
 typedef struct kc_ctx kc_ctx;
 
@@ -229,7 +237,7 @@ uint64_t kc_total_launches(const kc_ctx *ctx);
  * Results never depend on these options. */
 int kc_set_option(kc_ctx *ctx, const char *name, int value);
 /* Counters since kc_init: "sig_runs", "sig_fallbacks", "fast_runs", "fast_fallbacks", "total_launches"; current value of the
- * option "fast_max_ctas". */
+ * option "fast_max_ctas"; device arena: "arena_bytes" (reserved now), "arena_high" (most bytes in use at once since kc_init). */
 int kc_get_stat(const kc_ctx *ctx, const char *name, uint64_t *value);
 
 int kc_limbs_for_k(int k);

@@ -97,6 +97,19 @@ void check_params(const kc_params *p) {
     if (p->min_frequency != 1 && p->assume_simplitigs) KC_THROW(KC_ERR_ARG, "-z is not compatible with -S");   // :305-308
 }
 
+// Inputs of KC_POS32_BYTES or more need 64-bit window positions, which only the signature construction carries (the fixed-slot
+// and exact constructions move 32-bit positions, the -S path and the other entry points keep their 32-bit caps).
+#define KC_LARGE_ONLY "inputs of 2^32 bytes or more are built by the signature construction only (k >= 26, no -z, no -M, no -S)"
+void check_large_input(const kc_ctx *ctx, const kc_params *p, u64 n_bytes) {
+    if (n_bytes < KC_POS32_BYTES) return;
+    if (p->assume_simplitigs) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; -S was asked");
+    if (p->min_frequency > 1) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; -z (min_frequency > 1) was asked");
+    if (p->want_maxone) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; -M (want_maxone) was asked");
+    if (p->k < 26) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; k is below 26");
+    if (!ctx->sig.enabled) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; it is switched off (option sig_set = 0)");
+    if (!kc_sig_plan(n_bytes, p->k, ctx->sig).ok) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; its bucket plan does not fit this input");
+}
+
 // Make sure the arena can hold `need` bytes (bounded by what the device can give).
 void ensure_arena(kc_ctx *ctx, size_t need) {
     need = (need + 4095) & ~(size_t) 4095;  // both arena ends stay 256-byte aligned
@@ -121,12 +134,16 @@ void ensure_arena(kc_ctx *ctx, size_t need) {
 // stage depends on the number of nodes, which for a FASTA input (first-occurrence runs) is only known after stage 1:
 // `pessimistic = false` assumes one run per 64 sequence bytes (reads with 1 % errors give one per ~650), and a call that
 // runs out of arena is repeated once with the worst case (one run per 2 bytes), see run_with_arena.
+// Inputs of KC_POS32_BYTES or more take the signature construction alone (`sig`: its plan at this size): sequence, flags, code
+// words and record rows.
 size_t estimate_arena(u64 n_bytes, u64 n_recs, int limbs, bool complements, bool simplitigs, bool pessimistic = false,
-                      const KsfTuning *fast = nullptr) {
+                      const KsfTuning *fast = nullptr, const SigPlan *sig = nullptr) {
     const double wb = 8.0 * limbs;
     const double c = complements ? 2.0 : 1.0;
     double stage1 = n_bytes * (1.0 + 2.0 * (wb + 4.0) + 1.0 + 1.0 + 0.2);  // sequence, keys + positions x2, counts, control, flags
-    if (fast) {  // fixed-slot buckets of the histogram-free construction (tried first, released before the exact one runs)
+    if (n_bytes >= KC_POS32_BYTES && sig && sig->ok) {
+        stage1 = n_bytes * (1.0 + 0.125) + (double) kc_sig_arena_bytes(*sig, n_bytes);
+    } else if (fast) {  // fixed-slot buckets of the histogram-free construction (tried first, released before the exact one runs)
         const KsfPlan pl = kc_ksf_plan(n_bytes, *fast);
         if (pl.ok) {
             const double f = n_bytes * 1.2 + (double) (pl.slots[0] + pl.slots[1]) * (wb + 4.0) + (double) pl.n_leaf * 28.0 + 65536.0;
@@ -214,8 +231,10 @@ u64 run_stage1_runs(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_para
     const bool expect_duplicates = ctx->fast_heuristics && (p.min_frequency > 1 || (ctx->fast_overflow_bytes && nb >= ctx->fast_overflow_bytes / 2 && nb <= ctx->fast_overflow_bytes * 2));
     // Signature buckets first (kmerset_sig.cuh): records of ~7 windows instead of 12-byte items.  Read sets with coverage overflow
     // its buckets (every run of windows comes c times: sigma grows by sqrt(c)) and are remembered like a fixed-slot overflow.
+    // Inputs of KC_POS32_BYTES or more have no other construction (check_large_input): they always try it, and an overflow ends the call.
+    const bool large = nb >= KC_POS32_BYTES;
     const bool sig_overflowed = ctx->fast_heuristics && ctx->sig_overflow_bytes && nb >= ctx->sig_overflow_bytes / 2 && nb <= ctx->sig_overflow_bytes * 2;
-    if (!p.want_maxone && p.min_frequency == 1 && !sig_overflowed) {
+    if (!p.want_maxone && p.min_frequency == 1 && (large || !sig_overflowed)) {
         u64 *cells4 = ex.arena->alloc_top<u64>(4);  // {kept, runs, M, overflow status}
         ex.fill_bytes(cells4, 0, 32);
         if (kc_kmerset_build_sig<L>(ex, in.seq, nb, p.k, p.complements != 0, flags, cells4, ctx->sig, in.chunks)) {
@@ -232,9 +251,11 @@ u64 run_stage1_runs(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_para
             }
             ++ctx->sig_fallbacks;  // a bucket overflowed: discard the flags, fall through to the other constructions
             ctx->sig_overflow_bytes = nb;
+            if (large) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; it overflowed on this input (too repetitive)");
             ex.fill_bytes(flags, 0, fwords * 4);
         }
     }
+    if (large) KC_THROW(KC_ERR_INTERNAL, "an input of 2^32 bytes or more reached the 32-bit set constructions");
     if (!p.want_maxone && !expect_duplicates) {
         KsfPlan plan;
         u64 *cells4 = ex.arena->alloc_top<u64>(4);  // {kept, runs, M, overflow status}
@@ -738,7 +759,7 @@ int kc_compute_device(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_ou
     if (!ctx || !in || !out) return KC_ERR_ARG;
     KC_API_BEGIN
     check_params(p);
-    if (in->n_bytes >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "more than 2^32 sequence bytes on one GPU");
+    check_large_input(ctx, p, in->n_bytes);
     if ((reinterpret_cast<uintptr_t>(in->seq) & 15) != 0) KC_THROW(KC_ERR_ARG, "device sequence pointer must be 16-byte aligned");
     KC_CUDA(cudaSetDevice(ctx->device));
     const int limbs = kc_limbs_for_k(p->k);
@@ -749,8 +770,9 @@ int kc_compute_device(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_ou
     DevInput di{in->seq, in->n_bytes, in->rec_off, in->rec_len, in->n_recs};
     DevResult res;
     KC_TRACE_POINT("compute_device: start");
-    run_with_arena(ctx, estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, p->assume_simplitigs != 0, false, &ctx->fast),
-                   estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, p->assume_simplitigs != 0, true, &ctx->fast),
+    const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->sig);
+    run_with_arena(ctx, estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, p->assume_simplitigs != 0, false, &ctx->fast, &sig),
+                   estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, p->assume_simplitigs != 0, true, &ctx->fast, &sig),
                    [&] { dispatch_pipeline(ctx, ex, di, *p, res); });
     KC_TRACE_POINT("compute_device: launched");
     KC_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -773,7 +795,7 @@ int kc_compute(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_output *o
     if (!ctx || !in || !out) return KC_ERR_ARG;
     KC_API_BEGIN
     check_params(p);
-    if (in->n_bytes >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "more than 2^32 sequence bytes on one GPU");
+    check_large_input(ctx, p, in->n_bytes);
     KC_CUDA(cudaSetDevice(ctx->device));
     const int limbs = kc_limbs_for_k(p->k);
     const bool simplitigs = p->assume_simplitigs != 0;
@@ -782,8 +804,9 @@ int kc_compute(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_output *o
     ex.pinned = ctx->pin_small;
     ex.pinned_cap = ctx->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
     DevResult res;
-    run_with_arena(ctx, estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, false, &ctx->fast),
-                   estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, true, &ctx->fast), [&] {
+    const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->sig);
+    run_with_arena(ctx, estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, false, &ctx->fast, &sig),
+                   estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, true, &ctx->fast, &sig), [&] {
         // host -> device.  Large from-FASTA inputs go in chunks on the copy stream: the level-0 partition pass of chunk c starts
         // as soon as chunk c has landed (InputChunks), instead of after the whole copy.
         u8 *d_seq = ex.alloc<u8>(in->n_bytes + 64);
@@ -1471,6 +1494,8 @@ int kc_get_stat(const kc_ctx *ctx, const char *name, uint64_t *value) {
     else if (std::strcmp(name, "sig_runs") == 0) *value = ctx->sig_runs;
     else if (std::strcmp(name, "sig_fallbacks") == 0) *value = ctx->sig_fallbacks;
     else if (std::strcmp(name, "total_launches") == 0) *value = ctx->total_launches;
+    else if (std::strcmp(name, "arena_bytes") == 0) *value = ctx->arena.cap;
+    else if (std::strcmp(name, "arena_high") == 0) *value = ctx->arena.high;
     else if (std::strcmp(name, "fast_max_ctas") == 0) *value = (uint64_t) ctx->fast.max_ctas;
     else return KC_ERR_ARG;
     return KC_OK;

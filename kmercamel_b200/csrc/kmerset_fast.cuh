@@ -63,7 +63,7 @@ inline KsfFlagPeers kc_ksf_own_flags(u32 *flags) {
 
 // MULTI = false is the single-GPU instance: one RED on the GPU's own array, nothing else in the instruction stream (the loop over
 // the ranks cost the leaf resolve 9 % on one GPU although it almost never runs).
-template <bool MULTI> KC_D void kc_flag_clear_all(const KsfFlagPeers &fp, u32 pos) {
+template <bool MULTI, class Pos> KC_D void kc_flag_clear_all(const KsfFlagPeers &fp, Pos pos) {  // Pos: u32, or u64 past 2^32 bytes
     const u32 m = ~(1u << (pos & 31));
     if (MULTI) {
         for (int r = 0; r < fp.n; ++r) atomicAnd(&fp.f[r][pos >> 5], m);

@@ -35,7 +35,8 @@
 // words re-read, 16 bytes per record) = ~7.5 instead of 49.
 //
 // A bucket that exceeds its capacity (heavily repeated sequence, read sets with coverage) sets the status word; the caller
-// discards the flags and uses the other constructions, exactly like an overflow in kmerset_fast.cuh.
+// discards the flags and uses the other constructions, exactly like an overflow in kmerset_fast.cuh.  Inputs of 2^32 bytes or more
+// have no other construction (theirs carry 32-bit positions): there the call fails.
 #pragma once
 #include "kmerset_fast.cuh"
 
@@ -62,7 +63,7 @@ struct SigPlan {
 
 inline SigPlan kc_sig_plan(u64 n_bytes, int k, const SigTuning &t) {
     SigPlan p;
-    if (!t.enabled || n_bytes < t.min_items || n_bytes >= 0xFFFFFFFFULL) return p;
+    if (!t.enabled || n_bytes < t.min_items) return p;
     static const int ms[4] = {16, 15, 12, 11};
     for (int i = 0; i < 4 && !p.m; ++i) {
         const int d = k - ms[i] - (KC_SIG_W - 1);
@@ -93,6 +94,12 @@ inline SigPlan kc_sig_plan(u64 n_bytes, int k, const SigTuning &t) {
     p.n_buckets = (u32) (nb < 64 ? 64 : nb);
     p.ok = true;
     return p;
+}
+
+// Arena bytes of kc_kmerset_build_sig besides the sequence and the flags: record rows, code words, bucket counters.
+inline u64 kc_sig_arena_bytes(const SigPlan &p, u64 n_bytes) {
+    const u64 tiles = (n_bytes + 256 * 32 - 1) / (256 * 32);
+    return (u64) p.n_buckets * KC_SIG_REC_CAP * 8 + tiles * 256 * 8 + (u64) p.n_buckets * 4 + (3u << 10);
 }
 
 #ifdef __CUDACC__
@@ -140,8 +147,11 @@ KC_D u32 kc_sig_bucket(u32 sig, u32 n_buckets) {
     return __umulhi(~u13, n_buckets);
 }
 
-// A record: bits 0..31 END position of its first window, 32..34 windows - 1.
-KC_HD u64 kc_sig_record(u32 pos, u32 len) { return (u64) pos | ((u64) (len - 1) << 32); }
+// A record: END position of its first window in bits 0..31 (low half) and 35..63 (bits 32..60 of the position), windows - 1 in
+// bits 32..34.  Below 2^32 the word is the plain {position, length} of a 32-bit layout.
+KC_HD u64 kc_sig_record(u64 pos, u32 len) { return (pos & 0xFFFFFFFFULL) | ((u64) (len - 1) << 32) | ((pos >> 32) << 35); }
+KC_HD u64 kc_sig_record_pos(u64 rec) { return (rec & 0xFFFFFFFFULL) | ((rec >> 35) << 32); }
+KC_HD u32 kc_sig_record_len(u64 rec) { return ((u32) (rec >> 32) & 7u) + 1u; }
 
 // Multi-GPU (group.cuh): bucket b belongs to rank b % n; rank r's records for it go into the sub-slot (b / n, r) of the owner's
 // receive array (sub_cap records, reserved with a LOCAL counter: no remote atomics), the code words and the valid-window words of
@@ -159,7 +169,7 @@ struct SigPeers {
 // packed[s] = the 2-bit codes of bases 32 s .. 32 s + 31 (first base in the top bits); every strip of every tile is written.
 template <int M, bool P2P>
 __global__ void __launch_bounds__(256) kc_sig_scan_kernel(const u8 *__restrict__ seq, u64 n_bytes, int k, int a, u32 n_buckets, u32 *cursor,
-                                                          u64 *__restrict__ recs, u64 *__restrict__ packed, u32 *__restrict__ flags, u32 n_flag_words,
+                                                          u64 *__restrict__ recs, u64 *__restrict__ packed, u32 *__restrict__ flags, u64 n_flag_words,
                                                           u32 tile0, kc_ull *m_cell, u32 *status, const u32 *__restrict__ win_mask, const SigPeers sp) {
     constexpr int T = 256;
     constexpr int NH = 32 + KC_SIG_W - 1;  // M-mer hashes a strip needs
@@ -247,7 +257,8 @@ __global__ void __launch_bounds__(256) kc_sig_scan_kernel(const u8 *__restrict__
     const u32 bound = ps | ~emr;                         // a piece ends before the next piece or the next window that is not valid
     // eight pieces per round, so that their atomics are in flight together (one at a time, the thread waited ~0.7 us for each
     // slot: 51 % of the kernel's stall samples)
-    const u32 pos0 = (u32) block_pos0 + threadIdx.x * KC_EX_STRIP;
+    const u64 pos0 = (u64) block_pos0 + threadIdx.x * KC_EX_STRIP;
+    const u64 rec_hi = kc_sig_record(pos0, 1u) & ~0xFFFFFFFFULL;  // bits 35..63, the same for the whole strip (32 | 2^32)
     bool over = false;
     while (ps) {
         u32 bk[8], slot[8], e[8];
@@ -268,7 +279,7 @@ __global__ void __launch_bounds__(256) kc_sig_scan_kernel(const u8 *__restrict__
 #pragma unroll
         for (int u = 0; u < 8; ++u) {
             if (on[u]) {
-                const u64 rec = kc_sig_record(pos0 + (e[u] >> 3), (e[u] & 7u) + 1u);
+                const u64 rec = kc_sig_record((u32) pos0 + (e[u] >> 3), (e[u] & 7u) + 1u) | rec_hi;
                 if (P2P) {  // into the rank's own staging array; kc_sig_ship_kernel sends whole sub-slots
                     if (slot[u] < sp.sub_cap) recs[(u64) bk[u] * sp.sub_cap + slot[u]] = rec;
                     else over = true;
@@ -380,7 +391,7 @@ template <int L> struct SigCfg {
     static constexpr u32 T1N = 4 * KC_SIG_SLOTS, T2N = KC_SIG_SLOTS / 4;  // T2 takes the items that lose their T1 slot to another key (~4 %)
     static constexpr int T1_BITS = 13;
     static constexpr int MIN_CTAS = L == 1 ? 5 : (L == 2 ? 3 : 2);      // resident CTAs per SM the shared memory allows
-    static int smem() { return (int) (KC_SIG_SLOTS * (sizeof(KWord<L>) + 4) + T1N * 2 + T2N * 4); }
+    static int smem(bool pos64 = false) { return (int) (KC_SIG_SLOTS * (sizeof(KWord<L>) + 4) + (pos64 ? KC_SIG_REC_CAP * 8 : 0) + T1N * 2 + T2N * 4); }
 };
 
 // Reverse the 32 two-bit symbols of a limb through the bit-reversal instruction (kc_reverse_symbols64 of kword.cuh walks a
@@ -405,10 +416,16 @@ KC_D u32 kc_sig_hash2(u32 h) {
 }
 
 // The code words a record's windows can reach into: word NW - 1 = the strip of the record, the others to its left.
-template <int NW> KC_D void kc_sig_load_words(const u64 *__restrict__ packed, u64 rec, bool have, u64 (&w)[NW]) {
-    const u32 strip = (u32) rec >> 5;
+template <int NW, bool POS64> KC_D void kc_sig_load_words(const u64 *__restrict__ packed, u64 rec, bool have, u64 (&w)[NW]) {
+    if constexpr (POS64) {
+        const u64 strip = kc_sig_record_pos(rec) >> 5;
 #pragma unroll
-    for (int wi = 0; wi < NW; ++wi) w[wi] = have && strip >= (u32) (NW - 1 - wi) ? __ldg(&packed[strip - (u32) (NW - 1 - wi)]) : 0ULL;
+        for (int wi = 0; wi < NW; ++wi) w[wi] = have && strip >= (u64) (NW - 1 - wi) ? __ldg(&packed[strip - (u64) (NW - 1 - wi)]) : 0ULL;
+    } else {
+        const u32 strip = (u32) rec >> 5;
+#pragma unroll
+        for (int wi = 0; wi < NW; ++wi) w[wi] = have && strip >= (u32) (NW - 1 - wi) ? __ldg(&packed[strip - (u32) (NW - 1 - wi)]) : 0ULL;
+    }
 }
 
 // One bucket at a time, ONE THREAD PER RECORD: item t of record r lives in slot t * 256 + r of the shared-memory arrays
@@ -422,7 +439,12 @@ template <int NW> KC_D void kc_sig_load_words(const u64 *__restrict__ packed, u6
 // points (16 BSSY / BSYNC pairs per bucket) and the overlap of the eight independent hash / store chains (0.315 -> 0.289 ms on
 // configs[1]).  Fewer threads per CTA (160 / 192 with a second round for the records beyond, 6 CTAs per SM) were measured and change
 // nothing: 0.287 - 0.293 ms.
-template <int L, bool MULTI, bool UNI>
+//
+// POS64 (inputs of more than 2^32 bytes): window positions need 64 bits, and a shared array of them would cost the L = 1 instance one
+// of its five resident CTAs, so an item stands for its position by its slot (position = rp[slot % RC] + slot / RC, rp = the 256
+// record positions) and a duplicate folds by a CAS loop on slots.  A separate instance because this decode, in one code path for all
+// sizes, made the resolve 3 % slower on configs[1] (0.2442 -> 0.2515 ms, two back-to-back pairs on one B200 at 1000 W).
+template <int L, bool MULTI, bool UNI, bool POS64 = false>
 __global__ void __launch_bounds__(SigCfg<L>::THREADS, SigCfg<L>::MIN_CTAS) kc_sig_resolve_kernel(const u64 *__restrict__ packed, int k,
                                                                                                 const u32 *__restrict__ cursor, const u64 *__restrict__ recs,
                                                                                                 u32 n_buckets, KsfFlagPeers fl, kc_ull *n_unique, u32 *status,
@@ -434,7 +456,9 @@ __global__ void __launch_bounds__(SigCfg<L>::THREADS, SigCfg<L>::MIN_CTAS) kc_si
     static_assert((1u << Cfg::T1_BITS) == Cfg::T1N, "T1 size");
     extern __shared__ __align__(16) unsigned char kc_smem_raw[];
     KWord<L> *sk = reinterpret_cast<KWord<L> *>(kc_smem_raw);  // [SLOTS] canonical k-mer of the item in slot t * RC + r
-    u32 *sp = reinterpret_cast<u32 *>(sk + KC_SIG_SLOTS);       // [SLOTS] its window END position (the smallest one of its key, once folded)
+    u64 *rp = reinterpret_cast<u64 *>(sk + KC_SIG_SLOTS);       // POS64: [RC] END position of the first window of record r
+    // [SLOTS] its window END position (the smallest one of its key, once folded); POS64: the slot of that position
+    u32 *sp = reinterpret_cast<u32 *>(rp + (POS64 ? RC : 0));
     u32 *T2 = sp + KC_SIG_SLOTS;                                // [T2N]
     u16 *T1 = reinterpret_cast<u16 *>(T2 + T2N);                // [T1N]
     const KWord<L> kmask = KWord<L>::low_mask(2 * k);
@@ -450,7 +474,8 @@ __global__ void __launch_bounds__(SigCfg<L>::THREADS, SigCfg<L>::MIN_CTAS) kc_si
     };
     // record r (its code words in w) -> the canonical k-mers of its windows into slots t * RC + r, their T1 slots into h1
     auto spread = [&](const u64 rec, const u64 (&w)[NW], const u32 r, u32 (&h1)[P]) -> u32 {
-        const u32 pos = (u32) rec, len = ((u32) (rec >> 32) & 7u) + 1u;
+        const u32 pos = (u32) rec, len = kc_sig_record_len(rec);
+        if (POS64) rp[r] = kc_sig_record_pos(rec);
         const int sh = 2 * (31 - (int) (pos & 31u));
         const u64 mine = w[NW - 1];
         const u64 ms = sh ? mine << (64 - sh) : 0ULL;  // the bases behind the first window, left-aligned
@@ -490,7 +515,7 @@ __global__ void __launch_bounds__(SigCfg<L>::THREADS, SigCfg<L>::MIN_CTAS) kc_si
                 h1[t] = kc_sig_hash<1>(canon) >> (32 - Cfg::T1_BITS);
                 if ((u32) t < len) {
                     sk[slot] = canon;
-                    sp[slot] = pos + (u32) t;
+                    sp[slot] = POS64 ? slot : pos + (u32) t;
                     T1[h1[t]] = (u16) slot;
                 }
             }
@@ -528,23 +553,46 @@ __global__ void __launch_bounds__(SigCfg<L>::THREADS, SigCfg<L>::MIN_CTAS) kc_si
                 h1[t] = kc_sig_hash<L>(canon) >> (32 - Cfg::T1_BITS);
                 if ((u32) t < len) {
                     sk[slot] = canon;
-                    sp[slot] = pos + (u32) t;
+                    sp[slot] = POS64 ? slot : pos + (u32) t;
                     T1[h1[t]] = (u16) slot;
                 }
             }
         }
         return len;
     };
-    // an item that did not win its T1 slot: equal key = duplicate (fold the positions, clear the larger one's bit); different key ->
-    // T2 with CAS + linear probing
+    auto pos_of = [&](const u32 slot) -> u64 { return rp[slot % RC] + slot / RC; };
+    // a duplicate of the key that slot o represents: the smaller position stays in sp[o], the bit of the larger one is cleared
+    // (POS64: an atomicMin by position as a CAS loop on slots)
+    auto fold = [&](const u32 o, const u32 slot) {
+        if constexpr (!POS64) {
+            const u32 mine_p = sp[slot];
+            const u32 was = atomicMin(&sp[o], mine_p);
+            kc_flag_clear_all<MULTI>(fl, was > mine_p ? was : mine_p);
+            return;
+        }
+        const u64 mine_p = pos_of(slot);
+        u32 cur = sp[o];
+        for (;;) {
+            const u64 cur_p = pos_of(cur);
+            if (cur_p < mine_p) {
+                kc_flag_clear_all<MULTI>(fl, mine_p);
+                return;
+            }
+            const u32 was = atomicCAS(&sp[o], cur, slot);
+            if (was == cur) {
+                kc_flag_clear_all<MULTI>(fl, cur_p);
+                return;
+            }
+            cur = was;
+        }
+    };
+    // an item that did not win its T1 slot: equal key = duplicate (fold); different key -> T2 with CAS + linear probing
     auto settle = [&](const u32 slot) {
         const KWord<L> key = sk[slot];
         const u32 h = kc_sig_hash<L>(key);
         const u32 o = T1[h >> (32 - Cfg::T1_BITS)];
         if (sk[o] == key) {
-            const u32 mine_p = sp[slot];
-            const u32 was = atomicMin(&sp[o], mine_p);
-            kc_flag_clear_all<MULTI>(fl, was > mine_p ? was : mine_p);
+            fold(o, slot);
         } else {
             u32 s2 = kc_sig_hash2(h) & (T2N - 1);
 #pragma unroll 1
@@ -559,9 +607,7 @@ __global__ void __launch_bounds__(SigCfg<L>::THREADS, SigCfg<L>::MIN_CTAS) kc_si
                     break;
                 }
                 if (sk[old] == key) {
-                    const u32 mine_p = sp[slot];
-                    const u32 was = atomicMin(&sp[old], mine_p);
-                    kc_flag_clear_all<MULTI>(fl, was > mine_p ? was : mine_p);
+                    fold(old, slot);
                     break;
                 }
                 s2 = (s2 + 1) & (T2N - 1);
@@ -573,12 +619,12 @@ __global__ void __launch_bounds__(SigCfg<L>::THREADS, SigCfg<L>::MIN_CTAS) kc_si
     fetch(b, nr0, rec0);
     fetch(b + stride, nr1, rec1);
     u64 w0[NW], w1[NW];
-    kc_sig_load_words<NW>(packed, rec0, threadIdx.x < nr0 && nr0 <= RC, w0);
+    kc_sig_load_words<NW, POS64>(packed, rec0, threadIdx.x < nr0 && nr0 <= RC, w0);
     for (; b < n_buckets; b += stride) {
         u32 nr2;
         u64 rec2;
         fetch(b + 2 * stride, nr2, rec2);
-        kc_sig_load_words<NW>(packed, rec1, threadIdx.x < nr1 && nr1 <= RC, w1);
+        kc_sig_load_words<NW, POS64>(packed, rec1, threadIdx.x < nr1 && nr1 <= RC, w1);
         const u32 n_rec = nr0;
         const bool skip = n_rec == 0 || n_rec > RC;  // uniform over the CTA
         if (n_rec > RC && threadIdx.x == 0) status[0] = 1;  // the scan has set the status word already
@@ -635,6 +681,8 @@ template <int L> struct SigKernels {
             KC_CUDA(cudaFuncSetAttribute(kc_sig_resolve_kernel<L, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::smem()));
             KC_CUDA(cudaFuncSetAttribute(kc_sig_resolve_kernel<L, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::smem()));
             KC_CUDA(cudaFuncSetAttribute(kc_sig_resolve_kernel<L, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::smem()));
+            KC_CUDA(cudaFuncSetAttribute(kc_sig_resolve_kernel<L, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::smem(true)));
+            KC_CUDA(cudaFuncSetAttribute(kc_sig_resolve_kernel<L, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::smem(true)));
             dev[dv].n_sm = kc_sm_count(dv);
             KC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&dev[dv].occ, kc_sig_resolve_kernel<L, false, false>, Cfg::THREADS, Cfg::smem()));
         });
@@ -644,7 +692,7 @@ template <int L> struct SigKernels {
 
 template <bool P2P>
 inline void kc_sig_scan_launch(int m, u32 blocks, cudaStream_t st, const u8 *seq, u64 n_bytes, int k, int a, u32 n_buckets, u32 *cursor, u64 *recs, u64 *packed,
-                               u32 *flags, u32 n_flag_words, u32 tile0, kc_ull *m_cell, u32 *status, const u32 *win_mask, const SigPeers &sp) {
+                               u32 *flags, u64 n_flag_words, u32 tile0, kc_ull *m_cell, u32 *status, const u32 *win_mask, const SigPeers &sp) {
     switch (m) {
     case 16: kc_sig_scan_kernel<16, P2P><<<blocks, 256, 0, st>>>(seq, n_bytes, k, a, n_buckets, cursor, recs, packed, flags, n_flag_words, tile0, m_cell, status, win_mask, sp); break;
     case 15: kc_sig_scan_kernel<15, P2P><<<blocks, 256, 0, st>>>(seq, n_bytes, k, a, n_buckets, cursor, recs, packed, flags, n_flag_words, tile0, m_cell, status, win_mask, sp); break;
@@ -690,7 +738,7 @@ bool kc_kmerset_build_sig(CudaExec &ex, const u8 *seq, u64 n_bytes, int k, bool 
             const u64 part_bytes = std::min<u64>(n_bytes, (u64) t1 * TILE) - (u64) t0 * TILE;
             // sequence read, code words + flag words + records written
             CudaExec::Scope sc(ex, KP_KS_SCATTER0, part_bytes + part_bytes / 4 + part_bytes / 8 + (u64) (part_bytes * 8 / KC_SIG_WINDOWS_PER_RECORD));
-            kc_sig_scan_launch<false>(pl.m, t1 - t0, st, seq, n_bytes, k, pl.a, pl.n_buckets, cursor, recs, packed, flags, (u32) (kc_div_up(n_bytes, (u64) 32) + 1),
+            kc_sig_scan_launch<false>(pl.m, t1 - t0, st, seq, n_bytes, k, pl.a, pl.n_buckets, cursor, recs, packed, flags, kc_div_up(n_bytes, (u64) 32) + 1,
                                       t0, m_cell, status, win_mask, SigPeers());
             ++ex.launches;
         }
@@ -701,12 +749,11 @@ bool kc_kmerset_build_sig(CudaExec &ex, const u8 *seq, u64 n_bytes, int k, bool 
         const u32 grid = pl.n_buckets < fit ? pl.n_buckets : fit;
         // records read, two code words per record
         CudaExec::Scope sc(ex, KP_KS_RESOLVE, (u64) (n_bytes * (8 + 8 * Cfg::NW) / KC_SIG_WINDOWS_PER_RECORD));
-        if (complements)
-            kc_sig_resolve_kernel<L, false, false><<<grid, Cfg::THREADS, Cfg::smem(), st>>>(packed, k, cursor, recs, pl.n_buckets, kc_ksf_own_flags(flags),
-                                                                                          reinterpret_cast<kc_ull *>(cells), status, 1u, KC_SIG_REC_CAP, 0u);
-        else
-            kc_sig_resolve_kernel<L, false, true><<<grid, Cfg::THREADS, Cfg::smem(), st>>>(packed, k, cursor, recs, pl.n_buckets, kc_ksf_own_flags(flags),
-                                                                                         reinterpret_cast<kc_ull *>(cells), status, 1u, KC_SIG_REC_CAP, 0u);
+        const bool pos64 = n_bytes > 0xFFFFFFFFULL;  // a window END position may need more than 32 bits
+        auto *kern = complements ? (pos64 ? kc_sig_resolve_kernel<L, false, false, true> : kc_sig_resolve_kernel<L, false, false, false>)
+                                 : (pos64 ? kc_sig_resolve_kernel<L, false, true, true> : kc_sig_resolve_kernel<L, false, true, false>);
+        kern<<<grid, Cfg::THREADS, Cfg::smem(pos64), st>>>(packed, k, cursor, recs, pl.n_buckets, kc_ksf_own_flags(flags), reinterpret_cast<kc_ull *>(cells), status,
+                                                           1u, KC_SIG_REC_CAP, 0u);
         ++ex.launches;
         KC_CUDA(cudaGetLastError());
     }
@@ -746,7 +793,7 @@ inline void kc_sig_group_scan(CudaExec &ex, const u8 *seq, u64 n_bytes, int k, c
     if (t1 > t0) {
         slice_bytes = std::min<u64>(n_bytes, (u64) t1 * TILE) - (u64) t0 * TILE;
         CudaExec::Scope sc(ex, KP_KS_SCATTER0, slice_bytes + (slice_bytes / 4 + slice_bytes / 8) * (u64) sp.n + (u64) (slice_bytes * 8 / KC_SIG_WINDOWS_PER_RECORD));
-        kc_sig_scan_launch<true>(pl.m, t1 - t0, ex.stream, seq, n_bytes, k, pl.a, pl.n_buckets, cursor, staged, nullptr, nullptr, (u32) kc_div_up(n_bytes, (u64) 32), t0,
+        kc_sig_scan_launch<true>(pl.m, t1 - t0, ex.stream, seq, n_bytes, k, pl.a, pl.n_buckets, cursor, staged, nullptr, nullptr, kc_div_up(n_bytes, (u64) 32), t0,
                                  reinterpret_cast<kc_ull *>(cells + 2), status, nullptr, sp);
         ++ex.launches;
     }

@@ -115,6 +115,8 @@ inline RunNodes kc_runs_from_flags(CudaExec &ex, const u32 *flags, u64 n_pos, in
         return runs;
     }
     const u64 n_runs = host_cells[1];
+    // run numbers are 32-bit in the emit kernel (and node ids in the overlap stage); an input of 2^32 bytes or more can have more runs
+    if (n_runs >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "too many first-occurrence runs for one GPU");
     if (n_runs == 0) {
         ex.arena->release(mark);
         return runs;
