@@ -234,9 +234,13 @@ uint64_t kc_total_launches(const kc_ctx *ctx);
  * multi-level plan and the overflow fallback with small inputs; "fast_heuristics" (default 1): skip the attempt when
  * duplicates are expected (-z > 1, or the previous call on an input of similar size overflowed).
  * "fast_max_ctas": upper bound of the level >= 1 scatter grid.
+ * "tail_spec" (default 1): after the signature-bucket construction, queue the rest of the call sized for a few hundred
+ * first-occurrence runs (a genome) with no host round trip before the end; an input with more runs falls back to the
+ * ordinary path, and the context skips the attempt for inputs of similar size after that (with "fast_heuristics").
  * Results never depend on these options. */
 int kc_set_option(kc_ctx *ctx, const char *name, int value);
-/* Counters since kc_init: "sig_runs", "sig_fallbacks", "fast_runs", "fast_fallbacks", "total_launches"; current value of the
+/* Counters since kc_init: "sig_runs", "sig_fallbacks", "fast_runs", "fast_fallbacks", "total_launches", "tail_spec_runs",
+ * "tail_spec_fallbacks", "read_backs" (synchronising device -> host reads, i.e. host round trips); current value of the
  * option "fast_max_ctas"; device arena: "arena_bytes" (reserved now), "arena_high" (most bytes in use at once since kc_init). */
 int kc_get_stat(const kc_ctx *ctx, const char *name, uint64_t *value);
 

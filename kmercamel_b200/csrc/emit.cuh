@@ -99,12 +99,32 @@ template <int L> KmerIndex<L> kc_kmer_index_build(CudaExec &ex, const KWord<L> *
 
 static const u32 KC_RANK_SMALL = 1024;
 
+// Chunks of KC_EMIT_CHUNK output characters that node v writes, given its rank (the record-node emission of kc_emit_superstring).
+KC_HD u32 kc_emit_node_chunks(u64 cnt, u64 off, u64 s_begin, u64 s_end) {
+    if (cnt <= KC_EMIT_SHORT) return 0;
+    // the node's chunks start at its 16-byte aligned first byte; only those that meet the slice [s_begin, s_end) of this
+    // rank are enumerated (a rank of an 8-GPU job used to walk all chunks of the whole superstring: 0.26 ms instead of 0.06)
+    const u64 a0 = off & ~(u64) 15, a1 = off + cnt;
+    const u64 lo = a0 > s_begin ? a0 : s_begin, hi = a1 < s_end ? a1 : s_end;
+    return lo < hi ? (u32) ((hi - a0 + KC_EMIT_CHUNK - 1) / KC_EMIT_CHUNK - (lo - a0) / KC_EMIT_CHUNK) : 0u;
+}
+
 // List ranking of up to KC_RANK_SMALL nodes by one CTA in shared memory (same recurrences as the multi-kernel path).
+// chunks != nullptr (the deferred emission of a whole superstring): the same CTA also writes the exclusive prefix of the chunk counts
+// (chunks[0..N], N + 1 entries) and the characters of the short contributions into ms, which would otherwise take three more launches.
+// n_dev != nullptr: {n, N} on the device, and N is their cap (the entries past the real N get no chunks).
 template <int L>
-__global__ void __launch_bounds__(256) kc_rank_small_kernel(PathState s, NodeSeq<L> q, u32 N, u32 *fin_out, u64 *dist_out, u64 *cell) {
+__global__ void __launch_bounds__(256) kc_rank_small_kernel(PathState s, NodeSeq<L> q, u32 N, u32 *fin_out, u64 *dist_out, u64 *cell,
+                                                            const u32 *n_dev, u32 *chunks, u8 *ms) {
     __shared__ u32 jump[2][KC_RANK_SMALL], fin[2][KC_RANK_SMALL];
     __shared__ u64 dist[2][KC_RANK_SMALL];
     __shared__ u32 s_start, s_cyc;
+    __shared__ u32 sw[8];
+    const u32 n_cells = N;  // chunks[] has n_cells + 1 entries
+    if (n_dev) {
+        q.n = n_dev[0];
+        N = n_dev[1];
+    }
     if (threadIdx.x == 0) {
         s_start = KC_NONE;
         s_cyc = 0;
@@ -150,6 +170,43 @@ __global__ void __launch_bounds__(256) kc_rank_small_kernel(PathState s, NodeSeq
         cell[2] = st0 < N ? dist[cur][st0] : 0;
         cell[3] = st0 < N ? fin[cur][st0] : 0;
     }
+    if (!chunks) return;
+    const u32 st0 = s_start;
+    const u64 total = st0 < N ? dist[cur][st0] : 0;
+    const u32 fin_start = st0 < N ? fin[cur][st0] : 0;
+    u32 carry = 0;
+    for (u32 t0 = 0; t0 <= n_cells; t0 += 1024) {  // exclusive scan over n_cells + 1 entries, four per thread
+        const u32 base = t0 + threadIdx.x * 4;
+        u32 c4[4], c = 0;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const u32 v = base + j;
+            c4[j] = 0;
+            if (v < N && fin[cur][v] == fin_start) {
+                const u64 cnt = q.length(v) - (s.edge_from[v] != KC_NONE ? (u64) s.ovl[v] : 0);
+                c4[j] = kc_emit_node_chunks(cnt, total - dist[cur][v], 0, total);
+            }
+            c += c4[j];
+        }
+        u32 tile;
+        u32 p = kc_block_exclusive_scan_256(c, &tile, sw) + carry;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            if (base + j <= n_cells) chunks[base + j] = p;
+            p += c4[j];
+        }
+        carry += tile;
+        __syncthreads();  // sw is reused by the next tile
+    }
+    for (u32 v = threadIdx.x; v < N; v += 256) {  // the short contributions, one thread each
+        if (fin[cur][v] != fin_start) continue;
+        const u64 len = q.length(v);
+        const u64 cnt = len - (s.edge_from[v] != KC_NONE ? (u64) s.ovl[v] : 0);
+        if (cnt > KC_EMIT_SHORT) continue;
+        const u64 off = total - dist[cur][v];
+        const u64 n_upper = len - q.k + 1;
+        for (u64 j = 0; j < cnt && off + j < total; ++j) ms[off + j] = kc_letter(q.symbol(v, j), j < n_upper);
+    }
 }
 #endif
 
@@ -161,10 +218,25 @@ struct EmitResult {
     u64 slice_begin = 0, slice_len = 0;  // the part of it that `ms` holds (the whole superstring unless a slice was asked for)
 };
 
+// The speculative tail of kcgpu.cu: the node count is on the device ({n, N} at n_dev; nv and ns hold its cap) and the emission's
+// cell goes to `cell`, which the caller reads back with the rest of its status (kc_emit_check on words 0..3 of it).
+struct EmitSpec {
+    const u32 *n_dev;
+    u64 *cell;  // 6 words
+};
+
+// The host's checks of the emission's cell {start node, 0 if a cycle survived, length, ...}.
+inline void kc_emit_check(const u64 *info, u64 N, u64 total_ub) {
+    if (info[0] >= N) KC_THROW(KC_ERR_INTERNAL, "no start node: the path cover contains only cycles");
+    if (info[1] == 0) KC_THROW(KC_ERR_INTERNAL, "cycle in the final path cover");
+    if (total_ub && info[2] > total_ub) KC_THROW(KC_ERR_INTERNAL, "superstring longer than its bound");
+}
+
 // set_keys: sorted distinct (canonical when complements) k-mers, needed only for want_maxone.
 template <class Exec, int L>
 EmitResult kc_emit_superstring(Exec &ex, const NodeSeq<L> &ns, const NodeView<L> &nv, const PathState &st,
-                               const KWord<L> *set_keys, u64 n_set, bool want_maxone, u32 slice_index = 0, u32 n_slices = 1, u64 total_ub = 0) {
+                               const KWord<L> *set_keys, u64 n_set, bool want_maxone, u32 slice_index = 0, u32 n_slices = 1, u64 total_ub = 0,
+                               const EmitSpec *spec = nullptr) {
     // total_ub: an upper bound of the superstring length known to the caller (0 = none).  With it, a small problem (one-CTA list
     // ranking, record nodes, whole superstring) is emitted WITHOUT reading the length back first: the kernels take the length and the
     // printed strand from the device cell, the buffer and the launches are sized by the bound, and the one read-back comes after the
@@ -176,21 +248,31 @@ EmitResult kc_emit_superstring(Exec &ex, const NodeSeq<L> &ns, const NodeView<L>
     u32 *jump_a = ex.template alloc<u32>(N), *jump_b = ex.template alloc<u32>(N);
     u32 *fin_a = ex.template alloc<u32>(N), *fin_b = ex.template alloc<u32>(N);
     u64 *dist_a = ex.template alloc<u64>(N), *dist_b = ex.template alloc<u64>(N);
-    u64 *cell = ex.template alloc<u64>(6);  // [0] start node, [1] 0 if a cycle survived, [2..4] info for the host
+    u64 *cell = spec ? spec->cell : ex.template alloc<u64>(6);  // [0] start node, [1] 0 if a cycle survived, [2..4] info for the host
+    const u32 *n_dev = spec ? spec->n_dev : nullptr;
     const PathState s = st;
-    const NodeSeq<L> q = ns;
+    const NodeSeq<L> q = ns, q0 = ns;
     bool ranked = false;
+    bool deferred = false;
+    u8 *ms_pre = nullptr;
+    u32 *chunks_pre = nullptr;
 #ifdef __CUDACC__
     if constexpr (Exec::is_device) {
         if (N <= KC_RANK_SMALL) {  // the whole list ranking in one CTA (a genome leaves a few dozen nodes)
+            deferred = total_ub && !ns.kmers && !want_maxone && n_slices == 1;
+            if (deferred) {
+                ms_pre = ex.template alloc<u8>(total_ub + 1);
+                chunks_pre = ex.template alloc<u32>(N + 1);
+            }
             typename Exec::Scope sc(ex, KP_RANK, N * 25);
-            kc_rank_small_kernel<L><<<1, 256, 0, ex.stream>>>(s, q, (u32) N, fin_a, dist_a, cell);
+            kc_rank_small_kernel<L><<<1, 256, 0, ex.stream>>>(s, q, (u32) N, fin_a, dist_a, cell, n_dev, chunks_pre, ms_pre);
             ++ex.launches;
             KC_CUDA(cudaGetLastError());
             ranked = true;
         }
     }
 #endif
+    if (spec && !deferred) KC_THROW(KC_ERR_INTERNAL, "the speculative tail needs the deferred one-CTA emission");
     if (!ranked) {
         ex.fill_bytes(cell, 0xFF, 16);
         ex.for_each(N, [=] KC_HD_LAMBDA(u64 vv) {
@@ -238,17 +320,11 @@ EmitResult kc_emit_superstring(Exec &ex, const NodeSeq<L> &ns, const NodeView<L>
             });
         }
     }
-    bool deferred = false;
-#ifdef __CUDACC__
-    if constexpr (Exec::is_device) deferred = ranked && total_ub && !ns.kmers && !want_maxone && n_slices == 1;
-#endif
     const u64 *cellp = deferred ? cell : nullptr;  // deferred: the kernels below read the length and the printed strand from here
     u64 info[4] = {0, 1, total_ub, 0};
     if (!deferred) {
         ex.read_n(cell, info, 4);
-        const u64 start = info[0];
-        if (start >= N) KC_THROW(KC_ERR_INTERNAL, "no start node: the path cover contains only cycles");
-        if (info[1] == 0) KC_THROW(KC_ERR_INTERNAL, "cycle in the final path cover");
+        kc_emit_check(info, N, 0);
     }
     const u64 total_h = info[2];  // deferred: the bound (sizes the buffer and the launches)
     const u32 fin_start_h = (u32) info[3];
@@ -263,7 +339,7 @@ EmitResult kc_emit_superstring(Exec &ex, const NodeSeq<L> &ns, const NodeView<L>
     const u64 s_end_h = n_slices > 1 && slice_index + 1 < n_slices ? ((total / n_slices) * (slice_index + 1)) & ~(u64) 15 : total;
     const u64 s_end = s_end_h;
     const u32 fin_start = fin_start_h;
-    u8 *ms_base = ex.template alloc<u8>(s_end - s_begin + 1);
+    u8 *ms_base = deferred ? ms_pre : ex.template alloc<u8>(s_end - s_begin + 1);
     u8 *ms = ms_base - s_begin;
     res.ms = ms_base;
     res.length = total;
@@ -288,26 +364,19 @@ EmitResult kc_emit_superstring(Exec &ex, const NodeSeq<L> &ns, const NodeView<L>
         // Chunks are laid out on the OUTPUT: a chunk is 256 work items x 16 bytes, 16-byte aligned in `ms`, so a full
         // item is one st.global.v4 and a warp writes 512 contiguous bytes (the per-character version spent 0.16 ms
         // on 50 MB; byte stores, not DRAM, were the bound).
-        u32 *chunks = ex.template alloc<u32>(N + 1);
-        ex.for_each(N + 1, [=] KC_HD_LAMBDA(u64 vv) {
-            const u64 total = cellp ? cellp[2] : total_h;
-            const u32 fin_start = cellp ? (u32) cellp[3] : fin_start_h;
-            const u64 s_end = cellp ? total : s_end_h;
-            u32 c = 0;
-            if (vv < N && fa[vv] == fin_start) {
-                u32 v = (u32) vv;
-                u64 cnt = q.length(v) - (s.edge_from[v] != KC_NONE ? (u64) s.ovl[v] : 0);
-                if (cnt > KC_EMIT_SHORT) {
-                    u64 off = total - da[v];
-                    // the node's chunks start at its 16-byte aligned first byte; only those that meet the slice [s_begin, s_end) of this
-                    // rank are enumerated (a rank of an 8-GPU job used to walk all chunks of the whole superstring: 0.26 ms instead of 0.06)
-                    const u64 a0 = off & ~(u64) 15, a1 = off + cnt;
-                    const u64 lo = a0 > s_begin ? a0 : s_begin, hi = a1 < s_end ? a1 : s_end;
-                    if (lo < hi) c = (u32) ((hi - a0 + KC_EMIT_CHUNK - 1) / KC_EMIT_CHUNK - (lo - a0) / KC_EMIT_CHUNK);
+        // Deferred: kc_rank_small_kernel has written the chunk prefix and the short contributions already.
+        u32 *chunks = deferred ? chunks_pre : ex.template alloc<u32>(N + 1);
+        if (!deferred) {
+            ex.for_each(N + 1, [=] KC_HD_LAMBDA(u64 vv) {
+                u32 c = 0;
+                if (vv < N && fa[vv] == fin_start_h) {
+                    u32 v = (u32) vv;
+                    u64 cnt = q.length(v) - (s.edge_from[v] != KC_NONE ? (u64) s.ovl[v] : 0);
+                    c = kc_emit_node_chunks(cnt, total_h - da[v], s_begin, s_end_h);
                 }
-            }
-            chunks[vv] = c;
-        }, KP_EMIT, N * 12);
+                chunks[vv] = c;
+            }, KP_EMIT, N * 12);
+        }
         // Few nodes: launch for an upper bound of the chunk count (a node's chunks span at most its characters + 15 bytes of
         // alignment) and let the surplus work items exit, instead of reading the exact count back.
         u32 n_chunks = 0;
@@ -316,16 +385,16 @@ EmitResult kc_emit_superstring(Exec &ex, const NodeSeq<L> &ns, const NodeView<L>
         if constexpr (Exec::is_device) {
             if (N <= 65536) {
                 bounded = true;
-                ex.exclusive_scan_nosync(chunks, chunks, N + 1);
+                if (!deferred) ex.exclusive_scan_nosync(chunks, chunks, N + 1);
                 n_chunks = (u32) ((s_end - s_begin) / KC_EMIT_CHUNK + 2 * N + 1);
             }
         }
 #endif
         if (!bounded) n_chunks = ex.exclusive_scan(chunks, chunks, N + 1);
-        ex.for_each(N, [=] KC_HD_LAMBDA(u64 vv) {
-            const u64 total = cellp ? cellp[2] : total_h;
-            const u32 fin_start = cellp ? (u32) cellp[3] : fin_start_h;
-            const u64 s_end = cellp ? total : s_end_h;
+        if (!deferred) ex.for_each(N, [=] KC_HD_LAMBDA(u64 vv) {
+            const u64 total = total_h;
+            const u32 fin_start = fin_start_h;
+            const u64 s_end = s_end_h;
             u32 v = (u32) vv;
             if (fa[v] != fin_start) return;
             u64 len = q.length(v);
@@ -340,6 +409,8 @@ EmitResult kc_emit_superstring(Exec &ex, const NodeSeq<L> &ns, const NodeView<L>
         ex.for_each((u64) n_chunks * 256, [=] KC_HD_LAMBDA(u64 w) {
             const u64 total = cellp ? cellp[2] : total_h;
             const u64 s_end = cellp ? total : s_end_h;
+            NodeSeq<L> q = q0;
+            if (n_dev) q.n = n_dev[0];
             u32 chunk = (u32) (w >> 8), lane = (u32) (w & 255);
             if (chunk >= chunks[N]) return;  // chunks[N] = the exact number of chunks
             // node owning this chunk: last v with chunks[v] <= chunk (chunks[] is the exclusive prefix, N+1 entries)
@@ -444,11 +515,9 @@ EmitResult kc_emit_superstring(Exec &ex, const NodeSeq<L> &ns, const NodeView<L>
             mo[p] = present ? (u8) (c - ('a' - 'A')) : c;
         }, KP_MAXONE, 2 * total);
     }
-    if (deferred) {  // the one read-back of the stage, after its last kernel was queued
+    if (deferred && !spec) {  // the one read-back of the stage, after its last kernel was queued
         ex.read_n(cell, info, 4);
-        if (info[0] >= N) KC_THROW(KC_ERR_INTERNAL, "no start node: the path cover contains only cycles");
-        if (info[1] == 0) KC_THROW(KC_ERR_INTERNAL, "cycle in the final path cover");
-        if (info[2] > total_ub) KC_THROW(KC_ERR_INTERNAL, "superstring longer than its bound");
+        kc_emit_check(info, N, total_ub);
         res.length = info[2];
         res.slice_len = info[2];
     }

@@ -315,7 +315,13 @@ template <class Exec, int L> struct Engine {
 
     Engine(Exec &e, const NodeView<L> &v, bool strict_, bool lower_bound_) : ex(e), nv(v), strict(strict_), lower_bound(lower_bound_) {}
 
-    void init_state() {
+    // Speculative tail (kcgpu.cu): the real node count is on the device ({n, N} at n_dev) and nv holds its cap; the caller's kernel
+    // initialised the state, the identity live lists and the small engine's level masks (small_masks), and the status words of the
+    // single-CTA engine go to small_status, which the caller reads back with its own results (apply_small_status).
+    const u32 *n_dev = nullptr;
+    u32 *small_status = nullptr, *small_masks = nullptr;
+
+    void alloc_state() {
         const u64 N = nv.N;
         st.edge_from = ex.template alloc<u32>(N);
         st.edge_to = ex.template alloc<u32>(N);
@@ -331,6 +337,11 @@ template <class Exec, int L> struct Engine {
         ban_i = ex.template alloc<u32>(BAN_CAP);
         ban_j = ex.template alloc<u32>(BAN_CAP);
         ban_ctr = ex.template alloc<u32>(4);
+    }
+
+    void init_state() {
+        alloc_state();
+        const u64 N = nv.N;
         // one kernel instead of five fills and a kernel: on a genome the stage is a dozen tiny operations, each ~2 us of stream time
         PathState s = st;
         u8 *bf = ban_flag;
@@ -366,24 +377,29 @@ template <class Exec, int L> struct Engine {
 #ifdef __CUDACC__
         if constexpr (Exec::is_device) {
             if (!small_out) return;
-            u32 h[8 + 128 + 8];
-            ex.read_n(small_out, h, 8 + 128 + 8);
+            u32 h[KC_SMALL_STATUS_WORDS];
+            ex.read_n(small_out, h, KC_SMALL_STATUS_WORDS);
             small_out = nullptr;
-            if (std::getenv("KC_TRACE")) {
-                std::fprintf(stderr, "[kc_trace] small engine: n_s=%llu n_p=%llu levels=%u groups=%u edges=%u ban_rounds=%u bans=%u; clocks per level (* = run):",
-                             (unsigned long long) n_s, (unsigned long long) n_p, h[1], h[2], h[3], h[4], h[5]);
-                for (int dd = small_d; dd >= 0; --dd) std::fprintf(stderr, " d%d=%u%s", dd, h[8 + dd] & 0x7FFFFFFFu, (h[8 + dd] >> 31) ? "*" : "");
-                std::fprintf(stderr, "; phases: stage+mask=%u tuples=%u sort=%u groups=%u replay=%u validate+commit=%u lists=%u writeback=%u\n", h[136], h[137],
-                             h[138], h[139], h[140], h[141], h[142], h[143]);
-            }
-            if (h[0]) KC_THROW(KC_ERR_INTERNAL, "ban list overflow");
-            stats.levels_run += h[1];
-            stats.groups += h[2];
-            stats.edges += h[3];
-            stats.ban_rounds += h[4];
-            stats.bans += h[5];
+            apply_small_status(h);
         }
 #endif
+    }
+
+    // Statistics and error of a single-CTA engine run from its status words (read back by check_small or by the caller).
+    void apply_small_status(const u32 *h) {
+        if (std::getenv("KC_TRACE")) {
+            std::fprintf(stderr, "[kc_trace] small engine: n_s=%llu n_p=%llu levels=%u groups=%u edges=%u ban_rounds=%u bans=%u; clocks per level (* = run):",
+                         (unsigned long long) n_s, (unsigned long long) n_p, h[1], h[2], h[3], h[4], h[5]);
+            for (int dd = small_d; dd >= 0; --dd) std::fprintf(stderr, " d%d=%u%s", dd, h[8 + dd] & 0x7FFFFFFFu, (h[8 + dd] >> 31) ? "*" : "");
+            std::fprintf(stderr, "; phases: stage+mask=%u tuples=%u sort=%u groups=%u replay=%u validate+commit=%u lists=%u writeback=%u\n", h[136], h[137],
+                         h[138], h[139], h[140], h[141], h[142], h[143]);
+        }
+        if (h[0]) KC_THROW(KC_ERR_INTERNAL, "ban list overflow");
+        stats.levels_run += h[1];
+        stats.groups += h[2];
+        stats.edges += h[3];
+        stats.ban_rounds += h[4];
+        stats.bans += h[5];
     }
 
     // Runs levels d..0 in one kernel when the free ends fit in shared memory.  Device policy only.
@@ -422,9 +438,16 @@ template <class Exec, int L> struct Engine {
             a.strict = strict;
             // status words, then the level masks: [4] for the whole problem, then four words per end (two copies each: they travel with
             // the live lists); one allocation, one fill
-            a.out = ex.template alloc<u32>(8 + 128 + 8 + 4 + 8 * (n_s + n_p));
-            u32 *lvl_mask = a.out + (8 + 128 + 8);
-            ex.fill_bytes(a.out, 0, (8 + 128 + 8 + 4 + 4 * (n_s + n_p)) * 4);
+            u32 *lvl_mask;
+            if (n_dev) {
+                a.out = small_status;
+                lvl_mask = small_masks;
+            } else {
+                a.out = ex.template alloc<u32>(KC_SMALL_STATUS_WORDS + kc_small_mask_words(n_s, n_p) + 4 * (n_s + n_p));
+                lvl_mask = a.out + KC_SMALL_STATUS_WORDS;
+                ex.fill_bytes(a.out, 0, (KC_SMALL_STATUS_WORDS + kc_small_mask_words(n_s, n_p)) * 4);
+            }
+            a.n_dev = n_dev;
             a.lvl_mask_in = lvl_mask;
             a.end_mask_s_a = lvl_mask + 4;
             a.end_mask_p_a = a.end_mask_s_a + 4 * n_s;
@@ -441,7 +464,7 @@ template <class Exec, int L> struct Engine {
                 typename Exec::Scope sc(ex, KP_SMALL_ENGINE, 0);
                 const u32 per_cta = kc_small_mask_levels_per_cta<L>((u32) n_s, (u32) n_p);
                 kc_small_level_mask_kernel<L><<<(unsigned) kc_div_up((u64) d + 1, per_cta), 256, mask_smem, ex.stream>>>(nv, live_s, live_p, (u32) n_s, (u32) n_p, d,
-                                                                                                                      lvl_mask, a.end_mask_s_a, a.end_mask_p_a);
+                                                                                                                      lvl_mask, a.end_mask_s_a, a.end_mask_p_a, n_dev);
                 ++ex.launches;
             }
             {
@@ -451,14 +474,16 @@ template <class Exec, int L> struct Engine {
                 // 512 threads once the sort has work for them: two threads per tuple in the rank sort (129..256 tuples), more than two
                 // items per thread in the bitonic network (> 512 tuples)
                 const u64 nt0 = n_s + n_p;
-                const unsigned small_threads = small_threads_opt ? (unsigned) small_threads_opt : ((nt0 > 128 && nt0 <= 256) || nt0 > 512 ? 512u : 256u);
+                // (speculative tail: the count is not known here; 256 vs 512 threads is within 1.5 % at 50 records, r02z_small_engine_trace.txt)
+                const unsigned small_threads = small_threads_opt ? (unsigned) small_threads_opt
+                                               : n_dev || (nt0 > 128 && nt0 <= 256) || nt0 > 512 ? 512u : 256u;
                 kc_small_engine_kernel<L><<<1, small_threads, SmallCfg<L>::SMEM, ex.stream>>>(a);
             }
             ++ex.launches;
             KC_CUDA(cudaGetLastError());
             // The status words are read back by check_small() after the caller's next synchronisation point: the kernels of the
             // emission stage are queued behind this one without a host round trip.
-            small_out = a.out;
+            small_out = n_dev ? nullptr : a.out;
             small_d = d;
             return true;
         }

@@ -214,6 +214,7 @@ struct CudaExec {
     Arena *arena;
     KernelProf *prof = nullptr;
     u64 launches = 0;  // kernels launched through this policy (bench.py reports it as gpu_launches)
+    u64 read_backs = 0;  // synchronising read-backs (read_n), i.e. host round trips
     u8 *pinned = nullptr;  // page-locked host scratch of the context for the synchronising read-backs below: a pageable
     size_t pinned_cap = 0;  // destination makes the driver stage the copy, which costs several us per read on an idle stream
 
@@ -265,6 +266,7 @@ struct CudaExec {
     void sync() { KC_CUDA(cudaStreamSynchronize(stream)); }
     template <typename T> void read_n(const T *p, T *host, size_t n) {  // one synchronising read-back of n values
         const size_t bytes = n * sizeof(T);
+        ++read_backs;
         if (pinned && bytes <= pinned_cap) {
             KC_CUDA(cudaMemcpyAsync(pinned, p, bytes, cudaMemcpyDeviceToHost, stream));
             KC_CUDA(cudaStreamSynchronize(stream));

@@ -14,6 +14,7 @@
 #include "runs.cuh"
 #include "sort.cuh"
 #include "stage1.cuh"
+#include "tail_spec.cuh"
 
 #include <chrono>
 #include <mutex>
@@ -60,6 +61,10 @@ struct kc_ctx {
     bool fast_heuristics = true;  // skip the fixed-slot attempt when duplicates are expected (see run_stage1_runs)
     u64 fast_overflow_bytes = 0;  // input size of the last call whose fixed-slot attempt overflowed (0 = none)
     u64 total_launches = 0;  // kernels launched through this context since kc_init
+    u64 read_backs = 0;      // synchronising device -> host reads of this context since kc_init (host round trips)
+    bool tail_spec = true;   // option "tail_spec": queue the tail of the from-FASTA path without reading the run count (run_tail_spec)
+    u64 tail_spec_runs = 0, tail_spec_fallbacks = 0;
+    u64 spec_fail_bytes = 0;  // input size of the last call whose speculative tail did not hold (0 = none)
     KcGroup grp;             // multi-GPU: this context as one rank of a group (group.cuh)
     bool arena_limited = false;
     std::string last_error;
@@ -203,6 +208,93 @@ template <int L> u64 run_stage1(kc_ctx *ctx, CudaExec &ex, const DevInput &in, c
     return set.n_kept;
 }
 
+// The speculative tail (tail_spec.cuh): from the first-occurrence flags to the last emission kernel, sized for KC_SPEC_RUNS runs, with
+// ONE read-back of the status block `blk` (cells4 of the signature construction first, KC_SPEC_BLOCK_WORDS words, zeroed) at the end.
+// Returns the status: KC_SPEC_OK = `res` holds the result; otherwise nothing was done and the arena is as it was on entry.
+template <int L>
+u32 run_tail_spec(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &p, const u32 *flags, u64 *blk, DevResult &res) {
+    const u64 nb = in.n_bytes;
+    const int k = p.k;
+    const bool complements = p.complements != 0;
+    const size_t mark = ex.arena->mark();
+    const u32 C = KC_SPEC_RUNS, N_cap = complements ? 2 * C : C;
+    const u64 n_words = kc_div_up(nb, 32);
+    const u32 blocks = (u32) kc_div_up(nb, (u64) KC_RUN_TILE);
+    u32 *counts = ex.alloc<u32>(blocks);
+    u64 *rec_off = ex.alloc<u64>(C), *rec_len = ex.alloc<u64>(C);
+    kc_ull *n_runs = reinterpret_cast<kc_ull *>(blk + 1);
+    {
+        CudaExec::Scope sc(ex, KP_RUNS, nb / 8);
+        kc_runs_count_kernel<<<blocks, 256, 0, ex.stream>>>(flags, n_words, counts, n_runs);
+        kc_runs_emit_kernel<<<blocks, 256, 0, ex.stream>>>(flags, n_words, counts, rec_off, rec_len, n_runs, C);
+    }
+    ex.launches += 2;
+    KC_CUDA(cudaGetLastError());
+    KC_CUDA(cudaEventRecord(ctx->ev[2], ex.stream));
+    NodeView<L> nv;
+    nv.k = k;
+    nv.complements = complements;
+    nv.n = C;
+    nv.N = N_cap;
+    KWord<L> *first = ex.alloc<KWord<L>>(C), *last = ex.alloc<KWord<L>>(C);
+    nv.first = first;
+    nv.last = last;
+    Engine<CudaExec, L> eng(ex, nv, /*strict=*/false, /*lower_bound=*/false);
+    eng.small_threads_opt = ctx->small_threads;
+    eng.alloc_state();
+    u32 *spec = reinterpret_cast<u32 *>(blk + KC_SPEC_SPEC);
+    eng.n_dev = spec + 1;
+    eng.small_status = reinterpret_cast<u32 *>(blk + KC_SPEC_SMALL);
+    const u64 mask_words = kc_small_mask_words(N_cap, N_cap);
+    eng.small_masks = ex.alloc<u32>(mask_words + 4 * (u64) (2 * N_cap));  // + the second copies of the end masks
+    eng.live_s = ex.alloc<u32>(N_cap);
+    eng.live_p = ex.alloc<u32>(N_cap);
+    eng.n_s = eng.n_p = N_cap;
+    {
+        CudaExec::Scope sc(ex, KP_RUNS, 32 * (u64) C);
+        kc_spec_nodes_kernel<L><<<1, 1024, 0, ex.stream>>>(blk, spec, ctx->sparse_switch, complements, in.seq, k, rec_off, rec_len, first, last,
+                                                            eng.st, eng.ban_flag, eng.ban_ctr, eng.live_s, eng.live_p, eng.small_masks, (u32) mask_words);
+    }
+    ++ex.launches;
+    KC_CUDA(cudaGetLastError());
+    static_assert(4 * KC_SPEC_RUNS <= SmallCfg<L>::T && 2 * KC_SPEC_RUNS <= SmallCfg<L>::NS && 2 * KC_SPEC_RUNS <= KC_RANK_SMALL,
+                  "the speculative tail runs on the one-CTA kernels");
+    eng.run();  // all levels in the single-CTA engine
+    KC_CUDA(cudaEventRecord(ctx->ev[3], ex.stream));
+    NodeSeq<L> ns;
+    ns.k = k;
+    ns.kmers = nullptr;
+    ns.seq = in.seq;
+    ns.rec_off = rec_off;
+    ns.rec_len = rec_len;
+    ns.n = C;
+    const EmitSpec es{spec + 1, blk + KC_SPEC_EMIT};
+    // every character of the superstring is a character of some node: nodes are pieces of the input that overlap by < k
+    const u64 total_ub = nb + (u64) C * k + 16;
+    const EmitResult er = kc_emit_superstring<CudaExec, L>(ex, ns, nv, eng.st, nullptr, 0, false, 0, 1, total_ub, &es);
+    KC_CUDA(cudaEventRecord(ctx->ev[4], ex.stream));
+    KC_TRACE_POINT("tail_spec: queued");
+    u64 h[KC_SPEC_BLOCK_WORDS];
+    ex.read_n(blk, h, KC_SPEC_BLOCK_WORDS);
+    const u32 *hs = reinterpret_cast<const u32 *>(h + KC_SPEC_SPEC);
+    if (hs[0] != KC_SPEC_OK) {
+        ex.arena->release(mark);
+        return hs[0];
+    }
+    eng.apply_small_status(reinterpret_cast<const u32 *>(h + KC_SPEC_SMALL));  // a failed small-engine run is the cause, report that one
+    kc_emit_check(h + KC_SPEC_EMIT, hs[2], total_ub);
+    res.ms = er.ms;
+    res.maxone = nullptr;
+    res.length = h[KC_SPEC_EMIT + 2];
+    res.slice_begin = 0;
+    res.slice_len = res.length;
+    res.n_kmers = h[0];
+    res.n_occ = h[2];
+    res.n_nodes = hs[1];
+    res.n_simplitigs = hs[1];
+    return KC_SPEC_OK;
+}
+
 // From-FASTA regime: the nodes handed to the overlap stage are FIRST-OCCURRENCE RUNS.
 //
 // The reference turns the k-mer set into simplitigs by walking a hash table (src/simplitigs.h:105-205); which
@@ -213,8 +305,12 @@ template <int L> u64 run_stage1(kc_ctx *ctx, CudaExec &ex, const DevInput &in, c
 // simplitig read directly off the input, with no hash walk and no per-k-mer pointer chasing.  Runs are numbered
 // in input order and go through the same overlap levels d = k-1..0 as `-S` records, so run ends that overlap by
 // k-1 are still joined first, exactly as BIGREEDY requires.
+//
+// spec_res != nullptr: after the signature construction, try the speculative tail (run_tail_spec).  When it holds, *spec_res is the whole
+// result and *spec_done is set; otherwise the code below continues as if it had not been tried, on the same flags.
 template <int L>
-u64 run_stage1_runs(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &p, RunNodes *runs, KWord<L> **set_out, u64 *n_occ) {
+u64 run_stage1_runs(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &p, RunNodes *runs, KWord<L> **set_out, u64 *n_occ,
+                    DevResult *spec_res = nullptr, bool *spec_done = nullptr) {
     KC_CUDA(cudaEventRecord(ctx->ev[0], ex.stream));
     KC_CUDA(cudaEventRecord(ctx->ev[1], ex.stream));  // extraction is fused into the partition passes
     KC_TRACE_POINT("stage1: begin");
@@ -235,13 +331,30 @@ u64 run_stage1_runs(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_para
     const bool large = nb >= KC_POS32_BYTES;
     const bool sig_overflowed = ctx->fast_heuristics && ctx->sig_overflow_bytes && nb >= ctx->sig_overflow_bytes / 2 && nb <= ctx->sig_overflow_bytes * 2;
     if (!p.want_maxone && p.min_frequency == 1 && (large || !sig_overflowed)) {
-        u64 *cells4 = ex.arena->alloc_top<u64>(4);  // {kept, runs, M, overflow status}
-        ex.fill_bytes(cells4, 0, 32);
+        const size_t n_cells = spec_res ? KC_SPEC_BLOCK_WORDS : 4;
+        u64 *cells4 = ex.arena->alloc_top<u64>(n_cells);  // {kept, runs, M, overflow status} (+ the rest of the speculative tail's status block)
+        ex.fill_bytes(cells4, 0, n_cells * 8);
         if (kc_kmerset_build_sig<L>(ex, in.seq, nb, p.k, p.complements != 0, flags, cells4, ctx->sig, in.chunks)) {
             KC_TRACE_POINT("stage1: signature set launched");
             u64 hc[4];
             bool aborted = false;
-            *runs = kc_runs_from_flags(ex, flags, nb, p.k, cells4, hc, 4, &aborted);
+            if (spec_res) {
+                const u32 st = run_tail_spec<L>(ctx, ex, in, p, flags, cells4, *spec_res);
+                if (st == KC_SPEC_OK) {
+                    ++ctx->sig_runs;
+                    ++ctx->tail_spec_runs;
+                    *spec_done = true;
+                    return spec_res->n_kmers;
+                }
+                ++ctx->tail_spec_fallbacks;
+                if (st == KC_SPEC_SIG_OVERFLOW) {
+                    aborted = true;
+                } else {  // the flags stand: the ordinary tail counts the runs again
+                    if (st != KC_SPEC_EMPTY) ctx->spec_fail_bytes = nb;
+                    ex.fill_bytes(cells4 + 1, 0, 8);
+                }
+            }
+            if (!aborted) *runs = kc_runs_from_flags(ex, flags, nb, p.k, cells4, hc, 4, &aborted);
             if (!aborted) {
                 ++ctx->sig_runs;
                 *n_occ = hc[2];
@@ -354,7 +467,13 @@ void run_pipeline(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params
             n_occ = ext->n_occ;
             KC_CUDA(cudaEventRecord(ctx->ev[2], ex.stream));
         } else {
-            U = run_stage1_runs<L>(ctx, ex, in, p, &runs, &uniq, &n_occ);
+            // the speculative tail: a FASTA input with few runs (a genome) is computed behind one read-back (run_tail_spec)
+            const u64 nb = in.n_bytes;
+            const bool spec_failed = ctx->fast_heuristics && ctx->spec_fail_bytes && nb >= ctx->spec_fail_bytes / 2 && nb <= ctx->spec_fail_bytes * 2;
+            const bool spec = ctx->tail_spec && !spec_failed && !lower_bound && ctx->small_engine && nb > 0 && nb < KC_POS32_BYTES;
+            bool spec_done = false;
+            U = run_stage1_runs<L>(ctx, ex, in, p, &runs, &uniq, &n_occ, spec ? &res : nullptr, &spec_done);
+            if (spec_done) return;
         }
         if (U == 0) KC_THROW(KC_ERR_EMPTY, "the input contains no k-mers");  // src/main.cpp:155-158
         res.n_simplitigs = runs.n_runs;
@@ -787,6 +906,7 @@ int kc_compute_device(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_ou
     out->n_launches = ex.launches;
     fill_times(ctx, out);
     ctx->total_launches += ex.launches;
+    ctx->read_backs += ex.read_backs;
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -867,6 +987,7 @@ int kc_compute(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_output *o
     out->n_launches = ex.launches;
     fill_times(ctx, out);
     ctx->total_launches += ex.launches;
+    ctx->read_backs += ex.read_backs;
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -911,6 +1032,7 @@ int kc_lower_bound(kc_ctx *ctx, const kc_params *p, const kc_input *in, uint64_t
         fill_times(ctx, stats);
     }
     ctx->total_launches += ex.launches;
+    ctx->read_backs += ex.read_backs;
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -964,6 +1086,7 @@ int kc_streaming(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_output 
     out->n_launches = ex.launches;
     fill_times(ctx, out);
     ctx->total_launches += ex.launches;
+    ctx->read_backs += ex.read_backs;
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -1000,6 +1123,7 @@ int kc_maskopt(kc_ctx *ctx, const uint8_t *ms, uint64_t n, int k, int complement
     out->n_launches = ex.launches;
     fill_times(ctx, out);
     ctx->total_launches += ex.launches;
+    ctx->read_backs += ex.read_backs;
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -1035,6 +1159,7 @@ int kc_count_kmers(kc_ctx *ctx, const kc_params *p, const kc_input *in, uint64_t
     else if (p->k < 64) count_only<2>(ctx, ex, di, *p, keys, counts, n);
     else count_only<4>(ctx, ex, di, *p, keys, counts, n);
     ctx->total_launches += ex.launches;
+    ctx->read_backs += ex.read_backs;
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -1066,6 +1191,7 @@ int kc_partial_presort(kc_ctx *ctx, const uint64_t *kmers, uint64_t n, int k, ui
     KC_CUDA(cudaMemcpyAsync(out, dst, n * limbs * 8, cudaMemcpyDeviceToHost, ctx->stream));
     KC_CUDA(cudaStreamSynchronize(ctx->stream));
     ctx->total_launches += ex.launches;
+    ctx->read_backs += ex.read_backs;
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -1113,6 +1239,7 @@ int kc_kmer_digest(kc_ctx *ctx, const kc_params *p, const kc_input *in, int mask
     else if (limbs == 2) digest_only<2>(ctx, ex, di, *p, win_mask, digest);
     else digest_only<4>(ctx, ex, di, *p, win_mask, digest);
     ctx->total_launches += ex.launches;
+    ctx->read_backs += ex.read_backs;
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -1136,6 +1263,7 @@ int kc_overlap_path(kc_ctx *ctx, const uint64_t *first, const uint64_t *last, ui
     else if (k < 64) overlap_only<2>(ctx, ex, first, last, n, k, complements != 0, lower_bound != 0, strict != 0, edge_from, overlaps);
     else overlap_only<4>(ctx, ex, first, last, n, k, complements != 0, lower_bound != 0, strict != 0, edge_from, overlaps);
     ctx->total_launches += ex.launches;
+    ctx->read_backs += ex.read_backs;
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -1213,6 +1341,7 @@ int kc_group_compute_device(kc_ctx *ctx, const kc_params *p, const kc_input *in,
     out->n_launches = ex.launches;
     fill_times(ctx, out);
     ctx->total_launches += ex.launches;
+    ctx->read_backs += ex.read_backs;
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -1437,6 +1566,7 @@ int kc_group_compute(kc_group *g, const kc_params *p, const kc_input *in, kc_out
             R.launches = ex.launches;
             fill_times(ctx, &R.o);
             ctx->total_launches += ex.launches;
+            ctx->read_backs += ex.read_backs;
         } catch (const KcError &e) {
             R.code = e.code;
             char buf[512];
@@ -1494,6 +1624,9 @@ int kc_get_stat(const kc_ctx *ctx, const char *name, uint64_t *value) {
     else if (std::strcmp(name, "sig_runs") == 0) *value = ctx->sig_runs;
     else if (std::strcmp(name, "sig_fallbacks") == 0) *value = ctx->sig_fallbacks;
     else if (std::strcmp(name, "total_launches") == 0) *value = ctx->total_launches;
+    else if (std::strcmp(name, "read_backs") == 0) *value = ctx->read_backs;
+    else if (std::strcmp(name, "tail_spec_runs") == 0) *value = ctx->tail_spec_runs;
+    else if (std::strcmp(name, "tail_spec_fallbacks") == 0) *value = ctx->tail_spec_fallbacks;
     else if (std::strcmp(name, "arena_bytes") == 0) *value = ctx->arena.cap;
     else if (std::strcmp(name, "arena_high") == 0) *value = ctx->arena.high;
     else if (std::strcmp(name, "fast_max_ctas") == 0) *value = (uint64_t) ctx->fast.max_ctas;
@@ -1513,6 +1646,11 @@ int kc_set_option(kc_ctx *ctx, const char *name, int value) {
     }
     if (std::strcmp(name, "small_engine") == 0) {
         ctx->small_engine = value != 0;
+        return KC_OK;
+    }
+    if (std::strcmp(name, "tail_spec") == 0 && (value == 0 || value == 1)) {
+        ctx->tail_spec = value != 0;
+        ctx->spec_fail_bytes = 0;
         return KC_OK;
     }
     // histogram-free set construction (kmerset_fast.cuh); the last three exist so that tests can reach the multi-level
@@ -1537,6 +1675,7 @@ int kc_set_option(kc_ctx *ctx, const char *name, int value) {
         ctx->fast_heuristics = value != 0;
         ctx->fast_overflow_bytes = 0;
         ctx->sig_overflow_bytes = 0;
+        ctx->spec_fail_bytes = 0;
         return KC_OK;
     }
     if (std::strcmp(name, "fast_max_ctas") == 0 && value >= 0 && value <= (1 << 20)) {

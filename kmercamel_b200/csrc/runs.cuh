@@ -45,18 +45,34 @@ __global__ void __launch_bounds__(256) kc_runs_count_kernel(const u32 *flags, u6
 }
 
 // rec_off[r] = END position of the first window of run r, rec_len[r] = END position of its last window.
-__global__ void __launch_bounds__(256) kc_runs_emit_kernel(const u32 *flags, u64 n_words, const u32 *block_offsets, u64 *rec_off, u64 *rec_len) {
+// spec_total == nullptr: block_offsets = exclusive prefix of the per-block run counts.  Otherwise (speculative tail, kcgpu.cu) it holds
+// the counts themselves and *spec_total their sum: the kernel writes nothing when that exceeds spec_cap, and a block that holds a run
+// start or end sums the counts before it (one block in ~10^4 on a genome), instead of a scan launch in between.
+__global__ void __launch_bounds__(256) kc_runs_emit_kernel(const u32 *flags, u64 n_words, const u32 *block_offsets, u64 *rec_off, u64 *rec_len,
+                                                           const kc_ull *spec_total = nullptr, u64 spec_cap = 0) {
     __shared__ u32 sw[8];
+    if (spec_total && *spec_total > spec_cap) return;
     const u64 word = ((u64) blockIdx.x * 256 + threadIdx.x) * KC_RUN_WORDS;
     u32 f[KC_RUN_WORDS], prev, next;
     kc_runs_load(flags, word, n_words, f, prev, next);
-    u32 c = 0;
+    u32 c = 0, any = 0;
 #pragma unroll
-    for (int j = 0; j < KC_RUN_WORDS; ++j) c += __popc(kc_runs_starts(f[j], j ? f[j - 1] >> 31 : prev));
+    for (int j = 0; j < KC_RUN_WORDS; ++j) {
+        c += __popc(kc_runs_starts(f[j], j ? f[j - 1] >> 31 : prev));
+        any |= kc_runs_ends(f[j], j + 1 < KC_RUN_WORDS ? f[j + 1] & 1u : next);
+    }
+    if (!__syncthreads_or(c | any)) return;  // no run starts or ends here: nothing to write
     u32 total;
-    u32 before = kc_block_exclusive_scan<256>(c, &total, sw) + block_offsets[blockIdx.x];
-    if (c == 0 && (f[0] | f[1] | f[2] | f[3]) == 0) return;
-    static_assert(KC_RUN_WORDS == 4, "the early exit above spells the words out");
+    u32 before = kc_block_exclusive_scan<256>(c, &total, sw);
+    if (spec_total) {
+        u32 sum = 0;
+        for (u32 b = threadIdx.x; b < blockIdx.x; b += 256) sum += block_offsets[b];
+        u32 all;
+        kc_block_exclusive_scan<256>(sum, &all, sw);
+        before += all;
+    } else {
+        before += block_offsets[blockIdx.x];
+    }
 #pragma unroll
     for (int j = 0; j < KC_RUN_WORDS; ++j) {
         const u64 base = (word + j) * 32;

@@ -7,6 +7,11 @@
 #pragma once
 // (included from the middle of engine.cuh, after LevelCtx / SimulatePairFn)
 
+// Status words of one kc_small_engine_kernel run (SmallEngineArgs::out), and the zeroed words of its level masks that follow them:
+// [4] for the whole problem, then four words per end (the second copies of the ping-pong pairs need no zeroing).
+static const u32 KC_SMALL_STATUS_WORDS = 8 + 128 + 8;
+KC_HD u64 kc_small_mask_words(u64 n_s, u64 n_p) { return 4 + 4 * (n_s + n_p); }
+
 #ifdef __CUDACC__
 
 template <int L> struct SmallCfg {
@@ -37,6 +42,7 @@ template <int L> struct SmallEngineArgs {
     // [4 * n_s], [4 * n_p]: the same per END (bit d of the four words of initial list position i: end i has a partner at level d);
     // ping-pong copies travel with the live lists
     u32 *end_mask_s_a, *end_mask_p_a, *end_mask_s_b, *end_mask_p_b;
+    const u32 *n_dev;  // != nullptr: {n, N} on the device (speculative tail, kcgpu.cu); nv, n_s and n_p then hold their caps
 };
 
 // Levels of one CTA of kc_small_level_mask_kernel (host and device must agree): as many hash tables as fit next to the parked k-mers,
@@ -67,14 +73,19 @@ template <int L> KC_HD u32 kc_small_mask_levels_per_cta(u32 n_s, u32 n_p) {
 template <int L>
 __global__ void __launch_bounds__(256) kc_small_level_mask_kernel(NodeView<L> v, const u32 *__restrict__ ls, const u32 *__restrict__ lp, u32 n_s, u32 n_p,
                                                                   int d_start, u32 *mask_out /* [4], zeroed */, u32 *end_mask_s /* [4 n_s], zeroed */,
-                                                                  u32 *end_mask_p /* [4 n_p], zeroed */) {
+                                                                  u32 *end_mask_p /* [4 n_p], zeroed */, const u32 *n_dev /* see SmallEngineArgs */) {
     extern __shared__ __align__(16) unsigned char kc_smem_raw[];
     __shared__ u32 s_hits;
     const u32 tid = threadIdx.x, NT = blockDim.x;
+    const u32 G = kc_small_mask_levels_per_cta<L>(n_s, n_p);  // from the sizes the grid was launched for
+    if (n_dev) {  // the real counts are at most the caps: fewer k-mers to park, smaller tables
+        v.n = n_dev[0];
+        v.N = n_dev[1];
+        n_s = n_p = v.N;
+    }
     KWord<L> *pk = reinterpret_cast<KWord<L> *>(kc_smem_raw), *sk = pk + n_p;
     u32 *tab = reinterpret_cast<u32 *>(sk + n_s);
     const u32 H2 = kc_small_mask_table_slots<L>(n_p);
-    const u32 G = kc_small_mask_levels_per_cta<L>(n_s, n_p);
     const int d_hi = d_start - (int) (blockIdx.x * G);
     if (d_hi < 0) return;
     const u32 g = (u32) (d_hi + 1) < G ? (u32) (d_hi + 1) : G;  // levels d_hi, d_hi - 1, ..., d_hi - g + 1
@@ -168,6 +179,10 @@ template <int L> __global__ void __launch_bounds__(512) kc_small_engine_kernel(S
     const u32 tid = threadIdx.x;
     const u32 NT = blockDim.x;  // 256, or one warp for tiny problems (block barriers then cost next to nothing)
     NodeView<L> v = a.nv;
+    if (a.n_dev) {
+        v.n = a.n_dev[0];
+        v.N = a.n_dev[1];
+    }
     PathState s = a.st;
     u32 *head_w = a.head_w, *tail_w = a.tail_w, *slot_of = a.slot_of;
     u64 *stamp = a.stamp;
@@ -211,7 +226,7 @@ template <int L> __global__ void __launch_bounds__(512) kc_small_engine_kernel(S
         }
         __syncthreads();
     }
-    u32 n_s = a.n_s, n_p = a.n_p;
+    u32 n_s = a.n_dev ? v.N : a.n_s, n_p = a.n_dev ? v.N : a.n_p;
     u32 *ls = a.live_s_a, *lp = a.live_p_a, *ls2 = a.live_s_b, *lp2 = a.live_p_b;
     u32 *ms = a.end_mask_s_a, *mp = a.end_mask_p_a, *ms2 = a.end_mask_s_b, *mp2 = a.end_mask_p_b;
     __shared__ u32 s_nt;

@@ -225,6 +225,19 @@ u64 kc_extract_kmers(CudaExec &ex, const u8 *seq, u64 n_bytes, int k, bool compl
     return m;
 }
 
+// First and last k-mer of the node seq[off .. off + len), len >= k.
+template <int L> KC_D void kc_node_end_kmers(const u8 *seq, u64 off, u64 len, int k, KWord<L> &first, KWord<L> &last) {
+    KWord<L> f = KWord<L>::zero(), l = KWord<L>::zero();
+    for (int i = 0; i < k; ++i) {
+        f = f.shl(2);
+        f.w[0] |= kc_nucleotide_code(seq[off + i]) & 3;
+        l = l.shl(2);
+        l.w[0] |= kc_nucleotide_code(seq[off + len - k + i]) & 3;
+    }
+    first = f;
+    last = l;
+}
+
 // `-S`: first and last k-mer of every record (reference src/simplitigs.h:68-76) and input validation
 // (src/simplitigs.h:82 asserts ACGT only; records shorter than k have no k-mer and are rejected here).
 template <int L>
@@ -236,15 +249,7 @@ void kc_extract_node_ends(CudaExec &ex, const u8 *seq, u64 n_bytes, const u64 *r
             *error_flag = 1;
             return;
         }
-        KWord<L> f = KWord<L>::zero(), l = KWord<L>::zero();
-        for (int i = 0; i < k; ++i) {
-            f = f.shl(2);
-            f.w[0] |= kc_nucleotide_code(seq[off + i]) & 3;
-            l = l.shl(2);
-            l.w[0] |= kc_nucleotide_code(seq[off + len - k + i]) & 3;
-        }
-        first[r] = f;
-        last[r] = l;
+        kc_node_end_kmers<L>(seq, off, len, k, first[r], last[r]);
     });
     if (!validate_bytes) return;
     // every byte that is not a record separator must be a nucleotide
