@@ -39,11 +39,12 @@ extern "C" {
 #define KC_ERR_INTERNAL (-7)
 #define KC_ERR_NO_DEVICE (-8)
 
-/* Inputs of KC_POS32_BYTES sequence bytes or more (about 2^32) need 64-bit window positions.  kc_compute and
- * kc_compute_device take them on one GPU through the signature-bucket k-mer set construction, which applies with k >= 26,
- * min_frequency 1, no want_maxone and no assume_simplitigs; outside those conditions, or when a signature bucket overflows on
- * such an input (heavily repeated sequence), they fail with KC_ERR_TOO_LARGE.  Every other entry point (streaming, maskopt,
- * lower bound, count_kmers, kmer_digest, groups) refuses such inputs with KC_ERR_TOO_LARGE. */
+/* Inputs of KC_POS32_BYTES sequence bytes or more (about 2^32) need 64-bit window positions.  kc_compute, kc_compute_device,
+ * kc_lower_bound, kc_streaming and kc_kmer_digest take them on one GPU through the signature-bucket k-mer set construction, which
+ * applies with k >= 26, min_frequency 1, no want_maxone and no assume_simplitigs (kc_streaming: any min_frequency, every pass of
+ * -z is a first-occurrence construction; kc_kmer_digest ignores assume_simplitigs and want_maxone); outside those conditions, with
+ * option sig_set = 0, or when a signature bucket overflows on such an input (heavily repeated sequence), they fail with
+ * KC_ERR_TOO_LARGE.  kc_maskopt, kc_count_kmers and groups refuse such inputs with KC_ERR_TOO_LARGE. */
 #define KC_POS32_BYTES 0xFFFFFFF0ULL
 
 typedef struct kc_ctx kc_ctx;
@@ -114,7 +115,9 @@ int kc_lower_bound(kc_ctx *ctx, const kc_params *p, const kc_input *in, uint64_t
  *                src/streaming.h:12-107): out->ms = the masked superstring of the one-pass algorithm (the Z-th occurrence
  *                of every k-mer with at least Z occurrences is ON, the k-1 characters after an ON window are kept in
  *                lower case, everything else is dropped); out->n_kmers = k-mers turned ON.  assume_simplitigs and
- *                want_maxone must be 0.  An input without k-mers gives length 0 (the reference prints an empty line).
+ *                want_maxone must be 0.  An input without k-mers gives length 0 (the reference prints an empty line).  The
+ *                first-occurrence bits of every pass come from the signature construction where it applies (k >= 26), else from
+ *                the fixed-slot / exact ones; the output does not depend on which.
  * kc_maskopt     `maskopt -t max-one | min-one` (src/main.cpp:318-376, Optimize / OptimizeOnes src/masks.h:40-78,240-261):
  *                ms = the sequence of the single record (n letters, ACGTacgt only, else KC_ERR_BAD_SEQ); out->ms = the same
  *                letters with the mask that maximises (minimize = 0) or minimises (1) the number of ones while representing
@@ -159,7 +162,9 @@ int kc_partial_presort(kc_ctx *ctx, const uint64_t *kmers, uint64_t n, int k, ui
  * masked = 1: in->seq is ONE masked superstring of in->n_bytes letters; the set is the k-mers of the windows that start with an
  *             upper-case letter, i.e. the set the superstring REPRESENTS (what the reference's verify.py compares, and
  *             src/parser.h:41-42 case_sensitive); min_frequency must be 1.
- * `kmercamel compute` output verifies iff digest(masked = 1, output) == digest(masked = 0, input). */
+ * Without -z and with k >= 26 the set is built as first-occurrence bits by the signature construction and the flagged windows are
+ * hashed; otherwise (or after a bucket overflow below KC_POS32_BYTES) the sorted keys are.  The four words do not depend on which.
+ * `kmercamel compute` output verifies iff digest(masked = 1, output) == digest(masked = 0, input) (`kmercamel verify`). */
 int kc_kmer_digest(kc_ctx *ctx, const kc_params *p, const kc_input *in, int masked, uint64_t *digest);
 
 /* Overlap stage only (host buffers).  first/last: n * limbs limbs.  edge_from: N = n * (1 + complements) entries,
@@ -228,7 +233,8 @@ uint64_t kc_total_launches(const kc_ctx *ctx);
  * "small_engine" (default 1): run the tail of the overlap levels in the single-CTA kernel.
  * "sig_set" (default 1): try the signature-bucket k-mer set construction first (kmerset_sig.cuh: from-FASTA compute
  * with k >= 26, without -z and -M); "sig_load_pct" (0 = planned from the input size) and "sig_min_items": its plan
- * parameters, exposed so that tests reach the overflow fallback and small inputs.
+ * parameters, exposed so that tests reach the overflow fallback and small inputs.  kc_kmer_digest and kc_streaming try it first as
+ * well; an overflow there is counted in "sig_fallbacks" but not remembered by the context.
  * "fast_set" (default 1): then try the histogram-free fixed-slot construction (from-FASTA compute without -M);
  * "fast_leaf_target", "fast_sigmas", "fast_min_items": its plan parameters, exposed so that tests reach the
  * multi-level plan and the overflow fallback with small inputs; "fast_heuristics" (default 1): skip the attempt when

@@ -231,6 +231,11 @@ class ComputeResult:
     slice_len: int = 0     # of the superstring (length = the whole superstring)
 
 
+def _string_at(ptr, n: int) -> bytes:
+    """n bytes at host address ptr.  ctypes.string_at passes its length as a C int, which cuts results of 2^31 bytes and more."""
+    return bytes((C.c_char * n).from_address(ptr)) if n else b""
+
+
 class Context:
     """One context per process and GPU (kc_init / kc_destroy)."""
 
@@ -272,8 +277,8 @@ class Context:
         times = dict(extract=t.extract_ms, count=t.count_ms, path=t.path_ms, emit=t.emit_ms, total=t.total_ms)
         ms = mo = None
         if copy_host:
-            ms = C.string_at(out.ms, out.length)
-            mo = C.string_at(out.ms_maxone, out.length) if out.ms_maxone else None
+            ms = _string_at(out.ms, out.length)
+            mo = _string_at(out.ms_maxone, out.length) if out.ms_maxone else None
         return ComputeResult(ms, mo, out.length, out.n_kmers, out.n_occurrences, out.n_nodes, out.n_launches, out.n_simplitigs, times,
                              out.ms or 0, out.ms_maxone or 0)
 

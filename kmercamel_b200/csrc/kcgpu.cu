@@ -2,6 +2,7 @@
 // no CPU path and fails with KC_ERR_NO_DEVICE when no GPU is present.
 #include "../../include/kcgpu.h"
 
+#include "digest.cuh"
 #include "emit.cuh"
 #include "engine.cuh"
 #include "exec.cuh"
@@ -478,7 +479,11 @@ void run_pipeline(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params
         if (U == 0) KC_THROW(KC_ERR_EMPTY, "the input contains no k-mers");  // src/main.cpp:155-158
         res.n_simplitigs = runs.n_runs;
         // src/main.cpp:94,175-181: simplitigs barely longer than k-mers -> the greedy runs on the k-mers themselves (PartialPreSort order)
-        if (ctx->sparse_switch && runs.n_runs * 5 >= U) runs = kc_kmer_nodes_from_runs(ex, in.seq, runs, p.k);
+        if (ctx->sparse_switch && runs.n_runs * 5 >= U) {
+            // one node per k-mer; kc_kmer_nodes_from_runs numbers them with 32-bit offsets (inputs of 2^32 bytes or more can have that many)
+            if (U * (complements ? 2 : 1) >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "too many nodes for one GPU");
+            runs = kc_kmer_nodes_from_runs(ex, in.seq, runs, p.k);
+        }
         n_nodes = runs.n_runs;
         node_off = runs.rec_off;
         node_len = runs.rec_len;
@@ -597,20 +602,63 @@ void count_only(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &
     KC_CUDA(cudaStreamSynchronize(ex.stream));
 }
 
-// kc_kmer_digest: (n, sum h, xor h, sum h * c) over the kept (k-mer, c = min(occurrences, 256), or 1 without -z) pairs, h = the splitmix64 fold of
-// the limbs.  The same four numbers come out of oracle/ref_harness `full` for the reference's own hash table.
-KC_HD u64 kc_mix64(u64 x) {
-    x ^= x >> 30;
-    x *= 0xbf58476d1ce4e5b9ULL;
-    x ^= x >> 27;
-    x *= 0x94d049bb133111ebULL;
-    x ^= x >> 31;
-    return x;
+// The first-occurrence flags of a from-FASTA input built by the signature construction (kmerset_sig.cuh) alone, for the entry
+// points that need the k-mer set but not its runs: kc_kmer_digest and kc_streaming.  win_mask: optional window filter over END
+// positions, sized for the signature scan's tiles of 256 * 32 positions.  flags (fwords words) and cells {kept, -, M, status, ...}
+// arrive zeroed; after() queues the work that reads the flags before the one read-back of cells[0, n_cells) into hc.
+// Returns true when the flags stand.  Returns false when the construction does not apply, or when a bucket overflowed: then the overflow
+// is counted in sig_fallbacks, flags and cells are zeroed again, and the caller takes the other constructions.  Unlike run_stage1_runs
+// it leaves sig_overflow_bytes alone, so a digest or a streaming call does not change which construction a later compute tries.
+// Inputs of KC_POS32_BYTES or more have no other construction (check_large_input): there the call fails instead.
+template <int L, class After>
+bool sig_flags(kc_ctx *ctx, CudaExec &ex, const u8 *seq, u64 nb, const kc_params &p, u32 *flags, size_t fwords, const u32 *win_mask, u64 *cells,
+               u64 *hc, int n_cells, After after) {
+    const bool large = nb >= KC_POS32_BYTES;
+    if (!kc_kmerset_build_sig<L>(ex, seq, nb, p.k, p.complements != 0, flags, cells, ctx->sig, nullptr, win_mask)) {
+        if (large) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; its bucket plan does not fit this input");
+        return false;
+    }
+    after();
+    ex.read_n(cells, hc, (size_t) n_cells);
+    if (hc[3] == 0) {
+        ++ctx->sig_runs;
+        return true;
+    }
+    ++ctx->sig_fallbacks;
+    if (large) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; it overflowed on this input (too repetitive)");
+    ex.fill_bytes(flags, 0, fwords * 4);
+    ex.fill_bytes(cells, 0, (size_t) n_cells * 8);
+    return false;
 }
+
+// kc_kmer_digest: (n, sum h, xor h, sum h * c) over the kept (k-mer, c = min(occurrences, 256), or 1 without -z) pairs, h = the splitmix64 fold of
+// the limbs (kc_kmer_hash).  The same four numbers come out of oracle/ref_harness `full` for the reference's own hash table.
+// Without -z the set is first tried as first-occurrence flags of the signature construction, hashed window by window (digest.cuh); the
+// sorted keys of kc_kmerset_build are the other route.  The digest is a function of the set: both give the same four words.
 
 template <int L>
 void digest_only(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &p, const u32 *win_mask, uint64_t *digest) {
     KC_CUDA(cudaEventRecord(ctx->ev[0], ex.stream));
+    if (p.min_frequency == 1) {  // c = 1: digest[3] = digest[1]
+        const size_t top = ex.arena->top, mark = ex.arena->mark();
+        const size_t fwords = kc_runs_flag_words(in.n_bytes);
+        u32 *flags = ex.arena->alloc_top<u32>(fwords);
+        ex.fill_bytes(flags, 0, fwords * 4);
+        u64 *cells = ex.arena->alloc_top<u64>(8);  // {kept, -, M, status, n, sum h, xor h, -}
+        ex.fill_bytes(cells, 0, 64);
+        kc_ull *acc = reinterpret_cast<kc_ull *>(cells + 4);
+        u64 hc[7];
+        if (sig_flags<L>(ctx, ex, in.seq, in.n_bytes, p, flags, fwords, win_mask, cells, hc, 7,
+                         [&] { kc_flag_digest<L>(ex, in.seq, in.n_bytes, flags, fwords, p.k, p.complements != 0, acc); })) {
+            digest[0] = hc[4];
+            digest[1] = hc[5];
+            digest[2] = hc[6];
+            digest[3] = hc[5];
+            return;
+        }
+        ex.arena->release(mark);
+        ex.arena->top = top;
+    }
     KmerSet<L> set = kc_kmerset_build<L>(ex, in.seq, in.n_bytes, p.k, p.complements != 0, p.min_frequency, nullptr, true, nullptr, win_mask);
     const u64 U = set.n_kept;
     kc_ull *acc = reinterpret_cast<kc_ull *>(ex.alloc<u64>(4));
@@ -621,9 +669,7 @@ void digest_only(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params 
     ex.for_each(kc_div_up(U, 32) * 32, [=] __device__(u64 i) {
         u64 h = 0, wv = 0;
         if (i < U) {
-            h = kc_mix64(keys[i].w[0] + 0x9e3779b97f4a7c15ULL);
-#pragma unroll
-            for (int l = 1; l < L; ++l) h = kc_mix64(h ^ (keys[i].w[l] + 0x9e3779b97f4a7c15ULL * (u64) (l + 1)));
+            h = kc_kmer_hash<L>(keys[i]);
             wv = counted ? h * ((u64) cnt[i] + 1) : h;
         }
         u64 s = h, x = h;
@@ -645,6 +691,14 @@ void digest_only(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params 
     digest[1] = h4[1];
     digest[2] = h4[2];
     digest[3] = h4[3];
+}
+
+// kc_streaming: every pass of the first-occurrence construction tries the signature buckets first (sig_flags)
+template <int L> StreamingResult streaming_only(kc_ctx *ctx, CudaExec &ex, const u8 *seq, u64 nb, const kc_params &p) {
+    auto sig = [&](u32 *flags, size_t fwords, const u32 *win_mask, u64 *cells4, u64 *hc) {
+        return sig_flags<L>(ctx, ex, seq, nb, p, flags, fwords, win_mask, cells4, hc, 4, [] {});
+    };
+    return kc_streaming_run<L>(ex, seq, nb, p.k, p.complements != 0, p.min_frequency, ctx->fast, &ctx->fast_runs, &ctx->fast_fallbacks, sig);
 }
 
 template <int L>
@@ -997,7 +1051,7 @@ int kc_lower_bound(kc_ctx *ctx, const kc_params *p, const kc_input *in, uint64_t
     KC_API_BEGIN
     check_params(p);
     if (p->want_maxone) KC_THROW(KC_ERR_ARG, "lowerbound has no mask output");
-    if (in->n_bytes >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "more than 2^32 sequence bytes on one GPU");
+    check_large_input(ctx, p, in->n_bytes);
     KC_CUDA(cudaSetDevice(ctx->device));
     const int limbs = kc_limbs_for_k(p->k);
     const bool simplitigs = p->assume_simplitigs != 0;
@@ -1006,8 +1060,9 @@ int kc_lower_bound(kc_ctx *ctx, const kc_params *p, const kc_input *in, uint64_t
     ex.pinned = ctx->pin_small;
     ex.pinned_cap = ctx->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
     DevResult res;
-    run_with_arena(ctx, estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, false, &ctx->fast),
-                   estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, true, &ctx->fast), [&] {
+    const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->sig);
+    run_with_arena(ctx, estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, false, &ctx->fast, &sig),
+                   estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, true, &ctx->fast, &sig), [&] {
         u8 *d_seq = ex.alloc<u8>(in->n_bytes + 64);
         KC_CUDA(cudaMemcpyAsync(d_seq, in->seq, in->n_bytes, cudaMemcpyHostToDevice, ctx->stream));
         u64 *d_off = nullptr, *d_len = nullptr;
@@ -1057,10 +1112,15 @@ int kc_streaming(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_output 
     KC_API_BEGIN
     check_params(p);
     if (p->assume_simplitigs || p->want_maxone) KC_THROW(KC_ERR_ARG, "-S and -M belong to the greedy algorithm");  // src/main.cpp:296-301
-    if (in->n_bytes >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "more than 2^32 sequence bytes on one GPU");
+    {   // -z Z is Z first-occurrence passes, each of which the signature construction takes (kc_streaming_run)
+        kc_params q = *p;
+        q.min_frequency = 1;
+        check_large_input(ctx, &q, in->n_bytes);
+    }
     KC_CUDA(cudaSetDevice(ctx->device));
     const int limbs = kc_limbs_for_k(p->k);
-    ensure_arena(ctx, estimate_arena(in->n_bytes, 0, limbs, false, true, false, &ctx->fast));
+    const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->sig);
+    ensure_arena(ctx, estimate_arena(in->n_bytes, 0, limbs, false, true, false, &ctx->fast, &sig));
     ctx->arena.reset();
     CudaExec ex{ctx->stream, &ctx->arena};
     ex.prof = &ctx->prof;
@@ -1074,10 +1134,9 @@ int kc_streaming(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_output 
     KC_CUDA(cudaMemcpyAsync(d_seq, in->seq, in->n_bytes, cudaMemcpyHostToDevice, ctx->stream));
     KC_CUDA(cudaEventRecord(ctx->ev[1], ctx->stream));
     StreamingResult r;
-    const bool compl_ = p->complements != 0;
-    if (limbs == 1) r = kc_streaming_run<1>(ex, d_seq, in->n_bytes, p->k, compl_, p->min_frequency, ctx->fast, &ctx->fast_runs, &ctx->fast_fallbacks);
-    else if (limbs == 2) r = kc_streaming_run<2>(ex, d_seq, in->n_bytes, p->k, compl_, p->min_frequency, ctx->fast, &ctx->fast_runs, &ctx->fast_fallbacks);
-    else r = kc_streaming_run<4>(ex, d_seq, in->n_bytes, p->k, compl_, p->min_frequency, ctx->fast, &ctx->fast_runs, &ctx->fast_fallbacks);
+    if (limbs == 1) r = streaming_only<1>(ctx, ex, d_seq, in->n_bytes, *p);
+    else if (limbs == 2) r = streaming_only<2>(ctx, ex, d_seq, in->n_bytes, *p);
+    else r = streaming_only<4>(ctx, ex, d_seq, in->n_bytes, *p);
     for (int i = 2; i <= 4; ++i) KC_CUDA(cudaEventRecord(ctx->ev[i], ctx->stream));
     out->ms = copy_result_to_pinned(ctx, r.ms, r.length);
     out->length = r.length;
@@ -1201,12 +1260,19 @@ int kc_kmer_digest(kc_ctx *ctx, const kc_params *p, const kc_input *in, int mask
     KC_API_BEGIN
     check_params(p);
     if (masked && p->min_frequency != 1) KC_THROW(KC_ERR_ARG, "a masked superstring has no counts");
-    if (in->n_bytes + 1 >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "more than 2^32 sequence bytes on one GPU");
-    KC_CUDA(cudaSetDevice(ctx->device));
-    const int limbs = kc_limbs_for_k(p->k);
     // masked: the bytes are ONE masked superstring (no framing); a '\n' is appended so that it is a framed record
     const u64 nb = masked ? in->n_bytes + 1 : in->n_bytes;
+    {   // the digest ignores -S and -M: only -z and k decide whether an input of 2^32 bytes or more can be taken
+        kc_params q = *p;
+        q.assume_simplitigs = 0;
+        q.want_maxone = 0;
+        check_large_input(ctx, &q, nb);
+    }
+    KC_CUDA(cudaSetDevice(ctx->device));
+    const int limbs = kc_limbs_for_k(p->k);
+    // the sorted-keys route, or at 2^32 bytes and more the signature construction alone: sequence, flags, window mask, its buffers
     size_t need = (size_t) ((double) nb * (1.0 + 2.0 * 8 * limbs + 4.0 + 0.2) * 1.15) + (256u << 20);
+    if (nb >= KC_POS32_BYTES) need = (size_t) (((double) nb * 1.25 + (double) kc_sig_arena_bytes(kc_sig_plan(nb, p->k, ctx->sig), nb)) * 1.05) + (256u << 20);
     ensure_arena(ctx, need);
     ctx->arena.reset();
     CudaExec ex{ctx->stream, &ctx->arena};
@@ -1218,8 +1284,8 @@ int kc_kmer_digest(kc_ctx *ctx, const kc_params *p, const kc_input *in, int mask
     u32 *win_mask = nullptr;
     if (masked) {  // the windows whose first letter is upper case are the represented k-mers (reference verify.py / src/parser.h:41-42)
         ex.fill_bytes(d_seq + in->n_bytes, '\n', 64);
-        const u64 tile = kc_shard_granule(p->k);
-        const u64 mwords = kc_div_up(nb, tile) * (tile / 32) + 1;
+        // whole tiles of the signature scan (256 strips); the extraction tiles of the sorted-keys route divide them
+        const u64 mwords = kc_div_up(nb, (u64) 256 * KC_EX_STRIP) * 256 + 1;
         win_mask = ex.arena->alloc_top<u32>(mwords);
         const u64 len = in->n_bytes;
         const int k = p->k;

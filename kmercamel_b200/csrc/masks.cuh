@@ -4,7 +4,7 @@
 //              a window whose (canonical) k-mer has not been seen before prints its first character in upper case, and a
 //              character at most k-1 positions after the latest such window prints in lower case; every other character
 //              is dropped.  "Not seen before" is exactly the first-occurrence bit array the from-FASTA compute path builds
-//              (kmerset.cuh / kmerset_fast.cuh), so streaming = that construction + one stream compaction.
+//              (kmerset_sig.cuh / kmerset_fast.cuh / kmerset.cuh), so streaming = that construction + one stream compaction.
 //
 //   maskopt    `maskopt -t max-one | min-one` (reference src/masks.h:40-78 OptimizeOnes, 240-261 Optimize): the set S is the
 //              canonical k-mers of the windows that START with an upper-case letter (src/parser.h:41-42 case_sensitive);
@@ -16,6 +16,8 @@
 #include "emit.cuh"
 #include "kmerset_fast.cuh"
 #include "runs.cuh"
+
+#include <functional>
 
 #ifdef __CUDACC__
 
@@ -66,9 +68,35 @@ __global__ void __launch_bounds__(256) kc_streaming_count_kernel(const u32 *__re
     if (threadIdx.x == 0) block_counts[blockIdx.x] = total;
 }
 
+// Exclusive scan of the per-block counts into 64-bit offsets, out[n] = the total: the kept characters of an input of 2^32 bytes or more
+// can number 2^32 and more.  One CTA walks the counts with a running carry, as kc_scan_walk_kernel does (a tile of 1024 counts of at
+// most 8192 each sums within 32 bits).
+__global__ void __launch_bounds__(256) kc_streaming_offsets_kernel(const u32 *__restrict__ counts, u64 n, u64 *__restrict__ out) {
+    __shared__ u32 sw[8];
+    u64 carry = 0;
+    for (u64 t0 = 0; t0 < n; t0 += 1024) {
+        const u64 base = t0 + (u64) threadIdx.x * 4;
+        u32 v[4], c = 0;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            v[j] = base + j < n ? counts[base + j] : 0u;
+            c += v[j];
+        }
+        u32 total;
+        u64 q = carry + kc_block_exclusive_scan<256>(c, &total, sw);  // ends with a barrier: sw is free for the next tile
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            if (base + j < n) out[base + j] = q;
+            q += v[j];
+        }
+        carry += total;
+    }
+    if (threadIdx.x == 0) out[n] = carry;
+}
+
 // The kept characters of the block go through shared memory so that the stores to `out` are contiguous.
 __global__ void __launch_bounds__(256) kc_streaming_emit_kernel(const u8 *__restrict__ seq, const u32 *__restrict__ flags, u64 n_flag_words,
-                                                                u64 n_words, int k, const u32 *__restrict__ block_offsets, u8 *__restrict__ out) {
+                                                                u64 n_words, int k, const u64 *__restrict__ block_offsets, u8 *__restrict__ out) {
     __shared__ u32 sw[8];
     __shared__ u8 stage[256 * 32];
     const u64 w = (u64) blockIdx.x * 256 + threadIdx.x;
@@ -99,10 +127,13 @@ struct StreamingResult {
 };
 
 // seq: the framed records, resident in a buffer padded with '\n' up to a multiple of 32 bytes (+ 32).
+// sig(flags, fwords, win_mask, cells4, hc): the signature-bucket construction of the flags (kcgpu.cu sig_flags), tried first in every
+// pass; true = the flags stand and hc holds cells4, false = it did not apply or overflowed (flags and cells4 are zeroed again).  An input
+// of 2^32 bytes or more has no other construction: there sig fails the call instead of returning false.
+typedef std::function<bool(u32 *, size_t, const u32 *, u64 *, u64 *)> KcSigFlags;
 template <int L>
 StreamingResult kc_streaming_run(CudaExec &ex, const u8 *seq, u64 n_bytes, int k, bool complements, int min_freq, const KsfTuning &fast,
-                                 u64 *fast_runs, u64 *fast_fallbacks) {
-    typedef KsCfg<L> Cfg;
+                                 u64 *fast_runs, u64 *fast_fallbacks, const KcSigFlags &sig) {
     StreamingResult res;
     const size_t fwords = kc_runs_flag_words(n_bytes);
     u32 *flags = ex.arena->alloc_top<u32>(fwords);
@@ -110,8 +141,13 @@ StreamingResult kc_streaming_run(CudaExec &ex, const u8 *seq, u64 n_bytes, int k
     u64 *cells4 = ex.arena->alloc_top<u64>(4);  // {kept, -, M, overflow status}
     ex.fill_bytes(cells4, 0, 32);
     u64 hc[4] = {0, 0, 0, 0};
-    bool done = false;
-    if (min_freq == 1 && kc_kmerset_build_fast<L>(ex, seq, n_bytes, k, complements, 1, flags, cells4, fast)) {  // -z > 1: a read set, see run_stage1_runs
+    bool done = sig(flags, fwords, nullptr, cells4, hc);
+    const bool sig_ok = done;  // what did not apply or overflowed (a read set) is not tried again in the passes of -z
+    if (done) {
+        res.n_kept = hc[2] ? hc[0] : 0;
+        res.n_occ = hc[2];
+    }
+    if (!done && min_freq == 1 && kc_kmerset_build_fast<L>(ex, seq, n_bytes, k, complements, 1, flags, cells4, fast)) {  // -z > 1: a read set, see run_stage1_runs
         ex.read_n(cells4, hc, 4);
         if (hc[3] == 0) {
             done = true;
@@ -133,8 +169,8 @@ StreamingResult kc_streaming_run(CudaExec &ex, const u8 *seq, u64 n_bytes, int k
     // occurrence in file order.  Pass t = 2..Z repeats the first-occurrence construction over the windows that were not
     // flagged by the passes before it (window filter of the level-0 kernels): what it flags is every k-mer's t-th occurrence.
     if (min_freq > 1 && res.n_kept) {
-        const u64 tiles = kc_div_up(n_bytes, (u64) Cfg::EX_TILE);
-        const u64 mwords = tiles * (Cfg::EX_TILE / 32) + 1;
+        // whole tiles of the signature scan (256 strips); the extraction tiles of the other constructions divide them
+        const u64 mwords = kc_div_up(n_bytes, (u64) 256 * KC_EX_STRIP) * 256 + 1;
         u32 *avail = ex.arena->alloc_top<u32>(mwords);
         ex.fill_bytes(avail, 0xFF, mwords * 4);
         for (int t = 2; t <= min_freq && res.n_kept; ++t) {
@@ -145,6 +181,10 @@ StreamingResult kc_streaming_run(CudaExec &ex, const u8 *seq, u64 n_bytes, int k
             }, KP_MISC, mwords * 12);
             ex.fill_bytes(flags, 0, fwords * 4);
             ex.fill_bytes(cells4, 0, 32);
+            if (sig_ok && sig(flags, fwords, avail, cells4, hc)) {
+                res.n_kept = hc[2] ? hc[0] : 0;
+                continue;
+            }
             KmerSet<L> set = kc_kmerset_build_impl<L, true, false>(ex, seq, n_bytes, k, complements, 1, flags, cells4, nullptr, avail);
             res.n_kept = set.n_occ ? ex.read(cells4) : 0;
         }
@@ -159,12 +199,19 @@ StreamingResult kc_streaming_run(CudaExec &ex, const u8 *seq, u64 n_bytes, int k
         ++ex.launches;
         KC_CUDA(cudaGetLastError());
     }
-    // per-block counts are at most 8192, their running sum is bounded by n_bytes < 2^32
-    const u64 total = ex.exclusive_scan(counts, counts, blocks);
+    // per-block counts are at most 8192, their running sum is bounded by n_bytes: 64-bit offsets
+    u64 *offsets = ex.alloc<u64>((u64) blocks + 1);
+    {
+        CudaExec::Scope sc(ex, KP_SCAN, (u64) blocks * 12);
+        kc_streaming_offsets_kernel<<<1, 256, 0, ex.stream>>>(counts, blocks, offsets);
+        ++ex.launches;
+        KC_CUDA(cudaGetLastError());
+    }
+    const u64 total = ex.read(offsets + blocks);
     u8 *out = ex.alloc<u8>(total + 1);
     {
         CudaExec::Scope sc(ex, KP_EMIT, n_bytes + n_bytes / 8 + total);
-        kc_streaming_emit_kernel<<<blocks, 256, 0, ex.stream>>>(seq, flags, fwords, n_words, k, counts, out);
+        kc_streaming_emit_kernel<<<blocks, 256, 0, ex.stream>>>(seq, flags, fwords, n_words, k, offsets, out);
         ++ex.launches;
         KC_CUDA(cudaGetLastError());
     }
