@@ -247,7 +247,10 @@ uint64_t kc_total_launches(const kc_ctx *ctx);
 int kc_set_option(kc_ctx *ctx, const char *name, int value);
 /* Counters since kc_init: "sig_runs", "sig_fallbacks", "fast_runs", "fast_fallbacks", "total_launches", "tail_spec_runs",
  * "tail_spec_fallbacks", "read_backs" (synchronising device -> host reads, i.e. host round trips); current value of the
- * option "fast_max_ctas"; device arena: "arena_bytes" (reserved now), "arena_high" (most bytes in use at once since kc_init). */
+ * option "fast_max_ctas"; device arena: "arena_bytes" (reserved now), "arena_high" (most bytes in use at once since kc_init).
+ * Totals of the greedy overlap stage of the LAST call that ran it (kc_compute, kc_lower_bound, kc_overlap_path, a group
+ * compute), over the level loop and the single-CTA engine: "path_levels" (overlap levels replayed), "path_ban_rounds" (replays
+ * of a level after a cycle was found), "path_bans" (refused edges; with complements each one counts for both strands). */
 int kc_get_stat(const kc_ctx *ctx, const char *name, uint64_t *value);
 
 int kc_limbs_for_k(int k);

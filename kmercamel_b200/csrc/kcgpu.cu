@@ -66,6 +66,7 @@ struct kc_ctx {
     bool tail_spec = true;   // option "tail_spec": queue the tail of the from-FASTA path without reading the run count (run_tail_spec)
     u64 tail_spec_runs = 0, tail_spec_fallbacks = 0;
     u64 spec_fail_bytes = 0;  // input size of the last call whose speculative tail did not hold (0 = none)
+    EngineStats path_stats;   // the overlap stage of the last call that ran it (stats "path_levels", "path_ban_rounds", "path_bans")
     KcGroup grp;             // multi-GPU: this context as one rank of a group (group.cuh)
     bool arena_limited = false;
     std::string last_error;
@@ -283,6 +284,7 @@ u32 run_tail_spec(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params
         return hs[0];
     }
     eng.apply_small_status(reinterpret_cast<const u32 *>(h + KC_SPEC_SMALL));  // a failed small-engine run is the cause, report that one
+    ctx->path_stats = eng.stats;
     kc_emit_check(h + KC_SPEC_EMIT, hs[2], total_ub);
     res.ms = er.ms;
     res.maxone = nullptr;
@@ -540,6 +542,7 @@ void run_pipeline(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params
         u64 h[2];
         ex.read_n(reinterpret_cast<const u64 *>(acc), h, 2);
         eng.check_small();
+        ctx->path_stats = eng.stats;
         const u64 strands = complements ? 2 : 1;
         res.lower_bound = (h[0] * strands - h[1]) / strands;
         KC_CUDA(cudaEventRecord(ctx->ev[4], ex.stream));
@@ -558,6 +561,7 @@ void run_pipeline(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params
     }
     KC_CUDA(cudaEventRecord(ctx->ev[4], ex.stream));
     eng.check_small();  // deferred status of the single-CTA engine kernel: everything above is queued already
+    ctx->path_stats = eng.stats;
     res.ms = er.ms;
     res.maxone = er.maxone;
     res.length = er.length;
@@ -720,6 +724,7 @@ void overlap_only(kc_ctx *ctx, CudaExec &ex, const uint64_t *first, const uint64
     eng.init_state();
     eng.run();
     eng.check_small();
+    ctx->path_stats = eng.stats;
     std::vector<u32> ef(nv.N);
     KC_CUDA(cudaMemcpyAsync(ef.data(), eng.st.edge_from, (size_t) nv.N * 4, cudaMemcpyDeviceToHost, ex.stream));
     KC_CUDA(cudaMemcpyAsync(overlaps, eng.st.ovl, nv.N, cudaMemcpyDeviceToHost, ex.stream));
@@ -1696,6 +1701,9 @@ int kc_get_stat(const kc_ctx *ctx, const char *name, uint64_t *value) {
     else if (std::strcmp(name, "arena_bytes") == 0) *value = ctx->arena.cap;
     else if (std::strcmp(name, "arena_high") == 0) *value = ctx->arena.high;
     else if (std::strcmp(name, "fast_max_ctas") == 0) *value = (uint64_t) ctx->fast.max_ctas;
+    else if (std::strcmp(name, "path_levels") == 0) *value = ctx->path_stats.levels_run;
+    else if (std::strcmp(name, "path_ban_rounds") == 0) *value = ctx->path_stats.ban_rounds;
+    else if (std::strcmp(name, "path_bans") == 0) *value = ctx->path_stats.bans;
     else return KC_ERR_ARG;
     return KC_OK;
 }

@@ -174,12 +174,14 @@ int count_kmers(const uint8_t *seq, const uint64_t *rec_off, const uint64_t *rec
 
 // ---------------------------------------------------------------------------------------------------
 // Stage 3: src/global.h:43-133 line by line, with std::unordered_map standing in for the khash map.
+// `parts` is the number of prefix batches: 16 is the reference (MEMORY_REDUCTION_FACTOR, global.h:48,66); 1 puts every prefix into
+// one batch, the tie order of the product's from-FASTA engine (engine.cuh, strict = false).
 template <int L>
 int overlap_path(const uint64_t *first_in, const uint64_t *last_in, uint64_t n, int k, bool complements,
-                 bool lower_bound, int64_t *edge_from, uint8_t *overlaps) {
+                 bool lower_bound, int64_t *edge_from, uint8_t *overlaps, int parts = 16) {
     const size_t NONE = (size_t) -1;
     const size_t count = n * (1 + (complements ? 1 : 0));                         // global.h:47
-    const size_t batch = count / 16 + 1;                                          // global.h:48 (MEMORY_REDUCTION_FACTOR)
+    const size_t batch = count / parts + 1;                                       // global.h:48
     std::vector<Word<L>> node_first(count), node_last(count);                     // accessPrefix/accessSuffix, global.h:16-21
     for (size_t i = 0; i < n; ++i) {
         node_first[i] = load<L>(first_in + i * L);
@@ -201,7 +203,7 @@ int overlap_path(const uint64_t *first_in, const uint64_t *last_in, uint64_t n, 
     };
     std::unordered_map<Word<L>, size_t, WordHash<L>> prefixes;
     for (int d = k - 1; d >= 0; --d) {                                            // global.h:63
-        for (int part = 0; part < 16; ++part) {                                   // global.h:66
+        for (int part = 0; part < parts; ++part) {                                // global.h:66
             prefixes.clear();
             std::fill(next.begin(), next.end(), NONE);
             size_t to = std::min(count, (size_t) (part + 1) * batch);
@@ -259,6 +261,65 @@ int overlap_path(const uint64_t *first_in, const uint64_t *last_in, uint64_t n, 
     for (size_t i = 0; i < count; ++i) {
         edge_from[i] = ef[i] == NONE ? -1 : (int64_t) ef[i];
         overlaps[i] = ov[i];
+    }
+    return 0;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// The nodes of the product's from-FASTA regime (kmercamel_b200/csrc/runs.cuh): the window END position of the first occurrence, in
+// input order, of every kept canonical k-mer (occurring at least min_frequency times, counted as in count_kmers) is marked; a maximal
+// run of consecutive marked ends e_s..e_t is the node seq[e_s - k + 1 .. e_t].  Positions are seq offsets, so records must be
+// separated by a non-ACGT byte for runs not to cross them (the framing of records_to_arrays).
+template <int L>
+int first_occurrence_runs(const uint8_t *seq, const uint64_t *rec_off, const uint64_t *rec_len, uint64_t n_rec, int k,
+                          bool complements, int min_frequency, uint64_t **off_out, uint64_t **len_out, uint64_t *n_out,
+                          uint64_t *n_kept_out) {
+    std::vector<std::pair<Word<L>, uint64_t>> occ;  // (canonical k-mer, window end)
+    const Word<L> mask = Word<L>::low_mask(2 * k);
+    const int shift = 2 * (k - 1);
+    for (uint64_t r = 0; r < n_rec; ++r) {
+        const uint8_t *s = seq + rec_off[r];
+        int64_t current_length = 0;
+        Word<L> cur, rc;
+        for (uint64_t i = 0; i < rec_len[r]; ++i) {
+            int data = nucleotide_to_int(s[i]);
+            if (data >= 4) {
+                cur = Word<L>();
+                rc = Word<L>();
+                current_length = 0;
+                continue;
+            }
+            cur = (cur.shl(2) | Word<L>((uint64_t) data)) & mask;
+            rc = rc.shr(2) | Word<L>((uint64_t) (3 ^ data)).shl(shift);
+            if (++current_length >= k) occ.emplace_back((!complements || cur < rc) ? cur : rc, rec_off[r] + i);
+        }
+    }
+    std::sort(occ.begin(), occ.end(), [](const std::pair<Word<L>, uint64_t> &a, const std::pair<Word<L>, uint64_t> &b) {
+        return a.first < b.first || (a.first == b.first && a.second < b.second);
+    });
+    std::vector<uint64_t> ends;
+    for (size_t i = 0; i < occ.size();) {
+        size_t j = i;
+        while (j < occ.size() && occ[j].first == occ[i].first) ++j;
+        if (j - i >= (size_t) min_frequency) ends.push_back(occ[i].second);
+        i = j;
+    }
+    *n_kept_out = ends.size();
+    std::sort(ends.begin(), ends.end());
+    std::vector<uint64_t> offs, lens;
+    for (size_t i = 0; i < ends.size();) {
+        size_t j = i + 1;
+        while (j < ends.size() && ends[j] == ends[j - 1] + 1) ++j;
+        offs.push_back(ends[i] - (uint64_t) (k - 1));
+        lens.push_back(ends[j - 1] - ends[i] + (uint64_t) k);
+        i = j;
+    }
+    *n_out = offs.size();
+    *off_out = (uint64_t *) std::malloc(std::max<size_t>(1, offs.size() * 8));
+    *len_out = (uint64_t *) std::malloc(std::max<size_t>(1, lens.size() * 8));
+    if (!offs.empty()) {
+        std::memcpy(*off_out, offs.data(), offs.size() * 8);
+        std::memcpy(*len_out, lens.data(), lens.size() * 8);
     }
     return 0;
 }
@@ -580,7 +641,21 @@ void orc_bit_suffix(const uint64_t *in, int k, int d, uint64_t *out) {
 
 int orc_overlap_path(const uint64_t *first, const uint64_t *last, uint64_t n, int k, int complements,
                      int lower_bound, int64_t *edge_from, uint8_t *overlaps) {
-    DISPATCH(k, overlap_path, first, last, n, k, complements != 0, lower_bound != 0, edge_from, overlaps);
+    DISPATCH(k, overlap_path, first, last, n, k, complements != 0, lower_bound != 0, edge_from, overlaps, 16);
+}
+
+int orc_overlap_path_parts(const uint64_t *first, const uint64_t *last, uint64_t n, int k, int complements,
+                           int lower_bound, int parts, int64_t *edge_from, uint8_t *overlaps) {
+    if (parts < 1 || parts > 16) return -1;
+    DISPATCH(k, overlap_path, first, last, n, k, complements != 0, lower_bound != 0, edge_from, overlaps, parts);
+}
+
+int orc_first_occurrence_runs(const uint8_t *seq, const uint64_t *rec_off, const uint64_t *rec_len, uint64_t n_rec, int k,
+                              int complements, int min_frequency, uint64_t **off_out, uint64_t **len_out, uint64_t *n_out,
+                              uint64_t *n_kept_out) {
+    if (min_frequency < 1) return -1;
+    DISPATCH(k, first_occurrence_runs, seq, rec_off, rec_len, n_rec, k, complements != 0, min_frequency, off_out, len_out, n_out,
+             n_kept_out);
 }
 
 int orc_superstring(const uint8_t *seq, const uint64_t *rec_off, const uint64_t *rec_len, uint64_t n, int k,

@@ -39,6 +39,19 @@ void orc_bit_suffix(const uint64_t *in, int k, int d, uint64_t *out);
 int orc_overlap_path(const uint64_t *first, const uint64_t *last, uint64_t n, int k, int complements,
                      int lower_bound, int64_t *edge_from, uint8_t *overlaps);
 
+/* The same with `parts` prefix batches instead of the reference's 16 (1..16).  parts = 1 is the tie order of the product's
+ * from-FASTA engine (kmercamel_b200/csrc/engine.cuh with strict = false), which puts every prefix into one batch. */
+int orc_overlap_path_parts(const uint64_t *first, const uint64_t *last, uint64_t n, int k, int complements,
+                           int lower_bound, int parts, int64_t *edge_from, uint8_t *overlaps);
+
+/* The nodes of the product's from-FASTA regime (kmercamel_b200/csrc/runs.cuh), not a reference function: the window end of the
+ * first occurrence, in input order, of every canonical k-mer that occurs at least min_frequency times (counted as in
+ * orc_count_kmers) is marked, and the maximal runs of consecutive marked ends are returned as (start byte, length) pairs in seq
+ * coordinates, in input order.  n_kept_out = number of kept distinct k-mers.  Outputs are malloc'ed; release with orc_free. */
+int orc_first_occurrence_runs(const uint8_t *seq, const uint64_t *rec_off, const uint64_t *rec_len, uint64_t n_rec, int k,
+                              int complements, int min_frequency, uint64_t **off_out, uint64_t **len_out, uint64_t *n_out,
+                              uint64_t *n_kept_out);
+
 /* Superstring emission, reference src/global.h:149-210 (SuperstringFromPath).  Nodes are the framed records
  * (ACGT only, each at least k long).  set_keys (sorted unique canonical-or-not keys, n_set of them) is only
  * read when maxone_out != NULL and plays the role of kMersDict (src/global.h:165-167,185-195).

@@ -35,6 +35,9 @@ def lib():
         L.orc_limbs_for_k.restype = C.c_int
         L.orc_count_kmers.argtypes = [u8p, u64p, u64p, C.c_uint64, C.c_int, C.c_int, C.POINTER(u64p), C.POINTER(u8p), u64p]
         L.orc_overlap_path.argtypes = [u64p, u64p, C.c_uint64, C.c_int, C.c_int, C.c_int, i64p, u8p]
+        L.orc_overlap_path_parts.argtypes = [u64p, u64p, C.c_uint64, C.c_int, C.c_int, C.c_int, C.c_int, i64p, u8p]
+        L.orc_first_occurrence_runs.argtypes = [u8p, u64p, u64p, C.c_uint64, C.c_int, C.c_int, C.c_int, C.POINTER(u64p),
+                                                C.POINTER(u64p), u64p, u64p]
         L.orc_superstring.argtypes = [u8p, u64p, u64p, C.c_uint64, C.c_int, C.c_int, i64p, u8p, u64p, C.c_uint64,
                                       C.POINTER(u8p), C.POINTER(u8p), u64p]
         L.orc_compute_from_simplitigs.argtypes = [u8p, u64p, u64p, C.c_uint64, C.c_int, C.c_int, C.c_int,
@@ -218,17 +221,22 @@ def kmer_digest(keys, vals, min_frequency: int = 1):
                 int((h * (vals + np.uint64(1)) if min_frequency > 1 else h).sum(dtype=np.uint64))]
 
 
-def overlap_path(first, last, k: int, complements: bool, lower_bound: bool = False):
-    """first/last: [n, limbs] u64 -> (edge_from [N] i64, overlaps [N] u8)."""
+def overlap_path(first, last, k: int, complements: bool, lower_bound: bool = False, parts: int = 16):
+    """first/last: [n, limbs] u64 -> (edge_from [N] i64, overlaps [N] u8).  parts = number of prefix batches: 16 is the
+    reference, 1 the product's from-FASTA engine (engine.cuh with strict = false)."""
     first = np.ascontiguousarray(first, dtype=np.uint64)
     last = np.ascontiguousarray(last, dtype=np.uint64)
     n = first.shape[0]
     N = n * (2 if complements else 1)
     ef = np.zeros(N, dtype=np.int64)
     ov = np.zeros(N, dtype=np.uint8)
-    rc = lib().orc_overlap_path(_ptr(first, u64p), _ptr(last, u64p), n, k, int(complements), int(lower_bound),
-                                _ptr(ef, i64p), _ptr(ov, u8p))
-    assert rc == 0
+    if parts == 16:
+        rc = lib().orc_overlap_path(_ptr(first, u64p), _ptr(last, u64p), n, k, int(complements), int(lower_bound),
+                                    _ptr(ef, i64p), _ptr(ov, u8p))
+    else:
+        rc = lib().orc_overlap_path_parts(_ptr(first, u64p), _ptr(last, u64p), n, k, int(complements), int(lower_bound),
+                                          int(parts), _ptr(ef, i64p), _ptr(ov, u8p))
+    assert rc == 0, rc
     return ef, ov
 
 
@@ -267,14 +275,102 @@ def compute_from_simplitigs(records, k: int, complements: bool, want_maxone: boo
     return out, (_take(mo, n.value, np.uint8).tobytes() if want_maxone else None)
 
 
-def lower_bound_from_simplitigs(records, k: int, complements: bool) -> int:
+def lower_bound_from_simplitigs(records, k: int, complements: bool, parts: int = 16) -> int:
     """`kmercamel lowerbound -S` (reference src/lower_bound.h:9-22 LowerBoundLength): cycle cover of the records as
     nodes, (sum of lengths over the strands - sum of overlaps) / strands."""
     first = np.stack([kmer_from_string(r[:k].decode(), k) for r in records])
     last = np.stack([kmer_from_string(r[len(r) - k:].decode(), k) for r in records])
-    _, ov = overlap_path(first, last, k, complements, lower_bound=True)
+    _, ov = overlap_path(first, last, k, complements, lower_bound=True, parts=parts)
     strands = 2 if complements else 1
     return (sum(len(r) for r in records) * strands - int(ov.astype(np.int64).sum())) // strands
+
+
+def first_occurrence_runs(seq, rec_off, rec_len, k: int, complements: bool, min_frequency: int = 1):
+    """The from-FASTA nodes of the product (kmercamel_b200/csrc/runs.cuh): maximal runs of consecutive window ends that are the
+    first occurrence, in input order, of a kept canonical k-mer -> (run start byte [n] u64, run length [n] u64, kept k-mers)."""
+    seq = np.ascontiguousarray(seq, dtype=np.uint8)
+    rec_off = np.ascontiguousarray(rec_off, dtype=np.uint64)
+    rec_len = np.ascontiguousarray(rec_len, dtype=np.uint64)
+    ro, rl, n, kept = u64p(), u64p(), C.c_uint64(), C.c_uint64()
+    rc = lib().orc_first_occurrence_runs(_ptr(seq, u8p), _ptr(rec_off, u64p), _ptr(rec_len, u64p), len(rec_off), k,
+                                         int(complements), int(min_frequency), C.byref(ro), C.byref(rl), C.byref(n),
+                                         C.byref(kept))
+    assert rc == 0, rc
+    return _take(ro, n.value, np.uint64), _take(rl, n.value, np.uint64), kept.value
+
+
+_CODES = np.full(256, 4, dtype=np.uint8)
+for _i, _c in enumerate(b"ACGT"):
+    _CODES[_c] = _CODES[_c + 32] = _i
+
+
+def window_words(seq, starts, k: int):
+    """The k-mer (as read, not canonical) of the k bytes at each start -> [n, limbs] u64; the bytes must be ACGT or acgt."""
+    codes = _CODES[np.ascontiguousarray(seq, dtype=np.uint8)]
+    starts = np.asarray(starts, dtype=np.int64)
+    out = np.zeros((len(starts), limbs_for_k(k)), dtype=np.uint64)
+    for i in range(k):
+        c = codes[starts + i]
+        assert np.all(c < 4), "a node holds a non-ACGT byte"
+        bit = 2 * (k - 1 - i)  # base i (0 = leftmost) lies in one limb: 2-bit symbols never straddle a limb boundary
+        out[:, bit // 64] |= c.astype(np.uint64) << np.uint64(bit % 64)
+    return out
+
+
+def fasta_nodes(seq, rec_off, rec_len, k: int, complements: bool, min_frequency: int = 1, sparse_switch: bool = True):
+    """The nodes the product hands to its overlap stage from FASTA (kcgpu.cu run_pipeline) -> (node start [n] u64,
+    node length [n] u64, kept k-mers, first-occurrence runs).  The runs, unless there are at least U / 5 of them (the sparse
+    switch, reference src/main.cpp:94,175-181): then one node per k-mer of the runs, in run order and in the orientation it has
+    in the input, stably sorted on its first min(k, 4) bases (PartialPreSort, src/global_sparse.h:14-35)."""
+    off, ln, kept = first_occurrence_runs(seq, rec_off, rec_len, k, complements, min_frequency)
+    n_runs = len(off)
+    if kept == 0:
+        raise ValueError("the input contains no k-mers")
+    if sparse_switch and n_runs * 5 >= kept:
+        cnt = (ln - np.uint64(k - 1)).astype(np.int64)
+        base = np.repeat(off.astype(np.int64), cnt)
+        within = np.arange(int(cnt.sum())) - np.repeat(np.cumsum(cnt) - cnt, cnt)
+        starts = base + within
+        nb = min(k, 4)
+        codes = _CODES[np.ascontiguousarray(seq, dtype=np.uint8)].astype(np.int64)
+        digit = np.zeros(len(starts), dtype=np.int64)
+        for j in range(nb):
+            digit = (digit << 2) | codes[starts + j]
+        starts = starts[np.argsort(digit, kind="stable")]
+        off = starts.astype(np.uint64)
+        ln = np.full(len(starts), k, dtype=np.uint64)
+    return off, ln, kept, n_runs
+
+
+def compute_from_fasta(seq, rec_off, rec_len, k: int, complements: bool, min_frequency: int = 1, want_maxone: bool = False,
+                       sparse_switch: bool = True):
+    """The product's `compute` from FASTA, restated: fasta_nodes, then the greedy with one prefix batch (overlap_path
+    parts = 1, the engine's non-strict tie order), then the emission of the reference.  seq / rec_off / rec_len: framed
+    records (records_to_arrays, synth.frame_records).  -> dict(ms, maxone, n_kmers, n_nodes, n_simplitigs)."""
+    seq = np.ascontiguousarray(seq, dtype=np.uint8)
+    off, ln, kept, n_runs = fasta_nodes(seq, rec_off, rec_len, k, complements, min_frequency, sparse_switch)
+    first = window_words(seq, off, k)
+    last = window_words(seq, off + ln - np.uint64(k), k)
+    ef, ov = overlap_path(first, last, k, complements, parts=1)
+    set_keys = None
+    if want_maxone:
+        keys, vals = count_kmers(seq, rec_off, rec_len, k, complements)
+        set_keys = keys[vals.astype(np.int64) + 1 >= min_frequency]
+    ms, mo = superstring(seq, off, ln, k, complements, ef, ov, set_keys)
+    return dict(ms=ms, maxone=mo, n_kmers=kept, n_nodes=len(off), n_simplitigs=n_runs)
+
+
+def lower_bound_from_fasta(seq, rec_off, rec_len, k: int, complements: bool, min_frequency: int = 1,
+                           sparse_switch: bool = True) -> int:
+    """The product's `lowerbound` from FASTA, restated: the cycle cover (overlap_path lower_bound = True, parts = 1) of the
+    nodes of fasta_nodes, (sum of lengths over the strands - sum of overlaps) / strands (src/lower_bound.h:9-22)."""
+    seq = np.ascontiguousarray(seq, dtype=np.uint8)
+    off, ln, _, _ = fasta_nodes(seq, rec_off, rec_len, k, complements, min_frequency, sparse_switch)
+    _, ov = overlap_path(window_words(seq, off, k), window_words(seq, off + ln - np.uint64(k), k), k, complements,
+                         lower_bound=True, parts=1)
+    assert not np.any(ov == 255)  # a cycle cover: every node has a successor
+    strands = 2 if complements else 1
+    return (int(ln.astype(np.int64).sum()) * strands - int(ov.astype(np.int64).sum())) // strands
 
 
 def ms_kmers(ms: bytes, k: int, complements: bool):

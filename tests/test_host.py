@@ -169,6 +169,51 @@ def test_host_emul_simplitigs_md5(host_emul, golden, simplitigs_bytes):
     assert md5(out[0] + b"\n") == g["md5"] and md5(out[1] + b"\n") == g["maxone_md5"]
 
 
+def tie_heavy_node_set(seed):
+    """Seeded node set with many equal overlaps: records over a small alphabet, half of them periodic (a motif of 1-6 bases with a
+    few substitutions), the rest random; k from 3 to 127 so that all three word widths are covered.  -> (k, complements, records)"""
+    rng = np.random.default_rng(seed)
+    k = int(rng.choice([3, 4, 5, 6, 7, 8, 8, 12, 31, 32, 40, 63, 64, 100, 127]))
+    alpha = [b"AC", b"AT", b"ACG", b"ACGT"][seed % 4]
+    letters = np.frombuffer(alpha, dtype=np.uint8)
+    motifs = [rng.choice(letters, size=int(rng.integers(1, 7))).tobytes() for _ in range(4)]
+    recs = []
+    for _ in range(int(rng.integers(30, 401))):
+        n = k + int(rng.integers(0, k + 3))
+        if rng.random() < 0.5:
+            m = motifs[int(rng.integers(0, len(motifs)))]
+            ph = int(rng.integers(0, len(m)))
+            r = bytearray((m * (n // len(m) + 2))[ph:ph + n])
+            for _ in range(int(rng.integers(0, 3))):
+                r[int(rng.integers(0, n))] = int(rng.choice(letters))
+        else:
+            r = bytearray(rng.choice(letters, size=n).tobytes())
+        recs.append(bytes(r))
+    return k, bool(seed % 3), recs
+
+
+def test_host_emul_path_matches_oracle_batches(host_emul):
+    """The engine's tie order, compiled for the host, is the reference's greedy with the prefix nodes in one batch when it runs
+    non-strict (the from-FASTA regime: every prefix in batch 0, all cycle closers of a round banned at once) and with the
+    reference's 16 batches when it runs strict (-S).  Byte for byte, on node sets where equal overlaps and cycles abound."""
+    from test_oracle import node_ends
+    n_cases, banned, widths = 120, 0, set()
+    for seed in range(n_cases):
+        k, compl, recs = tie_heavy_node_set(seed)
+        widths.add(orc.limbs_for_k(k))
+        first, last = node_ends([r.decode() for r in recs], k)
+        for strict, parts in ((False, 1), (True, 16)):
+            out, err = host_emul("path", k, compl, strict, False, recs)
+            rows = np.array([list(map(int, ln.split())) for ln in out if ln], dtype=np.int64)
+            want_ef, want_ov = orc.overlap_path(first, last, k, compl, parts=parts)
+            assert np.array_equal(rows[:, 0], want_ef) and np.array_equal(rows[:, 1], want_ov), (seed, k, compl, strict)
+            if not strict and int(re.search(r"\bbans=(\d+)", err).group(1)) > 0:
+                banned += 1
+    assert widths == {1, 2, 4}
+    print(f"non-strict engine banned edges in {banned} of {n_cases} node sets")
+    assert 3 * banned >= n_cases  # the ban / replay path of the non-strict engine is covered, not avoided
+
+
 def test_host_emul_from_kmers_valid(host_emul):
     """From-FASTA regime (k-mer nodes, non-strict): the superstring represents exactly the k-mer set."""
     import random

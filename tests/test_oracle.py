@@ -118,6 +118,76 @@ def test_overlap_path_kats(records, k, compl, lb, want_ef, want_ov):
     assert ef.tolist() == want_ef and ov.tolist() == want_ov
 
 
+@pytest.mark.parametrize("records,k,compl,lb,want_ef,want_ov", PATH_KATS)
+def test_overlap_path_parts(records, k, compl, lb, want_ef, want_ov):
+    """parts = 16 is the reference's batching (the default); one batch agrees with it where no tie spans two batches."""
+    first, last = node_ends(records, k)
+    for parts in (16, 1):
+        ef, ov = orc.overlap_path(first, last, k, compl, lb, parts=parts)
+        assert ef.tolist() == want_ef and ov.tolist() == want_ov, parts
+
+
+# ---- the product's from-FASTA nodes: first-occurrence runs (kmercamel_b200/csrc/runs.cuh) --------------------------
+def _messy_records(seed):
+    """Records with N bytes, lower-case stretches, records shorter than k and repeated pieces."""
+    from kmercamel_b200 import synth
+    rng = np.random.default_rng(seed)
+    recs = [bytearray(r.tobytes()) for r in synth.random_genome_records(4, 900, seed)]
+    recs.append(bytearray(recs[0][200:500]))                                  # repeated piece: later occurrences are not first
+    recs[1][100:160] = bytes(recs[1][100:160]).lower()
+    recs[2][300:305] = b"NNNNN"
+    recs += [bytearray(b"ACGTA"), bytearray(b""), bytearray(b"acgtNacgtacgtt"), bytearray(recs[3][:40]).lower()]
+    for _ in range(30):                                                     # short pieces of earlier records
+        r = recs[int(rng.integers(0, 4))]
+        a = int(rng.integers(0, len(r) - 40))
+        recs.append(bytearray(r[a:a + int(rng.integers(1, 40))]))
+    return [bytes(r) for r in recs]
+
+
+@pytest.mark.parametrize("k", [1, 5, 11, 21, 31])
+@pytest.mark.parametrize("compl", [True, False])
+def test_first_occurrence_runs_vs_flags(k, compl):
+    """orc.first_occurrence_runs against the plain numpy first-occurrence flags of the sharded tests: the runs are exactly the
+    maximal stretches of flagged window ends, in input order, and the kept counts agree."""
+    from test_sharded import first_occurrence_flags, make_input
+    inputs = [make_input(3), make_input(4), orc.records_to_arrays(_messy_records(5))[0]]
+    for seq in inputs:
+        recs = bytes(seq).split(b"\n")[:-1]
+        s2, off, ln = orc.records_to_arrays(recs)
+        assert np.array_equal(s2, seq)
+        for z in (1, 2, 3):
+            words, kept = first_occurrence_flags(seq, k, compl, z)
+            ro, rl, n_kept = orc.first_occurrence_runs(seq, off, ln, k, compl, z)
+            assert n_kept == kept and int((rl - np.uint64(k - 1)).sum()) == kept, (k, compl, z)
+            got = np.zeros_like(words)
+            ends = np.concatenate([np.arange(int(o) + k - 1, int(o) + int(l)) for o, l in zip(ro, rl)]) if len(ro) else np.zeros(0, np.int64)
+            np.bitwise_or.at(got, ends >> 5, np.uint32(1) << (ends & 31).astype(np.uint32))
+            assert np.array_equal(got, words), (k, compl, z)
+            assert np.all(ro[1:] > ro[:-1] + rl[:-1] - np.uint64(k - 1))       # input order, maximal: no two runs touch
+
+
+def test_compute_from_fasta_is_a_min_one_superstring():
+    """The restated from-FASTA pipeline emits a superstring of exactly the kept k-mers with every k-mer ON once, in both node
+    regimes (runs and, past the sparse switch, k-mer nodes), and its lower bound does not exceed it."""
+    from kmercamel_b200 import synth
+    cases = [(_messy_records(7), 11, True, 1), (_messy_records(8), 31, False, 1), (_messy_records(9), 5, True, 2),
+             ([r.tobytes() for r in synth.short_records(300, 9, 11, 19)], 9, False, 1),
+             ([r.tobytes() for r in synth.short_records(200, 31, 34, 17)], 31, True, 1)]
+    for recs, k, compl, z in cases:
+        seq, off, ln = orc.records_to_arrays(recs)
+        keys, vals = orc.count_kmers(seq, off, ln, k, compl)
+        keys = keys[vals.astype(np.int64) + 1 >= z]
+        for sparse in (True, False):
+            r = orc.compute_from_fasta(seq, off, ln, k, compl, z, want_maxone=True, sparse_switch=sparse)
+            assert r["n_kmers"] == len(keys)
+            assert orc.verify_ms(r["ms"], k, compl, keys) and orc.verify_ms(r["maxone"], k, compl, keys)
+            assert sum(1 for c in r["ms"] if c <= 90) == len(keys)
+            assert r["ms"].upper() == r["maxone"].upper()
+            switched = sparse and r["n_simplitigs"] * 5 >= r["n_kmers"]
+            assert r["n_nodes"] == (r["n_kmers"] if switched else r["n_simplitigs"])
+            assert orc.lower_bound_from_fasta(seq, off, ln, k, compl, z, sparse_switch=sparse) <= len(r["ms"])
+
+
 # ---- lowerbound: tests/lower_bound_unittest.h:11-41 and the reference CLI on the fuzzed -S inputs -------------
 LOWER_BOUND_KATS = [(["ACG", "CGT", "TAA"], 3, False, 5), (["ACGT", "TAA"], 3, False, 5), (["AC", "GG"], 2, True, 3),
                     (["AAACCC", "CCCAAA", "TGGGGT"], 6, False, 11)]
