@@ -243,11 +243,16 @@ uint64_t kc_total_launches(const kc_ctx *ctx);
  * "tail_spec" (default 1): after the signature-bucket construction, queue the rest of the call sized for a few hundred
  * first-occurrence runs (a genome) with no host round trip before the end; an input with more runs falls back to the
  * ordinary path, and the context skips the attempt for inputs of similar size after that (with "fast_heuristics").
+ * "arena_poison" (default -1 = off, 0..255): fill every block the device arena hands out with this byte first (on the context
+ * stream), so that a kernel that reads memory no one wrote in this call gives a wrong result instead of an earlier call's bits.
+ * "arena_estimate_ppm" (default 1000000): scale the first arena estimate of kc_compute, kc_compute_device and kc_lower_bound, in
+ * parts per million, so that a small input runs out of arena and the call is repeated with the worst-case estimate.
  * Results never depend on these options. */
 int kc_set_option(kc_ctx *ctx, const char *name, int value);
 /* Counters since kc_init: "sig_runs", "sig_fallbacks", "fast_runs", "fast_fallbacks", "total_launches", "tail_spec_runs",
  * "tail_spec_fallbacks", "read_backs" (synchronising device -> host reads, i.e. host round trips); current value of the
- * option "fast_max_ctas"; device arena: "arena_bytes" (reserved now), "arena_high" (most bytes in use at once since kc_init).
+ * option "fast_max_ctas"; device arena: "arena_bytes" (reserved now), "arena_high" (most bytes in use at once since kc_init),
+ * "arena_retries" (calls repeated with the worst-case estimate after running out of arena).
  * Totals of the greedy overlap stage of the LAST call that ran it (kc_compute, kc_lower_bound, kc_overlap_path, a group
  * compute), over the level loop and the single-CTA engine: "path_levels" (overlap levels replayed), "path_ban_rounds" (replays
  * of a level after a cycle was found), "path_bans" (refused edges; with complements each one counts for both strands). */

@@ -78,16 +78,27 @@ inline int kc_sm_count(int dev) {
 }
 
 // Bump allocator over one device (or, in the host-emulation test build, host) slab.  All temporaries of a
-// kc_compute call live here so the timed path never calls cudaMalloc.
+// kc_compute call live here so the timed path never calls cudaMalloc.  The slab is never cleared: a block holds whatever an
+// earlier call, or an earlier block of the same call, left there, so everything a kernel reads must have been written in this call.
+// `poison` (option "arena_poison") makes that testable: every block handed out is first filled with that byte, on `stream`.
 struct Arena {
     char *base = nullptr;
     size_t cap = 0;
     size_t off = 0;   // bottom end: temporaries, stack discipline (mark / release)
     size_t top = 0;   // top end: small results that must outlive the temporaries below them
     size_t high = 0;
+    int poison = -1;  // 0..255: fill byte of every block handed out; -1 = off
+    cudaStream_t stream = nullptr;
     void reset() {
         off = 0;
         top = cap;
+    }
+    void fill_poison(void *p, size_t bytes) {
+#ifdef KC_HOST_EMUL
+        std::memset(p, poison, bytes);
+#else
+        KC_CUDA(cudaMemsetAsync(p, poison, bytes, stream));
+#endif
     }
     template <typename T> T *alloc(size_t n) {
         size_t bytes = kc_align_up((n ? n : 1) * sizeof(T), 256);
@@ -95,6 +106,7 @@ struct Arena {
         T *p = reinterpret_cast<T *>(base + off);
         off += bytes;
         if (off + (cap - top) > high) high = off + (cap - top);
+        if (poison >= 0) fill_poison(p, bytes);
         return p;
     }
     template <typename T> T *alloc_top(size_t n) {
@@ -102,6 +114,7 @@ struct Arena {
         if (off + bytes > top) KC_THROW(KC_ERR_OOM, "device arena exhausted");
         top -= bytes;
         if (off + (cap - top) > high) high = off + (cap - top);
+        if (poison >= 0) fill_poison(base + top, bytes);
         return reinterpret_cast<T *>(base + top);
     }
     size_t mark() const { return off; }

@@ -69,6 +69,8 @@ struct kc_ctx {
     EngineStats path_stats;   // the overlap stage of the last call that ran it (stats "path_levels", "path_ban_rounds", "path_bans")
     KcGroup grp;             // multi-GPU: this context as one rank of a group (group.cuh)
     bool arena_limited = false;
+    u32 arena_estimate_ppm = 1000000;  // option "arena_estimate_ppm": scales the first arena estimate of run_with_arena (tests)
+    u64 arena_retries = 0;         // calls repeated by run_with_arena after running out of arena
     std::string last_error;
 };
 
@@ -168,12 +170,13 @@ size_t estimate_arena(u64 n_bytes, u64 n_recs, int limbs, bool complements, bool
 // Runs body() with an arena of `need` bytes; if the arena is exhausted (more nodes than the estimate assumed) the call is
 // repeated once with `need_max`.
 template <class F> void run_with_arena(kc_ctx *ctx, size_t need, size_t need_max, F body) {
-    ensure_arena(ctx, need);
+    ensure_arena(ctx, (size_t) ((double) need * ctx->arena_estimate_ppm / 1e6));
     try {
         ctx->arena.reset();
         body();
     } catch (const KcError &e) {
         if (e.code != KC_ERR_OOM || need_max <= ctx->arena.cap || ctx->arena_limited) throw;
+        ++ctx->arena_retries;
         KC_CUDA(cudaStreamSynchronize(ctx->stream));
         ensure_arena(ctx, need_max);
         ctx->arena.reset();
@@ -899,6 +902,7 @@ int kc_init(int device, void *stream, kc_ctx **out) {
             KC_CUDA(cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
             ctx->own_stream = true;
         }
+        ctx->arena.stream = ctx->stream;
         for (int i = 0; i < 6; ++i) KC_CUDA(cudaEventCreate(&ctx->ev[i]));
         KC_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&ctx->pin_small), kc_ctx::KC_PIN_SMALL, cudaHostAllocDefault));
         if (const char *e = std::getenv("KC_FAST_SET")) ctx->fast.enabled = std::atoi(e) != 0;
@@ -987,7 +991,8 @@ int kc_compute(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_output *o
     run_with_arena(ctx, estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, false, &ctx->fast, &sig),
                    estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, true, &ctx->fast, &sig), [&] {
         // host -> device.  Large from-FASTA inputs go in chunks on the copy stream: the level-0 partition pass of chunk c starts
-        // as soon as chunk c has landed (InputChunks), instead of after the whole copy.
+        // as soon as chunk c has landed (InputChunks), instead of after the whole copy.  The 64 bytes past n_bytes are never written:
+        // every loader of the from-FASTA path is bounded by n_bytes (kc_compute_device gets a caller's buffer without them).
         u8 *d_seq = ex.alloc<u8>(in->n_bytes + 64);
         InputChunks chunks;
         const bool chunked = !simplitigs && in->n_bytes >= (8u << 20);
@@ -999,6 +1004,10 @@ int kc_compute(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_output *o
             const u64 granule = 32768;  // whole level-0 tiles for every word width
             chunks.chunk_bytes = (in->n_bytes / kc_ctx::KC_H2D_CHUNKS + granule) / granule * granule;
             chunks.ev = ctx->chunk_ev;
+            if (ctx->arena.poison >= 0) {  // the copy must land after the poison fill of d_seq on the context stream
+                KC_CUDA(cudaEventRecord(ctx->ev[5], ctx->stream));
+                KC_CUDA(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev[5], 0));
+            }
             for (u64 off = 0; off < in->n_bytes; off += chunks.chunk_bytes) {
                 const u64 len = std::min<u64>(chunks.chunk_bytes, in->n_bytes - off);
                 KC_CUDA(cudaMemcpyAsync(d_seq + off, in->seq + off, len, cudaMemcpyHostToDevice, ctx->copy_stream));
@@ -1700,6 +1709,7 @@ int kc_get_stat(const kc_ctx *ctx, const char *name, uint64_t *value) {
     else if (std::strcmp(name, "tail_spec_fallbacks") == 0) *value = ctx->tail_spec_fallbacks;
     else if (std::strcmp(name, "arena_bytes") == 0) *value = ctx->arena.cap;
     else if (std::strcmp(name, "arena_high") == 0) *value = ctx->arena.high;
+    else if (std::strcmp(name, "arena_retries") == 0) *value = ctx->arena_retries;
     else if (std::strcmp(name, "fast_max_ctas") == 0) *value = (uint64_t) ctx->fast.max_ctas;
     else if (std::strcmp(name, "path_levels") == 0) *value = ctx->path_stats.levels_run;
     else if (std::strcmp(name, "path_ban_rounds") == 0) *value = ctx->path_stats.ban_rounds;
@@ -1771,6 +1781,17 @@ int kc_set_option(kc_ctx *ctx, const char *name, int value) {
     }
     if (std::strcmp(name, "sig_min_items") == 0 && value >= 0) {
         ctx->sig.min_items = (u64) value;
+        return KC_OK;
+    }
+    // device arena (tests): fill every block it hands out with this byte (-1 = off), and scale the first estimate of a call (in
+    // parts per million: 1 % of an estimate is megabytes, more than a stage of a small input allocates) so that a small input runs
+    // out of arena at a chosen point and takes the retry with the worst-case estimate
+    if (std::strcmp(name, "arena_poison") == 0 && value >= -1 && value <= 255) {
+        ctx->arena.poison = value;
+        return KC_OK;
+    }
+    if (std::strcmp(name, "arena_estimate_ppm") == 0 && value >= 1 && value <= 1000000) {
+        ctx->arena_estimate_ppm = (u32) value;
         return KC_OK;
     }
     return KC_ERR_ARG;

@@ -12,6 +12,9 @@
 //       k-mers of the records (the from-FASTA regime) -> superstring [, max-one]
 //   host_emul plan <m_upper> <leaf_target> <sigmas> 0         the fixed-slot plan of csrc/ksf_plan.h for an input of m_upper
 //       windows -> "ok levels n_leaf slots0 slots1", then "bits cum cap" per level
+//
+// KC_ARENA_POISON=<0..255> in the environment fills every arena block with that byte before it is handed out (the option
+// "arena_poison" of the library): the output must not change.
 #include "../kmercamel_b200/csrc/emit.cuh"
 #include "../kmercamel_b200/csrc/engine.cuh"
 #include "../kmercamel_b200/csrc/ksf_plan.h"
@@ -29,10 +32,13 @@ template <int L> KWord<L> kmer_of(const std::string &s, size_t pos, int k) {
     return x;
 }
 
+static int arena_poison = -1;
+
 template <int L> int run(const std::string &mode, int k, bool complements, bool strict, bool flag, const std::vector<std::string> &recs) {
     Arena arena;
     arena.cap = (size_t) 1 << 30;
     arena.base = (char *) std::malloc(arena.cap);
+    arena.poison = arena_poison;
     arena.reset();
     HostExec ex{&arena};
     std::vector<KWord<L>> set;
@@ -101,6 +107,7 @@ template <int L> int run(const std::string &mode, int k, bool complements, bool 
 int main(int argc, char **argv) {
     if (argc < 6) return 64;
     std::string mode = argv[1];
+    if (const char *e = std::getenv("KC_ARENA_POISON")) arena_poison = std::atoi(e);
     if (mode == "plan") {
         KsfTuning t;
         t.leaf_target = (uint32_t) std::atoi(argv[3]);

@@ -5,6 +5,7 @@
 * the engine/emission control flow, compiled for the host (tests/host_emul, KC_HOST_EMUL), against the oracle.
 """
 import ctypes
+import functools
 import os
 import re
 import shutil
@@ -140,9 +141,13 @@ def host_emul():
     if shutil.which("nvcc") is not None:
         subprocess.check_call(["make", "-C", ROOT, "tests/host_emul"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
 
-    def run(mode, k, compl, strict, flag, records):
+    def run(mode, k, compl, strict, flag, records, poison=None):
+        env = dict(os.environ)
+        env.pop("KC_ARENA_POISON", None)
+        if poison is not None:
+            env["KC_ARENA_POISON"] = str(poison)
         p = subprocess.run([exe, mode, str(k), str(int(compl)), str(int(strict)), str(int(flag))],
-                           input=b"\n".join(records) + b"\n", capture_output=True)
+                           input=b"\n".join(records) + b"\n", capture_output=True, env=env)
         assert p.returncode == 0, p.stderr
         return p.stdout.split(b"\n"), p.stderr.decode()
     return run
@@ -226,6 +231,18 @@ def test_host_emul_from_kmers_valid(host_emul):
         exp, _ = orc.count_kmers(seq, off, ln, k, compl)
         assert orc.verify_ms(out[0], k, compl, exp) and orc.verify_ms(out[1], k, compl, exp)
         assert sum(1 for c in out[0] if c <= 90) == len(exp)  # min-one: every k-mer ON exactly once
+
+
+@pytest.mark.parametrize("poison", [0x00, 0xA5, 0xFF])
+def test_host_emul_poisoned_arena(host_emul, golden, simplitigs_bytes, poison):
+    """The cases above with every arena block filled with `poison` before it is handed out: the engine and the emission must
+    write everything they read.  0x00 looks like a finished zero-fill, 0xFF like KC_NONE."""
+    run = functools.partial(host_emul, poison=poison)
+    test_host_emul_path_kats(run)
+    test_host_emul_fuzz_S_byte_exact(run, golden)
+    test_host_emul_simplitigs_md5(run, golden, simplitigs_bytes)
+    test_host_emul_path_matches_oracle_batches(run)
+    test_host_emul_from_kmers_valid(run)
 
 
 # ---- plan of the fixed-slot k-mer set construction (csrc/ksf_plan.h) -----------------------------------------------
