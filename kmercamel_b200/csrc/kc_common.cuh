@@ -77,6 +77,10 @@ inline int kc_sm_count(int dev) {
     return n[dev];
 }
 
+struct ArenaMark {
+    size_t off, top;
+};
+
 // Bump allocator over one device (or, in the host-emulation test build, host) slab.  All temporaries of a
 // kc_compute call live here so the timed path never calls cudaMalloc.  The slab is never cleared: a block holds whatever an
 // earlier call, or an earlier block of the same call, left there, so everything a kernel reads must have been written in this call.
@@ -119,4 +123,10 @@ struct Arena {
     }
     size_t mark() const { return off; }
     void release(size_t m) { off = m; }
+    // both ends: restore() frees what either end handed out since checkpoint()
+    ArenaMark checkpoint() const { return {off, top}; }
+    void restore(const ArenaMark &m) {
+        off = m.off;
+        top = m.top;
+    }
 };

@@ -13,6 +13,7 @@
 #include "kword.cuh"
 #include "masks.cuh"
 #include "runs.cuh"
+#include "set_routes.cuh"
 #include "sort.cuh"
 #include "stage1.cuh"
 #include "tail_spec.cuh"
@@ -54,18 +55,11 @@ struct kc_ctx {
     bool small_engine = true;
     int small_threads = 0;   // 0 = chosen by the number of free ends (option "small_threads": 256 or 512)
     bool sparse_switch = true;  // src/main.cpp:175 (option "sparse_switch" = 0 keeps the runs as nodes whatever their number)
-    KsfTuning fast;          // histogram-free set construction (kmerset_fast.cuh); KC_FAST_* environment knobs for tests
-    u64 fast_runs = 0, fast_fallbacks = 0;
-    SigTuning sig;           // signature-bucket set construction (kmerset_sig.cuh), tried first in the FLAGS regime
-    u64 sig_runs = 0, sig_fallbacks = 0;
-    u64 sig_overflow_bytes = 0;   // input size of the last call whose signature buckets overflowed (0 = none)
-    bool fast_heuristics = true;  // skip the fixed-slot attempt when duplicates are expected (see run_stage1_runs)
-    u64 fast_overflow_bytes = 0;  // input size of the last call whose fixed-slot attempt overflowed (0 = none)
+    SetRoutes routes;        // the constructions of the first-occurrence bits, their tuning, counters and memories (set_routes.cuh)
     u64 total_launches = 0;  // kernels launched through this context since kc_init
     u64 read_backs = 0;      // synchronising device -> host reads of this context since kc_init (host round trips)
     bool tail_spec = true;   // option "tail_spec": queue the tail of the from-FASTA path without reading the run count (run_tail_spec)
     u64 tail_spec_runs = 0, tail_spec_fallbacks = 0;
-    u64 spec_fail_bytes = 0;  // input size of the last call whose speculative tail did not hold (0 = none)
     EngineStats path_stats;   // the overlap stage of the last call that ran it (stats "path_levels", "path_ban_rounds", "path_bans")
     KcGroup grp;             // multi-GPU: this context as one rank of a group (group.cuh)
     bool arena_limited = false;
@@ -108,15 +102,14 @@ void check_params(const kc_params *p) {
 
 // Inputs of KC_POS32_BYTES or more need 64-bit window positions, which only the signature construction carries (the fixed-slot
 // and exact constructions move 32-bit positions, the -S path and the other entry points keep their 32-bit caps).
-#define KC_LARGE_ONLY "inputs of 2^32 bytes or more are built by the signature construction only (k >= 26, no -z, no -M, no -S)"
 void check_large_input(const kc_ctx *ctx, const kc_params *p, u64 n_bytes) {
     if (n_bytes < KC_POS32_BYTES) return;
     if (p->assume_simplitigs) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; -S was asked");
     if (p->min_frequency > 1) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; -z (min_frequency > 1) was asked");
     if (p->want_maxone) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; -M (want_maxone) was asked");
     if (p->k < 26) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; k is below 26");
-    if (!ctx->sig.enabled) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; it is switched off (option sig_set = 0)");
-    if (!kc_sig_plan(n_bytes, p->k, ctx->sig).ok) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; its bucket plan does not fit this input");
+    if (!ctx->routes.sig.enabled) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; it is switched off (option sig_set = 0)");
+    if (!kc_sig_plan(n_bytes, p->k, ctx->routes.sig).ok) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; its bucket plan does not fit this input");
 }
 
 // Make sure the arena can hold `need` bytes (bounded by what the device can give).
@@ -312,11 +305,12 @@ u32 run_tail_spec(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params
 // in input order and go through the same overlap levels d = k-1..0 as `-S` records, so run ends that overlap by
 // k-1 are still joined first, exactly as BIGREEDY requires.
 //
+// The first-occurrence flags come from kc_set_ladder (set_routes.cuh), or else from the exact construction.
 // spec_res != nullptr: after the signature construction, try the speculative tail (run_tail_spec).  When it holds, *spec_res is the whole
-// result and *spec_done is set; otherwise the code below continues as if it had not been tried, on the same flags.
+// result and *spec_done is set; otherwise the runs are counted as if it had not been tried, on the same flags.
 template <int L>
 u64 run_stage1_runs(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &p, RunNodes *runs, KWord<L> **set_out, u64 *n_occ,
-                    DevResult *spec_res = nullptr, bool *spec_done = nullptr) {
+                    DevResult *spec_res, bool *spec_done) {
     KC_CUDA(cudaEventRecord(ctx->ev[0], ex.stream));
     KC_CUDA(cudaEventRecord(ctx->ev[1], ex.stream));  // extraction is fused into the partition passes
     KC_TRACE_POINT("stage1: begin");
@@ -326,82 +320,51 @@ u64 run_stage1_runs(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_para
     ex.fill_bytes(flags, 0, fwords * 4);
     u64 *cells = ex.arena->alloc_top<u64>(2);  // {kept distinct k-mers, runs}
     ex.fill_bytes(cells, 0, 16);
-    // FLAGS-only: try the histogram-free construction first (no host synchronisation until the runs are counted).  Its
-    // fixed slots assume mostly distinct k-mers; `-z Z > 1` announces a read set with coverage (every k-mer ~coverage times:
-    // the leaf slots overflow and the attempt is wasted — configs[3] at full size lost 70 ms to it), and so does an
-    // overflow in the previous call of this context on an input of similar size.
-    const bool expect_duplicates = ctx->fast_heuristics && (p.min_frequency > 1 || (ctx->fast_overflow_bytes && nb >= ctx->fast_overflow_bytes / 2 && nb <= ctx->fast_overflow_bytes * 2));
-    // Signature buckets first (kmerset_sig.cuh): records of ~7 windows instead of 12-byte items.  Read sets with coverage overflow
-    // its buckets (every run of windows comes c times: sigma grows by sqrt(c)) and are remembered like a fixed-slot overflow.
-    // Inputs of KC_POS32_BYTES or more have no other construction (check_large_input): they always try it, and an overflow ends the call.
-    const bool large = nb >= KC_POS32_BYTES;
-    const bool sig_overflowed = ctx->fast_heuristics && ctx->sig_overflow_bytes && nb >= ctx->sig_overflow_bytes / 2 && nb <= ctx->sig_overflow_bytes * 2;
-    if (!p.want_maxone && p.min_frequency == 1 && (large || !sig_overflowed)) {
-        const size_t n_cells = spec_res ? KC_SPEC_BLOCK_WORDS : 4;
-        u64 *cells4 = ex.arena->alloc_top<u64>(n_cells);  // {kept, runs, M, overflow status} (+ the rest of the speculative tail's status block)
+    u64 *cells4 = nullptr, hc[4];
+    KsfPlan plan;
+    auto launch = [&](KcRoute r) {
+        const size_t n_cells = r == KC_ROUTE_SIG && spec_res ? KC_SPEC_BLOCK_WORDS : 4;
+        cells4 = ex.arena->alloc_top<u64>(n_cells);  // {kept, runs, M, overflow status} (+ the rest of the speculative tail's status block)
         ex.fill_bytes(cells4, 0, n_cells * 8);
-        if (kc_kmerset_build_sig<L>(ex, in.seq, nb, p.k, p.complements != 0, flags, cells4, ctx->sig, in.chunks)) {
-            KC_TRACE_POINT("stage1: signature set launched");
-            u64 hc[4];
-            bool aborted = false;
-            if (spec_res) {
-                const u32 st = run_tail_spec<L>(ctx, ex, in, p, flags, cells4, *spec_res);
-                if (st == KC_SPEC_OK) {
-                    ++ctx->sig_runs;
-                    ++ctx->tail_spec_runs;
-                    *spec_done = true;
-                    return spec_res->n_kmers;
-                }
-                ++ctx->tail_spec_fallbacks;
-                if (st == KC_SPEC_SIG_OVERFLOW) {
-                    aborted = true;
-                } else {  // the flags stand: the ordinary tail counts the runs again
-                    if (st != KC_SPEC_EMPTY) ctx->spec_fail_bytes = nb;
-                    ex.fill_bytes(cells4 + 1, 0, 8);
-                }
+        return r == KC_ROUTE_SIG ? kc_kmerset_build_sig<L>(ex, in.seq, nb, p.k, p.complements != 0, flags, cells4, ctx->routes.sig, in.chunks)
+                                 : kc_kmerset_build_fast<L>(ex, in.seq, nb, p.k, p.complements != 0, p.min_frequency, flags, cells4, ctx->routes.fast,
+                                                            &plan, in.chunks);
+    };
+    auto consume = [&](KcRoute r) {
+        KC_TRACE_POINT(r == KC_ROUTE_SIG ? "stage1: signature set launched" : "stage1: fast set launched");
+        bool aborted = false;
+        if (r == KC_ROUTE_SIG && spec_res) {
+            const u32 st = run_tail_spec<L>(ctx, ex, in, p, flags, cells4, *spec_res);
+            if (st == KC_SPEC_OK) {
+                ++ctx->tail_spec_runs;
+                *spec_done = true;
+                return true;
             }
-            if (!aborted) *runs = kc_runs_from_flags(ex, flags, nb, p.k, cells4, hc, 4, &aborted);
-            if (!aborted) {
-                ++ctx->sig_runs;
-                *n_occ = hc[2];
-                *set_out = nullptr;
-                KC_CUDA(cudaEventRecord(ctx->ev[2], ex.stream));
-                return hc[2] ? hc[0] : 0;
+            ++ctx->tail_spec_fallbacks;
+            aborted = st == KC_SPEC_SIG_OVERFLOW;
+            if (!aborted) {  // the flags stand: the ordinary tail counts the runs again
+                if (st != KC_SPEC_EMPTY) ctx->routes.tail.remember(nb);
+                ex.fill_bytes(cells4 + 1, 0, 8);
             }
-            ++ctx->sig_fallbacks;  // a bucket overflowed: discard the flags, fall through to the other constructions
-            ctx->sig_overflow_bytes = nb;
-            if (large) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; it overflowed on this input (too repetitive)");
-            ex.fill_bytes(flags, 0, fwords * 4);
         }
-    }
-    if (large) KC_THROW(KC_ERR_INTERNAL, "an input of 2^32 bytes or more reached the 32-bit set constructions");
-    if (!p.want_maxone && !expect_duplicates) {
-        KsfPlan plan;
-        u64 *cells4 = ex.arena->alloc_top<u64>(4);  // {kept, runs, M, overflow status}
-        ex.fill_bytes(cells4, 0, 32);
-        if (kc_kmerset_build_fast<L>(ex, in.seq, nb, p.k, p.complements != 0, p.min_frequency, flags, cells4, ctx->fast, &plan, in.chunks)) {
-            KC_TRACE_POINT("stage1: fast set launched");
-            u64 hc[4];
-            bool aborted = false;
-            *runs = kc_runs_from_flags(ex, flags, nb, p.k, cells4, hc, 4, &aborted);
-            if (!aborted) {
-                ++ctx->fast_runs;
-                // the timers charged the partition passes with M = n_bytes; now that M is known, correct the byte counts
-                if (ex.prof && ex.prof->enabled && nb > hc[2]) {
-                    const u64 d = (nb - hc[2]) * (sizeof(KWord<L>) + 4);
-                    ex.prof->bytes[KP_KS_SCATTER0] -= d;
-                    ex.prof->bytes[KP_SORT_SCATTER] -= 2 * d * (u64) (plan.n_levels - 1);
-                    ex.prof->bytes[KP_KS_RESOLVE] -= d;
-                }
-                *n_occ = hc[2];
-                *set_out = nullptr;
-                KC_CUDA(cudaEventRecord(ctx->ev[2], ex.stream));
-                return hc[2] ? hc[0] : 0;
-            }
-            ++ctx->fast_fallbacks;  // a slot overflowed: discard the flags, fall through to the exact construction
-            ctx->fast_overflow_bytes = nb;
-            ex.fill_bytes(flags, 0, fwords * 4);
+        if (!aborted) *runs = kc_runs_from_flags(ex, flags, nb, p.k, cells4, hc, 4, &aborted);
+        if (aborted) ex.fill_bytes(flags, 0, fwords * 4);  // incomplete: the next construction starts from clear bits
+        return !aborted;
+    };
+    const KcRoute route = kc_set_ladder(ctx->routes, ctx->routes.compute_policy(p, nb), nb, *ex.arena, launch, consume);
+    if (route != KC_ROUTE_NONE) {
+        if (*spec_done) return spec_res->n_kmers;
+        // the timers charged the fixed-slot partition passes with M = n_bytes; now that M is known, correct the byte counts
+        if (route == KC_ROUTE_FAST && ex.prof && ex.prof->enabled && nb > hc[2]) {
+            const u64 d = (nb - hc[2]) * (sizeof(KWord<L>) + 4);
+            ex.prof->bytes[KP_KS_SCATTER0] -= d;
+            ex.prof->bytes[KP_SORT_SCATTER] -= 2 * d * (u64) (plan.n_levels - 1);
+            ex.prof->bytes[KP_KS_RESOLVE] -= d;
         }
+        *n_occ = hc[2];
+        *set_out = nullptr;
+        KC_CUDA(cudaEventRecord(ctx->ev[2], ex.stream));
+        return hc[2] ? hc[0] : 0;
     }
     // with -M the sorted k-mer set doubles as kMersDict of src/global.h:165-167; it stays at the arena bottom
     if (in.chunks) in.chunks->wait_all(ex.stream);
@@ -475,7 +438,7 @@ void run_pipeline(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params
         } else {
             // the speculative tail: a FASTA input with few runs (a genome) is computed behind one read-back (run_tail_spec)
             const u64 nb = in.n_bytes;
-            const bool spec_failed = ctx->fast_heuristics && ctx->spec_fail_bytes && nb >= ctx->spec_fail_bytes / 2 && nb <= ctx->spec_fail_bytes * 2;
+            const bool spec_failed = ctx->routes.heuristics && ctx->routes.tail.near(nb);
             const bool spec = ctx->tail_spec && !spec_failed && !lower_bound && ctx->small_engine && nb > 0 && nb < KC_POS32_BYTES;
             bool spec_done = false;
             U = run_stage1_runs<L>(ctx, ex, in, p, &runs, &uniq, &n_occ, spec ? &res : nullptr, &spec_done);
@@ -609,45 +572,16 @@ void count_only(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &
     KC_CUDA(cudaStreamSynchronize(ex.stream));
 }
 
-// The first-occurrence flags of a from-FASTA input built by the signature construction (kmerset_sig.cuh) alone, for the entry
-// points that need the k-mer set but not its runs: kc_kmer_digest and kc_streaming.  win_mask: optional window filter over END
-// positions, sized for the signature scan's tiles of 256 * 32 positions.  flags (fwords words) and cells {kept, -, M, status, ...}
-// arrive zeroed; after() queues the work that reads the flags before the one read-back of cells[0, n_cells) into hc.
-// Returns true when the flags stand.  Returns false when the construction does not apply, or when a bucket overflowed: then the overflow
-// is counted in sig_fallbacks, flags and cells are zeroed again, and the caller takes the other constructions.  Unlike run_stage1_runs
-// it leaves sig_overflow_bytes alone, so a digest or a streaming call does not change which construction a later compute tries.
-// Inputs of KC_POS32_BYTES or more have no other construction (check_large_input): there the call fails instead.
-template <int L, class After>
-bool sig_flags(kc_ctx *ctx, CudaExec &ex, const u8 *seq, u64 nb, const kc_params &p, u32 *flags, size_t fwords, const u32 *win_mask, u64 *cells,
-               u64 *hc, int n_cells, After after) {
-    const bool large = nb >= KC_POS32_BYTES;
-    if (!kc_kmerset_build_sig<L>(ex, seq, nb, p.k, p.complements != 0, flags, cells, ctx->sig, nullptr, win_mask)) {
-        if (large) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; its bucket plan does not fit this input");
-        return false;
-    }
-    after();
-    ex.read_n(cells, hc, (size_t) n_cells);
-    if (hc[3] == 0) {
-        ++ctx->sig_runs;
-        return true;
-    }
-    ++ctx->sig_fallbacks;
-    if (large) KC_THROW(KC_ERR_TOO_LARGE, KC_LARGE_ONLY "; it overflowed on this input (too repetitive)");
-    ex.fill_bytes(flags, 0, fwords * 4);
-    ex.fill_bytes(cells, 0, (size_t) n_cells * 8);
-    return false;
-}
-
 // kc_kmer_digest: (n, sum h, xor h, sum h * c) over the kept (k-mer, c = min(occurrences, 256), or 1 without -z) pairs, h = the splitmix64 fold of
 // the limbs (kc_kmer_hash).  The same four numbers come out of oracle/ref_harness `full` for the reference's own hash table.
-// Without -z the set is first tried as first-occurrence flags of the signature construction, hashed window by window (digest.cuh); the
-// sorted keys of kc_kmerset_build are the other route.  The digest is a function of the set: both give the same four words.
-
+// Without -z the set is first tried as first-occurrence flags (kc_set_ladder), hashed window by window (digest.cuh); the sorted keys
+// of kc_kmerset_build are the other route.  The digest is a function of the set: both give the same four words.  win_mask: optional
+// window filter over END positions, sized for the signature scan's tiles of 256 * 32 positions.
 template <int L>
 void digest_only(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &p, const u32 *win_mask, uint64_t *digest) {
     KC_CUDA(cudaEventRecord(ctx->ev[0], ex.stream));
     if (p.min_frequency == 1) {  // c = 1: digest[3] = digest[1]
-        const size_t top = ex.arena->top, mark = ex.arena->mark();
+        const ArenaMark mark = ex.arena->checkpoint();
         const size_t fwords = kc_runs_flag_words(in.n_bytes);
         u32 *flags = ex.arena->alloc_top<u32>(fwords);
         ex.fill_bytes(flags, 0, fwords * 4);
@@ -655,16 +589,23 @@ void digest_only(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params 
         ex.fill_bytes(cells, 0, 64);
         kc_ull *acc = reinterpret_cast<kc_ull *>(cells + 4);
         u64 hc[7];
-        if (sig_flags<L>(ctx, ex, in.seq, in.n_bytes, p, flags, fwords, win_mask, cells, hc, 7,
-                         [&] { kc_flag_digest<L>(ex, in.seq, in.n_bytes, flags, fwords, p.k, p.complements != 0, acc); })) {
+        RoutePolicy pol;
+        pol.sig = true;
+        const KcRoute route = kc_set_ladder(ctx->routes, pol, in.n_bytes, *ex.arena, [&](KcRoute) {
+            return kc_kmerset_build_sig<L>(ex, in.seq, in.n_bytes, p.k, p.complements != 0, flags, cells, ctx->routes.sig, nullptr, win_mask);
+        }, [&](KcRoute) {
+            kc_flag_digest<L>(ex, in.seq, in.n_bytes, flags, fwords, p.k, p.complements != 0, acc);
+            ex.read_n(cells, hc, 7);
+            return hc[3] == 0;
+        });
+        if (route == KC_ROUTE_SIG) {
             digest[0] = hc[4];
             digest[1] = hc[5];
             digest[2] = hc[6];
             digest[3] = hc[5];
             return;
         }
-        ex.arena->release(mark);
-        ex.arena->top = top;
+        ex.arena->restore(mark);
     }
     KmerSet<L> set = kc_kmerset_build<L>(ex, in.seq, in.n_bytes, p.k, p.complements != 0, p.min_frequency, nullptr, true, nullptr, win_mask);
     const u64 U = set.n_kept;
@@ -698,14 +639,6 @@ void digest_only(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params 
     digest[1] = h4[1];
     digest[2] = h4[2];
     digest[3] = h4[3];
-}
-
-// kc_streaming: every pass of the first-occurrence construction tries the signature buckets first (sig_flags)
-template <int L> StreamingResult streaming_only(kc_ctx *ctx, CudaExec &ex, const u8 *seq, u64 nb, const kc_params &p) {
-    auto sig = [&](u32 *flags, size_t fwords, const u32 *win_mask, u64 *cells4, u64 *hc) {
-        return sig_flags<L>(ctx, ex, seq, nb, p, flags, fwords, win_mask, cells4, hc, 4, [] {});
-    };
-    return kc_streaming_run<L>(ex, seq, nb, p.k, p.complements != 0, p.min_frequency, ctx->fast, &ctx->fast_runs, &ctx->fast_fallbacks, sig);
 }
 
 template <int L>
@@ -745,7 +678,7 @@ void group_alloc_common(kc_ctx *ctx, int n_ranks, int rank, int k, uint64_t n_by
     KC_CUDA(cudaSetDevice(ctx->device));
     G.n = n_ranks;
     G.rank = rank;
-    G.lay = kc_grp_layout(n_bytes_cap, kc_limbs_for_k(k), n_ranks, with_seq, kc_shard_granule(k), ctx->fast);
+    G.lay = kc_grp_layout(n_bytes_cap, kc_limbs_for_k(k), n_ranks, with_seq, kc_shard_granule(k), ctx->routes.fast);
     KC_CUDA(cudaMalloc(reinterpret_cast<void **>(&G.heap), G.lay.total));
     KC_CUDA(cudaMemset(G.heap, 0, G.lay.off_flags));  // sync words, cells, counts
     KC_CUDA(cudaMalloc(reinterpret_cast<void **>(&G.cnt0), 256 * 4));
@@ -807,61 +740,33 @@ template <int L> void group_compute_rank(kc_ctx *ctx, CudaExec &ex, const DevInp
         kc_grp_wait(G, ex, G.done_seq, ws);
         G.done_pending = false;
     }
-    auto finish = [&]() {
-        G.done_seq = ++G.seq;
-        kc_grp_signal(G, ex, G.done_seq);
-        G.done_pending = true;
-    };
-    // signature buckets first (kmerset_sig.cuh): every rank takes the same decision from values it sees identically
-    const bool sig_overflowed = ctx->fast_heuristics && ctx->sig_overflow_bytes && nb >= ctx->sig_overflow_bytes / 2 && nb <= ctx->sig_overflow_bytes * 2;
-    if (p.min_frequency == 1 && !sig_overflowed) {
-        const size_t top_mark = ex.arena->top, mark = ex.arena->mark();
-        ExtFlags ext;
-        ext.flags = reinterpret_cast<const u32 *>(G.heap + G.lay.off_flags);
-        ext.cells4 = kc_grp_sig_flags<L>(G, ex, in.seq, nb, p.k, p.complements != 0, ctx->sig);
-        if (ext.cells4) {
-            run_pipeline<L>(ctx, ex, in, p, res, &ext, false, (u32) G.rank, (u32) G.n);
-            if (!ext.aborted) {
-                ++ctx->sig_runs;
-                finish();
-                return;
-            }
-            if (ext.kept & 2u) {
-                G.failed = true;
-                KC_THROW(KC_ERR_INTERNAL, "a rank of the group did not arrive (wait timed out)");
-            }
-            ++ctx->sig_fallbacks;  // a bucket overflowed on some rank: every rank sees the same status word and falls back
-            ctx->sig_overflow_bytes = nb;
-        }
-        ex.arena->release(mark);
-        ex.arena->top = top_mark;
-    }
-    const KsfGroupPlan gp = kc_ksf_group_plan(nb, G.n, KsCfg<L>::EX_TILE, ctx->fast);
-    const bool expect_duplicates = ctx->fast_heuristics && (p.min_frequency > 1 || (ctx->fast_overflow_bytes && nb >= ctx->fast_overflow_bytes / 2 && nb <= ctx->fast_overflow_bytes * 2));
-    if (gp.ok && !expect_duplicates && gp.recv_items() <= G.lay.recv_items) {
-        const size_t top_mark = ex.arena->top, mark = ex.arena->mark();
-        ExtFlags ext;
-        ext.flags = reinterpret_cast<const u32 *>(G.heap + G.lay.off_flags);
-        ext.cells4 = kc_grp_fast_flags<L>(G, ex, in.seq, nb, p.k, p.complements != 0, p.min_frequency, gp, ctx->fast);
+    // every rank takes the same decisions from values it sees identically: a rung that overflowed on one rank sets the status
+    // word every rank reads
+    RoutePolicy pol = ctx->routes.compute_policy(p, nb);
+    const KsfGroupPlan gp = kc_ksf_group_plan(nb, G.n, KsCfg<L>::EX_TILE, ctx->routes.fast);
+    pol.fast = pol.fast && gp.ok && gp.recv_items() <= G.lay.recv_items;
+    ExtFlags ext;
+    ext.flags = reinterpret_cast<const u32 *>(G.heap + G.lay.off_flags);
+    const KcRoute route = kc_set_ladder(ctx->routes, pol, nb, *ex.arena, [&](KcRoute r) {
+        ext.cells4 = r == KC_ROUTE_SIG ? kc_grp_sig_flags<L>(G, ex, in.seq, nb, p.k, p.complements != 0, ctx->routes.sig)
+                                       : kc_grp_fast_flags<L>(G, ex, in.seq, nb, p.k, p.complements != 0, p.min_frequency, gp, ctx->routes.fast);
+        return ext.cells4 != nullptr;
+    }, [&](KcRoute) {
         run_pipeline<L>(ctx, ex, in, p, res, &ext, false, (u32) G.rank, (u32) G.n);
-        if (!ext.aborted) {
-            ++ctx->fast_runs;
-            finish();
-            return;
-        }
-        if (ext.kept & 2u) {
+        if (ext.aborted && (ext.kept & 2u)) {
             G.failed = true;
             KC_THROW(KC_ERR_INTERNAL, "a rank of the group did not arrive (wait timed out)");
         }
-        ++ctx->fast_fallbacks;  // a slot overflowed on some rank: every rank sees the same status word and falls back
-        ctx->fast_overflow_bytes = nb;
-        ex.arena->release(mark);
-        ex.arena->top = top_mark;
+        return !ext.aborted;
+    });
+    if (route == KC_ROUTE_NONE) {
+        ExtFlags exact;
+        exact.flags = kc_grp_exact_flags<L>(G, ex, in.seq, nb, p.k, p.complements != 0, p.min_frequency, &exact.kept, &exact.n_occ);
+        run_pipeline<L>(ctx, ex, in, p, res, &exact, false, (u32) G.rank, (u32) G.n);
     }
-    ExtFlags ext;
-    ext.flags = kc_grp_exact_flags<L>(G, ex, in.seq, nb, p.k, p.complements != 0, p.min_frequency, &ext.kept, &ext.n_occ);
-    run_pipeline<L>(ctx, ex, in, p, res, &ext, false, (u32) G.rank, (u32) G.n);
-    finish();
+    G.done_seq = ++G.seq;
+    kc_grp_signal(G, ex, G.done_seq);
+    G.done_pending = true;
 }
 
 void group_check_job(kc_ctx *ctx, const kc_params *p, u64 n_bytes) {
@@ -905,10 +810,10 @@ int kc_init(int device, void *stream, kc_ctx **out) {
         ctx->arena.stream = ctx->stream;
         for (int i = 0; i < 6; ++i) KC_CUDA(cudaEventCreate(&ctx->ev[i]));
         KC_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&ctx->pin_small), kc_ctx::KC_PIN_SMALL, cudaHostAllocDefault));
-        if (const char *e = std::getenv("KC_FAST_SET")) ctx->fast.enabled = std::atoi(e) != 0;
-        if (const char *e = std::getenv("KC_SIG_SET")) ctx->sig.enabled = std::atoi(e) != 0;
-        if (const char *e = std::getenv("KC_FAST_MAX_CTAS")) ctx->fast.max_ctas = std::atoi(e);
-        if (const char *e = std::getenv("KC_FAST_TMA")) ctx->fast.tma = std::atoi(e) != 0;
+        if (const char *e = std::getenv("KC_FAST_SET")) ctx->routes.fast.enabled = std::atoi(e) != 0;
+        if (const char *e = std::getenv("KC_SIG_SET")) ctx->routes.sig.enabled = std::atoi(e) != 0;
+        if (const char *e = std::getenv("KC_FAST_MAX_CTAS")) ctx->routes.fast.max_ctas = std::atoi(e);
+        if (const char *e = std::getenv("KC_FAST_TMA")) ctx->routes.fast.tma = std::atoi(e) != 0;
         if (const char *e = std::getenv("KC_SMALL_THREADS")) ctx->small_threads = std::atoi(e);
     } catch (const KcError &e) {
         int code = e.code;
@@ -952,9 +857,9 @@ int kc_compute_device(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_ou
     DevInput di{in->seq, in->n_bytes, in->rec_off, in->rec_len, in->n_recs};
     DevResult res;
     KC_TRACE_POINT("compute_device: start");
-    const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->sig);
-    run_with_arena(ctx, estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, p->assume_simplitigs != 0, false, &ctx->fast, &sig),
-                   estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, p->assume_simplitigs != 0, true, &ctx->fast, &sig),
+    const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->routes.sig);
+    run_with_arena(ctx, estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, p->assume_simplitigs != 0, false, &ctx->routes.fast, &sig),
+                   estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, p->assume_simplitigs != 0, true, &ctx->routes.fast, &sig),
                    [&] { dispatch_pipeline(ctx, ex, di, *p, res); });
     KC_TRACE_POINT("compute_device: launched");
     KC_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -987,9 +892,9 @@ int kc_compute(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_output *o
     ex.pinned = ctx->pin_small;
     ex.pinned_cap = ctx->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
     DevResult res;
-    const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->sig);
-    run_with_arena(ctx, estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, false, &ctx->fast, &sig),
-                   estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, true, &ctx->fast, &sig), [&] {
+    const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->routes.sig);
+    run_with_arena(ctx, estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, false, &ctx->routes.fast, &sig),
+                   estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, true, &ctx->routes.fast, &sig), [&] {
         // host -> device.  Large from-FASTA inputs go in chunks on the copy stream: the level-0 partition pass of chunk c starts
         // as soon as chunk c has landed (InputChunks), instead of after the whole copy.  The 64 bytes past n_bytes are never written:
         // every loader of the from-FASTA path is bounded by n_bytes (kc_compute_device gets a caller's buffer without them).
@@ -1074,9 +979,9 @@ int kc_lower_bound(kc_ctx *ctx, const kc_params *p, const kc_input *in, uint64_t
     ex.pinned = ctx->pin_small;
     ex.pinned_cap = ctx->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
     DevResult res;
-    const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->sig);
-    run_with_arena(ctx, estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, false, &ctx->fast, &sig),
-                   estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, true, &ctx->fast, &sig), [&] {
+    const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->routes.sig);
+    run_with_arena(ctx, estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, false, &ctx->routes.fast, &sig),
+                   estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, true, &ctx->routes.fast, &sig), [&] {
         u8 *d_seq = ex.alloc<u8>(in->n_bytes + 64);
         KC_CUDA(cudaMemcpyAsync(d_seq, in->seq, in->n_bytes, cudaMemcpyHostToDevice, ctx->stream));
         u64 *d_off = nullptr, *d_len = nullptr;
@@ -1133,8 +1038,8 @@ int kc_streaming(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_output 
     }
     KC_CUDA(cudaSetDevice(ctx->device));
     const int limbs = kc_limbs_for_k(p->k);
-    const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->sig);
-    ensure_arena(ctx, estimate_arena(in->n_bytes, 0, limbs, false, true, false, &ctx->fast, &sig));
+    const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->routes.sig);
+    ensure_arena(ctx, estimate_arena(in->n_bytes, 0, limbs, false, true, false, &ctx->routes.fast, &sig));
     ctx->arena.reset();
     CudaExec ex{ctx->stream, &ctx->arena};
     ex.prof = &ctx->prof;
@@ -1148,9 +1053,9 @@ int kc_streaming(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_output 
     KC_CUDA(cudaMemcpyAsync(d_seq, in->seq, in->n_bytes, cudaMemcpyHostToDevice, ctx->stream));
     KC_CUDA(cudaEventRecord(ctx->ev[1], ctx->stream));
     StreamingResult r;
-    if (limbs == 1) r = streaming_only<1>(ctx, ex, d_seq, in->n_bytes, *p);
-    else if (limbs == 2) r = streaming_only<2>(ctx, ex, d_seq, in->n_bytes, *p);
-    else r = streaming_only<4>(ctx, ex, d_seq, in->n_bytes, *p);
+    if (limbs == 1) r = kc_streaming_run<1>(ex, d_seq, in->n_bytes, p->k, p->complements != 0, p->min_frequency, ctx->routes);
+    else if (limbs == 2) r = kc_streaming_run<2>(ex, d_seq, in->n_bytes, p->k, p->complements != 0, p->min_frequency, ctx->routes);
+    else r = kc_streaming_run<4>(ex, d_seq, in->n_bytes, p->k, p->complements != 0, p->min_frequency, ctx->routes);
     for (int i = 2; i <= 4; ++i) KC_CUDA(cudaEventRecord(ctx->ev[i], ctx->stream));
     out->ms = copy_result_to_pinned(ctx, r.ms, r.length);
     out->length = r.length;
@@ -1286,7 +1191,8 @@ int kc_kmer_digest(kc_ctx *ctx, const kc_params *p, const kc_input *in, int mask
     const int limbs = kc_limbs_for_k(p->k);
     // the sorted-keys route, or at 2^32 bytes and more the signature construction alone: sequence, flags, window mask, its buffers
     size_t need = (size_t) ((double) nb * (1.0 + 2.0 * 8 * limbs + 4.0 + 0.2) * 1.15) + (256u << 20);
-    if (nb >= KC_POS32_BYTES) need = (size_t) (((double) nb * 1.25 + (double) kc_sig_arena_bytes(kc_sig_plan(nb, p->k, ctx->sig), nb)) * 1.05) + (256u << 20);
+    if (nb >= KC_POS32_BYTES)
+        need = (size_t) (((double) nb * 1.25 + (double) kc_sig_arena_bytes(kc_sig_plan(nb, p->k, ctx->routes.sig), nb)) * 1.05) + (256u << 20);
     ensure_arena(ctx, need);
     ctx->arena.reset();
     CudaExec ex{ctx->stream, &ctx->arena};
@@ -1545,9 +1451,9 @@ int kc_group_compute(kc_group *g, const kc_params *p, const kc_input *in, kc_out
             group_release_heaps(g);
             const u64 cap = std::min<u64>(0xFFFFFFE0ULL, in->n_bytes + in->n_bytes / 16 + (1u << 20));
             for (int r = 0; r < g->n; ++r) {
-                g->ctx[r]->fast = c0->fast;  // one plan for the whole group
-                g->ctx[r]->fast_heuristics = c0->fast_heuristics;
-                g->ctx[r]->fast_overflow_bytes = c0->fast_overflow_bytes;
+                g->ctx[r]->routes.fast = c0->routes.fast;  // one plan for the whole group
+                g->ctx[r]->routes.heuristics = c0->routes.heuristics;
+                g->ctx[r]->routes.fast_rung.overflow = c0->routes.fast_rung.overflow;
                 group_alloc_common(g->ctx[r], g->n, r, limbs == 1 ? 31 : (limbs == 2 ? 63 : 127), cap, true);
             }
             for (int r = 0; r < g->n; ++r) {
@@ -1699,10 +1605,10 @@ uint64_t kc_total_launches(const kc_ctx *ctx) { return ctx ? ctx->total_launches
 
 int kc_get_stat(const kc_ctx *ctx, const char *name, uint64_t *value) {
     if (!ctx || !name || !value) return KC_ERR_ARG;
-    if (std::strcmp(name, "fast_runs") == 0) *value = ctx->fast_runs;
-    else if (std::strcmp(name, "fast_fallbacks") == 0) *value = ctx->fast_fallbacks;
-    else if (std::strcmp(name, "sig_runs") == 0) *value = ctx->sig_runs;
-    else if (std::strcmp(name, "sig_fallbacks") == 0) *value = ctx->sig_fallbacks;
+    if (std::strcmp(name, "fast_runs") == 0) *value = ctx->routes.fast_rung.runs;
+    else if (std::strcmp(name, "fast_fallbacks") == 0) *value = ctx->routes.fast_rung.fallbacks;
+    else if (std::strcmp(name, "sig_runs") == 0) *value = ctx->routes.sig_rung.runs;
+    else if (std::strcmp(name, "sig_fallbacks") == 0) *value = ctx->routes.sig_rung.fallbacks;
     else if (std::strcmp(name, "total_launches") == 0) *value = ctx->total_launches;
     else if (std::strcmp(name, "read_backs") == 0) *value = ctx->read_backs;
     else if (std::strcmp(name, "tail_spec_runs") == 0) *value = ctx->tail_spec_runs;
@@ -1710,7 +1616,7 @@ int kc_get_stat(const kc_ctx *ctx, const char *name, uint64_t *value) {
     else if (std::strcmp(name, "arena_bytes") == 0) *value = ctx->arena.cap;
     else if (std::strcmp(name, "arena_high") == 0) *value = ctx->arena.high;
     else if (std::strcmp(name, "arena_retries") == 0) *value = ctx->arena_retries;
-    else if (std::strcmp(name, "fast_max_ctas") == 0) *value = (uint64_t) ctx->fast.max_ctas;
+    else if (std::strcmp(name, "fast_max_ctas") == 0) *value = (uint64_t) ctx->routes.fast.max_ctas;
     else if (std::strcmp(name, "path_levels") == 0) *value = ctx->path_stats.levels_run;
     else if (std::strcmp(name, "path_ban_rounds") == 0) *value = ctx->path_stats.ban_rounds;
     else if (std::strcmp(name, "path_bans") == 0) *value = ctx->path_stats.bans;
@@ -1734,53 +1640,51 @@ int kc_set_option(kc_ctx *ctx, const char *name, int value) {
     }
     if (std::strcmp(name, "tail_spec") == 0 && (value == 0 || value == 1)) {
         ctx->tail_spec = value != 0;
-        ctx->spec_fail_bytes = 0;
+        ctx->routes.tail = SizeMemo();
         return KC_OK;
     }
     // histogram-free set construction (kmerset_fast.cuh); the last three exist so that tests can reach the multi-level
     // plan and the overflow fallback with small inputs
     if (std::strcmp(name, "fast_set") == 0) {
-        ctx->fast.enabled = value != 0;
+        ctx->routes.fast.enabled = value != 0;
         return KC_OK;
     }
     if (std::strcmp(name, "fast_leaf_target") == 0 && value >= 1 && value <= 1024) {
-        ctx->fast.leaf_target = (u32) value;
+        ctx->routes.fast.leaf_target = (u32) value;
         return KC_OK;
     }
     if (std::strcmp(name, "fast_sigmas") == 0 && value >= 0) {
-        ctx->fast.sigmas = (double) value;
+        ctx->routes.fast.sigmas = (double) value;
         return KC_OK;
     }
     if (std::strcmp(name, "fast_tma") == 0 && (value == 0 || value == 1)) {
-        ctx->fast.tma = value != 0;
+        ctx->routes.fast.tma = value != 0;
         return KC_OK;
     }
     if (std::strcmp(name, "fast_heuristics") == 0 && (value == 0 || value == 1)) {
-        ctx->fast_heuristics = value != 0;
-        ctx->fast_overflow_bytes = 0;
-        ctx->sig_overflow_bytes = 0;
-        ctx->spec_fail_bytes = 0;
+        ctx->routes.heuristics = value != 0;
+        ctx->routes.sig_rung.overflow = ctx->routes.fast_rung.overflow = ctx->routes.tail = SizeMemo();
         return KC_OK;
     }
     if (std::strcmp(name, "fast_max_ctas") == 0 && value >= 0 && value <= (1 << 20)) {
-        ctx->fast.max_ctas = value;
+        ctx->routes.fast.max_ctas = value;
         return KC_OK;
     }
     if (std::strcmp(name, "fast_min_items") == 0 && value >= 0) {
-        ctx->fast.min_items = (u64) value;
+        ctx->routes.fast.min_items = (u64) value;
         return KC_OK;
     }
     // signature-bucket set construction (kmerset_sig.cuh)
     if (std::strcmp(name, "sig_set") == 0) {
-        ctx->sig.enabled = value != 0;
+        ctx->routes.sig.enabled = value != 0;
         return KC_OK;
     }
     if (std::strcmp(name, "sig_load_pct") == 0 && value >= 0 && value <= 400) {  // > 100 forces overflows (tests)
-        ctx->sig.load_pct = (u32) value;  // 0 = planned from the input size
+        ctx->routes.sig.load_pct = (u32) value;  // 0 = planned from the input size
         return KC_OK;
     }
     if (std::strcmp(name, "sig_min_items") == 0 && value >= 0) {
-        ctx->sig.min_items = (u64) value;
+        ctx->routes.sig.min_items = (u64) value;
         return KC_OK;
     }
     // device arena (tests): fill every block it hands out with this byte (-1 = off), and scale the first estimate of a call (in

@@ -2,7 +2,7 @@
 // src/khash_utils.h:143-159) as a fused  decode -> canonical k-mer -> radix partition -> shared-memory resolve.
 //
 // Items are kept as structure-of-arrays: the k-mer word (KWord<L>, 8L bytes) and, when the caller needs to know
-// WHERE a k-mer first occurs (the from-FASTA regime, see kcgpu.cu run_stage1_runs), a 32-bit payload = END position
+// WHERE a k-mer first occurs (the from-FASTA regime, see set_routes.cuh), a 32-bit payload = END position
 // of the window in the framed sequence.  Nothing else is ever materialised:
 //
 //   level 0   kc_ks_hist0_kernel      sequence bytes -> k-mers in registers -> 256-bin histogram of the top key bits

@@ -16,8 +16,7 @@
 #include "emit.cuh"
 #include "kmerset_fast.cuh"
 #include "runs.cuh"
-
-#include <functional>
+#include "set_routes.cuh"
 
 #ifdef __CUDACC__
 
@@ -126,14 +125,10 @@ struct StreamingResult {
     u64 length = 0, n_kept = 0, n_occ = 0;
 };
 
-// seq: the framed records, resident in a buffer padded with '\n' up to a multiple of 32 bytes (+ 32).
-// sig(flags, fwords, win_mask, cells4, hc): the signature-bucket construction of the flags (kcgpu.cu sig_flags), tried first in every
-// pass; true = the flags stand and hc holds cells4, false = it did not apply or overflowed (flags and cells4 are zeroed again).  An input
-// of 2^32 bytes or more has no other construction: there sig fails the call instead of returning false.
-typedef std::function<bool(u32 *, size_t, const u32 *, u64 *, u64 *)> KcSigFlags;
+// seq: the framed records, resident in a buffer padded with '\n' up to a multiple of 32 bytes (+ 32).  The constructions each pass
+// tries are those of kc_set_ladder (set_routes.cuh).
 template <int L>
-StreamingResult kc_streaming_run(CudaExec &ex, const u8 *seq, u64 n_bytes, int k, bool complements, int min_freq, const KsfTuning &fast,
-                                 u64 *fast_runs, u64 *fast_fallbacks, const KcSigFlags &sig) {
+StreamingResult kc_streaming_run(CudaExec &ex, const u8 *seq, u64 n_bytes, int k, bool complements, int min_freq, SetRoutes &routes) {
     StreamingResult res;
     const size_t fwords = kc_runs_flag_words(n_bytes);
     u32 *flags = ex.arena->alloc_top<u32>(fwords);
@@ -141,26 +136,26 @@ StreamingResult kc_streaming_run(CudaExec &ex, const u8 *seq, u64 n_bytes, int k
     u64 *cells4 = ex.arena->alloc_top<u64>(4);  // {kept, -, M, overflow status}
     ex.fill_bytes(cells4, 0, 32);
     u64 hc[4] = {0, 0, 0, 0};
-    bool done = sig(flags, fwords, nullptr, cells4, hc);
-    const bool sig_ok = done;  // what did not apply or overflowed (a read set) is not tried again in the passes of -z
-    if (done) {
+    const u32 *win_mask = nullptr;
+    auto launch = [&](KcRoute r) {
+        return r == KC_ROUTE_SIG ? kc_kmerset_build_sig<L>(ex, seq, n_bytes, k, complements, flags, cells4, routes.sig, nullptr, win_mask)
+                                 : kc_kmerset_build_fast<L>(ex, seq, n_bytes, k, complements, 1, flags, cells4, routes.fast);
+    };
+    auto consume = [&](KcRoute) {
+        ex.read_n(cells4, hc, 4);
+        if (hc[3] == 0) return true;
+        ex.fill_bytes(flags, 0, fwords * 4);
+        ex.fill_bytes(cells4, 0, 32);
+        return false;
+    };
+    RoutePolicy pol;
+    pol.sig = true;
+    pol.fast = min_freq == 1;
+    const KcRoute route = kc_set_ladder(routes, pol, n_bytes, *ex.arena, launch, consume);
+    if (route != KC_ROUTE_NONE) {
         res.n_kept = hc[2] ? hc[0] : 0;
         res.n_occ = hc[2];
-    }
-    if (!done && min_freq == 1 && kc_kmerset_build_fast<L>(ex, seq, n_bytes, k, complements, 1, flags, cells4, fast)) {  // -z > 1: a read set, see run_stage1_runs
-        ex.read_n(cells4, hc, 4);
-        if (hc[3] == 0) {
-            done = true;
-            ++*fast_runs;
-            res.n_kept = hc[2] ? hc[0] : 0;
-            res.n_occ = hc[2];
-        } else {
-            ++*fast_fallbacks;
-            ex.fill_bytes(flags, 0, fwords * 4);
-            ex.fill_bytes(cells4, 0, 32);
-        }
-    }
-    if (!done) {
+    } else {
         KmerSet<L> set = kc_kmerset_build<L>(ex, seq, n_bytes, k, complements, 1, flags, false, cells4);
         res.n_occ = set.n_occ;
         res.n_kept = set.n_occ ? ex.read(cells4) : 0;
@@ -173,6 +168,9 @@ StreamingResult kc_streaming_run(CudaExec &ex, const u8 *seq, u64 n_bytes, int k
         const u64 mwords = kc_div_up(n_bytes, (u64) 256 * KC_EX_STRIP) * 256 + 1;
         u32 *avail = ex.arena->alloc_top<u32>(mwords);
         ex.fill_bytes(avail, 0xFF, mwords * 4);
+        win_mask = avail;
+        pol.sig = route == KC_ROUTE_SIG;
+        pol.fast = false;
         for (int t = 2; t <= min_freq && res.n_kept; ++t) {
             const u32 *f = flags;
             const u64 fw = fwords;
@@ -181,7 +179,7 @@ StreamingResult kc_streaming_run(CudaExec &ex, const u8 *seq, u64 n_bytes, int k
             }, KP_MISC, mwords * 12);
             ex.fill_bytes(flags, 0, fwords * 4);
             ex.fill_bytes(cells4, 0, 32);
-            if (sig_ok && sig(flags, fwords, avail, cells4, hc)) {
+            if (kc_set_ladder(routes, pol, n_bytes, *ex.arena, launch, consume) == KC_ROUTE_SIG) {
                 res.n_kept = hc[2] ? hc[0] : 0;
                 continue;
             }

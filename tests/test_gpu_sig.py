@@ -136,6 +136,32 @@ def test_sig_overflow_falls_back(ctx):
         _restore(ctx)
 
 
+@pytest.mark.parametrize("call", ["digest", "streaming"])
+def test_sig_overflow_memory_is_compute_only(ctx, call):
+    """Only compute remembers a signature overflow: a digest or streaming call that overflows leaves the next compute on the same
+    input trying the buckets, and a remembered compute overflow does not stop the next digest or streaming call from trying them."""
+    recs = synth.random_genome_records(4, 60_000, 99)
+    seq, off, ln = synth.frame_records(recs)
+    other = {"digest": lambda: ctx.kmer_digest(seq, k=31), "streaming": lambda: ctx.streaming(seq, k=31)}[call]
+    try:
+        _options(ctx, sig_min_items=0, sig_load_pct=400, fast_heuristics=1)  # every bucket overflows; the memories start clear
+        want = ctx.compute(seq, k=31)
+        ctx.set_option("fast_heuristics", 1)
+        fb0 = ctx.stat("sig_fallbacks")
+        other()
+        assert ctx.stat("sig_fallbacks") == fb0 + 1
+        got = ctx.compute(seq, k=31)                 # tries the buckets: the overflow above was not remembered
+        assert ctx.stat("sig_fallbacks") == fb0 + 2 and got.ms == want.ms
+        got = ctx.compute(seq, k=31)                 # this overflow was: the buckets are skipped
+        assert ctx.stat("sig_fallbacks") == fb0 + 2 and got.ms == want.ms
+        other()                                      # ... but not by a digest or streaming call
+        assert ctx.stat("sig_fallbacks") == fb0 + 3
+        got = ctx.compute(seq, k=31)                 # which leaves the memory of compute as it was
+        assert ctx.stat("sig_fallbacks") == fb0 + 3 and got.ms == want.ms
+    finally:
+        _restore(ctx)
+
+
 @pytest.mark.parametrize("coverage", [2.0, 30.0])
 def test_sig_reads_with_coverage(ctx, coverage):
     """Reads: every run of windows comes `coverage` times, so the bucket sizes spread by sqrt(coverage): 2x still fits, 30x overflows
