@@ -258,6 +258,17 @@ int kc_set_option(kc_ctx *ctx, const char *name, int value);
  * of a level after a cycle was found), "path_bans" (refused edges; with complements each one counts for both strands). */
 int kc_get_stat(const kc_ctx *ctx, const char *name, uint64_t *value);
 
+/* ---- test hooks: not part of the compute path; they expose internals so that tests can hold them to a plain reference -------
+ *
+ * kc_debug_sort  the radix sort of the overlap levels and the sparse switch (kmercamel_b200/csrc/sort.cuh kc_sort<limbs>) on
+ *                n words of `limbs` little-endian uint64 limbs (host buffers): out = the words in ascending order of their low
+ *                key_bits bits.  limbs must be 1, 2, 3 or 5 (the widths the library sorts), 0 <= key_bits <= 64 limbs, and no
+ *                word may have a bit set at or above key_bits; otherwise KC_ERR_ARG.  stats (may be NULL) receives
+ *                {radix levels run, most buckets partitioned in one level, buckets sorted by the shared-memory kernel, buckets
+ *                that ran out of key bits, shared-memory buckets with more than 64 sub-buckets of more than 24 items (sorted whole
+ *                by the bitonic network; counted on the host with the kernel's rule)}. */
+int kc_debug_sort(kc_ctx *ctx, const uint64_t *words, uint64_t n, int limbs, int key_bits, uint64_t *out, uint64_t *stats);
+
 int kc_limbs_for_k(int k);
 void kc_free(void *p);
 const char *kc_strerror(int code);

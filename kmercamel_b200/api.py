@@ -81,6 +81,7 @@ def load_library():
     L.kc_count_kmers.argtypes = [C.c_void_p, C.POINTER(kc_params), C.POINTER(kc_input), C.POINTER(u64p), C.POINTER(u8p),
                                  u64p]
     L.kc_partial_presort.argtypes = [C.c_void_p, u64p, C.c_uint64, C.c_int, u64p]
+    L.kc_debug_sort.argtypes = [C.c_void_p, u64p, C.c_uint64, C.c_int, C.c_int, u64p, u64p]
     L.kc_kmer_digest.argtypes = [C.c_void_p, C.POINTER(kc_params), C.POINTER(kc_input), C.c_int, u64p]
     L.kc_overlap_path.argtypes = [C.c_void_p, u64p, u64p, C.c_uint64, C.c_int, C.c_int, C.c_int, C.c_int, i64p, u8p]
     L.kc_frame_fasta.argtypes = [C.c_char_p, C.c_uint64, C.POINTER(u8p), u64p, C.POINTER(u64p), C.POINTER(u64p), u64p]
@@ -120,7 +121,7 @@ def load_library():
     return L
 
 
-EXPORTED_SYMBOLS = ["kc_kmer_digest", "kc_partial_presort", "kc_init", "kc_destroy", "kc_compute", "kc_compute_device", "kc_lower_bound",
+EXPORTED_SYMBOLS = ["kc_kmer_digest", "kc_partial_presort", "kc_debug_sort", "kc_init", "kc_destroy", "kc_compute", "kc_compute_device", "kc_lower_bound",
                     "kc_copy_to_host", "kc_count_kmers", "kc_overlap_path", "kc_total_launches", "kc_shard_granule",
                     "kc_init_multi", "kc_group_destroy", "kc_group_size", "kc_group_ctx", "kc_group_compute", "kc_group_last_error",
                     "kc_group_alloc", "kc_group_open", "kc_group_compute_device", "kc_group_close", "kc_group_plan",
@@ -363,6 +364,18 @@ class Context:
         out = np.zeros_like(kmers)
         self._check(self._lib.kc_partial_presort(self._h, kmers.ctypes.data_as(u64p), kmers.shape[0], int(k), out.ctypes.data_as(u64p)))
         return out
+
+    def debug_sort(self, words, key_bits: int):
+        """Test hook kc_debug_sort: the radix sort of sort.cuh on words [n, limbs] u64 (limbs 1, 2, 3 or 5), ascending on their
+        low key_bits bits -> (sorted copy, stats).  stats: levels (radix levels run), max_big (most buckets partitioned in one
+        level), small (buckets sorted in shared memory), uniform (buckets that ran out of key bits), whole_bitonic (shared-memory
+        buckets sorted whole by the bitonic network)."""
+        words = np.ascontiguousarray(words, dtype=np.uint64)
+        out = np.zeros_like(words)
+        st = np.zeros(5, dtype=np.uint64)
+        self._check(self._lib.kc_debug_sort(self._h, words.ctypes.data_as(u64p), words.shape[0], words.shape[1], int(key_bits),
+                                            out.ctypes.data_as(u64p), st.ctypes.data_as(u64p)))
+        return out, dict(zip(("levels", "max_big", "small", "uniform", "whole_bitonic"), (int(x) for x in st)))
 
     def kmer_digest(self, seq, *, k, complements=True, min_frequency=1, masked=False):
         """Stage 1 as an order-independent digest [n, sum h, xor h, sum h * min(occurrences, 256)] (kc_kmer_digest).

@@ -1174,6 +1174,72 @@ int kc_partial_presort(kc_ctx *ctx, const uint64_t *kmers, uint64_t n, int k, ui
     KC_API_END(ctx)
 }
 
+int kc_debug_sort(kc_ctx *ctx, const uint64_t *words, uint64_t n, int limbs, int key_bits, uint64_t *out, uint64_t *stats) {
+    if (!ctx || (n && (!words || !out))) return KC_ERR_ARG;
+    KC_API_BEGIN
+    if (limbs != 1 && limbs != 2 && limbs != 3 && limbs != 5) KC_THROW(KC_ERR_ARG, "limbs must be 1, 2, 3 or 5");
+    if (key_bits < 0 || key_bits > 64 * limbs) KC_THROW(KC_ERR_ARG, "key_bits must be in 0..64 limbs");
+    for (u64 i = 0; i < n; ++i)
+        for (int j = 0; j < limbs; ++j) {
+            const int rem = key_bits - 64 * j;
+            const u64 high = rem >= 64 ? 0 : (rem <= 0 ? ~0ULL : ~0ULL << rem);
+            if (words[i * limbs + j] & high) KC_THROW(KC_ERR_ARG, "a word has a bit set at or above key_bits");
+        }
+    KC_CUDA(cudaSetDevice(ctx->device));
+    ensure_arena(ctx, (size_t) n * (16 * limbs + 8) + (64u << 20));
+    ctx->arena.reset();
+    CudaExec ex{ctx->stream, &ctx->arena};
+    ex.prof = &ctx->prof;
+    ex.pinned = ctx->pin_small;
+    ex.pinned_cap = ctx->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
+    u64 *a = ex.alloc<u64>(n * limbs), *b = ex.alloc<u64>(n * limbs);
+    if (n) KC_CUDA(cudaMemcpyAsync(a, words, n * limbs * 8, cudaMemcpyHostToDevice, ctx->stream));
+    KcSortStats st;
+    switch (limbs) {
+    case 1: kc_sort_impl<1, KC_SORT_ONLY>(ex, (KWord<1> *) a, (KWord<1> *) b, n, key_bits, 0, nullptr, &st); break;
+    case 2: kc_sort_impl<2, KC_SORT_ONLY>(ex, (KWord<2> *) a, (KWord<2> *) b, n, key_bits, 0, nullptr, &st); break;
+    case 3: kc_sort_impl<3, KC_SORT_ONLY>(ex, (KWord<3> *) a, (KWord<3> *) b, n, key_bits, 0, nullptr, &st); break;
+    default: kc_sort_impl<5, KC_SORT_ONLY>(ex, (KWord<5> *) a, (KWord<5> *) b, n, key_bits, 0, nullptr, &st); break;
+    }
+    if (n) KC_CUDA(cudaMemcpyAsync(out, a, n * limbs * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    KC_CUDA(cudaStreamSynchronize(ctx->stream));
+    ctx->total_launches += ex.launches;
+    ctx->read_backs += ex.read_backs;
+    if (stats) {
+        // the local kernel's path, from its rule (kc_sort_local_kernel): digit width about two sub-buckets per item, and a
+        // bucket with more than 64 sub-buckets of more than KC_SUB_SMALL items is sorted whole; a digit count does not depend
+        // on the order of the items, so the sorted words give the same counts
+        u64 whole = 0;
+        std::vector<u32> cnt(1u << KC_SUB_BITS_MAX);
+        for (const SortBucket &d : st.small) {
+            if (d.size < 2) continue;
+            int bits = 1;
+            while ((1u << bits) < 2 * d.size && bits < KC_SUB_BITS_MAX) ++bits;
+            if (bits > (int) d.rem) bits = d.rem;
+            const int shift = d.rem - bits;
+            std::fill(cnt.begin(), cnt.begin() + (1u << bits), 0u);
+            for (u64 i = d.off; i < d.off + d.size; ++i) {
+                u32 dg = 0;
+                for (int j = bits - 1; j >= 0; --j) {
+                    const int p = shift + j;
+                    dg = dg << 1 | (u32) ((out[i * limbs + (p >> 6)] >> (p & 63)) & 1);
+                }
+                ++cnt[dg];
+            }
+            u32 over = 0;
+            for (u32 s = 0; s < (1u << bits); ++s) over += cnt[s] > KC_SUB_SMALL;
+            whole += over > 64;
+        }
+        stats[0] = st.levels;
+        stats[1] = st.max_big;
+        stats[2] = st.small.size();
+        stats[3] = st.n_uniform;
+        stats[4] = whole;
+    }
+    return KC_OK;
+    KC_API_END(ctx)
+}
+
 int kc_kmer_digest(kc_ctx *ctx, const kc_params *p, const kc_input *in, int masked, uint64_t *digest) {
     if (!ctx || !in || !digest) return KC_ERR_ARG;
     KC_API_BEGIN

@@ -410,10 +410,26 @@ __global__ void __launch_bounds__(256) kc_sort_uniform_kernel(KWord<L> *buf0, co
     }
 }
 
+// Bookkeeping of one sort, kept only when the caller passes it (the test hook kc_debug_sort; the product path passes null).
+struct KcSortStats {
+    u32 levels = 0;                  // radix levels run
+    u32 max_big = 0;                 // most buckets partitioned in one level
+    u64 n_uniform = 0;               // buckets that ran out of key bits
+    std::vector<SortBucket> small;   // every bucket handed to the local kernel
+};
+
 // Radix levels consume the bits [low_bit, key_bits) from the top; bits below low_bit only matter to the final
 // shared-memory sort (which compares whole words).
+//
+// Bound of the small-bucket list.  Small buckets collect across levels, and the local kernel sorts them.  A level
+// partitioning nb buckets adds at most sum_b 2^bits_b children, and kc_sort_prep_kernel picks 2^bits_b = 2 or
+// 2^bits_b < 2 ceil(size_b / (CAP/4)) < 8 size_b / CAP + 2, so with q = n / CAP (rounded down) and nb <= q (each
+// partitioned bucket holds more than CAP items) a level adds at most 8 (q + 1) + 2 nb <= 10 q + 8 < small_cap = 16 q + 4096.
+// Before a level that could overflow the list, the local kernel sorts the buckets collected so far (they are final and
+// disjoint from every bucket still being partitioned) and the list starts empty.
 template <int L, int MODE>
-void kc_sort_impl(CudaExec &ex, KWord<L> *buf0, KWord<L> *buf1, u64 n, int key_bits, int low_bit, u8 *cnt_tmp) {
+void kc_sort_impl(CudaExec &ex, KWord<L> *buf0, KWord<L> *buf1, u64 n, int key_bits, int low_bit, u8 *cnt_tmp,
+                  KcSortStats *stats = nullptr) {
     typedef SortCfg<L> Cfg;
     if (n == 0) return;
     if (n >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "sort of more than 2^32 items");
@@ -463,8 +479,28 @@ void kc_sort_impl(CudaExec &ex, KWord<L> *buf0, KWord<L> *buf1, u64 n, int key_b
     ++ex.launches;
     SortBucket *cur = big_a, *nxt = big_b;
     const u32 max_ctas = 148 * 8;
+    auto run_local = [&](u64 bytes) {
+        if (stats) {
+            const size_t at = stats->small.size();
+            stats->small.resize(at + n_small);
+            KC_CUDA(cudaMemcpyAsync(stats->small.data() + at, small, (size_t) n_small * sizeof(SortBucket), cudaMemcpyDeviceToHost, st));
+            KC_CUDA(cudaStreamSynchronize(st));
+        }
+        CudaExec::Scope sc(ex, KP_SORT_LOCAL, bytes);
+        kc_sort_local_kernel<L, MODE><<<n_small, 256, local_smem, st>>>(buf0, buf1, small, cnt_tmp, low_bit);
+        ++ex.launches;
+    };
     bool first_level = true;
     while (nb > 0) {
+        if (n_small + 8 * (n / cap + 1) + 2 * (u64) nb > small_cap) {  // see the bound above
+            run_local(0);
+            ex.fill_bytes(ctr + 1, 0, 4);
+            n_small = 0;
+        }
+        if (stats) {
+            ++stats->levels;
+            if (nb > stats->max_big) stats->max_big = nb;
+        }
         kc_sort_prep_kernel<<<(unsigned) kc_div_up(nb, 256), 256, 0, st>>>(cur, nb, cap, Cfg::TILE, tile_count);
         ++ex.launches;
         ex.fill_bytes(tile_count + nb, 0, 4);
@@ -508,11 +544,8 @@ void kc_sort_impl(CudaExec &ex, KWord<L> *buf0, KWord<L> *buf1, u64 n, int key_b
         cur = nxt;
         nxt = t;
     }
-    if (n_small) {
-        CudaExec::Scope sc(ex, KP_SORT_LOCAL, 2 * n * sizeof(KWord<L>));
-        kc_sort_local_kernel<L, MODE><<<n_small, 256, local_smem, st>>>(buf0, buf1, small, cnt_tmp, low_bit);
-        ++ex.launches;
-    }
+    if (n_small) run_local(2 * n * sizeof(KWord<L>));
+    if (stats) stats->n_uniform = n_uniform;
     if (n_uniform) {
         kc_sort_uniform_kernel<L, MODE><<<n_uniform, 256, 0, st>>>(buf0, buf1, uniform, cnt_tmp);
         ++ex.launches;
