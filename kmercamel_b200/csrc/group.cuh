@@ -126,6 +126,8 @@ struct KcGroup {
     size_t tile_hist_cap = 0;
     u64 tab_n_bytes = ~0ull;              // the job geometry the device tables dst_k / dst_p were built for (fast path)
     int tab_limbs = 0;
+    u32 tab_n_digits = 0;                 // ... and the plan they encode (KsfGroupPlan n_digits, cap_sub)
+    u64 tab_cap_sub = 0;
     u64 timeout_ns = 30ull * 1000000000ull;
     bool attached() const { return n > 0 && heap != nullptr; }
     GrpDev dev() const {
@@ -251,10 +253,14 @@ u64 *kc_grp_fast_flags(KcGroup &G, CudaExec &ex, const u8 *seq, u64 n_bytes, int
     const u64 body_words = kc_div_up(n_bytes, (u64) 32);
     ex.fill_bytes(flags + body_words, 0, 8);  // the padding words nobody writes (kc_runs_load reads one past the end)
     // destination tables of this rank's sub-slots: digit d -> (owner's heap, slot (d - dig_begin(owner)) * n + rank)
-    if (G.tab_n_bytes != n_bytes || G.tab_limbs != L) {  // same geometry as the previous job: the tables on the device are still right
-        KC_CUDA(cudaStreamSynchronize(ex.stream));       // the staging table may still feed an earlier copy
+    // kept from the previous job only if it had the same geometry AND the same plan: the digit count and the sub-slot stride also
+    // follow the options fast_leaf_target / fast_sigmas, and stale ones would scatter items where no owner reads them
+    if (G.tab_n_bytes != n_bytes || G.tab_limbs != L || G.tab_n_digits != gp.n_digits || G.tab_cap_sub != gp.cap_sub) {
+        KC_CUDA(cudaStreamSynchronize(ex.stream));  // the staging table may still feed an earlier copy
         G.tab_n_bytes = n_bytes;
         G.tab_limbs = L;
+        G.tab_n_digits = gp.n_digits;
+        G.tab_cap_sub = gp.cap_sub;
         for (u32 d = 0; d < 256; ++d) {
             char *kp = nullptr, *pp = nullptr;
             if (d < gp.n_digits) {
