@@ -38,17 +38,6 @@ KC_HD u8 kc_letter(u32 sym, bool upper) {
     return upper ? c : (u8) (c + ('a' - 'A'));  // src/kmers.h:124-127 Masked
 }
 
-// first index in [0, n) with keys[i] >= x
-template <int L> KC_HD u64 kmer_lower_bound(const KWord<L> *keys, u64 n, const KWord<L> &x) {
-    u64 lo = 0, hi = n;
-    while (lo < hi) {
-        u64 mid = (lo + hi) >> 1;
-        if (keys[mid] < x) lo = mid + 1;
-        else hi = mid;
-    }
-    return lo;
-}
-
 // Bucket index over the top `bits` bits of the 2k-bit k-mers of a SORTED set: start[b] = first position whose k-mer has a
 // top-bits value >= b (start[2^bits] = n).  Cuts the ~log2(n) dependent DRAM probes of a binary search down to the index
 // read plus a search inside one bucket (about two keys when 2^bits ~ n / 2).

@@ -813,7 +813,6 @@ int kc_init(int device, void *stream, kc_ctx **out) {
         if (const char *e = std::getenv("KC_FAST_SET")) ctx->routes.fast.enabled = std::atoi(e) != 0;
         if (const char *e = std::getenv("KC_SIG_SET")) ctx->routes.sig.enabled = std::atoi(e) != 0;
         if (const char *e = std::getenv("KC_FAST_MAX_CTAS")) ctx->routes.fast.max_ctas = std::atoi(e);
-        if (const char *e = std::getenv("KC_FAST_TMA")) ctx->routes.fast.tma = std::atoi(e) != 0;
         if (const char *e = std::getenv("KC_SMALL_THREADS")) ctx->small_threads = std::atoi(e);
     } catch (const KcError &e) {
         int code = e.code;
@@ -1196,10 +1195,10 @@ int kc_debug_sort(kc_ctx *ctx, const uint64_t *words, uint64_t n, int limbs, int
     if (n) KC_CUDA(cudaMemcpyAsync(a, words, n * limbs * 8, cudaMemcpyHostToDevice, ctx->stream));
     KcSortStats st;
     switch (limbs) {
-    case 1: kc_sort_impl<1, KC_SORT_ONLY>(ex, (KWord<1> *) a, (KWord<1> *) b, n, key_bits, 0, nullptr, &st); break;
-    case 2: kc_sort_impl<2, KC_SORT_ONLY>(ex, (KWord<2> *) a, (KWord<2> *) b, n, key_bits, 0, nullptr, &st); break;
-    case 3: kc_sort_impl<3, KC_SORT_ONLY>(ex, (KWord<3> *) a, (KWord<3> *) b, n, key_bits, 0, nullptr, &st); break;
-    default: kc_sort_impl<5, KC_SORT_ONLY>(ex, (KWord<5> *) a, (KWord<5> *) b, n, key_bits, 0, nullptr, &st); break;
+    case 1: kc_sort<1>(ex, (KWord<1> *) a, (KWord<1> *) b, n, key_bits, &st); break;
+    case 2: kc_sort<2>(ex, (KWord<2> *) a, (KWord<2> *) b, n, key_bits, &st); break;
+    case 3: kc_sort<3>(ex, (KWord<3> *) a, (KWord<3> *) b, n, key_bits, &st); break;
+    default: kc_sort<5>(ex, (KWord<5> *) a, (KWord<5> *) b, n, key_bits, &st); break;
     }
     if (n) KC_CUDA(cudaMemcpyAsync(out, a, n * limbs * 8, cudaMemcpyDeviceToHost, ctx->stream));
     KC_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -1721,10 +1720,6 @@ int kc_set_option(kc_ctx *ctx, const char *name, int value) {
     }
     if (std::strcmp(name, "fast_sigmas") == 0 && value >= 0) {
         ctx->routes.fast.sigmas = (double) value;
-        return KC_OK;
-    }
-    if (std::strcmp(name, "fast_tma") == 0 && (value == 0 || value == 1)) {
-        ctx->routes.fast.tma = value != 0;
         return KC_OK;
     }
     if (std::strcmp(name, "fast_heuristics") == 0 && (value == 0 || value == 1)) {

@@ -882,27 +882,23 @@ __global__ void __launch_bounds__(256) kc_ks_uniform_kernel(KWord<L> *k0, const 
 }
 
 // ---- host driver -----------------------------------------------------------------------------------------------------
-// Multi-GPU use (hash-range sharding, see kmercamel_b200/sharded.py): the construction is cut at the level-0 boundary.
-//   KS_PARTITION  level 0 only, over the window END positions [pos_begin, pos_end) of a sequence that is resident in
-//                 full: the scrambled keys and their GLOBAL positions land in caller buffers, ordered by level-0 digit
-//                 (= by owner rank, owner = digit * n_ranks / 256); the 256 digit counts go back to the host.
-//   KS_RESOLVE    the items are given (after the all-to-all: every occurrence of this rank's hash range) and level 0
-//                 is skipped; first-occurrence bits are set at global positions.
-enum { KS_WHOLE = 0, KS_PARTITION = 1, KS_RESOLVE = 2, KS_HIST = 3, KS_SCATTER_P2P = 4 };
+// Multi-GPU use (hash-range sharding, kc_grp_exact_flags in group.cuh): the construction is cut at the level-0 boundary.
+//   kc_kmerset_hist_only, kc_kmerset_scatter_p2p   level 0 over the window END positions [pos_begin, pos_end) of a sequence
+//                 that is resident in full: the scrambled keys and their GLOBAL positions go straight into the owners'
+//                 buffers, ordered by level-0 digit (owner rank = digit * n_ranks / 256).
+//   kc_kmerset_resolve   the items are given (after the exchange: every occurrence of this rank's hash range, in its
+//                 n_pre level-0 buckets) and level 0 is skipped; first-occurrence bits are set at global positions.
 struct KsShard {
-    int mode = KS_WHOLE;
-    u64 pos_begin = 0, pos_end = 0;  // KS_PARTITION: multiples of EX_TILE (pos_end may also be n_bytes)
-    void *keys = nullptr;            // caller buffers (device): KS_PARTITION out (capacity pos_end - pos_begin), KS_RESOLVE in/scratch
+    u64 pos_begin = 0, pos_end = 0;  // hist / scatter: multiples of EX_TILE (pos_end may also be n_bytes)
+    void *keys = nullptr;            // resolve: the items (device, caller-owned)
     u32 *pos = nullptr;
-    u64 n_items = 0;                 // KS_RESOLVE
-    u32 host_hist[256];              // KS_PARTITION / KS_HIST out
-    // fused partition + exchange (peer memory): KS_HIST = histogram pass only (tile counts stay in tile_hist_keep),
-    // KS_SCATTER_P2P = scatter pass through the peer tables, KS_RESOLVE with n_pre > 0 = the owner's level-0 buckets
-    u16 *tile_hist_keep = nullptr;   // caller-owned, (tiles of the slice) * 256 entries
-    const u64 *cursor0 = nullptr;    // KS_SCATTER_P2P: host, 256 start cursors (this rank's segment inside each bucket)
-    void *const *dst_k = nullptr;    // KS_SCATTER_P2P: device tables of 256 pointers each
+    u64 n_items = 0;
+    u32 host_hist[256];              // hist out
+    u16 *tile_hist_keep = nullptr;   // caller-owned, (tiles of the slice) * 256 entries: hist out, scatter in
+    const u64 *cursor0 = nullptr;    // scatter: host, 256 start cursors (this rank's segment inside each bucket)
+    void *const *dst_k = nullptr;    // scatter: device tables of 256 pointers each
     u32 *const *dst_p = nullptr;
-    u32 n_pre = 0;                   // KS_RESOLVE: level-0 buckets already in place
+    u32 n_pre = 0;                   // resolve: level-0 buckets already in place (>= 1)
     const u64 *pre_off = nullptr, *pre_size = nullptr;  // host arrays
 };
 
@@ -917,6 +913,7 @@ template <int L> struct KmerSet {
 //   flags != nullptr (bit array over the n_bytes positions, zeroed by the caller): bit p = 1 iff a kept k-mer occurs for the FIRST time in the
 //                     window ending at p  (positions travel as the payload);
 //   want_keys:        the kept keys (sorted) and their counts are left at the arena position current on entry.
+//   shard != nullptr: level 0 is skipped, the construction resolves the level-0 buckets the shard gives (kc_kmerset_resolve).
 // Everything else this function allocates is released before it returns.
 
 template <int L, bool PAY, bool KEYS>
@@ -924,19 +921,12 @@ KmerSet<L> kc_kmerset_build_impl(CudaExec &ex, const u8 *seq, u64 n_bytes, int k
                                  u64 *ext_kept_cell, KsShard *shard = nullptr, const u32 *win_mask = nullptr) {
     typedef KsCfg<L> Cfg;
     KmerSet<L> res;
-    const int mode = shard ? shard->mode : KS_WHOLE;
-    if (mode != KS_WHOLE && (!PAY || KEYS)) KC_THROW(KC_ERR_INTERNAL, "sharded construction is FLAGS-only");
-    const u64 pos_begin = mode == KS_PARTITION ? shard->pos_begin : 0;
-    const u64 pos_end = mode == KS_PARTITION ? shard->pos_end : n_bytes;
-    if (mode == KS_PARTITION)
-        for (int i = 0; i < 256; ++i) shard->host_hist[i] = 0;
-    if (mode == KS_RESOLVE ? shard->n_items == 0 : pos_end <= pos_begin) return res;
-    if (mode == KS_PARTITION && (pos_begin % Cfg::EX_TILE != 0 || (pos_end % Cfg::EX_TILE != 0 && pos_end != n_bytes) || pos_end > n_bytes))
-        KC_THROW(KC_ERR_ARG, "shard boundaries must be multiples of the extraction tile");
+    if (shard && (!PAY || KEYS)) KC_THROW(KC_ERR_INTERNAL, "sharded construction is FLAGS-only");
+    if (shard ? shard->n_items == 0 : n_bytes == 0) return res;
     cudaStream_t st = ex.stream;
     const size_t base_mark = ex.arena->mark();
     const u32 cap = Cfg::CAP;
-    const u64 n = mode == KS_RESOLVE ? shard->n_items : pos_end - pos_begin;  // upper bound of M
+    const u64 n = shard ? shard->n_items : n_bytes;  // upper bound of M
     const u32 big_cap = (u32) (n / cap + 258);
     const u32 small_cap = (u32) (16 * (n / cap) + 4096);
     const u32 uniform_cap = big_cap;
@@ -954,8 +944,7 @@ KmerSet<L> kc_kmerset_build_impl(CudaExec &ex, const u8 *seq, u64 n_bytes, int k
     u8 *skip = ex.alloc<u8>(big_cap);
     u32 *ctr = ex.alloc<u32>(8);
     u64 *cells = ex.alloc<u64>(2);  // [0] = M, [1] = kept distinct keys
-    const u32 ex_blocks = mode == KS_RESOLVE ? 0u : (u32) kc_div_up(pos_end - pos_begin, (u64) Cfg::EX_TILE);
-    const u32 tile0 = (u32) (pos_begin / Cfg::EX_TILE);
+    const u32 ex_blocks = shard ? 0u : (u32) kc_div_up(n_bytes, (u64) Cfg::EX_TILE);
     u16 *tile_hist = ex.alloc<u16>((u64) (ex_blocks ? ex_blocks : 1) * 256);
     ex.fill_bytes(ctr, 0, 32);
     ex.fill_bytes(cells, 0, 16);
@@ -981,11 +970,11 @@ KmerSet<L> kc_kmerset_build_impl(CudaExec &ex, const u8 *seq, u64 n_bytes, int k
     KWord<L> *k0 = nullptr, *k1 = nullptr;
     u32 *p0 = nullptr, *p1 = nullptr;
     u8 *cnt_tmp = nullptr;
-    if (mode != KS_RESOLVE) {
+    if (!shard) {
         {
-            CudaExec::Scope sc(ex, KP_KS_HIST0, pos_end - pos_begin);
+            CudaExec::Scope sc(ex, KP_KS_HIST0, n_bytes);
             kc_ks_hist0_kernel<L, SCRAMBLE><<<ex_blocks, Cfg::EX_THREADS, 0, st>>>(seq, n_bytes, k, complements ? 1 : 0, shift0, bits0, hist, tile_hist,
-                                                                                   tile0, win_mask);
+                                                                                   0u, win_mask);
         }
         ++ex.launches;
         kc_ks_scan0_kernel<<<1, 256, 0, st>>>(hist, cursor, big_a, big_cap, small, small_cap, uniform, uniform_cap, ctr, cells, cap, Cfg::TILE,
@@ -994,7 +983,6 @@ KmerSet<L> kc_kmerset_build_impl(CudaExec &ex, const u8 *seq, u64 n_bytes, int k
         KC_CUDA(cudaGetLastError());
         KC_CUDA(cudaMemcpyAsync(h, ctr, 32, cudaMemcpyDeviceToHost, st));
         KC_CUDA(cudaMemcpyAsync(&M, cells, 8, cudaMemcpyDeviceToHost, st));
-        if (mode == KS_PARTITION) KC_CUDA(cudaMemcpyAsync(shard->host_hist, hist, 256 * 4, cudaMemcpyDeviceToHost, st));
         KC_CUDA(cudaStreamSynchronize(st));
         res.n_occ = M;
         if (M == 0) {
@@ -1007,61 +995,40 @@ KmerSet<L> kc_kmerset_build_impl(CudaExec &ex, const u8 *seq, u64 n_bytes, int k
         M = shard->n_items;
         res.n_occ = M;
         if (M >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "more than 2^32 k-mer occurrences on one GPU");
-        if (shard->n_pre) {
-            // the owner's level-0 buckets, delivered complete and contiguous by the peers' scatter passes
-            std::vector<SortBucket> hs, hb, hu;
-            for (u32 i = 0; i < shard->n_pre; ++i) {
-                if (shard->pre_size[i] == 0) continue;
-                SortBucket b;
-                b.off = shard->pre_off[i];
-                b.size = (u32) shard->pre_size[i];
-                b.rem = (u16) (key_bits - bits0);
-                b.parity = 0;
-                b.bits = 0;
-                if (b.size <= cap) {
-                    hs.push_back(b);
-                    if (b.size > 1024u) ++h[5];
-                } else if (b.rem == 0) {
-                    hu.push_back(b);
-                } else {
-                    hb.push_back(b);
-                    h[4] += (u32) kc_div_up(b.size, (u64) Cfg::TILE);
-                }
+        // the owner's level-0 buckets, delivered complete and contiguous by the peers' scatter passes
+        std::vector<SortBucket> hs, hb, hu;
+        for (u32 i = 0; i < shard->n_pre; ++i) {
+            if (shard->pre_size[i] == 0) continue;
+            SortBucket b;
+            b.off = shard->pre_off[i];
+            b.size = (u32) shard->pre_size[i];
+            b.rem = (u16) (key_bits - bits0);
+            b.parity = 0;
+            b.bits = 0;
+            if (b.size <= cap) {
+                hs.push_back(b);
+                if (b.size > 1024u) ++h[5];
+            } else if (b.rem == 0) {
+                hu.push_back(b);
+            } else {
+                hb.push_back(b);
+                h[4] += (u32) kc_div_up(b.size, (u64) Cfg::TILE);
             }
-            h[0] = (u32) hb.size();
-            h[1] = (u32) hs.size();
-            h[2] = (u32) hu.size();
-            if (h[0] > big_cap || h[1] > small_cap || h[2] > uniform_cap) KC_THROW(KC_ERR_INTERNAL, "k-mer set bucket list overflow");
-            if (h[0]) KC_CUDA(cudaMemcpyAsync(big_a, hb.data(), hb.size() * sizeof(SortBucket), cudaMemcpyHostToDevice, st));
-            if (h[1]) KC_CUDA(cudaMemcpyAsync(small, hs.data(), hs.size() * sizeof(SortBucket), cudaMemcpyHostToDevice, st));
-            if (h[2]) KC_CUDA(cudaMemcpyAsync(uniform, hu.data(), hu.size() * sizeof(SortBucket), cudaMemcpyHostToDevice, st));
-            u32 init[8] = {h[0], h[1], h[2], 0, h[4], h[5], 0, 0};
-            KC_CUDA(cudaMemcpyAsync(ctr, init, 32, cudaMemcpyHostToDevice, st));
-            KC_CUDA(cudaStreamSynchronize(st));  // the staging vectors live on this stack frame
-        } else {
-        SortBucket root;
-        root.off = 0;
-        root.size = (u32) M;
-        root.rem = (u16) key_bits;
-        root.parity = 0;
-        root.bits = 0;
-        if (M <= cap) {
-            KC_CUDA(cudaMemcpyAsync(small, &root, sizeof(root), cudaMemcpyHostToDevice, st));
-            h[1] = 1;
-            h[5] = M > 1024 ? 1 : 0;
-        } else {
-            KC_CUDA(cudaMemcpyAsync(big_a, &root, sizeof(root), cudaMemcpyHostToDevice, st));
-            h[0] = 1;
-            h[4] = (u32) kc_div_up(M, (u64) Cfg::TILE);
         }
-        u32 init[8] = {h[0], h[1], 0, 0, h[4], h[5], 0, 0};
+        h[0] = (u32) hb.size();
+        h[1] = (u32) hs.size();
+        h[2] = (u32) hu.size();
+        if (h[0] > big_cap || h[1] > small_cap || h[2] > uniform_cap) KC_THROW(KC_ERR_INTERNAL, "k-mer set bucket list overflow");
+        if (h[0]) KC_CUDA(cudaMemcpyAsync(big_a, hb.data(), hb.size() * sizeof(SortBucket), cudaMemcpyHostToDevice, st));
+        if (h[1]) KC_CUDA(cudaMemcpyAsync(small, hs.data(), hs.size() * sizeof(SortBucket), cudaMemcpyHostToDevice, st));
+        if (h[2]) KC_CUDA(cudaMemcpyAsync(uniform, hu.data(), hu.size() * sizeof(SortBucket), cudaMemcpyHostToDevice, st));
+        u32 init[8] = {h[0], h[1], h[2], 0, h[4], h[5], 0, 0};
         KC_CUDA(cudaMemcpyAsync(ctr, init, 32, cudaMemcpyHostToDevice, st));
-        KC_CUDA(cudaStreamSynchronize(st));  // root / init live on this stack frame
-        }
+        KC_CUDA(cudaStreamSynchronize(st));  // the staging vectors live on this stack frame
     }
     // k1 is allocated last: the KEYS result is compacted into k1 and then copied down to base_mark, and everything
     // allocated before k1 (control arrays, k0, payloads, counts: > U * (8L + 1) bytes) separates the two regions.
-    if (mode == KS_WHOLE) {
+    if (!shard) {
         k0 = ex.alloc<KWord<L>>(M);
         if (PAY) {
             p0 = ex.alloc<u32>(M);
@@ -1072,25 +1039,18 @@ KmerSet<L> kc_kmerset_build_impl(CudaExec &ex, const u8 *seq, u64 n_bytes, int k
     } else {
         k0 = reinterpret_cast<KWord<L> *>(shard->keys);
         p0 = shard->pos;
-        if (mode == KS_RESOLVE) {
-            k1 = ex.alloc<KWord<L>>(M);
-            p1 = ex.alloc<u32>(M);
-        }
+        k1 = ex.alloc<KWord<L>>(M);
+        p1 = ex.alloc<u32>(M);
     }
-    if (mode != KS_RESOLVE) {
+    if (!shard) {
         {
-            CudaExec::Scope sc(ex, KP_KS_SCATTER0, (pos_end - pos_begin) + M * (sizeof(KWord<L>) + (PAY ? 4 : 0)));
+            CudaExec::Scope sc(ex, KP_KS_SCATTER0, n_bytes + M * (sizeof(KWord<L>) + (PAY ? 4 : 0)));
             kc_ks_scatter0_kernel<L, PAY, SCRAMBLE><<<ex_blocks, Cfg::EX_THREADS, scatter0_smem, st>>>(seq, n_bytes, k, complements ? 1 : 0, shift0,
-                                                                                                   bits0, cursor, tile_hist, k0, p0, tile0, nullptr,
+                                                                                                   bits0, cursor, tile_hist, k0, p0, 0u, nullptr,
                                                                                                    nullptr, win_mask);
         }
         ++ex.launches;
         KC_CUDA(cudaGetLastError());
-    }
-    if (mode == KS_PARTITION) {
-        KC_CUDA(cudaStreamSynchronize(st));
-        ex.arena->release(base_mark);
-        return res;
     }
 
     // ---- levels >= 1 ----
@@ -1278,13 +1238,8 @@ template <int L> void kc_kmerset_scatter_p2p(CudaExec &ex, const u8 *seq, u64 n_
     ex.arena->release(mark);
 }
 
-// Sharded entry points (FLAGS-only; see KsShard).
-template <int L> u64 kc_kmerset_partition(CudaExec &ex, const u8 *seq, u64 n_bytes, int k, bool complements, KsShard *shard) {
-    shard->mode = KS_PARTITION;
-    return kc_kmerset_build_impl<L, true, false>(ex, seq, n_bytes, k, complements, 1, nullptr, nullptr, shard).n_occ;
-}
+// Phase C, on the owner: levels >= 1 and the resolve over the level-0 buckets delivered by phase B (FLAGS-only).
 template <int L> u64 kc_kmerset_resolve(CudaExec &ex, int k, int min_freq, u32 *flags, KsShard *shard) {
-    shard->mode = KS_RESOLVE;
     return kc_kmerset_build_impl<L, true, false>(ex, nullptr, 0, k, true, min_freq, flags, nullptr, shard).n_kept;
 }
 

@@ -434,52 +434,36 @@ __global__ void __launch_bounds__(256) kc_ksf_resolve_kernel(const KWord<L> *__r
     if ((threadIdx.x & 31) == 0 && kept) atomicAdd(n_unique, (kc_ull) kept);
 }
 
-template <int N> KC_D void kc_cp_async_wait_group() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N) : "memory"); }
-
 // ---- one-barrier leaf resolve with the thread's items staged in registers ------------------------------------------------------
-// The stage sweep of kc_ksf_resolve1_kernel (profiles/r01h_variant_sweep2.json) showed its time going with 1 / (CTAs per SM):
+// The stage sweep of the round-1 leaf resolve (profiles/r01h_variant_sweep2.json) showed its time going with 1 / (CTAs per SM):
 // 0.235 ms at 5 CTAs (2 stages), 0.270 at 4 (3 stages), 0.324 at 3 (4 stages) — the kernel is bound by the latency of one
 // leaf's dependent chain (LDS key -> hash -> STS/LDS table -> compare, item after item), not by DRAM.  Here a thread loads
 // ALL its keys first, hashes them together, then issues the table accesses together, so the chain is paid once per phase
 // instead of once per item; key and hash stay in registers between the phases.  THREADS = 512 halves the items per thread.
-// BAL (measured next, ncu r01h: 30 % of the samples wait at the barrier, 6 % on the load of the next leaf's size): with 16-byte
-// copy units a leaf of ~763 u64 keys gives threads 0..125 four items and the others two, so half the warps idle at the barrier;
-// 8-byte units (cp.async.ca) give every thread three.  The size of leaf n + 2 is loaded one iteration before it is needed.
-KC_D void kc_cp_async8(void *smem_dst, const void *gmem_src) {
-    const u32 d = (u32) __cvta_generic_to_shared(smem_dst);
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"(d), "l"(gmem_src) : "memory");
-}
-
-// TMA = true: the leaf arrives by two bulk copies (keys, positions) that one thread issues and that complete on an mbarrier, instead
-// of every thread issuing its own cp.async chunks and waiting for its own group; the items are then dealt out to the threads
-// round-robin (any thread may read any item once the barrier's phase has flipped).
-template <int L, int THREADS, bool MULTI, bool TMA, bool BAL = false>
+// The leaf arrives by two bulk copies (keys, positions) that one thread issues and that complete on an mbarrier; the items are
+// then dealt out to the threads round-robin (any thread may read any item once the barrier's phase has flipped).
+template <int L, int THREADS, bool MULTI>
 __global__ void __launch_bounds__(THREADS) kc_ksf_resolve2_kernel(const KWord<L> *__restrict__ keys, const u32 *__restrict__ pos, const u32 *__restrict__ cnt,
                                                                   u32 n_leaf, KsfFlagPeers fl, kc_ull *n_unique, u32 *status) {
     constexpr u32 CAP = KSF_LEAF_CAP;
     constexpr u32 T1N = 2 * CAP, T2N = CAP;
-    constexpr int KPC = (TMA || (BAL && L == 1)) ? 1 : (16 / (int) sizeof(KWord<L>) > 0 ? 16 / (int) sizeof(KWord<L>) : 1);
-    constexpr int CPK = (int) sizeof(KWord<L>) / 16 > 0 ? (int) sizeof(KWord<L>) / 16 : 1;
-    constexpr int UNITS = (int) CAP / KPC / THREADS;  // copy units (and hash rounds) per thread
-    constexpr int NI = UNITS * KPC;                   // items per thread
-    static_assert(UNITS >= 1 && UNITS * KPC * THREADS == (int) CAP, "CAP must be a whole number of units per thread");
+    constexpr int NI = (int) CAP / THREADS;  // items per thread
+    static_assert(NI >= 1 && NI * THREADS == (int) CAP, "CAP must be a whole number of items per thread");
     extern __shared__ __align__(16) unsigned char kc_smem_raw[];
     KWord<L> *sk0 = reinterpret_cast<KWord<L> *>(kc_smem_raw);
     u32 *sp0 = reinterpret_cast<u32 *>(sk0 + 2 * CAP);
     u32 *T2a = sp0 + 2 * CAP;                                  // [2][T2N]
     u16 *T1a = reinterpret_cast<u16 *>(T2a + 2 * T2N);         // [2][T1N]
-    __shared__ __align__(8) u64 full[2];  // TMA: "leaf in staging buffer b has landed"
+    __shared__ __align__(8) u64 full[2];  // "leaf in staging buffer b has landed"
     const u64 stride = gridDim.x;
     u64 c = blockIdx.x;
     if (c >= n_leaf) return;
-    if (TMA) {
-        if (threadIdx.x == 0) {
-            kc_mbar_init(&full[0], 1);
-            kc_mbar_init(&full[1], 1);
-            kc_mbar_fence_init();
-        }
-        __syncthreads();
+    if (threadIdx.x == 0) {
+        kc_mbar_init(&full[0], 1);
+        kc_mbar_init(&full[1], 1);
+        kc_mbar_fence_init();
     }
+    __syncthreads();
     u32 full_phase = 0;  // bit b: parity to wait for on full[b]
     auto leaf_size = [&](u64 leaf) -> u32 {
         if (leaf >= n_leaf) return 0u;
@@ -491,36 +475,12 @@ __global__ void __launch_bounds__(THREADS) kc_ksf_resolve2_kernel(const KWord<L>
         return sz;
     };
     auto fetch = [&](u64 bucket, u32 size, int buf) {
-        if constexpr (TMA) {
-            if (bucket < n_leaf && threadIdx.x == 0) {
-                const u32 kb = (size * (u32) sizeof(KWord<L>) + 15u) & ~15u, pb = (size * 4u + 15u) & ~15u;
-                kc_mbar_expect_tx(&full[buf], kb + pb);
-                if (kb) kc_bulk_g2s(sk0 + (u32) buf * CAP, keys + bucket * CAP, kb, &full[buf]);
-                if (pb) kc_bulk_g2s(sp0 + (u32) buf * CAP, pos + bucket * CAP, pb, &full[buf]);
-            }
-            return;
+        if (bucket < n_leaf && threadIdx.x == 0) {
+            const u32 kb = (size * (u32) sizeof(KWord<L>) + 15u) & ~15u, pb = (size * 4u + 15u) & ~15u;
+            kc_mbar_expect_tx(&full[buf], kb + pb);
+            if (kb) kc_bulk_g2s(sk0 + (u32) buf * CAP, keys + bucket * CAP, kb, &full[buf]);
+            if (pb) kc_bulk_g2s(sp0 + (u32) buf * CAP, pos + bucket * CAP, pb, &full[buf]);
         }
-        if (bucket < n_leaf) {
-            const char *gk = reinterpret_cast<const char *>(keys + bucket * CAP);
-            const char *gp = reinterpret_cast<const char *>(pos + bucket * CAP);
-            char *dk = reinterpret_cast<char *>(sk0 + (u32) buf * CAP);
-            char *dp = reinterpret_cast<char *>(sp0 + (u32) buf * CAP);
-            const u32 n_units = (size + KPC - 1) / KPC, pchunks = (size * 4 + 15) / 16;
-#pragma unroll
-            for (int m = 0; m < UNITS; ++m) {  // unit u holds items u * KPC .. u * KPC + KPC - 1: the ones this thread hashes
-                const u32 u = threadIdx.x + (u32) m * THREADS;
-                if (u < n_units) {
-                    if constexpr (BAL && L == 1) {
-                        kc_cp_async8(dk + 8 * u, gk + 8 * u);
-                    } else {
-#pragma unroll
-                        for (int cc = 0; cc < CPK; ++cc) kc_cp_async16(dk + 16 * (u * CPK + cc), gk + 16 * (u * CPK + cc));
-                    }
-                }
-            }
-            for (u32 q = threadIdx.x; q < pchunks; q += THREADS) kc_cp_async16(dp + 16 * q, gp + 16 * q);
-        }
-        kc_cp_async_commit();
     };
     u32 size = leaf_size(c);
     u32 size_n = leaf_size(c + stride);
@@ -529,27 +489,19 @@ __global__ void __launch_bounds__(THREADS) kc_ksf_resolve2_kernel(const KWord<L>
     u32 kept = 0;
     while (true) {
         const u64 cn = c + stride;
-        u32 raw_nn = 0;  // size of leaf c + 2 * stride: loaded here, first used at the bottom of the loop
-        if (BAL) {
-            if (cn + stride < n_leaf) raw_nn = cnt[cn + stride];
-        }
         KWord<L> *sk = sk0 + (u32) buf * CAP;
         u32 *sp = sp0 + (u32) buf * CAP;
         u32 *T2 = T2a + (u32) buf * T2N;
         u16 *T1 = T1a + (u32) buf * T1N;
-        if (TMA) {
-            kc_mbar_wait(&full[buf], (full_phase >> buf) & 1u);  // leaf c has landed (all of it, for every thread)
-            full_phase ^= 1u << buf;
-        } else {
-            kc_cp_async_wait_group<0>();  // the thread's own key units of leaf c have landed
-        }
+        kc_mbar_wait(&full[buf], (full_phase >> buf) & 1u);  // leaf c has landed (all of it, for every thread)
+        full_phase ^= 1u << buf;
         if (threadIdx.x < 256) reinterpret_cast<uint4 *>(T2)[threadIdx.x] = make_uint4(KC_NONE, KC_NONE, KC_NONE, KC_NONE);  // T2N = 256 x 4 slots
         // A: all keys, then all hashes, then all table stores
         KWord<L> key[NI];
         u32 h1[NI], h2[NI];
 #pragma unroll
         for (int m = 0; m < NI; ++m) {
-            const u32 i = (threadIdx.x + (u32) (m / KPC) * THREADS) * KPC + (u32) (m % KPC);
+            const u32 i = threadIdx.x + (u32) m * THREADS;
             if (i < size) key[m] = sk[i];
         }
 #pragma unroll
@@ -562,7 +514,7 @@ __global__ void __launch_bounds__(THREADS) kc_ksf_resolve2_kernel(const KWord<L>
         }
 #pragma unroll
         for (int m = 0; m < NI; ++m) {
-            const u32 i = (threadIdx.x + (u32) (m / KPC) * THREADS) * KPC + (u32) (m % KPC);
+            const u32 i = threadIdx.x + (u32) m * THREADS;
             if (i < size) T1[h1[m]] = (u16) i;
         }
         __syncthreads();
@@ -571,12 +523,12 @@ __global__ void __launch_bounds__(THREADS) kc_ksf_resolve2_kernel(const KWord<L>
         u32 o[NI];
 #pragma unroll
         for (int m = 0; m < NI; ++m) {
-            const u32 i = (threadIdx.x + (u32) (m / KPC) * THREADS) * KPC + (u32) (m % KPC);
+            const u32 i = threadIdx.x + (u32) m * THREADS;
             o[m] = i < size ? (u32) T1[h1[m]] : i;
         }
 #pragma unroll
         for (int m = 0; m < NI; ++m) {
-            const u32 i = (threadIdx.x + (u32) (m / KPC) * THREADS) * KPC + (u32) (m % KPC);
+            const u32 i = threadIdx.x + (u32) m * THREADS;
             if (i >= size) continue;
             if (o[m] == i) {
                 ++kept;
@@ -605,29 +557,21 @@ __global__ void __launch_bounds__(THREADS) kc_ksf_resolve2_kernel(const KWord<L>
         if (cn >= n_leaf) break;
         c = cn;
         size = size_n;
-        if (BAL) {
-            if (raw_nn > CAP) {
-                raw_nn = CAP;
-                if (threadIdx.x == 0) status[0] = 1;
-            }
-            size_n = raw_nn;
-        } else {
-            size_n = leaf_size(c + stride);
-        }
+        size_n = leaf_size(c + stride);
         buf ^= 1;
     }
-    if (!TMA) kc_cp_async_wait_group<0>();
 #pragma unroll
     for (int o2 = 16; o2 > 0; o2 >>= 1) kept += __shfl_down_sync(0xFFFFFFFFu, kept, o2);
     if ((threadIdx.x & 31) == 0 && kept) atomicAdd(n_unique, (kc_ull) kept);
 }
 
 // ---- levels >= 1 with the next tile in flight ---------------------------------------------------------------------------------
-// kc_ksf_scatter_kernel issues a tile's loads and then waits for them (ncu: long scoreboard, 47 % of the HBM peak).  Here the
-// tile after the current one streams into a shared-memory input buffer with cp.async while the current tile is ranked,
-// staged and written out: a thread takes its items out of the input buffer into registers, and the barrier that ends the
-// ranking phase frees the buffer for the next copy.  Tiles are contiguous in their parent slot, slots are 128-byte aligned.
-template <int L, int TILE, int MINB, int THREADS, bool TMA>
+// A scatter that issues a tile's loads and then waits for them (round 1, ncu: long scoreboard, 47 % of the HBM peak) is bound
+// by that wait.  Here the tile after the current one streams into a shared-memory input buffer by two bulk copies (issued by
+// one thread, completing on an mbarrier) while the current tile is ranked, staged and written out: a thread takes its items
+// out of the input buffer into registers, and the barrier that ends the ranking phase frees the buffer for the next copy.
+// Tiles are contiguous in their parent slot, slots are 128-byte aligned.
+template <int L, int TILE, int MINB, int THREADS>
 __global__ void __launch_bounds__(THREADS, MINB) kc_ksf_scatter_pf_kernel(const KWord<L> *__restrict__ ksrc, const u32 *__restrict__ psrc, KWord<L> *__restrict__ kdst,
                                                                 u32 *__restrict__ pdst, const u32 *__restrict__ P_size, const u32 *__restrict__ tile_prefix,
                                                                 u32 nP, u64 capP, u32 tiles_per_cta, int shift, int bits, u32 *C_cnt, u32 capC, u32 *status,
@@ -644,20 +588,18 @@ __global__ void __launch_bounds__(THREADS, MINB) kc_ksf_scatter_pf_kernel(const 
     __shared__ u64 dbase[256];  // slot index of the digit's first item of this tile, minus its staged position: at = dbase + q
     __shared__ u32 qlim[256];   // staged positions below this still fit into the child's slot
     __shared__ u32 sw[THREADS / 32];
-    __shared__ __align__(8) u64 full;  // TMA: "the tile in the input buffer has landed"
+    __shared__ __align__(8) u64 full;  // "the tile in the input buffer has landed"
     const u32 n_tiles = tile_prefix[nP];
     const u32 t0 = blockIdx.x * tiles_per_cta;
     const u32 t1 = min(n_tiles, t0 + tiles_per_cta);
     if (t0 >= t1) return;
     u32 b = kc_upper_bound_u32(tile_prefix, nP + 1, t0) - 1;
     if (threadIdx.x < 256) cnt[threadIdx.x] = 0;
-    if (TMA) {
-        if (threadIdx.x == 0) {
-            kc_mbar_init(&full, 1);
-            kc_mbar_fence_init();
-        }
-        __syncthreads();
+    if (threadIdx.x == 0) {
+        kc_mbar_init(&full, 1);
+        kc_mbar_fence_init();
     }
+    __syncthreads();
     u32 full_phase = 0;
     bool over = false;
     // tile t of the CTA -> (parent bucket, first item inside the source arrays, items)
@@ -667,34 +609,21 @@ __global__ void __launch_bounds__(THREADS, MINB) kc_ksf_scatter_pf_kernel(const 
         n_here = min((u32) TILE, P_size[bb] - start);
         first = (u64) bb * capP + start;
     };
-    auto prefetch = [&](u64 first, u32 n_here) {
-        if constexpr (TMA) {  // two bulk copies issued by one thread; tiles start on 128-byte boundaries of their slot
-            if (threadIdx.x == 0) {
-                const u32 kb = (n_here * (u32) sizeof(KWord<L>) + 15u) & ~15u, pb = (n_here * 4u + 15u) & ~15u;
-                kc_mbar_expect_tx(&full, kb + pb);
-                if (kb) kc_bulk_g2s(in_k, ksrc + first, kb, &full);
-                if (pb) kc_bulk_g2s(in_p, psrc + first, pb, &full);
-            }
-            return;
+    auto prefetch = [&](u64 first, u32 n_here) {  // tiles start on 128-byte boundaries of their slot
+        if (threadIdx.x == 0) {
+            const u32 kb = (n_here * (u32) sizeof(KWord<L>) + 15u) & ~15u, pb = (n_here * 4u + 15u) & ~15u;
+            kc_mbar_expect_tx(&full, kb + pb);
+            if (kb) kc_bulk_g2s(in_k, ksrc + first, kb, &full);
+            if (pb) kc_bulk_g2s(in_p, psrc + first, pb, &full);
         }
-        const char *gk = reinterpret_cast<const char *>(ksrc + first);
-        const char *gp = reinterpret_cast<const char *>(psrc + first);
-        const u32 kch = (n_here * (u32) sizeof(KWord<L>) + 15) / 16, pch = (n_here * 4 + 15) / 16;
-        for (u32 q = threadIdx.x; q < kch; q += THREADS) kc_cp_async16(reinterpret_cast<char *>(in_k) + 16 * q, gk + 16 * q);
-        for (u32 q = threadIdx.x; q < pch; q += THREADS) kc_cp_async16(reinterpret_cast<char *>(in_p) + 16 * q, gp + 16 * q);
-        kc_cp_async_commit();
     };
     u64 first;
     u32 n_here;
     describe(t0, b, first, n_here);
     prefetch(first, n_here);
     for (u32 t = t0; t < t1; ++t) {
-        if (TMA) {
-            kc_mbar_wait(&full, full_phase);
-            full_phase ^= 1u;
-        } else {
-            kc_cp_async_wait_all();
-        }
+        kc_mbar_wait(&full, full_phase);
+        full_phase ^= 1u;
         __syncthreads();  // tile t is complete in the input buffer; the write-out of tile t - 1 has left the staging buffers
         KWord<L> item[ITEMS];
         u32 pay[ITEMS];
@@ -798,15 +727,13 @@ template <int L> struct KsfKernels {  // the kernel instances this construction 
         const int d = once.run([&](int dv) {
             KC_CUDA(cudaFuncSetAttribute(kc_ksf_scatter0_kernel<L, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem0()));
             KC_CUDA(cudaFuncSetAttribute(kc_ksf_scatter0_kernel<L, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem0()));
-            KC_CUDA(cudaFuncSetAttribute(kc_ksf_scatter_pf_kernel<L, TILE1, 2, THREADS1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem1()));
-            KC_CUDA(cudaFuncSetAttribute(kc_ksf_scatter_pf_kernel<L, TILE1, 2, THREADS1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem1()));
-            KC_CUDA(cudaFuncSetAttribute(kc_ksf_resolve2_kernel<L, 256, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_r(false)));
-            KC_CUDA(cudaFuncSetAttribute(kc_ksf_resolve2_kernel<L, 256, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_r(false)));
-            KC_CUDA(cudaFuncSetAttribute(kc_ksf_resolve2_kernel<L, 256, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_r(false)));
+            KC_CUDA(cudaFuncSetAttribute(kc_ksf_scatter_pf_kernel<L, TILE1, 2, THREADS1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem1()));
+            KC_CUDA(cudaFuncSetAttribute(kc_ksf_resolve2_kernel<L, 256, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_r(false)));
+            KC_CUDA(cudaFuncSetAttribute(kc_ksf_resolve2_kernel<L, 256, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_r(false)));
             KC_CUDA(cudaFuncSetAttribute(kc_ksf_resolve_kernel<L, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_r(true)));
             KC_CUDA(cudaFuncSetAttribute(kc_ksf_resolve_kernel<L, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_r(true)));
             dev[dv].n_sm = kc_sm_count(dv);
-            KC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&dev[dv].occ_r[0], kc_ksf_resolve2_kernel<L, 256, false, true>, 256, smem_r(false)));
+            KC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&dev[dv].occ_r[0], kc_ksf_resolve2_kernel<L, 256, false>, 256, smem_r(false)));
             KC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&dev[dv].occ_r[1], kc_ksf_resolve_kernel<L, true, false>, 256, smem_r(true)));
         });
         return dev[d];
@@ -832,14 +759,9 @@ void kc_ksf_level(CudaExec &ex, const KWord<L> *ksrc, const u32 *psrc, KWord<L> 
     const u32 ctas = (u32) kc_div_up(tiles_ub, tiles_per_cta);
     {
         CudaExec::Scope sc(ex, KP_SORT_SCATTER, 2 * items_ub * (sizeof(KWord<L>) + 4));
-        if (tune.tma)
-            kc_ksf_scatter_pf_kernel<L, KK::TILE1, 2, KK::THREADS1, true><<<ctas, KK::THREADS1, KK::smem1(), st>>>(ksrc, psrc, kdst, pdst, P_size, tile_prefix, nP, capP,
-                                                                                                                tiles_per_cta, shift, bits, cnt_next, (u32) capC,
-                                                                                                                status, pdiv);
-        else
-            kc_ksf_scatter_pf_kernel<L, KK::TILE1, 2, KK::THREADS1, false><<<ctas, KK::THREADS1, KK::smem1(), st>>>(ksrc, psrc, kdst, pdst, P_size, tile_prefix, nP, capP,
-                                                                                                                 tiles_per_cta, shift, bits, cnt_next, (u32) capC,
-                                                                                                                 status, pdiv);
+        kc_ksf_scatter_pf_kernel<L, KK::TILE1, 2, KK::THREADS1><<<ctas, KK::THREADS1, KK::smem1(), st>>>(ksrc, psrc, kdst, pdst, P_size, tile_prefix, nP, capP,
+                                                                                                      tiles_per_cta, shift, bits, cnt_next, (u32) capC, status,
+                                                                                                      pdiv);
         ++ex.launches;
         KC_CUDA(cudaGetLastError());
     }
@@ -849,7 +771,7 @@ void kc_ksf_level(CudaExec &ex, const KWord<L> *ksrc, const u32 *psrc, KWord<L> 
 // Leaf slots (KSF_LEAF_CAP items each) -> losers cleared in fl, *n_unique += kept k-mers.
 template <int L>
 void kc_ksf_resolve(CudaExec &ex, const KWord<L> *keys, const u32 *pos, const u32 *cnt, u64 n_leaf, const KsfFlagPeers &fl, int min_freq, kc_ull *n_unique,
-                    u32 *status, u64 items_ub, bool tma = true) {
+                    u32 *status, u64 items_ub) {
     typedef KsfKernels<L> KK;
     if (n_leaf >= 0xFFFFFFFFULL) KC_THROW(KC_ERR_TOO_LARGE, "too many leaf buckets");
     const typename KK::Dev &dv = KK::prepare();
@@ -860,9 +782,8 @@ void kc_ksf_resolve(CudaExec &ex, const KWord<L> *keys, const u32 *pos, const u3
     const bool multi = fl.n > 1;
     if (counted && multi) kc_ksf_resolve_kernel<L, true, true><<<grid, 256, KK::smem_r(true), ex.stream>>>(keys, pos, cnt, (u32) n_leaf, fl, (u32) min_freq, n_unique, status);
     else if (counted) kc_ksf_resolve_kernel<L, true, false><<<grid, 256, KK::smem_r(true), ex.stream>>>(keys, pos, cnt, (u32) n_leaf, fl, (u32) min_freq, n_unique, status);
-    else if (multi) kc_ksf_resolve2_kernel<L, 256, true, true><<<grid, 256, KK::smem_r(false), ex.stream>>>(keys, pos, cnt, (u32) n_leaf, fl, n_unique, status);
-    else if (tma) kc_ksf_resolve2_kernel<L, 256, false, true><<<grid, 256, KK::smem_r(false), ex.stream>>>(keys, pos, cnt, (u32) n_leaf, fl, n_unique, status);
-    else kc_ksf_resolve2_kernel<L, 256, false, false><<<grid, 256, KK::smem_r(false), ex.stream>>>(keys, pos, cnt, (u32) n_leaf, fl, n_unique, status);
+    else if (multi) kc_ksf_resolve2_kernel<L, 256, true><<<grid, 256, KK::smem_r(false), ex.stream>>>(keys, pos, cnt, (u32) n_leaf, fl, n_unique, status);
+    else kc_ksf_resolve2_kernel<L, 256, false><<<grid, 256, KK::smem_r(false), ex.stream>>>(keys, pos, cnt, (u32) n_leaf, fl, n_unique, status);
     ++ex.launches;
     KC_CUDA(cudaGetLastError());
 }
@@ -939,7 +860,7 @@ bool kc_kmerset_build_fast(CudaExec &ex, const u8 *seq, u64 n_bytes, int k, bool
             if (c) atomicAdd(m_cell, (kc_ull) c);
         });
     }
-    kc_ksf_resolve<L>(ex, kb[last & 1], pb[last & 1], cnt_cur, pl.n_leaf, fl, min_freq, reinterpret_cast<kc_ull *>(cells), status, n_bytes, tune.tma);
+    kc_ksf_resolve<L>(ex, kb[last & 1], pb[last & 1], cnt_cur, pl.n_leaf, fl, min_freq, reinterpret_cast<kc_ull *>(cells), status, n_bytes);
     ex.arena->release(base_mark);
     return true;
 }

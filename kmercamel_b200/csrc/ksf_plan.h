@@ -3,7 +3,8 @@
 // tests/host_emul can check the invariants the kernels rely on:
 //   * a level's digit is at most 8 bits wide (the kernels keep 256 counters per tile);
 //   * every slot size is a multiple of 32 items, so slots stay 128-byte aligned for 4-byte positions and 256-byte aligned for
-//     8-byte keys — the cp.async (16-byte) tile and leaf copies of kc_ksf_scatter_pf_kernel / kc_ksf_resolve*_kernel need that;
+//     8-byte keys — the 16-byte bulk and cp.async copies of tiles and leaves (kc_ksf_scatter_pf_kernel, kc_ksf_resolve*_kernel)
+//     need that;
 //   * all partition digits together stay inside the top limb of the scrambled word (KWord::digit_top);
 //   * a leaf slot holds KSF_LEAF_CAP items, the capacity of the shared-memory resolve.
 #pragma once
@@ -18,7 +19,6 @@ struct KsfTuning {
     uint32_t leaf_target = 768;   // mean leaf size aimed at (the leaf slot holds KSF_LEAF_CAP)
     double sigmas = 8.0;     // slot = mean + sigmas * sqrt(mean) (+ 2 %) items; 0 forces overflows (tests)
     uint64_t min_items = 1u << 16;  // smaller inputs take the exact path (nothing to gain)
-    bool tma = true;         // tiles / leaves stream in through 1-D bulk copies (TMA) + mbarrier; false: per-thread cp.async (kept for A/B timing)
     int max_ctas = 148 * 16; // level >= 1 scatter grid: at most this many CTAs, each walking a run of consecutive tiles
 };
 

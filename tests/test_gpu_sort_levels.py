@@ -35,7 +35,7 @@ def _digits(w, pos, nbits):
 
 
 def _model(ref, key_bits):
-    """Counts-only model of kc_sort_impl's bucket bookkeeping on the sorted words `ref`: every bucket is a contiguous range of them
+    """Counts-only model of kc_sort's bucket bookkeeping on the sorted words `ref`: every bucket is a contiguous range of them
     (its items share the key bits already partitioned).  -> the statistics kc_debug_sort reports."""
     L = ref.shape[1]
     cap = CAP[L]
