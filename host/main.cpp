@@ -21,6 +21,7 @@
 #include <fstream>
 #include <iomanip>
 #include <iostream>
+#include <set>
 #include <string>
 #include <thread>
 #include <vector>
@@ -308,7 +309,7 @@ static int camel_compute(int argc, char **argv, bool lower_bound) {
     }
     std::vector<unsigned char>().swap(data);
     const double t_frame = now_ms();
-    // 64-bit window positions (include/kcgpu.h KC_POS32_BYTES): one GPU; -V would hold input and output at once, `verify` checks the file
+    // 64-bit window positions (include/kcgpu.h KC_POS32_BYTES): -V would hold input and output at once, `verify` checks the file
     const bool large = n_bytes >= KC_POS32_BYTES;
     if (large && verify) {
         std::cerr << "kmercamel compute: verification not available for inputs of 2^32 bytes or more (" << n_bytes << " sequence bytes)" << std::endl;
@@ -317,7 +318,8 @@ static int camel_compute(int argc, char **argv, bool lower_bound) {
 
     init_thread.join();
     rc = rc_init;
-    if (rc == KC_OK && multi && large) {
+    // such an input on ranks that all share one device: a group gains nothing there and holds the whole sequence once per rank
+    if (rc == KC_OK && multi && large && std::set<int>(devices.begin(), devices.end()).size() < 2) {
         kc_group_destroy(group);
         group = nullptr;
         ctx = nullptr;

@@ -44,7 +44,10 @@ extern "C" {
  * applies with k >= 26, min_frequency 1, no want_maxone and no assume_simplitigs (kc_streaming: any min_frequency, every pass of
  * -z is a first-occurrence construction; kc_kmer_digest ignores assume_simplitigs and want_maxone); outside those conditions, with
  * option sig_set = 0, or when a signature bucket overflows on such an input (heavily repeated sequence), they fail with
- * KC_ERR_TOO_LARGE.  kc_maskopt, kc_count_kmers and groups refuse such inputs with KC_ERR_TOO_LARGE. */
+ * KC_ERR_TOO_LARGE.  Groups (kc_group_compute, kc_group_compute_device) take them under the same conditions, with the same
+ * construction across their ranks and a byte-identical result; a group also refuses an input whose record streams would exceed
+ * 2^32 records on one rank (few ranks on tens of GB; kc_group_plan says so).  Such a refusal, and a bucket overflow seen by every
+ * rank, leaves the group usable.  kc_maskopt and kc_count_kmers refuse such inputs with KC_ERR_TOO_LARGE. */
 #define KC_POS32_BYTES 0xFFFFFFF0ULL
 
 typedef struct kc_ctx kc_ctx;
@@ -184,6 +187,9 @@ int kc_frame_fasta(const uint8_t *data, uint64_t n, uint8_t **seq, uint64_t *n_b
  * NVLink / NVSwitch); the level-0 partition pass stores each (k-mer, position) item straight into the heap of the GPU that owns
  * the k-mer's hash range, and ranks synchronise through device-side signal words — no collective library and no host round trip
  * on the data path (kmercamel_b200/csrc/group.cuh).  From-FASTA regime only (no -S, no -M); results are identical to kc_compute.
+ * Inputs of KC_POS32_BYTES or more run as on one GPU (see KC_POS32_BYTES): the signature construction alone, 64-bit positions.  A
+ * heap sized for such inputs (n_bytes_cap >= KC_POS32_BYTES) holds the receive regions of that construction only and takes no
+ * smaller job (KC_ERR_ARG); kc_group_compute rebuilds its heaps when the job size crosses KC_POS32_BYTES.
  *
  * (1) One process, one host thread per GPU — what §8(b) calls kc_init(n_gpus, device_ids):
  *       kc_init_multi     contexts on the given devices (an ordinal may repeat: several ranks then share a GPU, which is how the
@@ -203,7 +209,8 @@ int kc_frame_fasta(const uint8_t *data, uint64_t n, uint8_t **seq, uint64_t *n_b
  *       kc_group_close    releases the heap (all ranks must have finished their last job)
  *     kc_group_plan       host only, no GPU: plan[0] = fixed-slot path applies, [1], [2] = the rank's slice of window END positions,
  *                         [3], [4] = its range of level-0 digits (hash range), [5] = level-0 digits, [6] = items per (digit, sender)
- *                         sub-slot, [7] = heap bytes per rank. */
+ *                         sub-slot, [7] = heap bytes per rank (without the sequence).  From KC_POS32_BYTES on: plan[0] = plan[6] = 0,
+ *                         and KC_ERR_TOO_LARGE where the group cannot take the input at all (k < 26, or its 32-bit bounds). */
 typedef struct kc_group kc_group;
 int kc_init_multi(int n_gpus, const int *device_ids, kc_group **out);
 void kc_group_destroy(kc_group *g);

@@ -510,7 +510,7 @@ class Group:
             raise KcError(rc, self._lib.kc_group_last_error(self._g).decode())
         t = out.t
         times = dict(extract=t.extract_ms, count=t.count_ms, path=t.path_ms, emit=t.emit_ms, total=t.total_ms)
-        ms = C.string_at(out.ms, out.length) if copy else None
+        ms = _string_at(out.ms, out.length) if copy else None
         return ComputeResult(ms, None, out.length, out.n_kmers, out.n_occurrences, out.n_nodes, out.n_launches, out.n_simplitigs, times,
                              out.ms or 0, 0, 0, out.length)
 

@@ -28,24 +28,58 @@
 #include "kmerset_fast.cuh"
 #include "kmerset_sig.cuh"
 #include "runs.cuh"
+#include "set_routes.cuh"
+
+// The 32-bit quantities of the signature construction on a group (kmerset_sig.cuh), checked on the host for an input of n_bytes
+// (every rank computes the same values, so every rank refuses together).  Returns why the group cannot take the input, or nullptr.
+//   tiles, t0, t1 (kc_sig_group_scan)       u32 tile numbers: n_bytes < 2^45
+//   n_buckets                               < 2^27 (kc_sig_plan): b / n by SigPeers::magic needs b < 2^28; bucket indices, n_om and
+//                                           the grids of the counting, compacting and gathering kernels stay far below 2^32
+//   sub_cap                                 <= 256 records; a bucket's records over all senders <= n * 256 (kc_sig_gather_kernel)
+//   region_cap                              u32 stream length and ship offsets: < 2^32; products with the sender index are u64
+//   off_om, dense_cap                       the dense stream's offsets are u32 prefix sums: dense_cap < 2^32 for the largest slice.
+//                                           The stream holds at most dense_cap records: the first bucket past it raises the status
+//                                           word before any offset can wrap, and the ship kernel then sends empty tables
+// Window positions themselves are 61-bit (kc_sig_record) and the flags take u64 positions (kc_flag_clear_all).
+inline const char *kc_grp_large_bound(u64 n_bytes, int n_ranks) {
+    constexpr u64 TILE = 256 * KC_EX_STRIP;
+    if ((n_bytes + TILE - 1) / TILE >= (1ull << 32)) return KC_LARGE_ONLY "; on a group its 32-bit tile numbers do not reach this input";
+    if (kc_sig_region_cap(n_bytes, n_ranks) >= (1ull << 32)) return KC_LARGE_ONLY "; on a group of this size one rank's record stream to one owner would exceed 2^32 records (use more GPUs)";
+    if (kc_sig_dense_cap(kc_sig_max_slice(n_bytes, n_ranks), n_ranks) >= (1ull << 32)) return KC_LARGE_ONLY "; on a group of this size one rank's dense record stream would exceed 2^32 records (use more GPUs)";
+    return nullptr;
+}
 
 struct GrpLayout {
     u64 n_bytes_cap = 0;
     int limbs = 0, n_ranks = 0;
     u64 recv_items = 0, flag_words = 0;
+    u64 recv_k_bytes = 0, recv_p_bytes = 0;  // sizes of the two receive regions
     size_t off_sig = 0, off_cells = 0, off_cnt = 0, off_flags = 0, off_flags2 = 0, off_recv_k = 0, off_recv_p = 0, off_packed = 0, off_seq = 0, total = 0;
+    bool pos64() const { return n_bytes_cap >= KC_POS32_BYTES; }
 };
 
 // Heap of a rank for jobs of up to n_bytes_cap sequence bytes (identical on every rank).
+// From KC_POS32_BYTES on, only the signature construction runs (the others move 32-bit positions): the receive regions hold one
+// record stream per sender (kc_sig_region_cap records) and the senders' bucket offset tables, instead of the fixed-slot / exact
+// items (1.25 x n_bytes_cap / n_ranks of 8 L + 4 bytes), which would cost tens of GB per rank for nothing.  Such a heap takes no job
+// below KC_POS32_BYTES (group_check_job).
 inline GrpLayout kc_grp_layout(u64 n_bytes_cap, int limbs, int n_ranks, bool with_seq, u64 ex_tile, const KsfTuning &tune) {
     GrpLayout y;
     y.n_bytes_cap = n_bytes_cap;
     y.limbs = limbs;
     y.n_ranks = n_ranks;
-    const KsfGroupPlan gp = kc_ksf_group_plan(n_bytes_cap, n_ranks, ex_tile, tune);
-    const u64 by_plan = gp.ok ? gp.recv_items() + gp.recv_items() / 20 : 0;
-    const u64 by_share = (u64) ((double) n_bytes_cap / n_ranks * 1.25) + (1u << 20);  // exact path: a rank's hash range, back to back
-    y.recv_items = (by_plan > by_share ? by_plan : by_share) + 65536;
+    if (y.pos64()) {
+        const u64 nbr = (kc_sig_max_buckets(n_bytes_cap) + (u64) n_ranks - 1) / (u64) n_ranks;
+        y.recv_k_bytes = (u64) n_ranks * kc_sig_region_cap(n_bytes_cap, n_ranks) * 8;
+        y.recv_p_bytes = (u64) n_ranks * (nbr + 1) * 4;
+    } else {
+        const KsfGroupPlan gp = kc_ksf_group_plan(n_bytes_cap, n_ranks, ex_tile, tune);
+        const u64 by_plan = gp.ok ? gp.recv_items() + gp.recv_items() / 20 : 0;
+        const u64 by_share = (u64) ((double) n_bytes_cap / n_ranks * 1.25) + (1u << 20);  // exact path: a rank's hash range, back to back
+        y.recv_items = (by_plan > by_share ? by_plan : by_share) + 65536;
+        y.recv_k_bytes = y.recv_items * 8 * (u64) limbs;
+        y.recv_p_bytes = y.recv_items * 4;
+    }
     y.flag_words = n_bytes_cap / 32 + 66;
     size_t o = 0;
     auto take = [&](size_t bytes) {
@@ -58,8 +92,8 @@ inline GrpLayout kc_grp_layout(u64 n_bytes_cap, int limbs, int n_ranks, bool wit
     y.off_cnt = take((size_t) KC_MAX_PEERS * 256 * 4);
     y.off_flags = take(y.flag_words * 4);
     y.off_flags2 = take(y.flag_words * 4);
-    y.off_recv_k = take(y.recv_items * 8 * (u64) limbs);
-    y.off_recv_p = take(y.recv_items * 4);
+    y.off_recv_k = take(y.recv_k_bytes);
+    y.off_recv_p = take(y.recv_p_bytes);
     y.off_packed = take(n_bytes_cap / 4 + 4096);  // 2-bit code words of the whole sequence (signature construction, kmerset_sig.cuh)
     y.off_seq = take(with_seq ? n_bytes_cap + 256 : 0);
     y.total = o;
@@ -116,6 +150,7 @@ struct KcGroup {
     bool done_pending = false;            // a DONE signal (number done_seq) is out; the next job waits for it
     u32 done_seq = 0;
     bool failed = false;                  // a wait timed out or a rank left a job half way: the sync numbers no longer agree
+    bool refused = false;                 // the last job failed on every rank at the same point and was closed by a DONE signal
     // per-rank scratch outside the heap
     u32 *cnt0 = nullptr;                  // [256] level-0 fill counts of this rank's sub-slots
     u64 *cells_local = nullptr;           // [4]
@@ -323,11 +358,12 @@ template <int L>
 u64 *kc_grp_sig_flags(KcGroup &G, CudaExec &ex, const u8 *seq, u64 n_bytes, int k, bool complements, const SigTuning &tune) {
     const SigPlan pl = kc_sig_plan(n_bytes, k, tune);
     if (!pl.ok || G.n < 1 || pl.n_buckets >= (1u << 28)) return nullptr;
+    if (kc_grp_large_bound(n_bytes, G.n)) return nullptr;  // refused before the job (group_check_large)
     const u32 sub_cap = kc_sig_sub_cap(pl, G.n);
     const u32 nbr = kc_sig_owned_buckets(pl.n_buckets, G.n, 0);
-    const u32 region_cap = kc_sig_region_cap(n_bytes, G.n);
-    if ((u64) G.n * region_cap * 8 > G.lay.recv_items * 8 * (u64) G.lay.limbs) return nullptr;
-    if ((u64) G.n * ((u64) nbr + 1) * 4 > G.lay.recv_items * 4) return nullptr;
+    const u32 region_cap = (u32) kc_sig_region_cap(n_bytes, G.n);
+    if ((u64) G.n * region_cap * 8 > G.lay.recv_k_bytes) return nullptr;
+    if ((u64) G.n * ((u64) nbr + 1) * 4 > G.lay.recv_p_bytes) return nullptr;
     u32 *flags = reinterpret_cast<u32 *>(G.heap + G.lay.off_flags);
     const u64 body_words = kc_div_up(n_bytes, (u64) 32);
     ex.fill_bytes(flags + body_words, 0, 8);  // the padding words nobody writes (kc_runs_load reads one past the end)

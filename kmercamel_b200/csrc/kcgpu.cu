@@ -132,6 +132,13 @@ void ensure_arena(kc_ctx *ctx, size_t need) {
     ctx->arena.reset();
 }
 
+// Arena bytes of the overlap stage and the emission for `nodes` nodes per strand (the part of estimate_arena after stage 1).
+double overlap_emit_bytes(double nodes, int limbs, bool complements, u64 n_bytes) {
+    const double wb = 8.0 * limbs;
+    const double N = (complements ? 2.0 : 1.0) * nodes;
+    return N * (60.0 + 2.0 * 2.0 * (wb + 8.0) + 12.0 + 40.0) + N * 32.0 + 3.0 * n_bytes;
+}
+
 // Arena bytes one kc_compute needs (see DESIGN.md "Data layout in HBM").  Stage 1 is an exact upper bound; the overlap
 // stage depends on the number of nodes, which for a FASTA input (first-occurrence runs) is only known after stage 1:
 // `pessimistic = false` assumes one run per 64 sequence bytes (reads with 1 % errors give one per ~650), and a call that
@@ -141,7 +148,6 @@ void ensure_arena(kc_ctx *ctx, size_t need) {
 size_t estimate_arena(u64 n_bytes, u64 n_recs, int limbs, bool complements, bool simplitigs, bool pessimistic = false,
                       const KsfTuning *fast = nullptr, const SigPlan *sig = nullptr) {
     const double wb = 8.0 * limbs;
-    const double c = complements ? 2.0 : 1.0;
     double stage1 = n_bytes * (1.0 + 2.0 * (wb + 4.0) + 1.0 + 1.0 + 0.2);  // sequence, keys + positions x2, counts, control, flags
     if (n_bytes >= KC_POS32_BYTES && sig && sig->ok) {
         stage1 = n_bytes * (1.0 + 0.125) + (double) kc_sig_arena_bytes(*sig, n_bytes);
@@ -153,10 +159,7 @@ size_t estimate_arena(u64 n_bytes, u64 n_recs, int limbs, bool complements, bool
         }
     }
     double nodes = simplitigs ? (double) n_recs : (pessimistic ? n_bytes * 0.85 : n_bytes / 64.0 + 1e6);  // sparse switch: up to 5 k-mer nodes per 6 bytes
-    double N = c * nodes;
-    double engine = N * (60.0 + 2.0 * 2.0 * (wb + 8.0) + 12.0 + 40.0);
-    double emit = N * 32.0 + 3.0 * n_bytes;
-    double total = (stage1 + engine + emit) * 1.1 + (256u << 20);
+    double total = (stage1 + overlap_emit_bytes(nodes, limbs, complements, n_bytes)) * 1.1 + (256u << 20);
     return (size_t) total;
 }
 
@@ -672,7 +675,8 @@ void overlap_only(kc_ctx *ctx, CudaExec &ex, const uint64_t *first, const uint64
 void group_alloc_common(kc_ctx *ctx, int n_ranks, int rank, int k, uint64_t n_bytes_cap, bool with_seq) {
     if (n_ranks < 1 || n_ranks > KC_MAX_PEERS || rank < 0 || rank >= n_ranks) KC_THROW(KC_ERR_ARG, "bad rank / group size");
     if (k < 1 || k > 127) KC_THROW(KC_ERR_ARG, "k must be in 1..127");
-    if (n_bytes_cap >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "more than 2^32 sequence bytes");
+    if (n_bytes_cap >= KC_POS32_BYTES)
+        if (const char *why = kc_grp_large_bound(n_bytes_cap, n_ranks)) KC_THROW(KC_ERR_TOO_LARGE, why);
     KcGroup &G = ctx->grp;
     if (G.heap) KC_THROW(KC_ERR_ARG, "this context already belongs to a group");
     KC_CUDA(cudaSetDevice(ctx->device));
@@ -692,6 +696,7 @@ void group_alloc_common(kc_ctx *ctx, int n_ranks, int rank, int k, uint64_t n_by
     G.seq = 0;
     G.done_pending = false;
     G.failed = false;
+    G.refused = false;
     G.tab_n_bytes = ~0ull;
     if (const char *e = std::getenv("KC_GROUP_TIMEOUT_MS")) G.timeout_ns = (u64) std::atoll(e) * 1000000ull;
 }
@@ -719,7 +724,14 @@ void group_detach(kc_ctx *ctx) {
 
 // Arena of one rank for a job of n_bytes: the owner-side levels over its hash range (two ping-pong generations of fixed slots, or
 // the exact construction's buffers), the node-dependent part of the overlap stage and the emission scratch.
-size_t group_arena_need(u64 n_bytes, int n_ranks, int limbs, bool complements, bool pessimistic) {
+// Inputs of KC_POS32_BYTES or more take the signature construction alone (`sig`: its plan at this size).  Its scratch is released
+// before the runs are counted (kc_grp_sig_flags), so a rank needs the larger of it and the overlap stage + emission of one GPU
+// (estimate_arena): the sequence, the flags and the code words live in the heap.  Ranks that share a device need this once each.
+size_t group_arena_need(u64 n_bytes, int n_ranks, int limbs, bool complements, bool pessimistic, const SigPlan *sig = nullptr) {
+    if (n_bytes >= KC_POS32_BYTES && sig && sig->ok) {
+        const double tail = overlap_emit_bytes(pessimistic ? n_bytes * 0.85 : n_bytes / 64.0 + 1e6, limbs, complements, n_bytes);
+        return (size_t) (std::max(tail, (double) kc_sig_group_arena_bytes(*sig, n_bytes, n_ranks)) * 1.1) + (256u << 20);
+    }
     const double owned = (double) n_bytes / n_ranks * 1.3 + (1u << 20);
     const double stage1 = owned * (8.0 * limbs + 4.0 + 2.0) * 4.0;
     const double c = complements ? 2.0 : 1.0;
@@ -747,18 +759,38 @@ template <int L> void group_compute_rank(kc_ctx *ctx, CudaExec &ex, const DevInp
     pol.fast = pol.fast && gp.ok && gp.recv_items() <= G.lay.recv_items;
     ExtFlags ext;
     ext.flags = reinterpret_cast<const u32 *>(G.heap + G.lay.off_flags);
-    const KcRoute route = kc_set_ladder(ctx->routes, pol, nb, *ex.arena, [&](KcRoute r) {
-        ext.cells4 = r == KC_ROUTE_SIG ? kc_grp_sig_flags<L>(G, ex, in.seq, nb, p.k, p.complements != 0, ctx->routes.sig)
-                                       : kc_grp_fast_flags<L>(G, ex, in.seq, nb, p.k, p.complements != 0, p.min_frequency, gp, ctx->routes.fast);
-        return ext.cells4 != nullptr;
-    }, [&](KcRoute) {
-        run_pipeline<L>(ctx, ex, in, p, res, &ext, false, (u32) G.rank, (u32) G.n);
-        if (ext.aborted && (ext.kept & 2u)) {
-            G.failed = true;
-            KC_THROW(KC_ERR_INTERNAL, "a rank of the group did not arrive (wait timed out)");
+    auto ladder = [&] {
+        return kc_set_ladder(ctx->routes, pol, nb, *ex.arena, [&](KcRoute r) {
+            ext.cells4 = r == KC_ROUTE_SIG ? kc_grp_sig_flags<L>(G, ex, in.seq, nb, p.k, p.complements != 0, ctx->routes.sig)
+                                           : kc_grp_fast_flags<L>(G, ex, in.seq, nb, p.k, p.complements != 0, p.min_frequency, gp, ctx->routes.fast);
+            return ext.cells4 != nullptr;
+        }, [&](KcRoute) {
+            run_pipeline<L>(ctx, ex, in, p, res, &ext, false, (u32) G.rank, (u32) G.n);
+            if (ext.aborted && (ext.kept & 2u)) {
+                G.failed = true;
+                KC_THROW(KC_ERR_INTERNAL, "a rank of the group did not arrive (wait timed out)");
+            }
+            return !ext.aborted;
+        });
+    };
+    KcRoute route = KC_ROUTE_NONE;
+    if (nb < KC_POS32_BYTES) {
+        route = ladder();
+    } else {
+        // The signature rung alone.  Its refusals (a bucket overflow, seen by every rank through the shared status word; too many
+        // runs or nodes, from totals every rank reads) come on every rank at the same point: the job is closed like a finished one,
+        // so that the sync numbers stay aligned and the next job waits for every rank's DONE as usual.
+        try {
+            route = ladder();
+        } catch (const KcError &e) {
+            if (e.code != KC_ERR_TOO_LARGE || G.failed) throw;
+            G.done_seq = ++G.seq;
+            kc_grp_signal(G, ex, G.done_seq);
+            G.done_pending = true;
+            G.refused = true;
+            throw;
         }
-        return !ext.aborted;
-    });
+    }
     if (route == KC_ROUTE_NONE) {
         ExtFlags exact;
         exact.flags = kc_grp_exact_flags<L>(G, ex, in.seq, nb, p.k, p.complements != 0, p.min_frequency, &exact.kept, &exact.n_occ);
@@ -767,6 +799,15 @@ template <int L> void group_compute_rank(kc_ctx *ctx, CudaExec &ex, const DevInp
     G.done_seq = ++G.seq;
     kc_grp_signal(G, ex, G.done_seq);
     G.done_pending = true;
+}
+
+// A group takes an input of KC_POS32_BYTES or more wherever one GPU does (check_large_input), through the same construction with
+// 64-bit positions, within the 32-bit bounds of its exchange (kc_grp_large_bound).  Every rank refuses from the same values, before
+// anything of the job is queued, so a refusal leaves the group in step.
+void group_check_large(const kc_ctx *ctx, const kc_params *p, u64 n_bytes, int n_ranks) {
+    if (n_bytes < KC_POS32_BYTES) return;
+    check_large_input(ctx, p, n_bytes);
+    if (const char *why = kc_grp_large_bound(n_bytes, n_ranks)) KC_THROW(KC_ERR_TOO_LARGE, why);
 }
 
 void group_check_job(kc_ctx *ctx, const kc_params *p, u64 n_bytes) {
@@ -779,6 +820,9 @@ void group_check_job(kc_ctx *ctx, const kc_params *p, u64 n_bytes) {
     if (p->assume_simplitigs || p->want_maxone) KC_THROW(KC_ERR_ARG, "the multi-GPU construction supports neither -S nor -M");
     if (kc_limbs_for_k(p->k) > G.lay.limbs) KC_THROW(KC_ERR_ARG, "the group heap was sized for a narrower k-mer word");
     if (n_bytes > G.lay.n_bytes_cap) KC_THROW(KC_ERR_TOO_LARGE, "the input exceeds the capacity the group heap was sized for");
+    if (G.lay.pos64() && n_bytes < KC_POS32_BYTES)
+        KC_THROW(KC_ERR_ARG, "the group heap was sized for inputs of 2^32 bytes or more (signature construction only); smaller inputs need a heap with a cap below 2^32");
+    group_check_large(ctx, p, n_bytes, G.n);
 }
 
 
@@ -1369,14 +1413,19 @@ int kc_group_compute_device(kc_ctx *ctx, const kc_params *p, const kc_input *in,
     DevInput di{in->seq, in->n_bytes, nullptr, nullptr, 0};
     DevResult res;
     // no retry with a larger arena here: a rank that repeated its job alone would leave the group's sync numbers behind
-    ensure_arena(ctx, group_arena_need(in->n_bytes, ctx->grp.n, limbs, p->complements != 0, false));
+    const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->routes.sig);
+    const size_t need = group_arena_need(in->n_bytes, ctx->grp.n, limbs, p->complements != 0, false, &sig);
+    ensure_arena(ctx, need);
+    if (in->n_bytes >= KC_POS32_BYTES && ctx->arena.cap < need) KC_THROW(KC_ERR_OOM, "the device cannot hold this rank's arena for an input of 2^32 bytes or more");
     ctx->arena.reset();
+    ctx->grp.refused = false;
     try {
         if (limbs == 1) group_compute_rank<1>(ctx, ex, di, *p, res);
         else if (limbs == 2) group_compute_rank<2>(ctx, ex, di, *p, res);
         else group_compute_rank<4>(ctx, ex, di, *p, res);
     } catch (const KcError &e) {
-        if (e.code != KC_ERR_EMPTY) ctx->grp.failed = true;  // "no k-mers" is found by every rank at the same point
+        // "no k-mers" and the refusals of group_compute_rank are found by every rank at the same point
+        if (e.code != KC_ERR_EMPTY && !ctx->grp.refused) ctx->grp.failed = true;
         throw;
     }
     KC_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -1407,16 +1456,21 @@ int kc_group_plan(int n_ranks, int rank, int k, uint64_t n_bytes, uint64_t *plan
     if (!plan || n_ranks < 1 || n_ranks > KC_MAX_PEERS || rank < 0 || rank >= n_ranks || k < 1 || k > 127) return KC_ERR_ARG;
     const u64 tile = kc_shard_granule(k);
     KsfTuning tune;
+    if (n_bytes >= KC_POS32_BYTES) {  // the signature construction alone (default options), within the group's 32-bit bounds
+        const SigTuning sig;
+        if (k < 26 || !kc_sig_plan(n_bytes, k, sig).ok || kc_grp_large_bound(n_bytes, n_ranks)) return KC_ERR_TOO_LARGE;
+    }
     const KsfGroupPlan gp = kc_ksf_group_plan(n_bytes, n_ranks, tile, tune);
+    const bool fixed = gp.ok && n_bytes < KC_POS32_BYTES;  // the fixed slots move 32-bit positions
     const GrpLayout lay = kc_grp_layout(n_bytes, kc_limbs_for_k(k), n_ranks, false, tile, tune);
     const u64 tiles = kc_div_up(n_bytes, tile);
-    plan[0] = gp.ok ? 1 : 0;
+    plan[0] = fixed ? 1 : 0;
     plan[1] = std::min<u64>(n_bytes, tiles * (u64) rank / (u64) n_ranks * tile);
     plan[2] = std::min<u64>(n_bytes, tiles * (u64) (rank + 1) / (u64) n_ranks * tile);
-    plan[3] = gp.ok ? gp.dig_begin(rank) : (u64) ((rank * 256 + n_ranks - 1) / n_ranks);
-    plan[4] = gp.ok ? gp.dig_begin(rank + 1) : (u64) (((rank + 1) * 256 + n_ranks - 1) / n_ranks);
-    plan[5] = gp.ok ? gp.n_digits : 256;
-    plan[6] = gp.cap_sub;
+    plan[3] = fixed ? gp.dig_begin(rank) : (u64) ((rank * 256 + n_ranks - 1) / n_ranks);
+    plan[4] = fixed ? gp.dig_begin(rank + 1) : (u64) (((rank + 1) * 256 + n_ranks - 1) / n_ranks);
+    plan[5] = fixed ? gp.n_digits : 256;
+    plan[6] = n_bytes < KC_POS32_BYTES ? gp.cap_sub : 0;
     plan[7] = lay.total;
     return KC_OK;
 }
@@ -1508,13 +1562,15 @@ int kc_group_compute(kc_group *g, const kc_params *p, const kc_input *in, kc_out
     try {
         check_params(p);
         if (p->assume_simplitigs || p->want_maxone) KC_THROW(KC_ERR_ARG, "the multi-GPU construction supports neither -S nor -M");
-        if (in->n_bytes >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "more than 2^32 sequence bytes");
+        const bool large = in->n_bytes >= KC_POS32_BYTES;
+        for (int r = 0; r < g->n; ++r) group_check_large(g->ctx[r], p, in->n_bytes, g->n);  // options are per rank
         const int limbs = kc_limbs_for_k(p->k);
-        // (re)build the heaps when the job does not fit the ones in place
+        // (re)build the heaps when the job does not fit the ones in place; a heap for inputs of 2^32 bytes or more takes no smaller job
         const KcGroup &G0 = c0->grp;
-        if (!G0.attached() || in->n_bytes > G0.lay.n_bytes_cap || limbs > G0.lay.limbs || G0.failed) {
+        if (!G0.attached() || in->n_bytes > G0.lay.n_bytes_cap || limbs > G0.lay.limbs || G0.failed || (G0.lay.pos64() && !large)) {
             group_release_heaps(g);
-            const u64 cap = std::min<u64>(0xFFFFFFE0ULL, in->n_bytes + in->n_bytes / 16 + (1u << 20));
+            const u64 want = in->n_bytes + in->n_bytes / 16 + (1u << 20);
+            const u64 cap = large ? want : std::min<u64>(0xFFFFFFE0ULL, want);
             for (int r = 0; r < g->n; ++r) {
                 g->ctx[r]->routes.fast = c0->routes.fast;  // one plan for the whole group
                 g->ctx[r]->routes.heuristics = c0->routes.heuristics;
@@ -1533,15 +1589,24 @@ int kc_group_compute(kc_group *g, const kc_params *p, const kc_input *in, kc_out
         }
         // every allocation happens BEFORE the first kernel of the job is queued anywhere: cudaMalloc / cudaFree wait for the whole
         // device, which would include a peer rank's wait kernel when two ranks share a GPU (tests)
-        {   // (one thread per rank: cudaMalloc of tens of GB takes ~0.1 s per device)
+        {   // (one thread per rank: cudaMalloc of tens of GB takes ~0.1 s per device; ranks that share a device take turns, so that
+            //  each one sees what the others took)
             KcError errs[KC_MAX_PEERS];
             bool bad[KC_MAX_PEERS] = {};
+            std::mutex dev_mutex[KC_MAX_DEVICES];
             std::vector<std::thread> th;
             for (int r = 0; r < g->n; ++r)
                 th.emplace_back([&, r] {
                     try {
-                        KC_CUDA(cudaSetDevice(g->ctx[r]->device));
-                        ensure_arena(g->ctx[r], group_arena_need(in->n_bytes, g->n, limbs, p->complements != 0, false));
+                        kc_ctx *ctx = g->ctx[r];
+                        std::lock_guard<std::mutex> lk(dev_mutex[ctx->device % KC_MAX_DEVICES]);
+                        KC_CUDA(cudaSetDevice(ctx->device));
+                        const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->routes.sig);
+                        const size_t need = group_arena_need(in->n_bytes, g->n, limbs, p->complements != 0, false, &sig);
+                        ensure_arena(ctx, need);
+                        // a rank that ran out of arena half way would strand the others: refuse before anything is queued
+                        if (large && ctx->arena.cap < need)
+                            KC_THROW(KC_ERR_OOM, "the device cannot hold every rank's arena for an input of 2^32 bytes or more (ranks sharing a device need it once each)");
                     } catch (const KcError &e) {
                         errs[r] = e;
                         bad[r] = true;
@@ -1570,6 +1635,7 @@ int kc_group_compute(kc_group *g, const kc_params *p, const kc_input *in, kc_out
             KC_CUDA(cudaSetDevice(ctx->device));
             KcGroup &G = ctx->grp;
             ctx->arena.reset();
+            G.refused = false;
             CudaExec ex{ctx->stream, &ctx->arena};
             ex.prof = &ctx->prof;
             ex.pinned = ctx->pin_small;
@@ -1623,7 +1689,8 @@ int kc_group_compute(kc_group *g, const kc_params *p, const kc_input *in, kc_out
             char buf[512];
             std::snprintf(buf, sizeof(buf), "rank %d: %s (%s:%d)", r, e.what, e.file, e.line);
             R.what = buf;
-            if (e.code != KC_ERR_EMPTY) {  // "no k-mers" is found by every rank at the same point; anything else strands the others
+            // "no k-mers" and the refusals of group_compute_rank are found by every rank at the same point; anything else strands the others
+            if (e.code != KC_ERR_EMPTY && !ctx->grp.refused) {
                 ctx->grp.failed = true;
                 g->hs.abort();
             }
@@ -1638,9 +1705,11 @@ int kc_group_compute(kc_group *g, const kc_params *p, const kc_input *in, kc_out
     for (int r = 1; r < g->n; ++r) th.emplace_back(worker, r);
     worker(0);
     for (auto &t : th) t.join();
+    bool all_refused = true;
+    for (int r = 0; r < g->n; ++r) all_refused = all_refused && g->ctx[r]->grp.refused;
     for (int r = 0; r < g->n; ++r)
         if (ro[r].code != KC_OK) {
-            if (ro[r].code != KC_ERR_EMPTY)
+            if (ro[r].code != KC_ERR_EMPTY && !all_refused)
                 for (int s = 0; s < g->n; ++s) g->ctx[s]->grp.failed = true;
             g->last_error = ro[r].what;
             c0->last_error = ro[r].what;

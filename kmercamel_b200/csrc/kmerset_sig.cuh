@@ -672,6 +672,7 @@ template <int L> struct SigKernels {
     typedef SigCfg<L> Cfg;
     struct Dev {
         int n_sm = 0, occ = 0;
+        int occ_multi64 = 0;  // the group's instance for inputs of 2^32 bytes or more
     };
     static const Dev &prepare() {
         static KcDevOnce once;
@@ -683,8 +684,11 @@ template <int L> struct SigKernels {
             KC_CUDA(cudaFuncSetAttribute(kc_sig_resolve_kernel<L, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::smem()));
             KC_CUDA(cudaFuncSetAttribute(kc_sig_resolve_kernel<L, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::smem(true)));
             KC_CUDA(cudaFuncSetAttribute(kc_sig_resolve_kernel<L, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::smem(true)));
+            KC_CUDA(cudaFuncSetAttribute(kc_sig_resolve_kernel<L, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::smem(true)));
+            KC_CUDA(cudaFuncSetAttribute(kc_sig_resolve_kernel<L, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::smem(true)));
             dev[dv].n_sm = kc_sm_count(dv);
             KC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&dev[dv].occ, kc_sig_resolve_kernel<L, false, false>, Cfg::THREADS, Cfg::smem()));
+            KC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&dev[dv].occ_multi64, kc_sig_resolve_kernel<L, true, false, true>, Cfg::THREADS, Cfg::smem(true)));
         });
         return dev[d];
     }
@@ -771,10 +775,32 @@ inline u32 kc_sig_sub_cap(const SigPlan &pl, int n_ranks) {
 }
 inline u32 kc_sig_owned_buckets(u32 n_buckets, int n_ranks, int rank) { return (n_buckets + (u32) n_ranks - 1u - (u32) rank) / (u32) n_ranks; }
 
-// Records one (sender, owner) stream must hold: the pair's share of the slice's records + 15 % + slack.
-inline u32 kc_sig_region_cap(u64 n_bytes, int n_ranks) {
+// Records one (sender, owner) stream must hold: the pair's share of the slice's records + 15 % + slack.  The kernels take it as a
+// u32: kc_grp_large_bound (group.cuh) refuses the inputs where it reaches 2^32.
+inline u64 kc_sig_region_cap(u64 n_bytes, int n_ranks) {
     const double per_pair = (double) n_bytes / n_ranks / KC_SIG_WINDOWS_PER_RECORD / n_ranks;
-    return (u32) (((u64) (per_pair * 1.15) + 8192 + 31) / 32 * 32);
+    return ((u64) (per_pair * 1.15) + 8192 + 31) / 32 * 32;
+}
+// Records the dense stream of a slice of slice_bytes may hold (kc_sig_compact_kernel reports more through the status word).
+inline u64 kc_sig_dense_cap(u64 slice_bytes, int n_ranks) { return (u64) (slice_bytes / KC_SIG_WINDOWS_PER_RECORD * 1.3) + (u64) n_ranks * 8192 + 65536; }
+// The most buckets any plan gives an input of up to n_bytes: kc_sig_plan keeps at least 32 records per bucket and fewer than 2^27 buckets.
+inline u64 kc_sig_max_buckets(u64 n_bytes) {
+    const u64 nb = (u64) ((double) n_bytes / (32.0 * KC_SIG_WINDOWS_PER_RECORD)) + 1;
+    return nb < 64 ? 64 : (nb < (1u << 27) ? nb : (1u << 27));
+}
+// Bytes of the largest slice of the tiles a rank of n_ranks scans (kc_sig_group_scan).
+inline u64 kc_sig_max_slice(u64 n_bytes, int n_ranks) {
+    constexpr u64 TILE = 256 * KC_EX_STRIP;
+    const u64 tiles = (n_bytes + TILE - 1) / TILE;
+    return std::min<u64>(n_bytes, (tiles + (u64) n_ranks - 1) / (u64) n_ranks * TILE);
+}
+
+// Arena bytes of kc_grp_sig_flags on one rank: bucket counters, records staged per bucket, owner-major offsets and the dense stream
+// of its slice (kc_sig_group_scan), then the gathered rows of the buckets it owns (kc_sig_group_resolve), + scan scratch.
+inline u64 kc_sig_group_arena_bytes(const SigPlan &p, u64 n_bytes, int n_ranks) {
+    const u64 nb = p.n_buckets, nbr = (nb + (u64) n_ranks - 1) / (u64) n_ranks;
+    const u64 scan = nb * 4 + nb * kc_sig_sub_cap(p, n_ranks) * 8 + ((u64) n_ranks * nbr + 1) * 8 + kc_sig_dense_cap(kc_sig_max_slice(n_bytes, n_ranks), n_ranks) * 8;
+    return scan + nbr * (4 + 8 * (u64) KC_SIG_REC_CAP) + (64u << 20);
 }
 
 // The scan of this rank's slice of the tiles (records staged per bucket, code words and valid-window words to every rank), then the
@@ -801,7 +827,7 @@ inline void kc_sig_group_scan(CudaExec &ex, const u8 *seq, u64 n_bytes, int k, c
     ++ex.launches;
     KC_CUDA(cudaGetLastError());
     ex.exclusive_scan_nosync(off_om, off_om, (u64) n_om + 1);
-    const u64 dense_cap = (u64) (slice_bytes / KC_SIG_WINDOWS_PER_RECORD * 1.3) + (u64) sp.n * 8192 + 65536;
+    const u64 dense_cap = kc_sig_dense_cap(slice_bytes, sp.n);
     u64 *dense = ex.alloc<u64>(dense_cap);
     {
         const u64 rec_bytes = (u64) (slice_bytes * 8 / KC_SIG_WINDOWS_PER_RECORD);
@@ -834,7 +860,12 @@ void kc_sig_group_resolve(CudaExec &ex, const u64 *packed, int k, bool complemen
         KC_CUDA(cudaGetLastError());
     }
     CudaExec::Scope sc(ex, KP_KS_RESOLVE, (u64) (n_bytes / n_ranks * (8 + 8 * Cfg::NW) / KC_SIG_WINDOWS_PER_RECORD));
-    if (complements)
+    if (n_bytes > 0xFFFFFFFFULL) {  // a window END position may need more than 32 bits (as in kc_kmerset_build_sig)
+        const u32 fit64 = (u32) (dv.n_sm * (dv.occ_multi64 > 0 ? dv.occ_multi64 : 1));
+        auto *kern = complements ? kc_sig_resolve_kernel<L, true, false, true> : kc_sig_resolve_kernel<L, true, true, true>;
+        kern<<<n_owned < fit64 ? n_owned : fit64, Cfg::THREADS, Cfg::smem(true), ex.stream>>>(packed, k, cnt_bm, recs_bm, n_owned, all_flags, reinterpret_cast<kc_ull *>(cells),
+                                                                                         reinterpret_cast<u32 *>(cells + 3), (u32) n_ranks, KC_SIG_REC_CAP, 0u);
+    } else if (complements)
         kc_sig_resolve_kernel<L, true, false><<<grid, Cfg::THREADS, Cfg::smem(), ex.stream>>>(packed, k, cnt_bm, recs_bm, n_owned, all_flags, reinterpret_cast<kc_ull *>(cells),
                                                                                             reinterpret_cast<u32 *>(cells + 3), (u32) n_ranks, KC_SIG_REC_CAP, 0u);
     else
