@@ -19,10 +19,12 @@
 #include "tail_spec.cuh"
 
 #include <chrono>
+#include <exception>
 #include <mutex>
 #include <new>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 static double kc_now_ms() {
@@ -34,17 +36,28 @@ static const bool kc_trace = std::getenv("KC_TRACE") != nullptr;
         if (kc_trace) std::fprintf(stderr, "[kc_trace] %-28s %.3f ms\n", (label), kc_now_ms()); \
     } while (0)
 
+// Page-locked host buffer, grown on demand and reused across calls.
+struct PinnedBuf {
+    u8 *p = nullptr;
+    size_t cap = 0;
+    unsigned flags = cudaHostAllocDefault;
+    void reserve(size_t need) {
+        if (cap >= need) return;
+        if (p) KC_CUDA(cudaFreeHost(p));
+        p = nullptr;
+        cap = 0;
+        KC_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&p), need + need / 8, flags));
+        cap = need + need / 8;
+    }
+};
+
 struct kc_ctx {
     int device = 0;
     cudaStream_t stream = nullptr;
     bool own_stream = false;
     Arena arena;
     KernelProf prof;
-    // pinned host staging for kc_compute (grown on demand, reused across calls)
-    u8 *pin_in = nullptr;
-    size_t pin_in_cap = 0;
-    u8 *pin_out = nullptr;
-    size_t pin_out_cap = 0;
+    PinnedBuf pin_out;  // the host results of kc_compute, kc_streaming and kc_maskopt
     static const size_t KC_PIN_SMALL = 4096;
     u8 *pin_small = nullptr;  // page-locked scratch for the small synchronising read-backs (CudaExec::read_n)
     cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
@@ -92,6 +105,33 @@ void set_error(kc_ctx *ctx, const KcError &e) {
         if (ctx) (ctx)->last_error = "unknown failure";                \
         return KC_ERR_INTERNAL;                                        \
     }
+
+// The state of one call on a context: its device is made current, and `ex` runs on the context's stream, arena, profiler and
+// pinned scratch.  The call's launches and read-backs are added to the context's totals when it returns; a failed call (one that
+// leaves by an exception) adds nothing.
+struct CallFrame {
+    kc_ctx *ctx;
+    CudaExec ex{ctx->stream, &ctx->arena};
+    const int exceptions = std::uncaught_exceptions();
+    explicit CallFrame(kc_ctx *c) : ctx(c) {
+        KC_CUDA(cudaSetDevice(c->device));
+        ex.prof = &c->prof;
+        ex.pinned = c->pin_small;
+        ex.pinned_cap = c->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
+    }
+    ~CallFrame() {
+        if (std::uncaught_exceptions() > exceptions) return;
+        ctx->total_launches += ex.launches;
+        ctx->read_backs += ex.read_backs;
+    }
+};
+
+// f(std::integral_constant<int, L>()) for the k-mer word of `limbs` 64-bit limbs (kc_limbs_for_k: 1, 2 or 4).
+template <class F> decltype(auto) with_limbs(int limbs, F &&f) {
+    if (limbs == 1) return f(std::integral_constant<int, 1>());
+    if (limbs == 2) return f(std::integral_constant<int, 2>());
+    return f(std::integral_constant<int, 4>());
+}
 
 void check_params(const kc_params *p) {
     if (!p) KC_THROW(KC_ERR_ARG, "params is NULL");
@@ -163,9 +203,15 @@ size_t estimate_arena(u64 n_bytes, u64 n_recs, int limbs, bool complements, bool
     return (size_t) total;
 }
 
-// Runs body() with an arena of `need` bytes; if the arena is exhausted (more nodes than the estimate assumed) the call is
-// repeated once with `need_max`.
-template <class F> void run_with_arena(kc_ctx *ctx, size_t need, size_t need_max, F body) {
+// Runs body() with an arena of estimate_arena's bytes for this input; if the arena is exhausted (more nodes than the estimate
+// assumed) the call is repeated once with the pessimistic estimate.
+template <class F> void run_with_arena(kc_ctx *ctx, const kc_params &p, const kc_input &in, F body) {
+    const SigPlan sig = kc_sig_plan(in.n_bytes, p.k, ctx->routes.sig);
+    auto estimate = [&](bool pessimistic) {
+        return estimate_arena(in.n_bytes, in.n_recs, kc_limbs_for_k(p.k), p.complements != 0, p.assume_simplitigs != 0, pessimistic,
+                              &ctx->routes.fast, &sig);
+    };
+    const size_t need = estimate(false), need_max = estimate(true);
     ensure_arena(ctx, (size_t) ((double) need * ctx->arena_estimate_ppm / 1e6));
     try {
         ctx->arena.reset();
@@ -191,8 +237,62 @@ struct DevInput {
 struct DevResult {
     const u8 *ms = nullptr, *maxone = nullptr;
     u64 length = 0, n_kmers = 0, n_occ = 0, n_nodes = 0, n_simplitigs = 0;
-    u64 lower_bound = 0;  // only with run_pipeline(..., lower_bound = true)
+    u64 lower_bound = 0;  // only with run_tail(..., lower_bound = true)
     u64 slice_begin = 0, slice_len = 0;
+};
+
+// Host -> device: the sequence and, with `records` (-S), the records.  The 64 bytes past n_bytes are never written: every loader
+// of the from-FASTA path is bounded by n_bytes (kc_compute_device gets a caller's buffer without them).  With `chunks`, a large
+// from-FASTA input goes in chunks on the copy stream: the level-0 partition pass of chunk c starts as soon as chunk c has landed
+// (InputChunks), instead of after the whole copy.  The returned input carries `chunks` when it was used.
+DevInput upload_input(kc_ctx *ctx, CudaExec &ex, const kc_input *in, bool records, InputChunks *chunks) {
+    u8 *d_seq = ex.alloc<u8>(in->n_bytes + 64);
+    if (records || in->n_bytes < (8u << 20)) chunks = nullptr;
+    if (chunks) {
+        if (!ctx->copy_stream) {
+            KC_CUDA(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
+            for (int c = 0; c < kc_ctx::KC_H2D_CHUNKS; ++c) KC_CUDA(cudaEventCreateWithFlags(&ctx->chunk_ev[c], cudaEventDisableTiming));
+        }
+        const u64 granule = 32768;  // whole level-0 tiles for every word width
+        chunks->chunk_bytes = (in->n_bytes / kc_ctx::KC_H2D_CHUNKS + granule) / granule * granule;
+        chunks->ev = ctx->chunk_ev;
+        if (ctx->arena.poison >= 0) {  // the copy must land after the poison fill of d_seq on the context stream
+            KC_CUDA(cudaEventRecord(ctx->ev[5], ctx->stream));
+            KC_CUDA(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev[5], 0));
+        }
+        for (u64 off = 0; off < in->n_bytes; off += chunks->chunk_bytes) {
+            const u64 len = std::min<u64>(chunks->chunk_bytes, in->n_bytes - off);
+            KC_CUDA(cudaMemcpyAsync(d_seq + off, in->seq + off, len, cudaMemcpyHostToDevice, ctx->copy_stream));
+            KC_CUDA(cudaEventRecord(ctx->chunk_ev[chunks->n++], ctx->copy_stream));
+        }
+    } else {
+        KC_CUDA(cudaMemcpyAsync(d_seq, in->seq, in->n_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    }
+    u64 *d_off = nullptr, *d_len = nullptr;
+    if (records) {
+        d_off = ex.alloc<u64>(in->n_recs);
+        d_len = ex.alloc<u64>(in->n_recs);
+        KC_CUDA(cudaMemcpyAsync(d_off, in->rec_off, in->n_recs * 8, cudaMemcpyHostToDevice, ctx->stream));
+        KC_CUDA(cudaMemcpyAsync(d_len, in->rec_len, in->n_recs * 8, cudaMemcpyHostToDevice, ctx->stream));
+    }
+    return DevInput{d_seq, in->n_bytes, d_off, d_len, in->n_recs, chunks};
+}
+
+// Host -> device for the mask passes: n bytes, then '\n' from the last whole 32-byte word on through 64 bytes past the end.
+u8 *upload_padded(CudaExec &ex, const u8 *src, u64 n) {
+    const u64 padded = (n + 31) / 32 * 32 + 64;
+    u8 *d = ex.alloc<u8>(padded);
+    ex.fill_bytes(d + (n & ~(u64) 31), '\n', padded - (n & ~(u64) 31));
+    if (n) KC_CUDA(cudaMemcpyAsync(d, src, n, cudaMemcpyHostToDevice, ex.stream));
+    return d;
+}
+
+// What stage 1 hands to run_tail: the nodes (first-occurrence runs, or with -S the records), the kept distinct k-mers U, the k-mer
+// occurrences and, for -M, the sorted k-mer set (kMersDict of src/global.h:165-167).
+template <int L> struct Stage1 {
+    RunNodes nodes;
+    u64 U = 0, n_occ = 0;
+    KWord<L> *uniq = nullptr;
 };
 
 // Stage 1 alone.  Leaves the sorted distinct k-mers (and their counts) at the current arena top and returns them.
@@ -312,8 +412,8 @@ u32 run_tail_spec(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params
 // spec_res != nullptr: after the signature construction, try the speculative tail (run_tail_spec).  When it holds, *spec_res is the whole
 // result and *spec_done is set; otherwise the runs are counted as if it had not been tried, on the same flags.
 template <int L>
-u64 run_stage1_runs(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &p, RunNodes *runs, KWord<L> **set_out, u64 *n_occ,
-                    DevResult *spec_res, bool *spec_done) {
+Stage1<L> run_stage1_runs(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &p, DevResult *spec_res, bool *spec_done) {
+    Stage1<L> s;
     KC_CUDA(cudaEventRecord(ctx->ev[0], ex.stream));
     KC_CUDA(cudaEventRecord(ctx->ev[1], ex.stream));  // extraction is fused into the partition passes
     KC_TRACE_POINT("stage1: begin");
@@ -350,13 +450,13 @@ u64 run_stage1_runs(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_para
                 ex.fill_bytes(cells4 + 1, 0, 8);
             }
         }
-        if (!aborted) *runs = kc_runs_from_flags(ex, flags, nb, p.k, cells4, hc, 4, &aborted);
+        if (!aborted) s.nodes = kc_runs_from_flags(ex, flags, nb, p.k, cells4, hc, 4, &aborted);
         if (aborted) ex.fill_bytes(flags, 0, fwords * 4);  // incomplete: the next construction starts from clear bits
         return !aborted;
     };
     const KcRoute route = kc_set_ladder(ctx->routes, ctx->routes.compute_policy(p, nb), nb, *ex.arena, launch, consume);
     if (route != KC_ROUTE_NONE) {
-        if (*spec_done) return spec_res->n_kmers;
+        if (*spec_done) return s;
         // the timers charged the fixed-slot partition passes with M = n_bytes; now that M is known, correct the byte counts
         if (route == KC_ROUTE_FAST && ex.prof && ex.prof->enabled && nb > hc[2]) {
             const u64 d = (nb - hc[2]) * (sizeof(KWord<L>) + 4);
@@ -364,114 +464,51 @@ u64 run_stage1_runs(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_para
             ex.prof->bytes[KP_SORT_SCATTER] -= 2 * d * (u64) (plan.n_levels - 1);
             ex.prof->bytes[KP_KS_RESOLVE] -= d;
         }
-        *n_occ = hc[2];
-        *set_out = nullptr;
-        KC_CUDA(cudaEventRecord(ctx->ev[2], ex.stream));
-        return hc[2] ? hc[0] : 0;
+        s.n_occ = hc[2];
+        s.U = hc[2] ? hc[0] : 0;
+        return s;
     }
     // with -M the sorted k-mer set doubles as kMersDict of src/global.h:165-167; it stays at the arena bottom
     if (in.chunks) in.chunks->wait_all(ex.stream);
     KmerSet<L> set = kc_kmerset_build<L>(ex, in.seq, nb, p.k, p.complements != 0, p.min_frequency, flags, p.want_maxone != 0, cells);
     KC_TRACE_POINT("stage1: set built");
-    *n_occ = set.n_occ;
-    *set_out = set.keys;
-    if (set.n_occ == 0 || set.n_kept == 0) {
-        KC_CUDA(cudaEventRecord(ctx->ev[2], ex.stream));
-        return 0;
-    }
+    s.n_occ = set.n_occ;
+    s.uniq = set.keys;
+    if (set.n_occ == 0 || set.n_kept == 0) return s;
     if (p.want_maxone) {  // the KEYS path has read the count back already
         const u64 kept = set.n_kept;
         KC_CUDA(cudaMemcpyAsync(cells, &kept, 8, cudaMemcpyHostToDevice, ex.stream));
     }
     u64 host_cells[2];
-    *runs = kc_runs_from_flags(ex, flags, nb, p.k, cells, host_cells);
-    const u64 n_kept = p.want_maxone ? set.n_kept : host_cells[0];
+    s.nodes = kc_runs_from_flags(ex, flags, nb, p.k, cells, host_cells);
+    s.U = p.want_maxone ? set.n_kept : host_cells[0];
     KC_TRACE_POINT("stage1: runs built");
-    KC_CUDA(cudaEventRecord(ctx->ev[2], ex.stream));
-    return n_kept;
+    return s;
 }
 
-// First-occurrence flags that were built outside run_pipeline (multi-GPU construction, group.cuh).
-struct ExtFlags {
-    const u32 *flags = nullptr;
-    u64 kept = 0, n_occ = 0;   // totals, when they are known on the host already (exact path)
-    u64 *cells4 = nullptr;     // fast path: device words {kept, 0, M, status}, read back together with the run count
-    bool aborted = false;      // out: the status word was set (a slot overflowed somewhere): nothing was done
-};
-
+// From stage 1's outcome to the result: the sparse switch, the node ends, the overlap stage, then the lower bound or the emission
+// (of slice `slice_index` of `n_slices`).  Stage 1 ends here, at event 2.
 template <int L>
-void run_pipeline(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &p, DevResult &res, ExtFlags *ext = nullptr,
-                  bool lower_bound = false, u32 slice_index = 0, u32 n_slices = 1) {
+void run_tail(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &p, Stage1<L> s, DevResult &res, bool lower_bound,
+              u32 slice_index = 0, u32 n_slices = 1) {
     const bool complements = p.complements != 0;
-    KWord<L> *uniq = nullptr;
-    u8 *cnt = nullptr;
-    u64 U = 0, n_occ = 0;
+    KC_CUDA(cudaEventRecord(ctx->ev[2], ex.stream));
+    res.n_simplitigs = s.nodes.n_runs;
+    if (!p.assume_simplitigs) {
+        if (s.U == 0) KC_THROW(KC_ERR_EMPTY, "the input contains no k-mers");  // src/main.cpp:155-158
+        // src/main.cpp:94,175-181: simplitigs barely longer than k-mers -> the greedy runs on the k-mers themselves (PartialPreSort order)
+        if (ctx->sparse_switch && s.nodes.n_runs * 5 >= s.U) {
+            // one node per k-mer; kc_kmer_nodes_from_runs numbers them with 32-bit offsets (inputs of 2^32 bytes or more can have that many)
+            if (s.U * (complements ? 2 : 1) >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "too many nodes for one GPU");
+            s.nodes = kc_kmer_nodes_from_runs(ex, in.seq, s.nodes, p.k);
+        }
+        if (s.nodes.n_runs * (complements ? 2 : 1) >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "too many nodes for one GPU");
+    }
+    const u64 n_nodes = s.nodes.n_runs;
+    const u64 *node_off = s.nodes.rec_off, *node_len = s.nodes.rec_len;
     NodeView<L> nv;
-    NodeSeq<L> ns;
     nv.k = p.k;
     nv.complements = complements;
-    ns.k = p.k;
-    ns.kmers = nullptr;
-    ns.seq = in.seq;
-    ns.rec_off = in.rec_off;
-    ns.rec_len = in.rec_len;
-    u64 n_nodes = 0;
-    const u64 *node_off = in.rec_off, *node_len = in.rec_len;
-    if (in.chunks && (p.assume_simplitigs || ext)) in.chunks->wait_all(ex.stream);
-    if (!p.assume_simplitigs) {
-        RunNodes runs;
-        if (ext && ext->cells4) {  // multi-GPU fast path: totals and status arrive with the run count, in ONE read-back
-            u64 hc[4];
-            runs = kc_runs_from_flags(ex, ext->flags, in.n_bytes, p.k, ext->cells4, hc, 4, &ext->aborted);
-            if (ext->aborted) {
-                ext->kept = hc[3];  // the status word, for the caller's diagnosis
-                return;
-            }
-            U = hc[2] ? hc[0] : 0;
-            n_occ = hc[2];
-            KC_CUDA(cudaEventRecord(ctx->ev[2], ex.stream));
-        } else if (ext) {          // multi-GPU exact path
-            u64 *cells = ex.arena->alloc_top<u64>(2);
-            ex.fill_bytes(cells, 0, 16);
-            u64 host_cells[2];
-            runs = kc_runs_from_flags(ex, ext->flags, in.n_bytes, p.k, cells, host_cells);
-            U = runs.n_runs ? ext->kept : 0;
-            n_occ = ext->n_occ;
-            KC_CUDA(cudaEventRecord(ctx->ev[2], ex.stream));
-        } else {
-            // the speculative tail: a FASTA input with few runs (a genome) is computed behind one read-back (run_tail_spec)
-            const u64 nb = in.n_bytes;
-            const bool spec_failed = ctx->routes.heuristics && ctx->routes.tail.near(nb);
-            const bool spec = ctx->tail_spec && !spec_failed && !lower_bound && ctx->small_engine && nb > 0 && nb < KC_POS32_BYTES;
-            bool spec_done = false;
-            U = run_stage1_runs<L>(ctx, ex, in, p, &runs, &uniq, &n_occ, spec ? &res : nullptr, &spec_done);
-            if (spec_done) return;
-        }
-        if (U == 0) KC_THROW(KC_ERR_EMPTY, "the input contains no k-mers");  // src/main.cpp:155-158
-        res.n_simplitigs = runs.n_runs;
-        // src/main.cpp:94,175-181: simplitigs barely longer than k-mers -> the greedy runs on the k-mers themselves (PartialPreSort order)
-        if (ctx->sparse_switch && runs.n_runs * 5 >= U) {
-            // one node per k-mer; kc_kmer_nodes_from_runs numbers them with 32-bit offsets (inputs of 2^32 bytes or more can have that many)
-            if (U * (complements ? 2 : 1) >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "too many nodes for one GPU");
-            runs = kc_kmer_nodes_from_runs(ex, in.seq, runs, p.k);
-        }
-        n_nodes = runs.n_runs;
-        node_off = runs.rec_off;
-        node_len = runs.rec_len;
-        if (n_nodes * (complements ? 2 : 1) >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "too many nodes for one GPU");
-    } else {
-        if (in.n_recs == 0) KC_THROW(KC_ERR_EMPTY, "input cannot be empty");  // src/global.h:219-221
-        if (in.n_recs * (complements ? 2 : 1) >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "too many records for one GPU");
-        KC_CUDA(cudaEventRecord(ctx->ev[0], ex.stream));
-        if (p.want_maxone) {  // kMersDict of src/global.h:165-167 = every k-mer of the records
-            U = run_stage1<L>(ctx, ex, in, p, &uniq, &cnt, &n_occ);
-        } else {
-            KC_CUDA(cudaEventRecord(ctx->ev[1], ex.stream));
-            KC_CUDA(cudaEventRecord(ctx->ev[2], ex.stream));
-        }
-        n_nodes = in.n_recs;
-        res.n_simplitigs = in.n_recs;
-    }
     {
         KWord<L> *first = ex.alloc<KWord<L>>(n_nodes), *last = ex.alloc<KWord<L>>(n_nodes);
         u32 *err = ex.alloc<u32>(1);
@@ -483,10 +520,14 @@ void run_pipeline(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params
         nv.first = first;
         nv.last = last;
         nv.n = (u32) n_nodes;
-        ns.rec_off = node_off;
-        ns.rec_len = node_len;
     }
     nv.N = nv.n * (complements ? 2u : 1u);
+    NodeSeq<L> ns;
+    ns.k = p.k;
+    ns.kmers = nullptr;
+    ns.seq = in.seq;
+    ns.rec_off = node_off;
+    ns.rec_len = node_len;
     ns.n = nv.n;
     KC_TRACE_POINT("pipeline: nodes ready");
     Engine<CudaExec, L> eng(ex, nv, /*strict=*/p.assume_simplitigs != 0, lower_bound);
@@ -501,7 +542,7 @@ void run_pipeline(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params
         // In this mode every virtual node has an out-edge after d = 0, so no 255 is left among the overlaps.
         kc_ull *acc = reinterpret_cast<kc_ull *>(ex.alloc<u64>(2));
         ex.fill_bytes(acc, 0, 16);
-        const u64 *len = node_off == in.rec_off ? in.rec_len : node_len;
+        const u64 *len = node_len;
         const u8 *ovl = eng.st.ovl;
         const u32 n = nv.n;
         ex.for_each(nv.N, [=] __device__(u64 i) {
@@ -515,15 +556,15 @@ void run_pipeline(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params
         const u64 strands = complements ? 2 : 1;
         res.lower_bound = (h[0] * strands - h[1]) / strands;
         KC_CUDA(cudaEventRecord(ctx->ev[4], ex.stream));
-        res.n_kmers = U;
-        res.n_occ = n_occ;
+        res.n_kmers = s.U;
+        res.n_occ = s.n_occ;
         res.n_nodes = nv.n;
         return;
     }
     EmitResult er;
     try {
         // every character of the superstring is a character of some node: nodes are pieces of the input that overlap by < k
-        er = kc_emit_superstring<CudaExec, L>(ex, ns, nv, eng.st, uniq, U, p.want_maxone != 0, slice_index, n_slices, in.n_bytes + n_nodes * (u64) p.k + 16);
+        er = kc_emit_superstring<CudaExec, L>(ex, ns, nv, eng.st, s.uniq, s.U, p.want_maxone != 0, slice_index, n_slices, in.n_bytes + n_nodes * (u64) p.k + 16);
     } catch (const KcError &) {
         eng.check_small();  // a failed small-engine run is the cause, report that one
         throw;
@@ -536,15 +577,36 @@ void run_pipeline(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params
     res.length = er.length;
     res.slice_begin = er.slice_begin;
     res.slice_len = er.slice_len;
-    res.n_kmers = U;
-    res.n_occ = n_occ;
+    res.n_kmers = s.U;
+    res.n_occ = s.n_occ;
     res.n_nodes = nv.n;
 }
 
-void dispatch_pipeline(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &p, DevResult &res, bool lower_bound = false) {
-    if (p.k < 32) run_pipeline<1>(ctx, ex, in, p, res, nullptr, lower_bound);
-    else if (p.k < 64) run_pipeline<2>(ctx, ex, in, p, res, nullptr, lower_bound);
-    else run_pipeline<4>(ctx, ex, in, p, res, nullptr, lower_bound);
+// One GPU: stage 1 (the -S records, or the first-occurrence runs, behind which the speculative tail may finish the call), then
+// run_tail.
+template <int L> void run_pipeline(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &p, DevResult &res, bool lower_bound) {
+    Stage1<L> s;
+    if (p.assume_simplitigs) {
+        if (in.n_recs == 0) KC_THROW(KC_ERR_EMPTY, "input cannot be empty");  // src/global.h:219-221
+        if (in.n_recs * (p.complements ? 2 : 1) >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "too many records for one GPU");
+        KC_CUDA(cudaEventRecord(ctx->ev[0], ex.stream));
+        if (p.want_maxone) {  // kMersDict of src/global.h:165-167 = every k-mer of the records
+            u8 *cnt = nullptr;
+            s.U = run_stage1<L>(ctx, ex, in, p, &s.uniq, &cnt, &s.n_occ);
+        } else {
+            KC_CUDA(cudaEventRecord(ctx->ev[1], ex.stream));
+        }
+        s.nodes = RunNodes{in.rec_off, in.rec_len, in.n_recs};
+    } else {
+        // the speculative tail: a FASTA input with few runs (a genome) is computed behind one read-back (run_tail_spec)
+        const u64 nb = in.n_bytes;
+        const bool spec_failed = ctx->routes.heuristics && ctx->routes.tail.near(nb);
+        const bool spec = ctx->tail_spec && !spec_failed && !lower_bound && ctx->small_engine && nb > 0 && nb < KC_POS32_BYTES;
+        bool spec_done = false;
+        s = run_stage1_runs<L>(ctx, ex, in, p, spec ? &res : nullptr, &spec_done);
+        if (spec_done) return;
+    }
+    run_tail<L>(ctx, ex, in, p, s, res, lower_bound);
 }
 
 void fill_times(kc_ctx *ctx, kc_output *out) {
@@ -556,6 +618,28 @@ void fill_times(kc_ctx *ctx, kc_output *out) {
     if (cudaEventElapsedTime(&t, ctx->ev[3], ctx->ev[4]) == cudaSuccess) out->t.emit_ms = t;
     if (cudaEventElapsedTime(&t, ctx->ev[0], ctx->ev[4]) == cudaSuccess) out->t.total_ms = t;
     (void) cudaGetLastError();
+}
+
+// A call's result in the ABI's form, with the device pointers of `res` (kc_compute points them at its pinned copy).
+void fill_output(kc_ctx *ctx, const DevResult &res, u64 launches, kc_output *out) {
+    out->ms = const_cast<u8 *>(res.ms);
+    out->ms_maxone = const_cast<u8 *>(res.maxone);
+    out->length = res.length;
+    out->n_kmers = res.n_kmers;
+    out->n_occurrences = res.n_occ;
+    out->n_nodes = res.n_nodes;
+    out->n_simplitigs = res.n_simplitigs;
+    out->n_launches = launches;
+    fill_times(ctx, out);
+}
+
+// Device result -> the context's pinned host buffer; with -M the max-one mask follows the superstring there.
+u8 *copy_to_pinned(kc_ctx *ctx, const u8 *ms, const u8 *maxone, u64 n) {
+    ctx->pin_out.reserve((size_t) n * (maxone ? 2 : 1) + 64);
+    if (n) KC_CUDA(cudaMemcpyAsync(ctx->pin_out.p, ms, n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (maxone) KC_CUDA(cudaMemcpyAsync(ctx->pin_out.p + n, maxone, n, cudaMemcpyDeviceToHost, ctx->stream));
+    KC_CUDA(cudaStreamSynchronize(ctx->stream));
+    return ctx->pin_out.p;
 }
 
 template <int L>
@@ -757,20 +841,27 @@ template <int L> void group_compute_rank(kc_ctx *ctx, CudaExec &ex, const DevInp
     RoutePolicy pol = ctx->routes.compute_policy(p, nb);
     const KsfGroupPlan gp = kc_ksf_group_plan(nb, G.n, KsCfg<L>::EX_TILE, ctx->routes.fast);
     pol.fast = pol.fast && gp.ok && gp.recv_items() <= G.lay.recv_items;
-    ExtFlags ext;
-    ext.flags = reinterpret_cast<const u32 *>(G.heap + G.lay.off_flags);
+    const u32 *flags = reinterpret_cast<const u32 *>(G.heap + G.lay.off_flags);
+    u64 *cells4 = nullptr;  // device words {kept, 0, M, status}, read back together with the run count
     auto ladder = [&] {
         return kc_set_ladder(ctx->routes, pol, nb, *ex.arena, [&](KcRoute r) {
-            ext.cells4 = r == KC_ROUTE_SIG ? kc_grp_sig_flags<L>(G, ex, in.seq, nb, p.k, p.complements != 0, ctx->routes.sig)
-                                           : kc_grp_fast_flags<L>(G, ex, in.seq, nb, p.k, p.complements != 0, p.min_frequency, gp, ctx->routes.fast);
-            return ext.cells4 != nullptr;
+            cells4 = r == KC_ROUTE_SIG ? kc_grp_sig_flags<L>(G, ex, in.seq, nb, p.k, p.complements != 0, ctx->routes.sig)
+                                       : kc_grp_fast_flags<L>(G, ex, in.seq, nb, p.k, p.complements != 0, p.min_frequency, gp, ctx->routes.fast);
+            return cells4 != nullptr;
         }, [&](KcRoute) {
-            run_pipeline<L>(ctx, ex, in, p, res, &ext, false, (u32) G.rank, (u32) G.n);
-            if (ext.aborted && (ext.kept & 2u)) {
+            Stage1<L> s;
+            u64 hc[4];
+            bool aborted = false;  // the status word was set (a slot overflowed somewhere): nothing was done
+            s.nodes = kc_runs_from_flags(ex, flags, nb, p.k, cells4, hc, 4, &aborted);
+            if (aborted && (hc[3] & 2u)) {
                 G.failed = true;
                 KC_THROW(KC_ERR_INTERNAL, "a rank of the group did not arrive (wait timed out)");
             }
-            return !ext.aborted;
+            if (aborted) return false;
+            s.U = hc[2] ? hc[0] : 0;
+            s.n_occ = hc[2];
+            run_tail<L>(ctx, ex, in, p, s, res, false, (u32) G.rank, (u32) G.n);
+            return true;
         });
     };
     KcRoute route = KC_ROUTE_NONE;
@@ -791,10 +882,16 @@ template <int L> void group_compute_rank(kc_ctx *ctx, CudaExec &ex, const DevInp
             throw;
         }
     }
-    if (route == KC_ROUTE_NONE) {
-        ExtFlags exact;
-        exact.flags = kc_grp_exact_flags<L>(G, ex, in.seq, nb, p.k, p.complements != 0, p.min_frequency, &exact.kept, &exact.n_occ);
-        run_pipeline<L>(ctx, ex, in, p, res, &exact, false, (u32) G.rank, (u32) G.n);
+    if (route == KC_ROUTE_NONE) {  // the exact construction: its totals are on the host already
+        Stage1<L> s;
+        u64 kept = 0;
+        const u32 *xflags = kc_grp_exact_flags<L>(G, ex, in.seq, nb, p.k, p.complements != 0, p.min_frequency, &kept, &s.n_occ);
+        u64 *cells = ex.arena->alloc_top<u64>(2);
+        ex.fill_bytes(cells, 0, 16);
+        u64 host_cells[2];
+        s.nodes = kc_runs_from_flags(ex, xflags, nb, p.k, cells, host_cells);
+        s.U = s.nodes.n_runs ? kept : 0;
+        run_tail<L>(ctx, ex, in, p, s, res, false, (u32) G.rank, (u32) G.n);
     }
     G.done_seq = ++G.seq;
     kc_grp_signal(G, ex, G.done_seq);
@@ -825,6 +922,33 @@ void group_check_job(kc_ctx *ctx, const kc_params *p, u64 n_bytes) {
     group_check_large(ctx, p, n_bytes, G.n);
 }
 
+// Readies this rank's arena for a job (group_arena_need).  There is no retry with a larger arena: a rank that repeated its job alone
+// would leave the group's sync numbers behind.  A rank that ran out of arena half way would strand the others, so an input of
+// KC_POS32_BYTES or more whose arena the device cannot hold is refused with `refusal` before anything is queued.
+void group_prepare_arena(kc_ctx *ctx, const kc_params &p, u64 n_bytes, const char *refusal) {
+    const SigPlan sig = kc_sig_plan(n_bytes, p.k, ctx->routes.sig);
+    const size_t need = group_arena_need(n_bytes, ctx->grp.n, kc_limbs_for_k(p.k), p.complements != 0, false, &sig);
+    ensure_arena(ctx, need);
+    if (n_bytes >= KC_POS32_BYTES && ctx->arena.cap < need) KC_THROW(KC_ERR_OOM, refusal);
+}
+
+// Marks the group failed unless error `code` leaves it in step: "no k-mers" and the refusals of group_compute_rank are found by
+// every rank at the same point, anything else strands the other ranks.  Returns whether it did.
+bool group_fail(kc_ctx *ctx, int code) {
+    if (code == KC_ERR_EMPTY || ctx->grp.refused) return false;
+    ctx->grp.failed = true;
+    return true;
+}
+
+// This rank's job (group_compute_rank), at the word width of k.
+void group_run_job(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &p, DevResult &res) {
+    try {
+        with_limbs(kc_limbs_for_k(p.k), [&](auto l) { group_compute_rank<decltype(l)::value>(ctx, ex, in, p, res); });
+    } catch (const KcError &e) {
+        group_fail(ctx, e.code);
+        throw;
+    }
+}
 
 }  // namespace
 
@@ -871,8 +995,7 @@ void kc_destroy(kc_ctx *ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
     if (ctx->arena.base) cudaFree(ctx->arena.base);
-    if (ctx->pin_in) cudaFreeHost(ctx->pin_in);
-    if (ctx->pin_out) cudaFreeHost(ctx->pin_out);
+    if (ctx->pin_out.p) cudaFreeHost(ctx->pin_out.p);
     if (ctx->pin_small) cudaFreeHost(ctx->pin_small);
     group_detach(ctx);
     for (int i = 0; i < 6; ++i)
@@ -891,33 +1014,17 @@ int kc_compute_device(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_ou
     check_params(p);
     check_large_input(ctx, p, in->n_bytes);
     if ((reinterpret_cast<uintptr_t>(in->seq) & 15) != 0) KC_THROW(KC_ERR_ARG, "device sequence pointer must be 16-byte aligned");
-    KC_CUDA(cudaSetDevice(ctx->device));
-    const int limbs = kc_limbs_for_k(p->k);
-    CudaExec ex{ctx->stream, &ctx->arena};
-    ex.prof = &ctx->prof;
-    ex.pinned = ctx->pin_small;
-    ex.pinned_cap = ctx->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
+    CallFrame f(ctx);
     DevInput di{in->seq, in->n_bytes, in->rec_off, in->rec_len, in->n_recs};
     DevResult res;
     KC_TRACE_POINT("compute_device: start");
-    const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->routes.sig);
-    run_with_arena(ctx, estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, p->assume_simplitigs != 0, false, &ctx->routes.fast, &sig),
-                   estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, p->assume_simplitigs != 0, true, &ctx->routes.fast, &sig),
-                   [&] { dispatch_pipeline(ctx, ex, di, *p, res); });
+    run_with_arena(ctx, *p, *in, [&] {
+        with_limbs(kc_limbs_for_k(p->k), [&](auto l) { run_pipeline<decltype(l)::value>(ctx, f.ex, di, *p, res, false); });
+    });
     KC_TRACE_POINT("compute_device: launched");
     KC_CUDA(cudaStreamSynchronize(ctx->stream));
     KC_TRACE_POINT("compute_device: synced");
-    out->ms = const_cast<u8 *>(res.ms);
-    out->ms_maxone = const_cast<u8 *>(res.maxone);
-    out->length = res.length;
-    out->n_kmers = res.n_kmers;
-    out->n_occurrences = res.n_occ;
-    out->n_nodes = res.n_nodes;
-    out->n_simplitigs = res.n_simplitigs;
-    out->n_launches = ex.launches;
-    fill_times(ctx, out);
-    ctx->total_launches += ex.launches;
-    ctx->read_backs += ex.read_backs;
+    fill_output(ctx, res, f.ex.launches, out);
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -927,83 +1034,23 @@ int kc_compute(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_output *o
     KC_API_BEGIN
     check_params(p);
     check_large_input(ctx, p, in->n_bytes);
-    KC_CUDA(cudaSetDevice(ctx->device));
-    const int limbs = kc_limbs_for_k(p->k);
-    const bool simplitigs = p->assume_simplitigs != 0;
-    CudaExec ex{ctx->stream, &ctx->arena};
-    ex.prof = &ctx->prof;
-    ex.pinned = ctx->pin_small;
-    ex.pinned_cap = ctx->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
+    CallFrame f(ctx);
     DevResult res;
-    const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->routes.sig);
-    run_with_arena(ctx, estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, false, &ctx->routes.fast, &sig),
-                   estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, true, &ctx->routes.fast, &sig), [&] {
-        // host -> device.  Large from-FASTA inputs go in chunks on the copy stream: the level-0 partition pass of chunk c starts
-        // as soon as chunk c has landed (InputChunks), instead of after the whole copy.  The 64 bytes past n_bytes are never written:
-        // every loader of the from-FASTA path is bounded by n_bytes (kc_compute_device gets a caller's buffer without them).
-        u8 *d_seq = ex.alloc<u8>(in->n_bytes + 64);
+    run_with_arena(ctx, *p, *in, [&] {
         InputChunks chunks;
-        const bool chunked = !simplitigs && in->n_bytes >= (8u << 20);
-        if (chunked) {
-            if (!ctx->copy_stream) {
-                KC_CUDA(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-                for (int c = 0; c < kc_ctx::KC_H2D_CHUNKS; ++c) KC_CUDA(cudaEventCreateWithFlags(&ctx->chunk_ev[c], cudaEventDisableTiming));
-            }
-            const u64 granule = 32768;  // whole level-0 tiles for every word width
-            chunks.chunk_bytes = (in->n_bytes / kc_ctx::KC_H2D_CHUNKS + granule) / granule * granule;
-            chunks.ev = ctx->chunk_ev;
-            if (ctx->arena.poison >= 0) {  // the copy must land after the poison fill of d_seq on the context stream
-                KC_CUDA(cudaEventRecord(ctx->ev[5], ctx->stream));
-                KC_CUDA(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev[5], 0));
-            }
-            for (u64 off = 0; off < in->n_bytes; off += chunks.chunk_bytes) {
-                const u64 len = std::min<u64>(chunks.chunk_bytes, in->n_bytes - off);
-                KC_CUDA(cudaMemcpyAsync(d_seq + off, in->seq + off, len, cudaMemcpyHostToDevice, ctx->copy_stream));
-                KC_CUDA(cudaEventRecord(ctx->chunk_ev[chunks.n++], ctx->copy_stream));
-            }
-        } else {
-            KC_CUDA(cudaMemcpyAsync(d_seq, in->seq, in->n_bytes, cudaMemcpyHostToDevice, ctx->stream));
-        }
-        u64 *d_off = nullptr, *d_len = nullptr;
-        if (simplitigs) {
-            d_off = ex.alloc<u64>(in->n_recs);
-            d_len = ex.alloc<u64>(in->n_recs);
-            KC_CUDA(cudaMemcpyAsync(d_off, in->rec_off, in->n_recs * 8, cudaMemcpyHostToDevice, ctx->stream));
-            KC_CUDA(cudaMemcpyAsync(d_len, in->rec_len, in->n_recs * 8, cudaMemcpyHostToDevice, ctx->stream));
-        }
-        DevInput di{d_seq, in->n_bytes, d_off, d_len, in->n_recs, chunked ? &chunks : nullptr};
+        const DevInput di = upload_input(ctx, f.ex, in, p->assume_simplitigs != 0, &chunks);
         try {
-            dispatch_pipeline(ctx, ex, di, *p, res);
+            with_limbs(kc_limbs_for_k(p->k), [&](auto l) { run_pipeline<decltype(l)::value>(ctx, f.ex, di, *p, res, false); });
         } catch (...) {
-            if (chunked) cudaStreamSynchronize(ctx->copy_stream);  // `chunks` and the caller's buffer must outlive the copy
+            if (di.chunks) cudaStreamSynchronize(ctx->copy_stream);  // `chunks` and the caller's buffer must outlive the copy
             throw;
         }
-        if (chunked) chunks.wait_all(ctx->stream);
+        if (di.chunks) chunks.wait_all(ctx->stream);
     });
-    // device -> pinned host
-    const size_t need = (size_t) res.length * (res.maxone ? 2 : 1) + 64;
-    if (ctx->pin_out_cap < need) {
-        if (ctx->pin_out) KC_CUDA(cudaFreeHost(ctx->pin_out));
-        ctx->pin_out = nullptr;
-        ctx->pin_out_cap = 0;
-        KC_CUDA(cudaMallocHost(&ctx->pin_out, need + need / 8));
-        ctx->pin_out_cap = need + need / 8;
-    }
-    KC_CUDA(cudaMemcpyAsync(ctx->pin_out, res.ms, res.length, cudaMemcpyDeviceToHost, ctx->stream));
-    if (res.maxone)
-        KC_CUDA(cudaMemcpyAsync(ctx->pin_out + res.length, res.maxone, res.length, cudaMemcpyDeviceToHost, ctx->stream));
-    KC_CUDA(cudaStreamSynchronize(ctx->stream));
-    out->ms = ctx->pin_out;
-    out->ms_maxone = res.maxone ? ctx->pin_out + res.length : nullptr;
-    out->length = res.length;
-    out->n_kmers = res.n_kmers;
-    out->n_occurrences = res.n_occ;
-    out->n_nodes = res.n_nodes;
-    out->n_simplitigs = res.n_simplitigs;
-    out->n_launches = ex.launches;
-    fill_times(ctx, out);
-    ctx->total_launches += ex.launches;
-    ctx->read_backs += ex.read_backs;
+    u8 *host = copy_to_pinned(ctx, res.ms, res.maxone, res.length);
+    fill_output(ctx, res, f.ex.launches, out);
+    out->ms = host;
+    out->ms_maxone = res.maxone ? host + res.length : nullptr;
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -1014,59 +1061,17 @@ int kc_lower_bound(kc_ctx *ctx, const kc_params *p, const kc_input *in, uint64_t
     check_params(p);
     if (p->want_maxone) KC_THROW(KC_ERR_ARG, "lowerbound has no mask output");
     check_large_input(ctx, p, in->n_bytes);
-    KC_CUDA(cudaSetDevice(ctx->device));
-    const int limbs = kc_limbs_for_k(p->k);
-    const bool simplitigs = p->assume_simplitigs != 0;
-    CudaExec ex{ctx->stream, &ctx->arena};
-    ex.prof = &ctx->prof;
-    ex.pinned = ctx->pin_small;
-    ex.pinned_cap = ctx->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
+    CallFrame f(ctx);
     DevResult res;
-    const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->routes.sig);
-    run_with_arena(ctx, estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, false, &ctx->routes.fast, &sig),
-                   estimate_arena(in->n_bytes, in->n_recs, limbs, p->complements != 0, simplitigs, true, &ctx->routes.fast, &sig), [&] {
-        u8 *d_seq = ex.alloc<u8>(in->n_bytes + 64);
-        KC_CUDA(cudaMemcpyAsync(d_seq, in->seq, in->n_bytes, cudaMemcpyHostToDevice, ctx->stream));
-        u64 *d_off = nullptr, *d_len = nullptr;
-        if (simplitigs) {
-            d_off = ex.alloc<u64>(in->n_recs);
-            d_len = ex.alloc<u64>(in->n_recs);
-            KC_CUDA(cudaMemcpyAsync(d_off, in->rec_off, in->n_recs * 8, cudaMemcpyHostToDevice, ctx->stream));
-            KC_CUDA(cudaMemcpyAsync(d_len, in->rec_len, in->n_recs * 8, cudaMemcpyHostToDevice, ctx->stream));
-        }
-        DevInput di{d_seq, in->n_bytes, d_off, d_len, in->n_recs};
-        dispatch_pipeline(ctx, ex, di, *p, res, /*lower_bound=*/true);
+    run_with_arena(ctx, *p, *in, [&] {
+        const DevInput di = upload_input(ctx, f.ex, in, p->assume_simplitigs != 0, nullptr);
+        with_limbs(kc_limbs_for_k(p->k), [&](auto l) { run_pipeline<decltype(l)::value>(ctx, f.ex, di, *p, res, true); });
     });
     KC_CUDA(cudaStreamSynchronize(ctx->stream));
     *lower_bound = res.lower_bound;
-    if (stats) {
-        std::memset(stats, 0, sizeof(*stats));
-        stats->n_kmers = res.n_kmers;
-        stats->n_occurrences = res.n_occ;
-        stats->n_nodes = res.n_nodes;
-        stats->n_simplitigs = res.n_simplitigs;
-        stats->n_launches = ex.launches;
-        fill_times(ctx, stats);
-    }
-    ctx->total_launches += ex.launches;
-    ctx->read_backs += ex.read_backs;
+    if (stats) fill_output(ctx, res, f.ex.launches, stats);
     return KC_OK;
     KC_API_END(ctx)
-}
-
-// device result -> the context's pinned host buffer
-static u8 *copy_result_to_pinned(kc_ctx *ctx, const u8 *dev, u64 n) {
-    const size_t need = (size_t) n + 64;
-    if (ctx->pin_out_cap < need) {
-        if (ctx->pin_out) KC_CUDA(cudaFreeHost(ctx->pin_out));
-        ctx->pin_out = nullptr;
-        ctx->pin_out_cap = 0;
-        KC_CUDA(cudaMallocHost(&ctx->pin_out, need + need / 8));
-        ctx->pin_out_cap = need + need / 8;
-    }
-    if (n) KC_CUDA(cudaMemcpyAsync(ctx->pin_out, dev, n, cudaMemcpyDeviceToHost, ctx->stream));
-    KC_CUDA(cudaStreamSynchronize(ctx->stream));
-    return ctx->pin_out;
 }
 
 int kc_streaming(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_output *out) {
@@ -1079,35 +1084,25 @@ int kc_streaming(kc_ctx *ctx, const kc_params *p, const kc_input *in, kc_output 
         q.min_frequency = 1;
         check_large_input(ctx, &q, in->n_bytes);
     }
-    KC_CUDA(cudaSetDevice(ctx->device));
+    CallFrame f(ctx);
     const int limbs = kc_limbs_for_k(p->k);
     const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->routes.sig);
     ensure_arena(ctx, estimate_arena(in->n_bytes, 0, limbs, false, true, false, &ctx->routes.fast, &sig));
     ctx->arena.reset();
-    CudaExec ex{ctx->stream, &ctx->arena};
-    ex.prof = &ctx->prof;
-    ex.pinned = ctx->pin_small;
-    ex.pinned_cap = ctx->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
     std::memset(out, 0, sizeof(*out));
     KC_CUDA(cudaEventRecord(ctx->ev[0], ctx->stream));
-    const u64 padded = (in->n_bytes + 31) / 32 * 32 + 64;
-    u8 *d_seq = ex.alloc<u8>(padded);
-    ex.fill_bytes(d_seq + (in->n_bytes & ~(u64) 31), '\n', padded - (in->n_bytes & ~(u64) 31));
-    KC_CUDA(cudaMemcpyAsync(d_seq, in->seq, in->n_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    const u8 *d_seq = upload_padded(f.ex, in->seq, in->n_bytes);
     KC_CUDA(cudaEventRecord(ctx->ev[1], ctx->stream));
-    StreamingResult r;
-    if (limbs == 1) r = kc_streaming_run<1>(ex, d_seq, in->n_bytes, p->k, p->complements != 0, p->min_frequency, ctx->routes);
-    else if (limbs == 2) r = kc_streaming_run<2>(ex, d_seq, in->n_bytes, p->k, p->complements != 0, p->min_frequency, ctx->routes);
-    else r = kc_streaming_run<4>(ex, d_seq, in->n_bytes, p->k, p->complements != 0, p->min_frequency, ctx->routes);
+    const StreamingResult r = with_limbs(limbs, [&](auto l) {
+        return kc_streaming_run<decltype(l)::value>(f.ex, d_seq, in->n_bytes, p->k, p->complements != 0, p->min_frequency, ctx->routes);
+    });
     for (int i = 2; i <= 4; ++i) KC_CUDA(cudaEventRecord(ctx->ev[i], ctx->stream));
-    out->ms = copy_result_to_pinned(ctx, r.ms, r.length);
+    out->ms = copy_to_pinned(ctx, r.ms, nullptr, r.length);
     out->length = r.length;
     out->n_kmers = r.n_kept;
     out->n_occurrences = r.n_occ;
-    out->n_launches = ex.launches;
+    out->n_launches = f.ex.launches;
     fill_times(ctx, out);
-    ctx->total_launches += ex.launches;
-    ctx->read_backs += ex.read_backs;
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -1117,34 +1112,25 @@ int kc_maskopt(kc_ctx *ctx, const uint8_t *ms, uint64_t n, int k, int complement
     KC_API_BEGIN
     if (k < 1 || k > 127) KC_THROW(KC_ERR_ARG, "k must be in 1..127");
     if (n + 1 >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "more than 2^32 sequence bytes on one GPU");
-    KC_CUDA(cudaSetDevice(ctx->device));
+    CallFrame f(ctx);
     const int limbs = kc_limbs_for_k(k);
     // min-one keeps the sorted key set of the first construction (n * (8 limbs + 1) bytes) at the arena bottom while a second,
     // flags-only construction runs above it
     ensure_arena(ctx, estimate_arena(n + 1, 0, limbs, false, true) + 2 * n + (minimize ? (size_t) n * (8 * limbs + 1) + n / 4 : 0));
     ctx->arena.reset();
-    CudaExec ex{ctx->stream, &ctx->arena};
-    ex.prof = &ctx->prof;
-    ex.pinned = ctx->pin_small;
-    ex.pinned_cap = ctx->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
     std::memset(out, 0, sizeof(*out));
     KC_CUDA(cudaEventRecord(ctx->ev[0], ctx->stream));
-    u8 *d_seq = ex.alloc<u8>(n + 64);
-    ex.fill_bytes(d_seq + (n & ~(u64) 31), '\n', n + 64 - (n & ~(u64) 31));
-    if (n) KC_CUDA(cudaMemcpyAsync(d_seq, ms, n, cudaMemcpyHostToDevice, ctx->stream));
+    const u8 *d_seq = upload_padded(f.ex, ms, n);
     KC_CUDA(cudaEventRecord(ctx->ev[1], ctx->stream));
-    MaskoptResult r;
-    if (limbs == 1) r = kc_maskopt_run<1>(ex, d_seq, n, k, complements != 0, minimize != 0);
-    else if (limbs == 2) r = kc_maskopt_run<2>(ex, d_seq, n, k, complements != 0, minimize != 0);
-    else r = kc_maskopt_run<4>(ex, d_seq, n, k, complements != 0, minimize != 0);
+    const MaskoptResult r = with_limbs(limbs, [&](auto l) {
+        return kc_maskopt_run<decltype(l)::value>(f.ex, d_seq, n, k, complements != 0, minimize != 0);
+    });
     for (int i = 2; i <= 4; ++i) KC_CUDA(cudaEventRecord(ctx->ev[i], ctx->stream));
-    out->ms = copy_result_to_pinned(ctx, r.ms, r.length);
+    out->ms = copy_to_pinned(ctx, r.ms, nullptr, r.length);
     out->length = r.length;
     out->n_kmers = r.n_kmers;
-    out->n_launches = ex.launches;
+    out->n_launches = f.ex.launches;
     fill_times(ctx, out);
-    ctx->total_launches += ex.launches;
-    ctx->read_backs += ex.read_backs;
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -1164,23 +1150,13 @@ int kc_count_kmers(kc_ctx *ctx, const kc_params *p, const kc_input *in, uint64_t
     KC_API_BEGIN
     check_params(p);
     if (in->n_bytes >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "more than 2^32 sequence bytes on one GPU");
-    KC_CUDA(cudaSetDevice(ctx->device));
+    CallFrame f(ctx);
     const int limbs = kc_limbs_for_k(p->k);
     size_t need = (size_t) ((double) in->n_bytes * (1.0 + 2.0 * 8 * limbs + 4.0) * 1.15) + (256u << 20);
     ensure_arena(ctx, need);
     ctx->arena.reset();
-    CudaExec ex{ctx->stream, &ctx->arena};
-    ex.prof = &ctx->prof;
-    ex.pinned = ctx->pin_small;
-    ex.pinned_cap = ctx->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
-    u8 *d_seq = ex.alloc<u8>(in->n_bytes + 64);
-    KC_CUDA(cudaMemcpyAsync(d_seq, in->seq, in->n_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    DevInput di{d_seq, in->n_bytes, nullptr, nullptr, in->n_recs};
-    if (p->k < 32) count_only<1>(ctx, ex, di, *p, keys, counts, n);
-    else if (p->k < 64) count_only<2>(ctx, ex, di, *p, keys, counts, n);
-    else count_only<4>(ctx, ex, di, *p, keys, counts, n);
-    ctx->total_launches += ex.launches;
-    ctx->read_backs += ex.read_backs;
+    const DevInput di = upload_input(ctx, f.ex, in, false, nullptr);
+    with_limbs(limbs, [&](auto l) { count_only<decltype(l)::value>(ctx, f.ex, di, *p, keys, counts, n); });
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -1191,14 +1167,11 @@ int kc_partial_presort(kc_ctx *ctx, const uint64_t *kmers, uint64_t n, int k, ui
     if (k < 1 || k > 127) KC_THROW(KC_ERR_ARG, "k must be in 1..127");
     if (n >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "too many k-mers");
     if (n == 0) return KC_OK;
-    KC_CUDA(cudaSetDevice(ctx->device));
+    CallFrame f(ctx);
+    CudaExec &ex = f.ex;
     const int limbs = kc_limbs_for_k(k);
     ensure_arena(ctx, (size_t) (n * (16.0 * limbs + 64.0)) + (64u << 20));
     ctx->arena.reset();
-    CudaExec ex{ctx->stream, &ctx->arena};
-    ex.prof = &ctx->prof;
-    ex.pinned = ctx->pin_small;
-    ex.pinned_cap = ctx->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
     u64 *src = ex.alloc<u64>(n * limbs), *dst = ex.alloc<u64>(n * limbs);
     KC_CUDA(cudaMemcpyAsync(src, kmers, n * limbs * 8, cudaMemcpyHostToDevice, ctx->stream));
     const int sfb = 2 * k < 8 ? 2 * k : 8;  // SORT_FIRST_BITS, src/global_sparse.h:16
@@ -1211,8 +1184,6 @@ int kc_partial_presort(kc_ctx *ctx, const uint64_t *kmers, uint64_t n, int k, ui
     ex.for_each(n * limbs, [=] __device__(u64 t) { dst[t] = src[(perm[t / limbs] & 0xFFFFFFFFULL) * limbs + t % limbs]; });
     KC_CUDA(cudaMemcpyAsync(out, dst, n * limbs * 8, cudaMemcpyDeviceToHost, ctx->stream));
     KC_CUDA(cudaStreamSynchronize(ctx->stream));
-    ctx->total_launches += ex.launches;
-    ctx->read_backs += ex.read_backs;
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -1228,13 +1199,10 @@ int kc_debug_sort(kc_ctx *ctx, const uint64_t *words, uint64_t n, int limbs, int
             const u64 high = rem >= 64 ? 0 : (rem <= 0 ? ~0ULL : ~0ULL << rem);
             if (words[i * limbs + j] & high) KC_THROW(KC_ERR_ARG, "a word has a bit set at or above key_bits");
         }
-    KC_CUDA(cudaSetDevice(ctx->device));
+    CallFrame f(ctx);
+    CudaExec &ex = f.ex;
     ensure_arena(ctx, (size_t) n * (16 * limbs + 8) + (64u << 20));
     ctx->arena.reset();
-    CudaExec ex{ctx->stream, &ctx->arena};
-    ex.prof = &ctx->prof;
-    ex.pinned = ctx->pin_small;
-    ex.pinned_cap = ctx->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
     u64 *a = ex.alloc<u64>(n * limbs), *b = ex.alloc<u64>(n * limbs);
     if (n) KC_CUDA(cudaMemcpyAsync(a, words, n * limbs * 8, cudaMemcpyHostToDevice, ctx->stream));
     KcSortStats st;
@@ -1246,8 +1214,6 @@ int kc_debug_sort(kc_ctx *ctx, const uint64_t *words, uint64_t n, int limbs, int
     }
     if (n) KC_CUDA(cudaMemcpyAsync(out, a, n * limbs * 8, cudaMemcpyDeviceToHost, ctx->stream));
     KC_CUDA(cudaStreamSynchronize(ctx->stream));
-    ctx->total_launches += ex.launches;
-    ctx->read_backs += ex.read_backs;
     if (stats) {
         // the local kernel's path, from its rule (kc_sort_local_kernel): digit width about two sub-buckets per item, and a
         // bucket with more than 64 sub-buckets of more than KC_SUB_SMALL items is sorted whole; a digit count does not depend
@@ -1296,7 +1262,8 @@ int kc_kmer_digest(kc_ctx *ctx, const kc_params *p, const kc_input *in, int mask
         q.want_maxone = 0;
         check_large_input(ctx, &q, nb);
     }
-    KC_CUDA(cudaSetDevice(ctx->device));
+    CallFrame f(ctx);
+    CudaExec &ex = f.ex;
     const int limbs = kc_limbs_for_k(p->k);
     // the sorted-keys route, or at 2^32 bytes and more the signature construction alone: sequence, flags, window mask, its buffers
     size_t need = (size_t) ((double) nb * (1.0 + 2.0 * 8 * limbs + 4.0 + 0.2) * 1.15) + (256u << 20);
@@ -1304,10 +1271,6 @@ int kc_kmer_digest(kc_ctx *ctx, const kc_params *p, const kc_input *in, int mask
         need = (size_t) (((double) nb * 1.25 + (double) kc_sig_arena_bytes(kc_sig_plan(nb, p->k, ctx->routes.sig), nb)) * 1.05) + (256u << 20);
     ensure_arena(ctx, need);
     ctx->arena.reset();
-    CudaExec ex{ctx->stream, &ctx->arena};
-    ex.prof = &ctx->prof;
-    ex.pinned = ctx->pin_small;
-    ex.pinned_cap = ctx->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
     u8 *d_seq = ex.alloc<u8>(nb + 64);
     if (in->n_bytes) KC_CUDA(cudaMemcpyAsync(d_seq, in->seq, in->n_bytes, cudaMemcpyHostToDevice, ctx->stream));
     u32 *win_mask = nullptr;
@@ -1330,11 +1293,7 @@ int kc_kmer_digest(kc_ctx *ctx, const kc_params *p, const kc_input *in, int mask
         }, KP_MISC, len + len / 8);
     }
     DevInput di{d_seq, nb, nullptr, nullptr, in->n_recs};
-    if (limbs == 1) digest_only<1>(ctx, ex, di, *p, win_mask, digest);
-    else if (limbs == 2) digest_only<2>(ctx, ex, di, *p, win_mask, digest);
-    else digest_only<4>(ctx, ex, di, *p, win_mask, digest);
-    ctx->total_launches += ex.launches;
-    ctx->read_backs += ex.read_backs;
+    with_limbs(limbs, [&](auto l) { digest_only<decltype(l)::value>(ctx, ex, di, *p, win_mask, digest); });
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -1346,26 +1305,19 @@ int kc_overlap_path(kc_ctx *ctx, const uint64_t *first, const uint64_t *last, ui
     if (k < 1 || k > 127) KC_THROW(KC_ERR_ARG, "k must be in 1..127");
     if (n == 0) KC_THROW(KC_ERR_EMPTY, "input cannot be empty");
     if (n * (complements ? 2 : 1) >= 0xFFFFFFF0ULL) KC_THROW(KC_ERR_TOO_LARGE, "too many nodes for one GPU");
-    KC_CUDA(cudaSetDevice(ctx->device));
+    CallFrame f(ctx);
     const int limbs = kc_limbs_for_k(k);
     ensure_arena(ctx, estimate_arena(0, n, limbs, complements != 0, true) + n * 16 * limbs);
     ctx->arena.reset();
-    CudaExec ex{ctx->stream, &ctx->arena};
-    ex.prof = &ctx->prof;
-    ex.pinned = ctx->pin_small;
-    ex.pinned_cap = ctx->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
-    if (k < 32) overlap_only<1>(ctx, ex, first, last, n, k, complements != 0, lower_bound != 0, strict != 0, edge_from, overlaps);
-    else if (k < 64) overlap_only<2>(ctx, ex, first, last, n, k, complements != 0, lower_bound != 0, strict != 0, edge_from, overlaps);
-    else overlap_only<4>(ctx, ex, first, last, n, k, complements != 0, lower_bound != 0, strict != 0, edge_from, overlaps);
-    ctx->total_launches += ex.launches;
-    ctx->read_backs += ex.read_backs;
+    with_limbs(limbs, [&](auto l) {
+        overlap_only<decltype(l)::value>(ctx, f.ex, first, last, n, k, complements != 0, lower_bound != 0, strict != 0, edge_from, overlaps);
+    });
     return KC_OK;
     KC_API_END(ctx)
 }
 
 uint64_t kc_shard_granule(int k) {
-    const int limbs = kc_limbs_for_k(k);
-    return limbs == 1 ? KsCfg<1>::EX_TILE : (limbs == 2 ? KsCfg<2>::EX_TILE : KsCfg<4>::EX_TILE);
+    return with_limbs(kc_limbs_for_k(k), [](auto l) -> uint64_t { return KsCfg<decltype(l)::value>::EX_TILE; });
 }
 
 int kc_group_alloc(kc_ctx *ctx, int n_ranks, int rank, int k, uint64_t n_bytes_cap, uint8_t *handle_out) {
@@ -1404,44 +1356,17 @@ int kc_group_compute_device(kc_ctx *ctx, const kc_params *p, const kc_input *in,
     KC_API_BEGIN
     group_check_job(ctx, p, in->n_bytes);
     if ((reinterpret_cast<uintptr_t>(in->seq) & 15) != 0) KC_THROW(KC_ERR_ARG, "device sequence pointer must be 16-byte aligned");
-    KC_CUDA(cudaSetDevice(ctx->device));
-    const int limbs = kc_limbs_for_k(p->k);
-    CudaExec ex{ctx->stream, &ctx->arena};
-    ex.prof = &ctx->prof;
-    ex.pinned = ctx->pin_small;
-    ex.pinned_cap = ctx->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
+    CallFrame f(ctx);
     DevInput di{in->seq, in->n_bytes, nullptr, nullptr, 0};
     DevResult res;
-    // no retry with a larger arena here: a rank that repeated its job alone would leave the group's sync numbers behind
-    const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->routes.sig);
-    const size_t need = group_arena_need(in->n_bytes, ctx->grp.n, limbs, p->complements != 0, false, &sig);
-    ensure_arena(ctx, need);
-    if (in->n_bytes >= KC_POS32_BYTES && ctx->arena.cap < need) KC_THROW(KC_ERR_OOM, "the device cannot hold this rank's arena for an input of 2^32 bytes or more");
+    group_prepare_arena(ctx, *p, in->n_bytes, "the device cannot hold this rank's arena for an input of 2^32 bytes or more");
     ctx->arena.reset();
     ctx->grp.refused = false;
-    try {
-        if (limbs == 1) group_compute_rank<1>(ctx, ex, di, *p, res);
-        else if (limbs == 2) group_compute_rank<2>(ctx, ex, di, *p, res);
-        else group_compute_rank<4>(ctx, ex, di, *p, res);
-    } catch (const KcError &e) {
-        // "no k-mers" and the refusals of group_compute_rank are found by every rank at the same point
-        if (e.code != KC_ERR_EMPTY && !ctx->grp.refused) ctx->grp.failed = true;
-        throw;
-    }
+    group_run_job(ctx, f.ex, di, *p, res);
     KC_CUDA(cudaStreamSynchronize(ctx->stream));
     if (slice_begin) *slice_begin = res.slice_begin;
     if (slice_len) *slice_len = res.slice_len;
-    out->ms = const_cast<u8 *>(res.ms);
-    out->ms_maxone = nullptr;
-    out->length = res.length;
-    out->n_kmers = res.n_kmers;
-    out->n_occurrences = res.n_occ;
-    out->n_nodes = res.n_nodes;
-    out->n_simplitigs = res.n_simplitigs;
-    out->n_launches = ex.launches;
-    fill_times(ctx, out);
-    ctx->total_launches += ex.launches;
-    ctx->read_backs += ex.read_backs;
+    fill_output(ctx, res, f.ex.launches, out);
     return KC_OK;
     KC_API_END(ctx)
 }
@@ -1482,8 +1407,7 @@ struct kc_group {
     int n = 0;
     kc_ctx *ctx[KC_MAX_PEERS] = {};
     GrpHostSync hs;
-    u8 *pin_out = nullptr;
-    size_t pin_out_cap = 0;
+    PinnedBuf pin_out{nullptr, 0, cudaHostAllocPortable};  // every rank copies its slice in
     std::mutex out_mutex;
     std::string last_error;
 };
@@ -1548,7 +1472,7 @@ void kc_group_destroy(kc_group *g) {
     for (int r = 0; r < g->n; ++r)
         for (int i = 0; i < 2; ++i)
             if (g->hs.ev[r][i]) cudaEventDestroy(g->hs.ev[r][i]);
-    if (g->pin_out) cudaFreeHost(g->pin_out);
+    if (g->pin_out.p) cudaFreeHost(g->pin_out.p);
     delete g;
 }
 
@@ -1575,7 +1499,7 @@ int kc_group_compute(kc_group *g, const kc_params *p, const kc_input *in, kc_out
                 g->ctx[r]->routes.fast = c0->routes.fast;  // one plan for the whole group
                 g->ctx[r]->routes.heuristics = c0->routes.heuristics;
                 g->ctx[r]->routes.fast_rung.overflow = c0->routes.fast_rung.overflow;
-                group_alloc_common(g->ctx[r], g->n, r, limbs == 1 ? 31 : (limbs == 2 ? 63 : 127), cap, true);
+                group_alloc_common(g->ctx[r], g->n, r, 32 * limbs - 1, cap, true);  // the largest k of this word width
             }
             for (int r = 0; r < g->n; ++r) {
                 for (int s = 0; s < g->n; ++s) g->ctx[r]->grp.peer[s] = g->ctx[s]->grp.heap;
@@ -1601,12 +1525,8 @@ int kc_group_compute(kc_group *g, const kc_params *p, const kc_input *in, kc_out
                         kc_ctx *ctx = g->ctx[r];
                         std::lock_guard<std::mutex> lk(dev_mutex[ctx->device % KC_MAX_DEVICES]);
                         KC_CUDA(cudaSetDevice(ctx->device));
-                        const SigPlan sig = kc_sig_plan(in->n_bytes, p->k, ctx->routes.sig);
-                        const size_t need = group_arena_need(in->n_bytes, g->n, limbs, p->complements != 0, false, &sig);
-                        ensure_arena(ctx, need);
-                        // a rank that ran out of arena half way would strand the others: refuse before anything is queued
-                        if (large && ctx->arena.cap < need)
-                            KC_THROW(KC_ERR_OOM, "the device cannot hold every rank's arena for an input of 2^32 bytes or more (ranks sharing a device need it once each)");
+                        group_prepare_arena(ctx, *p, in->n_bytes,
+                                            "the device cannot hold every rank's arena for an input of 2^32 bytes or more (ranks sharing a device need it once each)");
                     } catch (const KcError &e) {
                         errs[r] = e;
                         bad[r] = true;
@@ -1625,21 +1545,17 @@ int kc_group_compute(kc_group *g, const kc_params *p, const kc_input *in, kc_out
         int code = KC_OK;
         std::string what;
         DevResult res;
-        u64 launches = 0;
         kc_output o;
     } ro[KC_MAX_PEERS];
     auto worker = [&](int r) {
         kc_ctx *ctx = g->ctx[r];
         RankOut &R = ro[r];
         try {
-            KC_CUDA(cudaSetDevice(ctx->device));
+            CallFrame f(ctx);
+            CudaExec &ex = f.ex;
             KcGroup &G = ctx->grp;
             ctx->arena.reset();
             G.refused = false;
-            CudaExec ex{ctx->stream, &ctx->arena};
-            ex.prof = &ctx->prof;
-            ex.pinned = ctx->pin_small;
-            ex.pinned_cap = ctx->pin_small ? kc_ctx::KC_PIN_SMALL : 0;
             // the sequence: this rank brings in its share over its own PCIe link and hands it to every peer over NVLink
             u8 *seq = reinterpret_cast<u8 *>(G.heap + G.lay.off_seq);
             const u64 nb = in->n_bytes;
@@ -1661,39 +1577,22 @@ int kc_group_compute(kc_group *g, const kc_params *p, const kc_input *in, kc_out
             kc_grp_signal(G, ex, s0);
             kc_grp_wait(G, ex, s0, ws);
             DevInput di{seq, nb, nullptr, nullptr, 0};
-            const int limbs = kc_limbs_for_k(p->k);
-            if (limbs == 1) group_compute_rank<1>(ctx, ex, di, *p, R.res);
-            else if (limbs == 2) group_compute_rank<2>(ctx, ex, di, *p, R.res);
-            else group_compute_rank<4>(ctx, ex, di, *p, R.res);
+            group_run_job(ctx, ex, di, *p, R.res);
             {   // the first rank to get here sizes the common result buffer
                 std::lock_guard<std::mutex> lk(g->out_mutex);
-                const size_t need = (size_t) R.res.length + 64;
-                if (g->pin_out_cap < need) {
-                    if (g->pin_out) KC_CUDA(cudaFreeHost(g->pin_out));
-                    g->pin_out = nullptr;
-                    g->pin_out_cap = 0;
-                    KC_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&g->pin_out), need + need / 8, cudaHostAllocPortable));
-                    g->pin_out_cap = need + need / 8;
-                }
+                g->pin_out.reserve((size_t) R.res.length + 64);
             }
             if (R.res.slice_len)
-                KC_CUDA(cudaMemcpyAsync(g->pin_out + R.res.slice_begin, R.res.ms, R.res.slice_len, cudaMemcpyDeviceToHost, ctx->stream));
+                KC_CUDA(cudaMemcpyAsync(g->pin_out.p + R.res.slice_begin, R.res.ms, R.res.slice_len, cudaMemcpyDeviceToHost, ctx->stream));
             KC_CUDA(cudaStreamSynchronize(ctx->stream));
             if (ex.read(ws) & 2u) KC_THROW(KC_ERR_INTERNAL, "a rank of the group did not arrive (wait timed out)");
-            R.launches = ex.launches;
-            fill_times(ctx, &R.o);
-            ctx->total_launches += ex.launches;
-            ctx->read_backs += ex.read_backs;
+            fill_output(ctx, R.res, ex.launches, &R.o);
         } catch (const KcError &e) {
             R.code = e.code;
             char buf[512];
             std::snprintf(buf, sizeof(buf), "rank %d: %s (%s:%d)", r, e.what, e.file, e.line);
             R.what = buf;
-            // "no k-mers" and the refusals of group_compute_rank are found by every rank at the same point; anything else strands the others
-            if (e.code != KC_ERR_EMPTY && !ctx->grp.refused) {
-                ctx->grp.failed = true;
-                g->hs.abort();
-            }
+            if (group_fail(ctx, e.code)) g->hs.abort();
         } catch (...) {
             R.code = KC_ERR_INTERNAL;
             R.what = "rank " + std::to_string(r) + ": unknown failure";
@@ -1720,16 +1619,11 @@ int kc_group_compute(kc_group *g, const kc_params *p, const kc_input *in, kc_out
             g->last_error = "the ranks disagree on the result";
             return KC_ERR_INTERNAL;
         }
-    std::memset(out, 0, sizeof(*out));
-    out->ms = g->pin_out;
-    out->length = ro[0].res.length;
-    out->n_kmers = ro[0].res.n_kmers;
-    out->n_occurrences = ro[0].res.n_occ;
-    out->n_nodes = ro[0].res.n_nodes;
-    out->n_simplitigs = ro[0].res.n_simplitigs;
-    out->t = ro[0].o.t;
+    *out = ro[0].o;
+    out->ms = g->pin_out.p;
+    out->n_launches = 0;
     for (int r = 0; r < g->n; ++r) {
-        out->n_launches += ro[r].launches;
+        out->n_launches += ro[r].o.n_launches;
         if (ro[r].o.t.total_ms > out->t.total_ms) out->t = ro[r].o.t;  // the slowest rank's stage times
     }
     return KC_OK;

@@ -1,4 +1,4 @@
-// First-occurrence runs: the nodes of the overlap stage in the from-FASTA regime (see kcgpu.cu run_stage1_runs).
+// First-occurrence runs: the nodes of the overlap stage in the from-FASTA regime (see kcgpu.cu run_stage1_runs and run_tail).
 //
 // Bit p of the flag array marks a window END position p whose k-mer is a kept k-mer occurring there for the first time.  A
 // maximal run of consecutive flagged positions e_s..e_t is the node seq[e_s - k + 1 .. e_t].  Every run has one
@@ -96,7 +96,7 @@ __global__ void __launch_bounds__(256) kc_runs_emit_kernel(const u32 *flags, u64
 }
 
 struct RunNodes {
-    u64 *rec_off = nullptr, *rec_len = nullptr;  // arena top end
+    const u64 *rec_off = nullptr, *rec_len = nullptr;  // arena top end (or the -S records)
     u64 n_runs = 0;
 };
 

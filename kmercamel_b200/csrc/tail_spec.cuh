@@ -39,7 +39,7 @@ __global__ void __launch_bounds__(1024) kc_spec_nodes_kernel(const u64 *cells, u
     const u32 status = cells[3] ? KC_SPEC_SIG_OVERFLOW
                        : U == 0 ? KC_SPEC_EMPTY
                        : runs > KC_SPEC_RUNS ? KC_SPEC_TOO_MANY
-                       : sparse_switch && runs * 5 >= U ? KC_SPEC_SPARSE  // src/main.cpp:175-181, as in run_pipeline
+                       : sparse_switch && runs * 5 >= U ? KC_SPEC_SPARSE  // src/main.cpp:175-181, as in run_tail
                                                         : KC_SPEC_OK;
     const u32 n = status == KC_SPEC_OK ? (u32) runs : 0u, N = complements ? 2 * n : n;
     if (threadIdx.x == 0) {

@@ -318,7 +318,7 @@ def window_words(seq, starts, k: int):
 
 
 def fasta_nodes(seq, rec_off, rec_len, k: int, complements: bool, min_frequency: int = 1, sparse_switch: bool = True):
-    """The nodes the product hands to its overlap stage from FASTA (kcgpu.cu run_pipeline) -> (node start [n] u64,
+    """The nodes the product hands to its overlap stage from FASTA (kcgpu.cu run_tail) -> (node start [n] u64,
     node length [n] u64, kept k-mers, first-occurrence runs).  The runs, unless there are at least U / 5 of them (the sparse
     switch, reference src/main.cpp:94,175-181): then one node per k-mer of the runs, in run order and in the orientation it has
     in the input, stably sorted on its first min(k, 4) bases (PartialPreSort, src/global_sparse.h:14-35)."""
