@@ -109,6 +109,8 @@ __global__ void __launch_bounds__(256) kc_rank_small_kernel(PathState s, NodeSeq
     __shared__ u64 dist[2][KC_RANK_SMALL];
     __shared__ u32 s_start, s_cyc;
     __shared__ u32 sw[8];
+    kc_pdl_wait();
+    kc_pdl_trigger();  // one CTA: the next kernel's launch overlaps this one
     const u32 n_cells = N;  // chunks[] has n_cells + 1 entries
     if (n_dev) {
         q.n = n_dev[0];
@@ -254,9 +256,7 @@ EmitResult kc_emit_superstring(Exec &ex, const NodeSeq<L> &ns, const NodeView<L>
                 chunks_pre = ex.template alloc<u32>(N + 1);
             }
             typename Exec::Scope sc(ex, KP_RANK, N * 25);
-            kc_rank_small_kernel<L><<<1, 256, 0, ex.stream>>>(s, q, (u32) N, fin_a, dist_a, cell, n_dev, chunks_pre, ms_pre);
-            ++ex.launches;
-            KC_CUDA(cudaGetLastError());
+            ex.launch(kc_rank_small_kernel<L>, 1, 256, 0, s, q, (u32) N, fin_a, dist_a, cell, n_dev, chunks_pre, ms_pre);
             ranked = true;
         }
     }

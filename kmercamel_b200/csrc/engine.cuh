@@ -463,9 +463,8 @@ template <class Exec, int L> struct Engine {
             {   // which levels can accept an edge at all: one CTA per two levels (the engine kernel used to do this alone)
                 typename Exec::Scope sc(ex, KP_SMALL_ENGINE, 0);
                 const u32 per_cta = kc_small_mask_levels_per_cta<L>((u32) n_s, (u32) n_p);
-                kc_small_level_mask_kernel<L><<<(unsigned) kc_div_up((u64) d + 1, per_cta), 256, mask_smem, ex.stream>>>(nv, live_s, live_p, (u32) n_s, (u32) n_p, d,
-                                                                                                                      lvl_mask, a.end_mask_s_a, a.end_mask_p_a, n_dev);
-                ++ex.launches;
+                ex.launch(kc_small_level_mask_kernel<L>, (unsigned) kc_div_up((u64) d + 1, per_cta), 256, mask_smem, nv, (const u32 *) live_s,
+                          (const u32 *) live_p, (u32) n_s, (u32) n_p, d, lvl_mask, a.end_mask_s_a, a.end_mask_p_a, n_dev);
             }
             {
                 typename Exec::Scope sc(ex, KP_SMALL_ENGINE, 0);
@@ -477,10 +476,8 @@ template <class Exec, int L> struct Engine {
                 // (speculative tail: the count is not known here; 256 vs 512 threads is within 1.5 % at 50 records, r02z_small_engine_trace.txt)
                 const unsigned small_threads = small_threads_opt ? (unsigned) small_threads_opt
                                                : n_dev || (nt0 > 128 && nt0 <= 256) || nt0 > 512 ? 512u : 256u;
-                kc_small_engine_kernel<L><<<1, small_threads, SmallCfg<L>::SMEM, ex.stream>>>(a);
+                ex.launch(kc_small_engine_kernel<L>, 1, small_threads, SmallCfg<L>::SMEM, a);
             }
-            ++ex.launches;
-            KC_CUDA(cudaGetLastError());
             // The status words are read back by check_small() after the caller's next synchronisation point: the kernels of the
             // emission stage are queued behind this one without a host round trip.
             small_out = n_dev ? nullptr : a.out;

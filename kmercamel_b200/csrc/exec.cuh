@@ -13,6 +13,7 @@
 #pragma once
 #include <cstring>
 #include "kc_common.cuh"
+#include <utility>
 #include <vector>
 
 #ifdef __CUDA_ARCH__
@@ -50,6 +51,7 @@ static const char *const kc_prof_names[KP_COUNT] = {
 static const int KC_FE_THREADS = 256;
 
 template <typename F> __global__ void __launch_bounds__(KC_FE_THREADS) kc_for_each_kernel(u64 n, F f) {
+    kc_pdl_wait();
     u64 i = (u64) blockIdx.x * KC_FE_THREADS + threadIdx.x;
     if (i < n) f(i);
 }
@@ -209,10 +211,40 @@ struct KernelProf {
     }
 };
 
+// The kernel nodes of a captured graph whose arguments hold the input pointer `seq`, so that a replay can point them at another input
+// of the same size (cudaGraphExecKernelNodeSetParams).  They are found at capture by value: every 8-byte word of an argument that
+// equals `seq`.  The input is a caller's buffer or the arena block it was copied to, never an address that another argument holds.
+struct SeqPatch {
+    const void *seq = nullptr;
+    struct Node {
+        cudaGraphNode_t node;
+        void *func;
+        dim3 grid, block;
+        size_t smem;
+        std::vector<std::vector<u8>> args;  // the captured argument bytes
+        std::vector<std::pair<u32, u32>> at;  // (argument, byte offset) of every copy of seq
+    };
+    std::vector<Node> nodes;
+
+    void set_seq(cudaGraphExec_t exec, const void *s) {
+        if (s == seq) return;
+        for (Node &n : nodes) {
+            std::vector<void *> ptrs;
+            for (const auto &[i, off] : n.at) std::memcpy(n.args[i].data() + off, &s, 8);
+            for (auto &a : n.args) ptrs.push_back(a.data());
+            cudaKernelNodeParams kp{n.func, n.grid, n.block, (unsigned) n.smem, ptrs.data(), nullptr};
+            KC_CUDA(cudaGraphExecKernelNodeSetParams(exec, n.node, &kp));
+        }
+        seq = s;
+    }
+};
+
 struct CudaExec {
     cudaStream_t stream;
     Arena *arena;
     KernelProf *prof = nullptr;
+    bool pdl = false;            // launch with programmatic stream serialization (the kernels wait in kc_pdl_wait)
+    SeqPatch *patch = nullptr;   // != nullptr while a graph is captured from this policy's launches
     u64 launches = 0;  // kernels launched through this policy (bench.py reports it as gpu_launches)
     u64 read_backs = 0;  // synchronising read-backs (read_n), i.e. host round trips
     u8 *pinned = nullptr;  // page-locked host scratch of the context for the synchronising read-backs below: a pageable
@@ -242,14 +274,52 @@ struct CudaExec {
 
     template <typename T> T *alloc(size_t n) { return arena->alloc<T>(n); }
 
+    // One kernel launch on the stream; with `pdl`, the kernel may start before the previous one ends (it waits in kc_pdl_wait).
+    template <typename... P, typename... A> void launch(void (*kern)(P...), dim3 grid, dim3 block, size_t smem, const A &...a) {
+        cudaLaunchConfig_t cfg = {};
+        cfg.gridDim = grid;
+        cfg.blockDim = block;
+        cfg.dynamicSmemBytes = smem;
+        cfg.stream = stream;
+        cudaLaunchAttribute attr[1];
+        if (pdl) {
+            attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+            attr[0].val.programmaticStreamSerializationAllowed = 1;
+            cfg.attrs = attr;
+            cfg.numAttrs = 1;
+        }
+        KC_CUDA(cudaLaunchKernelEx(&cfg, kern, a...));
+        ++launches;
+        if (patch) note_seq<P...>(reinterpret_cast<void *>(kern), grid, block, smem, a...);
+    }
+
+    // While capturing: the node just added, if any of its arguments holds patch->seq (see SeqPatch).
+    template <typename... P> void note_seq(void *func, dim3 grid, dim3 block, size_t smem, const P &...p) {
+        SeqPatch::Node n{};
+        (n.args.emplace_back(reinterpret_cast<const u8 *>(&p), reinterpret_cast<const u8 *>(&p) + sizeof(P)), ...);
+        for (u32 i = 0; i < (u32) n.args.size(); ++i)
+            for (u32 off = 0; off + 8 <= n.args[i].size(); off += 8)
+                if (std::memcmp(n.args[i].data() + off, &patch->seq, 8) == 0) n.at.emplace_back(i, off);
+        if (n.at.empty()) return;
+        cudaStreamCaptureStatus cs;
+        const cudaGraphNode_t *deps = nullptr;
+        size_t n_deps = 0;
+        KC_CUDA(cudaStreamGetCaptureInfo(stream, &cs, nullptr, nullptr, &deps, &n_deps));
+        if (cs != cudaStreamCaptureStatusActive || n_deps != 1) KC_THROW(KC_ERR_INTERNAL, "graph capture: no kernel node to patch");
+        n.node = deps[0];
+        n.func = func;
+        n.grid = grid;
+        n.block = block;
+        n.smem = smem;
+        patch->nodes.push_back(std::move(n));
+    }
+
     template <typename F> void for_each(u64 n, F f, int id = KP_MISC, u64 bytes = 0) {
         if (n == 0) return;
         Scope sc(*this, id, bytes);
         u64 blocks = kc_div_up(n, KC_FE_THREADS);
         if (blocks > 0x7FFFFFFFULL) KC_THROW(KC_ERR_TOO_LARGE, "for_each grid too large");
-        kc_for_each_kernel<<<(unsigned) blocks, KC_FE_THREADS, 0, stream>>>(n, f);
-        ++launches;
-        KC_CUDA(cudaGetLastError());
+        launch(kc_for_each_kernel<F>, (unsigned) blocks, KC_FE_THREADS, 0, n, f);
     }
 
     void fill_bytes(void *p, int value, size_t bytes) {

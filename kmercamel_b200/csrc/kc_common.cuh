@@ -18,6 +18,22 @@ typedef int64_t i64;
 #define KC_D __device__ __forceinline__
 #define KC_HD_LAMBDA __host__ __device__
 
+// Programmatic dependent launch (CudaExec::launch with ex.pdl): a kernel may start while the one before it in the stream is still
+// running, so every kernel launched that way waits here before it touches memory; without the launch attribute the wait returns at once.
+// kc_pdl_trigger lets the next kernel start its launch early; that is safe because the next kernel waits here for this one to finish.
+#ifdef __CUDACC__
+KC_D void kc_pdl_wait() {
+#if defined(__CUDA_ARCH__) && __CUDA_ARCH__ >= 900
+    asm volatile("griddepcontrol.wait;" ::: "memory");
+#endif
+}
+KC_D void kc_pdl_trigger() {
+#if defined(__CUDA_ARCH__) && __CUDA_ARCH__ >= 900
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+#endif
+}
+#endif
+
 // Status codes of the C ABI: KC_OK / KC_ERR_* from include/kcgpu.h.
 
 struct KcError {

@@ -51,6 +51,45 @@ struct PinnedBuf {
     }
 };
 
+// What the host needs of a queued speculative tail once its status block is back (tail_spec_queue -> tail_spec_finish).
+struct SpecTail {
+    size_t mark = 0;  // arena bottom before the tail
+    const u8 *ms = nullptr;
+    u64 total_ub = 0;
+    u64 n_s = 0, n_p = 0;  // the small engine's sizes (apply_small_status)
+    int small_d = 0;
+};
+
+// The from-FASTA call of one genome on one GPU (signature construction + speculative tail, up to the copy of the status block into
+// pinned memory) captured as a CUDA graph and replayed by later calls of the same shape: the launches of the step cost one
+// cudaGraphLaunch.  Everything the key holds fixes the arena layout and the launch shapes; options that change either clear the cache
+// (kc_set_option), and so does a new arena.  The input pointer is the one argument that changes between calls (SeqPatch).
+struct SpecGraph {
+    int limbs = 0, k = 0;
+    bool complements = false;
+    u64 n_bytes = 0;
+    const char *arena_base = nullptr;
+    ArenaMark arena_at;  // both arena ends when the call reached the construction
+    const u32 *flags = nullptr;
+    cudaGraph_t graph = nullptr;
+    cudaGraphExec_t exec = nullptr;
+    SeqPatch patch;
+    u64 launches = 0, arena_high = 0;
+    ArenaMark arena_after;
+    u64 *blk = nullptr;
+    SpecTail tail;
+    bool same_shape(const SpecGraph &o) const {
+        return limbs == o.limbs && k == o.k && complements == o.complements && n_bytes == o.n_bytes && arena_base == o.arena_base &&
+               arena_at.off == o.arena_at.off && arena_at.top == o.arena_at.top && flags == o.flags;
+    }
+    void destroy() {
+        if (exec) cudaGraphExecDestroy(exec);
+        if (graph) cudaGraphDestroy(graph);
+        exec = nullptr;
+        graph = nullptr;
+    }
+};
+
 struct kc_ctx {
     int device = 0;
     cudaStream_t stream = nullptr;
@@ -64,6 +103,7 @@ struct kc_ctx {
     // kc_compute with host buffers: the input is copied in chunks on its own stream, the first partition pass follows the copy front
     static const int KC_H2D_CHUNKS = 4;
     cudaStream_t copy_stream = nullptr;
+    cudaStream_t capture_stream = nullptr;  // SpecGraph captures (the context's stream may be the legacy default stream, which cannot capture)
     cudaEvent_t chunk_ev[KC_H2D_CHUNKS] = {nullptr, nullptr, nullptr, nullptr};
     bool small_engine = true;
     int small_threads = 0;   // 0 = chosen by the number of free ends (option "small_threads": 256 or 512)
@@ -71,14 +111,21 @@ struct kc_ctx {
     SetRoutes routes;        // the constructions of the first-occurrence bits, their tuning, counters and memories (set_routes.cuh)
     u64 total_launches = 0;  // kernels launched through this context since kc_init
     u64 read_backs = 0;      // synchronising device -> host reads of this context since kc_init (host round trips)
-    bool tail_spec = true;   // option "tail_spec": queue the tail of the from-FASTA path without reading the run count (run_tail_spec)
+    bool tail_spec = true;   // option "tail_spec": queue the tail of the from-FASTA path without reading the run count (run_sig_spec)
     u64 tail_spec_runs = 0, tail_spec_fallbacks = 0;
     EngineStats path_stats;   // the overlap stage of the last call that ran it (stats "path_levels", "path_ban_rounds", "path_bans")
     KcGroup grp;             // multi-GPU: this context as one rank of a group (group.cuh)
     bool arena_limited = false;
     u32 arena_estimate_ppm = 1000000;  // option "arena_estimate_ppm": scales the first arena estimate of run_with_arena (tests)
     u64 arena_retries = 0;         // calls repeated by run_with_arena after running out of arena
+    std::vector<SpecGraph> spec_graphs;  // cached graphs of the speculative from-FASTA call (SpecGraph), at most KC_SPEC_GRAPHS
+    static const size_t KC_SPEC_GRAPHS = 8;
+    u64 spec_graph_captures = 0, spec_graph_replays = 0;
     std::string last_error;
+    void clear_spec_graphs() {
+        for (SpecGraph &g : spec_graphs) g.destroy();
+        spec_graphs.clear();
+    }
 };
 
 namespace {
@@ -157,6 +204,7 @@ void ensure_arena(kc_ctx *ctx, size_t need) {
     need = (need + 4095) & ~(size_t) 4095;  // both arena ends stay 256-byte aligned
     if (ctx->arena.cap >= need) return;
     if (ctx->arena.cap && ctx->arena_limited && need >= ctx->arena.cap) return;  // already holds all the device can give
+    ctx->clear_spec_graphs();
     if (ctx->arena.base) {
         KC_CUDA(cudaFree(ctx->arena.base));
         ctx->arena.base = nullptr;
@@ -309,29 +357,31 @@ template <int L> u64 run_stage1(kc_ctx *ctx, CudaExec &ex, const DevInput &in, c
     return set.n_kept;
 }
 
-// The speculative tail (tail_spec.cuh): from the first-occurrence flags to the last emission kernel, sized for KC_SPEC_RUNS runs, with
-// ONE read-back of the status block `blk` (cells4 of the signature construction first, KC_SPEC_BLOCK_WORDS words, zeroed) at the end.
-// Returns the status: KC_SPEC_OK = `res` holds the result; otherwise nothing was done and the arena is as it was on entry.
+// The speculative tail (tail_spec.cuh): from the first-occurrence flags to the last emission kernel, sized for KC_SPEC_RUNS runs, and
+// the copy of the status block `blk` (cells4 of the signature construction first, KC_SPEC_BLOCK_WORDS words, zeroed) into the pinned
+// scratch behind them.  tail_spec_finish reads it.
 template <int L>
-u32 run_tail_spec(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &p, const u32 *flags, u64 *blk, DevResult &res) {
+SpecTail tail_spec_queue(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &p, const u32 *flags, u64 *blk) {
+    SpecTail t;
     const u64 nb = in.n_bytes;
     const int k = p.k;
     const bool complements = p.complements != 0;
-    const size_t mark = ex.arena->mark();
+    t.mark = ex.arena->mark();
     const u32 C = KC_SPEC_RUNS, N_cap = complements ? 2 * C : C;
     const u64 n_words = kc_div_up(nb, 32);
     const u32 blocks = (u32) kc_div_up(nb, (u64) KC_RUN_TILE);
     u32 *counts = ex.alloc<u32>(blocks);
     u64 *rec_off = ex.alloc<u64>(C), *rec_len = ex.alloc<u64>(C);
     kc_ull *n_runs = reinterpret_cast<kc_ull *>(blk + 1);
+    auto stage_event = [&](int i) {  // a captured graph is timed as a whole (run_sig_spec)
+        if (!ex.patch) KC_CUDA(cudaEventRecord(ctx->ev[i], ex.stream));
+    };
     {
         CudaExec::Scope sc(ex, KP_RUNS, nb / 8);
-        kc_runs_count_kernel<<<blocks, 256, 0, ex.stream>>>(flags, n_words, counts, n_runs);
-        kc_runs_emit_kernel<<<blocks, 256, 0, ex.stream>>>(flags, n_words, counts, rec_off, rec_len, n_runs, C);
+        ex.launch(kc_runs_count_kernel, blocks, 256, 0, flags, n_words, counts, n_runs);
+        ex.launch(kc_runs_emit_kernel, blocks, 256, 0, flags, n_words, (const u32 *) counts, rec_off, rec_len, (const kc_ull *) n_runs, (u64) C);
     }
-    ex.launches += 2;
-    KC_CUDA(cudaGetLastError());
-    KC_CUDA(cudaEventRecord(ctx->ev[2], ex.stream));
+    stage_event(2);
     NodeView<L> nv;
     nv.k = k;
     nv.complements = complements;
@@ -353,15 +403,13 @@ u32 run_tail_spec(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params
     eng.n_s = eng.n_p = N_cap;
     {
         CudaExec::Scope sc(ex, KP_RUNS, 32 * (u64) C);
-        kc_spec_nodes_kernel<L><<<1, 1024, 0, ex.stream>>>(blk, spec, ctx->sparse_switch, complements, in.seq, k, rec_off, rec_len, first, last,
-                                                            eng.st, eng.ban_flag, eng.ban_ctr, eng.live_s, eng.live_p, eng.small_masks, (u32) mask_words);
+        ex.launch(kc_spec_nodes_kernel<L>, 1, 1024, 0, (const u64 *) blk, spec, ctx->sparse_switch, complements, in.seq, k, rec_off, rec_len, first, last,
+                  eng.st, eng.ban_flag, eng.ban_ctr, eng.live_s, eng.live_p, eng.small_masks, (u32) mask_words);
     }
-    ++ex.launches;
-    KC_CUDA(cudaGetLastError());
     static_assert(4 * KC_SPEC_RUNS <= SmallCfg<L>::T && 2 * KC_SPEC_RUNS <= SmallCfg<L>::NS && 2 * KC_SPEC_RUNS <= KC_RANK_SMALL,
                   "the speculative tail runs on the one-CTA kernels");
     eng.run();  // all levels in the single-CTA engine
-    KC_CUDA(cudaEventRecord(ctx->ev[3], ex.stream));
+    stage_event(3);
     NodeSeq<L> ns;
     ns.k = k;
     ns.kmers = nullptr;
@@ -371,21 +419,38 @@ u32 run_tail_spec(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params
     ns.n = C;
     const EmitSpec es{spec + 1, blk + KC_SPEC_EMIT};
     // every character of the superstring is a character of some node: nodes are pieces of the input that overlap by < k
-    const u64 total_ub = nb + (u64) C * k + 16;
-    const EmitResult er = kc_emit_superstring<CudaExec, L>(ex, ns, nv, eng.st, nullptr, 0, false, 0, 1, total_ub, &es);
-    KC_CUDA(cudaEventRecord(ctx->ev[4], ex.stream));
+    t.total_ub = nb + (u64) C * k + 16;
+    t.ms = kc_emit_superstring<CudaExec, L>(ex, ns, nv, eng.st, nullptr, 0, false, 0, 1, t.total_ub, &es).ms;
+    stage_event(4);
+    if (!ex.pinned || ex.pinned_cap < KC_SPEC_BLOCK_WORDS * 8) KC_THROW(KC_ERR_INTERNAL, "no pinned scratch for the status block");
+    KC_CUDA(cudaMemcpyAsync(ex.pinned, blk, KC_SPEC_BLOCK_WORDS * 8, cudaMemcpyDeviceToHost, ex.stream));
+    t.n_s = eng.n_s;
+    t.n_p = eng.n_p;
+    t.small_d = eng.small_d;
     KC_TRACE_POINT("tail_spec: queued");
+    return t;
+}
+
+// The one read-back of the speculative tail.  Returns the status: KC_SPEC_OK = `res` holds the result; otherwise nothing was done and
+// the arena bottom is as it was before the tail.
+template <int L> u32 tail_spec_finish(kc_ctx *ctx, CudaExec &ex, const SpecTail &t, DevResult &res) {
     u64 h[KC_SPEC_BLOCK_WORDS];
-    ex.read_n(blk, h, KC_SPEC_BLOCK_WORDS);
+    ex.sync();
+    std::memcpy(h, ex.pinned, sizeof(h));
+    ++ex.read_backs;
     const u32 *hs = reinterpret_cast<const u32 *>(h + KC_SPEC_SPEC);
     if (hs[0] != KC_SPEC_OK) {
-        ex.arena->release(mark);
+        ex.arena->release(t.mark);
         return hs[0];
     }
+    Engine<CudaExec, L> eng(ex, NodeView<L>(), false, false);
+    eng.n_s = t.n_s;
+    eng.n_p = t.n_p;
+    eng.small_d = t.small_d;
     eng.apply_small_status(reinterpret_cast<const u32 *>(h + KC_SPEC_SMALL));  // a failed small-engine run is the cause, report that one
     ctx->path_stats = eng.stats;
-    kc_emit_check(h + KC_SPEC_EMIT, hs[2], total_ub);
-    res.ms = er.ms;
+    kc_emit_check(h + KC_SPEC_EMIT, hs[2], t.total_ub);
+    res.ms = t.ms;
     res.maxone = nullptr;
     res.length = h[KC_SPEC_EMIT + 2];
     res.slice_begin = 0;
@@ -395,6 +460,94 @@ u32 run_tail_spec(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params
     res.n_nodes = hs[1];
     res.n_simplitigs = hs[1];
     return KC_SPEC_OK;
+}
+
+// The signature construction into `flags` and the speculative tail behind it, with programmatic dependent launches: directly while
+// the kernel-class timers are on (they bracket every launch with events) or the input is still being copied in, otherwise as a cached
+// graph (SpecGraph) that the first call of a shape captures from the same launches.  Returns false (nothing queued) when the
+// signature plan does not apply.
+template <int L>
+bool run_sig_spec(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &p, u32 *flags, u64 **blk, SpecTail &t) {
+    if (!kc_sig_plan(in.n_bytes, p.k, ctx->routes.sig).ok) {
+        ex.arena->alloc_top<u64>(KC_SPEC_BLOCK_WORDS);  // as every rung, the block stays allocated when the plan does not apply
+        return false;
+    }
+    auto queue = [&] {
+        *blk = ex.arena->alloc_top<u64>(KC_SPEC_BLOCK_WORDS);
+        kc_kmerset_build_sig<L>(ex, in.seq, in.n_bytes, p.k, p.complements != 0, flags, *blk, ctx->routes.sig, in.chunks, nullptr, nullptr,
+                                KC_SPEC_BLOCK_WORDS);
+        t = tail_spec_queue<L>(ctx, ex, in, p, flags, *blk);
+    };
+    ex.pdl = true;
+    if ((ex.prof && ex.prof->enabled) || in.chunks) {
+        queue();
+        ex.pdl = false;
+        return true;
+    }
+    Arena &A = *ex.arena;
+    SpecGraph key;
+    key.limbs = L;
+    key.k = p.k;
+    key.complements = p.complements != 0;
+    key.n_bytes = in.n_bytes;
+    key.arena_base = A.base;
+    key.arena_at = A.checkpoint();
+    key.flags = flags;
+    SpecGraph *g = nullptr;
+    for (SpecGraph &c : ctx->spec_graphs)
+        if (c.same_shape(key)) g = &c;
+    if (g) {
+        A.restore(g->arena_after);
+        if (g->arena_high > A.high) A.high = g->arena_high;
+        *blk = g->blk;
+        t = g->tail;
+        ++ctx->spec_graph_replays;
+    } else {
+        if (ctx->spec_graphs.size() >= kc_ctx::KC_SPEC_GRAPHS) ctx->clear_spec_graphs();
+        if (!ctx->capture_stream) KC_CUDA(cudaStreamCreateWithFlags(&ctx->capture_stream, cudaStreamNonBlocking));
+        key.patch.seq = in.seq;
+        const u64 launches0 = ex.launches;
+        cudaStream_t run_stream = ex.stream;
+        auto end_capture = [&](cudaGraph_t *graph) {  // the capture stream only records: nothing runs until the graph is launched
+            ex.patch = nullptr;
+            ex.stream = A.stream = run_stream;
+            return cudaStreamEndCapture(ctx->capture_stream, graph);
+        };
+        KC_CUDA(cudaStreamBeginCapture(ctx->capture_stream, cudaStreamCaptureModeRelaxed));
+        ex.stream = A.stream = ctx->capture_stream;
+        ex.patch = &key.patch;
+        try {
+            queue();
+        } catch (...) {
+            ex.pdl = false;
+            cudaGraph_t partial = nullptr;
+            end_capture(&partial);
+            if (partial) cudaGraphDestroy(partial);
+            (void) cudaGetLastError();
+            throw;
+        }
+        KC_CUDA(end_capture(&key.graph));
+        if (cudaGraphInstantiate(&key.exec, key.graph, 0) != cudaSuccess) {
+            key.destroy();
+            ex.pdl = false;
+            KC_THROW(KC_ERR_CUDA, "cudaGraphInstantiate failed");
+        }
+        key.launches = ex.launches - launches0;
+        ex.launches = launches0;
+        key.arena_after = A.checkpoint();
+        key.arena_high = A.high;
+        key.blk = *blk;
+        key.tail = t;
+        ctx->spec_graphs.push_back(std::move(key));
+        g = &ctx->spec_graphs.back();
+        ++ctx->spec_graph_captures;
+    }
+    ex.pdl = false;
+    g->patch.set_seq(g->exec, in.seq);
+    KC_CUDA(cudaGraphLaunch(g->exec, ex.stream));
+    ex.launches += g->launches;
+    for (int i = 2; i <= 4; ++i) KC_CUDA(cudaEventRecord(ctx->ev[i], ex.stream));  // the stage timers see the graph as one piece
+    return true;
 }
 
 // From-FASTA regime: the nodes handed to the overlap stage are FIRST-OCCURRENCE RUNS.
@@ -409,7 +562,7 @@ u32 run_tail_spec(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params
 // k-1 are still joined first, exactly as BIGREEDY requires.
 //
 // The first-occurrence flags come from kc_set_ladder (set_routes.cuh), or else from the exact construction.
-// spec_res != nullptr: after the signature construction, try the speculative tail (run_tail_spec).  When it holds, *spec_res is the whole
+// spec_res != nullptr: after the signature construction, try the speculative tail (run_sig_spec).  When it holds, *spec_res is the whole
 // result and *spec_done is set; otherwise the runs are counted as if it had not been tried, on the same flags.
 template <int L>
 Stage1<L> run_stage1_runs(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const kc_params &p, DevResult *spec_res, bool *spec_done) {
@@ -419,25 +572,24 @@ Stage1<L> run_stage1_runs(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const k
     KC_TRACE_POINT("stage1: begin");
     const u64 nb = in.n_bytes;
     const size_t fwords = kc_runs_flag_words(nb);
-    u32 *flags = ex.arena->alloc_top<u32>(fwords);
-    ex.fill_bytes(flags, 0, fwords * 4);
+    u32 *flags = ex.arena->alloc_top<u32>(fwords);  // zeroed by the construction that fills it (the signature scan writes every word)
     u64 *cells = ex.arena->alloc_top<u64>(2);  // {kept distinct k-mers, runs}
-    ex.fill_bytes(cells, 0, 16);
     u64 *cells4 = nullptr, hc[4];
     KsfPlan plan;
+    SpecTail tail;
     auto launch = [&](KcRoute r) {
-        const size_t n_cells = r == KC_ROUTE_SIG && spec_res ? KC_SPEC_BLOCK_WORDS : 4;
-        cells4 = ex.arena->alloc_top<u64>(n_cells);  // {kept, runs, M, overflow status} (+ the rest of the speculative tail's status block)
-        ex.fill_bytes(cells4, 0, n_cells * 8);
-        return r == KC_ROUTE_SIG ? kc_kmerset_build_sig<L>(ex, in.seq, nb, p.k, p.complements != 0, flags, cells4, ctx->routes.sig, in.chunks)
-                                 : kc_kmerset_build_fast<L>(ex, in.seq, nb, p.k, p.complements != 0, p.min_frequency, flags, cells4, ctx->routes.fast,
-                                                            &plan, in.chunks);
+        if (r == KC_ROUTE_SIG && spec_res) return run_sig_spec<L>(ctx, ex, in, p, flags, &cells4, tail);
+        cells4 = ex.arena->alloc_top<u64>(4);  // {kept, runs, M, overflow status}
+        if (r == KC_ROUTE_SIG) return kc_kmerset_build_sig<L>(ex, in.seq, nb, p.k, p.complements != 0, flags, cells4, ctx->routes.sig, in.chunks, nullptr, nullptr, 4);
+        ex.fill_bytes(flags, 0, fwords * 4);
+        ex.fill_bytes(cells4, 0, 32);
+        return kc_kmerset_build_fast<L>(ex, in.seq, nb, p.k, p.complements != 0, p.min_frequency, flags, cells4, ctx->routes.fast, &plan, in.chunks);
     };
     auto consume = [&](KcRoute r) {
         KC_TRACE_POINT(r == KC_ROUTE_SIG ? "stage1: signature set launched" : "stage1: fast set launched");
         bool aborted = false;
         if (r == KC_ROUTE_SIG && spec_res) {
-            const u32 st = run_tail_spec<L>(ctx, ex, in, p, flags, cells4, *spec_res);
+            const u32 st = tail_spec_finish<L>(ctx, ex, tail, *spec_res);
             if (st == KC_SPEC_OK) {
                 ++ctx->tail_spec_runs;
                 *spec_done = true;
@@ -451,8 +603,7 @@ Stage1<L> run_stage1_runs(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const k
             }
         }
         if (!aborted) s.nodes = kc_runs_from_flags(ex, flags, nb, p.k, cells4, hc, 4, &aborted);
-        if (aborted) ex.fill_bytes(flags, 0, fwords * 4);  // incomplete: the next construction starts from clear bits
-        return !aborted;
+        return !aborted;  // incomplete flags: the next construction clears them first
     };
     const KcRoute route = kc_set_ladder(ctx->routes, ctx->routes.compute_policy(p, nb), nb, *ex.arena, launch, consume);
     if (route != KC_ROUTE_NONE) {
@@ -470,6 +621,8 @@ Stage1<L> run_stage1_runs(kc_ctx *ctx, CudaExec &ex, const DevInput &in, const k
     }
     // with -M the sorted k-mer set doubles as kMersDict of src/global.h:165-167; it stays at the arena bottom
     if (in.chunks) in.chunks->wait_all(ex.stream);
+    ex.fill_bytes(flags, 0, fwords * 4);
+    ex.fill_bytes(cells, 0, 16);
     KmerSet<L> set = kc_kmerset_build<L>(ex, in.seq, nb, p.k, p.complements != 0, p.min_frequency, flags, p.want_maxone != 0, cells);
     KC_TRACE_POINT("stage1: set built");
     s.n_occ = set.n_occ;
@@ -598,7 +751,7 @@ template <int L> void run_pipeline(kc_ctx *ctx, CudaExec &ex, const DevInput &in
         }
         s.nodes = RunNodes{in.rec_off, in.rec_len, in.n_recs};
     } else {
-        // the speculative tail: a FASTA input with few runs (a genome) is computed behind one read-back (run_tail_spec)
+        // the speculative tail: a FASTA input with few runs (a genome) is computed behind one read-back (run_sig_spec)
         const u64 nb = in.n_bytes;
         const bool spec_failed = ctx->routes.heuristics && ctx->routes.tail.near(nb);
         const bool spec = ctx->tail_spec && !spec_failed && !lower_bound && ctx->small_engine && nb > 0 && nb < KC_POS32_BYTES;
@@ -994,6 +1147,7 @@ int kc_init(int device, void *stream, kc_ctx **out) {
 void kc_destroy(kc_ctx *ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
+    ctx->clear_spec_graphs();
     if (ctx->arena.base) cudaFree(ctx->arena.base);
     if (ctx->pin_out.p) cudaFreeHost(ctx->pin_out.p);
     if (ctx->pin_small) cudaFreeHost(ctx->pin_small);
@@ -1003,6 +1157,7 @@ void kc_destroy(kc_ctx *ctx) {
     for (int i = 0; i < kc_ctx::KC_H2D_CHUNKS; ++i)
         if (ctx->chunk_ev[i]) cudaEventDestroy(ctx->chunk_ev[i]);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
+    if (ctx->capture_stream) cudaStreamDestroy(ctx->capture_stream);
     for (cudaEvent_t e : ctx->prof.pool) cudaEventDestroy(e);
     if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
     delete ctx;
@@ -1641,6 +1796,8 @@ int kc_get_stat(const kc_ctx *ctx, const char *name, uint64_t *value) {
     else if (std::strcmp(name, "read_backs") == 0) *value = ctx->read_backs;
     else if (std::strcmp(name, "tail_spec_runs") == 0) *value = ctx->tail_spec_runs;
     else if (std::strcmp(name, "tail_spec_fallbacks") == 0) *value = ctx->tail_spec_fallbacks;
+    else if (std::strcmp(name, "spec_graph_captures") == 0) *value = ctx->spec_graph_captures;
+    else if (std::strcmp(name, "spec_graph_replays") == 0) *value = ctx->spec_graph_replays;
     else if (std::strcmp(name, "arena_bytes") == 0) *value = ctx->arena.cap;
     else if (std::strcmp(name, "arena_high") == 0) *value = ctx->arena.high;
     else if (std::strcmp(name, "arena_retries") == 0) *value = ctx->arena_retries;
@@ -1654,6 +1811,8 @@ int kc_get_stat(const kc_ctx *ctx, const char *name, uint64_t *value) {
 
 int kc_set_option(kc_ctx *ctx, const char *name, int value) {
     if (!ctx || !name) return KC_ERR_ARG;
+    cudaSetDevice(ctx->device);
+    ctx->clear_spec_graphs();  // an option may change the launch shapes or the arena layout of the cached calls
     if (std::strcmp(name, "sparse_switch") == 0) {
         ctx->sparse_switch = value != 0;
         return KC_OK;

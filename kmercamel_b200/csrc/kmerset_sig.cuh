@@ -171,6 +171,7 @@ template <int M, bool P2P>
 __global__ void __launch_bounds__(256) kc_sig_scan_kernel(const u8 *__restrict__ seq, u64 n_bytes, int k, int a, u32 n_buckets, u32 *cursor,
                                                           u64 *__restrict__ recs, u64 *__restrict__ packed, u32 *__restrict__ flags, u64 n_flag_words,
                                                           u32 tile0, kc_ull *m_cell, u32 *status, const u32 *__restrict__ win_mask, const SigPeers sp) {
+    kc_pdl_wait();
     constexpr int T = 256;
     constexpr int NH = 32 + KC_SIG_W - 1;  // M-mer hashes a strip needs
     __shared__ u64 pk[KC_EX_HALO + T];
@@ -194,13 +195,16 @@ __global__ void __launch_bounds__(256) kc_sig_scan_kernel(const u8 *__restrict__
         em = all ? 0xFFFFFFFFu : kc_strip_emit_mask(vm, widx, k);
     }
     em &= kc_strip_window_filter(win_mask, block_pos0);
-    {   // clear-the-losers flags: every window starts as "first occurrence" (bit p & 31 of word p >> 5 = window END p)
+    {   // clear-the-losers flags: every window starts as "first occurrence" (bit p & 31 of word p >> 5 = window END p).  The flags do
+        // not arrive zeroed: every word is written, the ones past the last tile (the padding word) by the last thread of that tile
         const u64 w = (u64) (block_pos0 >> 5) + threadIdx.x;
-        if (P2P) {  // the arrays of a group do not arrive zeroed: every word of the slice is written
+        if (P2P) {
             if (w < n_flag_words)
                 for (int r = 0; r < sp.n; ++r) sp.flags[r][w] = __brev(em);
-        } else if (em && w < n_flag_words) {
+        } else if (w < n_flag_words) {
             flags[w] = __brev(em);
+            if (threadIdx.x == T - 1 && (u64) block_pos0 + T * KC_EX_STRIP >= n_bytes)
+                for (u64 x = w + 1; x < n_flag_words; ++x) flags[x] = 0;
         }
     }
     {
@@ -450,6 +454,9 @@ __global__ void __launch_bounds__(SigCfg<L>::THREADS, SigCfg<L>::MIN_CTAS) kc_si
                                                                                                 u32 n_buckets, KsfFlagPeers fl, kc_ull *n_unique, u32 *status,
                                                                                                 u32 n_senders, u32 sub_cap, u32 off_stride) {
     // MULTI: the buckets are this rank's (kc_sig_gather_kernel has lined their records up), a duplicate clears its bit on every rank
+    kc_pdl_wait();
+    // the CTAs finish unevenly: the next kernel (the run count) may place its CTAs on the SMs this one leaves
+    kc_pdl_trigger();
     typedef SigCfg<L> Cfg;
     constexpr u32 RC = KC_SIG_REC_CAP, T2N = Cfg::T2N;
     constexpr int NW = Cfg::NW, P = KC_SIG_PIECE;
@@ -695,23 +702,20 @@ template <int L> struct SigKernels {
 };
 
 template <bool P2P>
-inline void kc_sig_scan_launch(int m, u32 blocks, cudaStream_t st, const u8 *seq, u64 n_bytes, int k, int a, u32 n_buckets, u32 *cursor, u64 *recs, u64 *packed,
+inline void kc_sig_scan_launch(CudaExec &ex, int m, u32 blocks, const u8 *seq, u64 n_bytes, int k, int a, u32 n_buckets, u32 *cursor, u64 *recs, u64 *packed,
                                u32 *flags, u64 n_flag_words, u32 tile0, kc_ull *m_cell, u32 *status, const u32 *win_mask, const SigPeers &sp) {
-    switch (m) {
-    case 16: kc_sig_scan_kernel<16, P2P><<<blocks, 256, 0, st>>>(seq, n_bytes, k, a, n_buckets, cursor, recs, packed, flags, n_flag_words, tile0, m_cell, status, win_mask, sp); break;
-    case 15: kc_sig_scan_kernel<15, P2P><<<blocks, 256, 0, st>>>(seq, n_bytes, k, a, n_buckets, cursor, recs, packed, flags, n_flag_words, tile0, m_cell, status, win_mask, sp); break;
-    case 12: kc_sig_scan_kernel<12, P2P><<<blocks, 256, 0, st>>>(seq, n_bytes, k, a, n_buckets, cursor, recs, packed, flags, n_flag_words, tile0, m_cell, status, win_mask, sp); break;
-    default: kc_sig_scan_kernel<11, P2P><<<blocks, 256, 0, st>>>(seq, n_bytes, k, a, n_buckets, cursor, recs, packed, flags, n_flag_words, tile0, m_cell, status, win_mask, sp); break;
-    }
-    KC_CUDA(cudaGetLastError());
+    auto *kern = m == 16 ? kc_sig_scan_kernel<16, P2P> : m == 15 ? kc_sig_scan_kernel<15, P2P> : m == 12 ? kc_sig_scan_kernel<12, P2P> : kc_sig_scan_kernel<11, P2P>;
+    ex.launch(kern, blocks, 256, 0, seq, n_bytes, k, a, n_buckets, cursor, recs, packed, flags, n_flag_words, tile0, m_cell, status, win_mask, sp);
 }
 
 // Launches the construction on ex.stream and returns without synchronising; same contract as kc_kmerset_build_fast:
-//   cells[0] += distinct k-mers, cells[2] = M (k-mer windows), low word of cells[3] = overflow status; flags arrive zeroed.
+//   cells[0] += distinct k-mers, cells[2] = M (k-mer windows), low word of cells[3] = overflow status.  The flags (kc_runs_flag_words
+// of n_bytes) need not arrive zeroed; the cells must, unless zero_cells > 0: then the construction zeroes cells[0, zero_cells) first
+// (with its bucket counters in the same memset when `cells` is the arena's top block).
 // Returns false (nothing launched) when the plan does not apply.
 template <int L>
 bool kc_kmerset_build_sig(CudaExec &ex, const u8 *seq, u64 n_bytes, int k, bool complements, u32 *flags, u64 *cells, const SigTuning &tune,
-                          InputChunks *chunks = nullptr, const u32 *win_mask = nullptr, SigPlan *plan_out = nullptr) {
+                          InputChunks *chunks = nullptr, const u32 *win_mask = nullptr, SigPlan *plan_out = nullptr, u32 zero_cells = 0) {
     typedef SigCfg<L> Cfg;
     typedef SigKernels<L> KK;
     const SigPlan pl = kc_sig_plan(n_bytes, k, tune);
@@ -724,8 +728,17 @@ bool kc_kmerset_build_sig(CudaExec &ex, const u8 *seq, u64 n_bytes, int k, bool 
     const u32 blocks = (u32) kc_div_up(n_bytes, TILE);
     u64 *recs = ex.alloc<u64>((u64) pl.n_buckets * KC_SIG_REC_CAP);
     u64 *packed = ex.alloc<u64>((u64) blocks * 256);
-    u32 *cursor = ex.alloc<u32>(pl.n_buckets);
-    ex.fill_bytes(cursor, 0, (size_t) pl.n_buckets * 4);
+    // the bucket counters go to the arena top, right below `cells` when the caller has just allocated them there: one memset for both
+    const ArenaMark top_mark = ex.arena->checkpoint();
+    u32 *cursor = ex.arena->alloc_top<u32>(pl.n_buckets);
+    const size_t cursor_bytes = kc_align_up((u64) pl.n_buckets * 4, 256);
+    if (zero_cells && reinterpret_cast<char *>(cursor) + cursor_bytes == reinterpret_cast<char *>(cells)) {
+        ex.fill_bytes(cursor, 0, cursor_bytes + (size_t) zero_cells * 8);
+    } else {
+        ex.fill_bytes(cursor, 0, cursor_bytes);
+        ex.fill_bytes(cells, 0, (size_t) zero_cells * 8);
+    }
+    const u64 n_flag_words = kc_div_up(n_bytes, (u64) 32) + 1;
     u32 *status = reinterpret_cast<u32 *>(cells + 3);
     kc_ull *m_cell = reinterpret_cast<kc_ull *>(cells + 2);
     {
@@ -742,9 +755,8 @@ bool kc_kmerset_build_sig(CudaExec &ex, const u8 *seq, u64 n_bytes, int k, bool 
             const u64 part_bytes = std::min<u64>(n_bytes, (u64) t1 * TILE) - (u64) t0 * TILE;
             // sequence read, code words + flag words + records written
             CudaExec::Scope sc(ex, KP_KS_SCATTER0, part_bytes + part_bytes / 4 + part_bytes / 8 + (u64) (part_bytes * 8 / KC_SIG_WINDOWS_PER_RECORD));
-            kc_sig_scan_launch<false>(pl.m, t1 - t0, st, seq, n_bytes, k, pl.a, pl.n_buckets, cursor, recs, packed, flags, kc_div_up(n_bytes, (u64) 32) + 1,
-                                      t0, m_cell, status, win_mask, SigPeers());
-            ++ex.launches;
+            kc_sig_scan_launch<false>(ex, pl.m, t1 - t0, seq, n_bytes, k, pl.a, pl.n_buckets, cursor, recs, packed, flags, n_flag_words, t0, m_cell,
+                                      status, win_mask, SigPeers());
         }
         if (chunks) chunks->waited = true;
     }
@@ -756,12 +768,10 @@ bool kc_kmerset_build_sig(CudaExec &ex, const u8 *seq, u64 n_bytes, int k, bool 
         const bool pos64 = n_bytes > 0xFFFFFFFFULL;  // a window END position may need more than 32 bits
         auto *kern = complements ? (pos64 ? kc_sig_resolve_kernel<L, false, false, true> : kc_sig_resolve_kernel<L, false, false, false>)
                                  : (pos64 ? kc_sig_resolve_kernel<L, false, true, true> : kc_sig_resolve_kernel<L, false, true, false>);
-        kern<<<grid, Cfg::THREADS, Cfg::smem(pos64), st>>>(packed, k, cursor, recs, pl.n_buckets, kc_ksf_own_flags(flags), reinterpret_cast<kc_ull *>(cells), status,
-                                                           1u, KC_SIG_REC_CAP, 0u);
-        ++ex.launches;
-        KC_CUDA(cudaGetLastError());
+        ex.launch(kern, grid, Cfg::THREADS, Cfg::smem(pos64), packed, k, cursor, recs, pl.n_buckets, kc_ksf_own_flags(flags), reinterpret_cast<kc_ull *>(cells),
+                  status, 1u, KC_SIG_REC_CAP, 0u);
     }
-    ex.arena->release(base_mark);
+    ex.arena->restore({base_mark, top_mark.top});
     return true;
 }
 
@@ -819,9 +829,8 @@ inline void kc_sig_group_scan(CudaExec &ex, const u8 *seq, u64 n_bytes, int k, c
     if (t1 > t0) {
         slice_bytes = std::min<u64>(n_bytes, (u64) t1 * TILE) - (u64) t0 * TILE;
         CudaExec::Scope sc(ex, KP_KS_SCATTER0, slice_bytes + (slice_bytes / 4 + slice_bytes / 8) * (u64) sp.n + (u64) (slice_bytes * 8 / KC_SIG_WINDOWS_PER_RECORD));
-        kc_sig_scan_launch<true>(pl.m, t1 - t0, ex.stream, seq, n_bytes, k, pl.a, pl.n_buckets, cursor, staged, nullptr, nullptr, kc_div_up(n_bytes, (u64) 32), t0,
+        kc_sig_scan_launch<true>(ex, pl.m, t1 - t0, seq, n_bytes, k, pl.a, pl.n_buckets, cursor, staged, nullptr, nullptr, kc_div_up(n_bytes, (u64) 32), t0,
                                  reinterpret_cast<kc_ull *>(cells + 2), status, nullptr, sp);
-        ++ex.launches;
     }
     kc_sig_om_counts_kernel<<<(unsigned) kc_div_up((u64) n_om + 1, 256), 256, 0, ex.stream>>>(cursor, pl.n_buckets, nbr, (u32) sp.n, sp.sub_cap, off_om);
     ++ex.launches;

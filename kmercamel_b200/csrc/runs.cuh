@@ -29,6 +29,7 @@ KC_D u32 kc_runs_starts(u32 f, u32 prev) { return f & ~((f << 1) | prev); }
 KC_D u32 kc_runs_ends(u32 f, u32 next) { return f & ~((f >> 1) | (next << 31)); }
 
 __global__ void __launch_bounds__(256) kc_runs_count_kernel(const u32 *flags, u64 n_words, u32 *block_counts, kc_ull *total_runs) {
+    kc_pdl_wait();
     __shared__ u32 sw[8];
     const u64 word = ((u64) blockIdx.x * 256 + threadIdx.x) * KC_RUN_WORDS;
     u32 f[KC_RUN_WORDS], prev, next;
@@ -50,6 +51,7 @@ __global__ void __launch_bounds__(256) kc_runs_count_kernel(const u32 *flags, u6
 // start or end sums the counts before it (one block in ~10^4 on a genome), instead of a scan launch in between.
 __global__ void __launch_bounds__(256) kc_runs_emit_kernel(const u32 *flags, u64 n_words, const u32 *block_offsets, u64 *rec_off, u64 *rec_len,
                                                            const kc_ull *spec_total = nullptr, u64 spec_cap = 0) {
+    kc_pdl_wait();
     __shared__ u32 sw[8];
     if (spec_total && *spec_total > spec_cap) return;
     const u64 word = ((u64) blockIdx.x * 256 + threadIdx.x) * KC_RUN_WORDS;

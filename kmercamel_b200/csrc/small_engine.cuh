@@ -74,6 +74,7 @@ template <int L>
 __global__ void __launch_bounds__(256) kc_small_level_mask_kernel(NodeView<L> v, const u32 *__restrict__ ls, const u32 *__restrict__ lp, u32 n_s, u32 n_p,
                                                                   int d_start, u32 *mask_out /* [4], zeroed */, u32 *end_mask_s /* [4 n_s], zeroed */,
                                                                   u32 *end_mask_p /* [4 n_p], zeroed */, const u32 *n_dev /* see SmallEngineArgs */) {
+    kc_pdl_wait();
     extern __shared__ __align__(16) unsigned char kc_smem_raw[];
     __shared__ u32 s_hits;
     const u32 tid = threadIdx.x, NT = blockDim.x;
@@ -163,6 +164,8 @@ __global__ void __launch_bounds__(256) kc_small_level_mask_kernel(NodeView<L> v,
 }
 
 template <int L> __global__ void __launch_bounds__(512) kc_small_engine_kernel(SmallEngineArgs<L> a) {
+    kc_pdl_wait();
+    kc_pdl_trigger();  // one CTA: the next kernel's launch overlaps this one
     typedef KWord<L + 1> TW;
     constexpr u32 TCAP = SmallCfg<L>::T, HCAP = SmallCfg<L>::H;
     extern __shared__ __align__(16) unsigned char kc_smem_raw[];

@@ -1,4 +1,4 @@
-// Speculative tail of the from-FASTA single-GPU path (kcgpu.cu run_tail_spec).
+// Speculative tail of the from-FASTA single-GPU path (kcgpu.cu tail_spec_queue, run_sig_spec).
 //
 // A genome leaves a few dozen first-occurrence runs, far below what the one-CTA kernels of the tail take.  So instead of reading the run
 // count back after the signature construction and sizing the tail from it, the host queues the whole tail sized for KC_SPEC_RUNS runs
@@ -34,6 +34,8 @@ template <int L>
 __global__ void __launch_bounds__(1024) kc_spec_nodes_kernel(const u64 *cells, u32 *spec, bool sparse_switch, bool complements, const u8 *seq, int k,
                                                             u64 *rec_off, u64 *rec_len, KWord<L> *first, KWord<L> *last, PathState st, u8 *ban_flag,
                                                             u32 *ban_ctr, u32 *live_s, u32 *live_p, u32 *masks, u32 mask_words) {
+    kc_pdl_wait();
+    kc_pdl_trigger();  // one CTA: the next kernel's launch overlaps this one
     const u64 kept = cells[0], runs = cells[1], M = cells[2];
     const u64 U = M ? kept : 0;
     const u32 status = cells[3] ? KC_SPEC_SIG_OVERFLOW
